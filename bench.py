@@ -5,6 +5,7 @@ trainPNHigh.py:131-144) on synthetic QWS-shaped instances, per the driver contra
     python bench.py --gpus 1 --steps 5 --warmup 3                       # our CUDA path
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...                                 # reference CPU algorithm (oracle port)
+    python bench.py --dump-outputs DIR ...                               # also write the last step's outputs as .npy
 
 One "step" = one pass of the hot path over one batch of n instances per GPU:
 encoder LSTM (L steps) + fused greedy decode (K steps) for PNLow, the same for PNHigh with PNLow's
@@ -98,6 +99,11 @@ class ClockSampler:
     def stop(self):
         if self.proc:
             self.proc.terminate()
+            try:                                           # reap it: the benchmark leaves no process behind
+                self.proc.wait(timeout=10)
+            except subprocess.TimeoutExpired:
+                self.proc.kill()
+                self.proc.wait()
         sm = [float(r[0]) for r in self.rows if r and r[0].replace(".", "").isdigit()]
         mx = [float(r[1]) for r in self.rows if len(r) > 1 and r[1].replace(".", "").isdigit()]
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
@@ -289,6 +295,25 @@ def pipeline_block(dev, shape: str, n: int, steps: int, warmup: int):
             "note": "ML stage inside the timed region; stage_ms from CUDA events at the stage boundaries inside compose"}
 
 
+DUMP_INSTANCES = 8192          # at most 8192 x 1,040 floats (34 MB) for the qws shape, whatever the batch
+
+
+def dump_outputs(path: str, n: int, arrays):
+    """``--dump-outputs``: write ``{name: (device tensor, instance axis)}`` as ``path/<name>.npy`` in float32 (picks and
+    violation counts are small integers, exact in float32).  Batches above DUMP_INSTANCES instances keep a fixed, seeded
+    sample of instances, the same in every array; ``instances.npy`` lists them (float64)."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    rows = np.arange(n)
+    if n > DUMP_INSTANCES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_INSTANCES, replace=False))
+    np.save(os.path.join(path, "instances.npy"), rows.astype(np.float64))
+    for name, (t, axis) in arrays.items():
+        sel = t.index_select(axis, torch.from_numpy(rows).to(t.device))
+        np.save(os.path.join(path, f"{name}.npy"), sel.cpu().numpy().astype(np.float32))
+
+
 # ----------------------------------------------------------------------------- our arm
 def run_ours(args):
     import torch
@@ -330,6 +355,7 @@ def run_ours(args):
              torch.empty(n, L_SEQ, device=dev), torch.empty(n, L_SEQ, device=dev)) for _ in range(2)]
     enc_ev, dec_ev = [], []
     enc_mib = (enc_out.numel() * 4) >> 20
+    reward = [None]                                        # pn_reward of the latest step (violations, objFunc, reward)
 
     def device_step(record: bool):
         lat = None
@@ -348,7 +374,7 @@ def run_ours(args):
                 e2.record()
                 dec_ev.append((e1, e2))
             lat = wl
-        return ops.pn_reward(x, idx)[2], idx
+        reward[0] = ops.pn_reward(x, idx)
 
     from gnnpn_sc_b200.pipeline import GreedyLowHigh
     composer = GreedyLowHigh(low, high, dev)
@@ -386,6 +412,12 @@ def run_ours(args):
     launches0 = _lib.launch_count()
     ms_total = timed(lambda: device_step(True), args.steps)
     launches = _lib.launch_count() - launches0
+    if rank == 0 and args.dump_outputs:
+        # bufs[level] = (dec_h, picks [K, n], window logits [n, L], window probabilities [n, L]) of the last step
+        dump_outputs(args.dump_outputs, n, {
+            "pnlow_picks": (bufs[0][1], 1), "pnlow_window_logits": (bufs[0][2], 0), "pnlow_window_probs": (bufs[0][3], 0),
+            "pnhigh_picks": (bufs[1][1], 1), "pnhigh_window_logits": (bufs[1][2], 0), "pnhigh_window_probs": (bufs[1][3], 0),
+            "violations": (reward[0][0], 0), "objective": (reward[0][1], 0), "reward": (reward[0][2], 0)})
     enc_launch_ms = sum(a.elapsed_time(b) for a, b in enc_ev) / len(enc_ev)        # avg encoder-scan launch, ms
     dec_launch_ms = sum(a.elapsed_time(b) for a, b in dec_ev) / len(dec_ev)        # avg fused-decode launch, ms
     seq_on = args.kernel == "tc" and (ops.get_option("persistent") & 1)
@@ -652,7 +684,12 @@ def main():
                     help="recurrence kernel: tcgen05 3xTF32 (default) or strict-fp32 FFMA")
     ap.add_argument("--workload", default="qws", choices=["qws", "scaleup"],
                     help="qws: the headline (BASELINE config 2/3); scaleup: 100 tasks x 1000 candidates (config 4)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (picks, window logits and probabilities "
+                         "of PNLow and PNHigh, objective and reward; rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "qws"):
+        ap.error("--dump-outputs writes the outputs of the headline workload (--impl ours --workload qws)")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "scaleup":

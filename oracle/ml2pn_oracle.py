@@ -1,8 +1,7 @@
 """TEST INFRASTRUCTURE (oracle): CPU restatement of ``src/ML2PN.py`` -- never imported by the product path.
 
 ``calc`` follows ML2PN.py:6-12 and ``scores`` the list handling of ``check`` (ML2PN.py:34-56): python lists of
-python floats (the JSON the trainers wrote), numpy float64 reductions.  Pinned by
-``tests/test_oracle_ml2pn.py`` against the reference module executed live where ``/root/reference`` is mounted.
+python floats (the JSON the trainers wrote), numpy float64 reductions.
 """
 from __future__ import annotations
 

@@ -21,11 +21,9 @@ bit-identical to the reference; the Python-level per-row loops of the reference
 is set, which replays them op for op (used for the CPU timing baseline so the
 timed work equals what the reference executes).
 
-Pinning: ``oracle/make_golden.py`` imports the *real* reference from
-``/root/reference`` (only available in the build container), runs both on the
-same tensors and writes ``tests/golden/pn_*.npz``; ``tests/test_oracle_pn.py``
-checks this restatement against those fixtures everywhere and against the live
-reference when it is present.
+Pinning: ``oracle/make_golden.py`` runs the *real* reference on the same tensors
+and writes its outputs to ``tests/golden/pn_*.npz``; ``tests/test_oracle_pn.py``
+checks this restatement against those fixtures, bit for bit.
 """
 from __future__ import annotations
 

@@ -8,7 +8,6 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE = "/root/reference"
 
 
 def pytest_configure(config):
@@ -33,11 +32,6 @@ def pytest_collection_modifyitems(config, items):
 @pytest.fixture(scope="session")
 def golden_dir():
     return GOLDEN
-
-
-@pytest.fixture(scope="session")
-def reference_available():
-    return os.path.isdir(os.path.join(REFERENCE, "src", "models"))
 
 
 PARITY_LOG = os.path.join(ROOT, "gpurun_out", "parity.jsonl")

@@ -195,13 +195,13 @@ def test_pnlow_then_pnhigh_trainers_and_ml2pn(tmp_path):
     assert allR["averageQ"] == sum(allR["quality"]) / 16
 
 
-def test_reinforce_step_reduces_loss_surrogate():
+def test_reinforce_step_reduces_loss_surrogate(tmp_path):
     """A few REINFORCE updates on one batch move the sampled reward mean down (sanity of sign and plumbing)."""
     from gnnpn_sc_b200 import trainPN
     K, N = 5, 4
     torch.manual_seed(0)
     data = _toy_pn_data(256, K, N, seed=4)
-    low = trainPN.PNLow("toy", 0, 1, K, 1, N, 256, 0, 10, 1, 0.9, 2.0, 3e-3, -1, root="/tmp/gnnpn_toy")
+    low = trainPN.PNLow("toy", 0, 1, K, 1, N, 256, 0, 10, 1, 0.9, 2.0, 3e-3, -1, root=str(tmp_path))
     tr = low.start(data=data, n_epochs=16)
     first, last = np.mean(tr.train_tour[:6]), np.mean(tr.train_tour[-6:])
     print(f"mean sampled reward (violations): first epochs {first:.3f} -> last epochs {last:.3f}")
