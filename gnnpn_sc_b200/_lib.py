@@ -98,7 +98,7 @@ def lib():
                 fn = getattr(h, name)          # AttributeError if the ABI lost a symbol
                 fn.restype = res
                 fn.argtypes = args
-            if h.gnnpn_abi_version() != 7:
+            if h.gnnpn_abi_version() != 8:
                 raise GnnpnError("libgnnpn_b200.so ABI version mismatch")
             _lib = h
     return _lib

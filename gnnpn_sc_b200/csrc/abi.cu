@@ -4,6 +4,7 @@
 #include <string.h>
 #include <vector>
 #include "common.cuh"
+#include "internal.cuh"
 #include "options.cuh"
 
 namespace gnnpn {
@@ -37,19 +38,6 @@ static std::atomic<int>* option_slot(const char* name) {
   if (!strcmp(name, "spmm_chunk")) return &o.spmm_chunk;
   return nullptr;
 }
-int launch_gemm_ffma(const float* A, int64_t lda, const float* W, int64_t ldw, const float* bias,
-                     const float* scale, const float* shift, int act, float* C, int64_t ldc, int64_t M, int N,
-                     int K, cudaStream_t st);
-size_t tc_gemm_workspace_bytes(int64_t M, int N, int K);
-int launch_gemm_tc(const float* A, int64_t lda, const float* W, int64_t ldw, const float* bias, const float* scale,
-                   const float* shift, int act, float* C, int64_t ldc, int64_t M, int N, int K, void* workspace,
-                   cudaStream_t st);
-// persistent fp16-split node transform (node_transform.cu): K <= 256, N <= 256, N % 16 == 0, K % 4 == 0
-bool node_transform_supported(int64_t M, int N, int K);
-size_t node_transform_workspace_bytes(int N, int K);
-int launch_node_transform(const float* A, int64_t lda, const float* W, int64_t ldw, const float* bias,
-                          const float* scale, const float* shift, int act, float* C, int64_t ldc, int64_t M, int N,
-                          int K, void* workspace, cudaStream_t st);
 }  // namespace gnnpn
 
 using namespace gnnpn;

@@ -2,6 +2,7 @@
 // Parity anchor and small-shape path (request graphs have <= ~100 nodes per batch, K = 28/128/256);
 // the large service-side transforms go through the tcgen05 3xTF32 kernel in gemm_tc.cu.
 #include "common.cuh"
+#include "internal.cuh"
 
 namespace gnnpn {
 namespace {

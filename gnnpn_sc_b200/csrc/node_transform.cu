@@ -22,35 +22,14 @@
 // workspace and launch_node_transform's guarded strict-fp32 FFMA pass (gemm_ffma.cu) recomputes C -- on the device,
 // no host round trip; it returns immediately when the flag is clear (the normal case).
 // Shapes outside (K > 256, N > 256, N % 16 != 0, K % 4 != 0) use the 3xTF32 mainloop in tc_kernels.cu.
-#include <stdlib.h>
 #include <cuda_fp16.h>
 #include "tc_common.cuh"
 #include "common.cuh"
+#include "internal.cuh"
 #include "tc_seq_dev.cuh"
 
 namespace gnnpn {
-int launch_gemm_ffma_if(const int* only_if, const float* A, int64_t lda, const float* W, int64_t ldw, const float* bias,
-                        const float* scale, const float* shift, int act, float* C, int64_t ldc, int64_t M, int N,
-                        int K, cudaStream_t st);
-namespace tc {
-int make_map_2d(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows, bool f16);
-}
 namespace nt {
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult qr;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qr) == cudaSuccess &&
-        qr == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)ptr;
-  }
-  return fn;
-}
 
 using namespace tc;
 using namespace seq;       // cluster / cta_group::2 helpers
@@ -351,8 +330,7 @@ __global__ void split_w_kernel(const float* __restrict__ W, int64_t ldw, int N, 
 }  // namespace nt
 
 bool node_transform_supported(int64_t M, int N, int K) {
-  static const int off = getenv("GNNPN_GEMM_V1") ? atoi(getenv("GNNPN_GEMM_V1")) : 0;   // A/B: force the 3xTF32 mainloop
-  return !off && M >= 1 && N >= 16 && N <= nt::MAX_N && (N % 16) == 0 && K >= 4 && K <= nt::MAX_KB * nt::KB && (K % 4) == 0;
+  return M >= 1 && N >= 16 && N <= nt::MAX_N && (N % 16) == 0 && K >= 4 && K <= nt::MAX_KB * nt::KB && (K % 4) == 0;
 }
 
 size_t node_transform_workspace_bytes(int N, int K) {
@@ -384,8 +362,7 @@ int launch_node_transform(const float* A, int64_t lda, const float* W, int64_t l
   p.st_tab = st_tab;
   p.status = status;
   CUtensorMap map_c;
-  static const int direct = getenv("GNNPN_GEMM_DIRECT_STORE") ? atoi(getenv("GNNPN_GEMM_DIRECT_STORE")) : 0;   // A/B knob
-  if (p.c_vec >= 4 && !direct) {
+  if (p.c_vec >= 4) {
     // C as a 2-D fp32 tensor {N, M}; box = 32 columns x 32 rows, 128B swizzle (one epilogue warp's tile)
     EncodeTiledFn fn = encode_fn();
     if (!fn) return GNNPN_EUNSUPPORTED;

@@ -1,6 +1,6 @@
 // Library-wide run-time options (gnnpn_set_option / gnnpn_get_option, include/gnnpn_b200.h).  The matching
 // environment variables are read ONCE, when the library is loaded, to set the initial values; kernels and dispatchers
-// read the atomics -- nothing on a call path calls getenv.
+// read the atomics -- nothing on a call path reads the environment.
 #pragma once
 #include <atomic>
 

@@ -1,7 +1,6 @@
 // Pointer-network entry points: weight packing, encoder scan, fused greedy decode,
 // interface-faithful logits materialisation, composition objective / reward.
 #include <math.h>
-#include <stdlib.h>
 #include <cuda_fp16.h>
 #include "lstm_step.cuh"
 #include "tc_lstm.cuh"
@@ -29,36 +28,23 @@ __device__ float folded_weight(const float* __restrict__ w_ih, const float* __re
 __global__ void pack_lstm_kernel(const float* __restrict__ w_ih, const float* __restrict__ w_hh,
                                  const float* __restrict__ b_ih, const float* __restrict__ b_hh,
                                  const float* __restrict__ w_e, const float* __restrict__ b_e,
-                                 const float* __restrict__ start, int H, int F, int Fpad, int Kp,
+                                 const float* __restrict__ start, int H, int F, int Fpad,
                                  float* __restrict__ packed) {
   const int G = 4 * H;
   const int rows = H + Fpad + 2;  // + bias row + start row
   const int64_t ffma_total = (int64_t)rows * G;
-  const int64_t tc_total = (int64_t)G * Kp;
   const int64_t tc16_total = (int64_t)G * kKp16;
-  for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < ffma_total + tc_total + tc16_total;
+  for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < ffma_total + tc16_total;
        e += (int64_t)gridDim.x * blockDim.x) {
-    if (e >= ffma_total + tc_total) {              // fp16-split tcgen05 operand: [4H][kKp16] halfs, weights x 2^4
-      const int64_t t = e - ffma_total - tc_total;
+    if (e >= ffma_total) {                         // fp16-split tcgen05 operand: [4H][kKp16] halfs, weights x 2^4
+      const int64_t t = e - ffma_total;
       const int nn = (int)(t / kKp16), k = (int)(t % kKp16);
       const int r = (nn & 3) * H + (nn >> 2);
       const float w = kW16Scale * folded_weight(w_ih, w_hh, w_e, H, F, r, k);
       const __half hi = __float2half_rn(w);
-      __half* base = reinterpret_cast<__half*>(packed + ffma_total + 2 * tc_total);
+      __half* base = reinterpret_cast<__half*>(packed + ffma_total);
       base[t] = hi;
       base[tc16_total + t] = __float2half_rn(w - __half2float(hi));
-      continue;
-    }
-    if (e >= ffma_total) {                         // tcgen05 operand: [4H gate columns][Kp], K contiguous
-      const int64_t t = e - ffma_total;
-      const int nn = (int)(t / Kp), k = (int)(t % Kp);
-      const int r = (nn & 3) * H + (nn >> 2);
-      const float w = folded_weight(w_ih, w_hh, w_e, H, F, r, k);
-      uint32_t hb;
-      asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(w));
-      const float hi = __uint_as_float(hb);
-      packed[ffma_total + t] = hi;
-      packed[ffma_total + tc_total + t] = w - hi;
       continue;
     }
     const int k = (int)(e / G), nn = (int)(e % G);
@@ -93,27 +79,23 @@ __global__ void pack_lstm_kernel(const float* __restrict__ w_ih, const float* __
 // ---------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) pointer_step_dot_kernel(
     const PointerStepArgs pa, int k, const float* __restrict__ q, int64_t q_ld, const float* __restrict__ inputs, int F,
-    void* __restrict__ a_hi_next, void* __restrict__ a_lo_next, int64_t a_ld, int a_f16) {
+    const LstmXSlot x_next) {
   const int lane = threadIdx.x & 31;
   const int64_t b = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (b >= pa.n) return;
   const float4* qp = reinterpret_cast<const float4*>(q + b * q_ld);
   const float4 q0 = __ldg(qp + 2 * lane), q1 = __ldg(qp + 2 * lane + 1);     // the lane's floats [8*lane, 8*lane+8)
   const int fed = pointer_step_warp(pa, k, b, q0, q1, lane);
-  if (a_hi_next && lane < F) {
-    // tensor-core path: the chosen candidate's raw row becomes columns [H, H+F) of the next step's A operand
-    const float v = __ldg(inputs + (b * pa.L + fed) * (int64_t)F + lane);
-    if (a_f16) {
-      const __half hi = __float2half_rn(v);
-      reinterpret_cast<__half*>(a_hi_next)[b * a_ld + kH + lane] = hi;
-      reinterpret_cast<__half*>(a_lo_next)[b * a_ld + kH + lane] = __float2half_rn(v - __half2float(hi));
-    } else {
-      uint32_t hb;
-      asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(v));
-      reinterpret_cast<float*>(a_hi_next)[b * a_ld + kH + lane] = __uint_as_float(hb);
-      reinterpret_cast<float*>(a_lo_next)[b * a_ld + kH + lane] = v - __uint_as_float(hb);
-    }
-  }
+  if (x_next.hi && lane < F)     // tensor-core path: the fed candidate's raw row is the next step's input
+    stage_x_f16(x_next.hi, x_next.lo, x_next.ld, b, lane, __ldg(inputs + (b * pa.L + fed) * (int64_t)F + lane));
+}
+
+// argument block of the pointer steps over row-major encodings [n, L, kH]
+PointerStepArgs pointer_step_args(const float* enc_out, const float* latent_win, float alpha, int use_tanh, float C,
+                                  int64_t n, int L, int N, int32_t* idx_out, float* win_logits, float* win_probs,
+                                  const int32_t* forced, const float* uniform) {
+  return PointerStepArgs{enc_out, (int64_t)L * kH, latent_win, alpha, use_tanh, C, n, L, N, idx_out, win_logits,
+                         win_probs, forced, uniform};
 }
 
 // ---------------------------------------------------------------------------
@@ -270,8 +252,7 @@ int gnnpn_pn_pack_lstm_f32(const float* w_ih, const float* w_hh, const float* b_
   GNNPN_REQUIRE(w_ih && w_hh && b_ih && b_hh && w_embed && b_embed && packed, GNNPN_ENULL);
   GNNPN_REQUIRE(hidden == kH && in_features >= 1 && in_features <= kXPad, GNNPN_ESHAPE);
   pack_lstm_kernel<<<kNumSMs * 4, 256, 0, (cudaStream_t)stream>>>(w_ih, w_hh, b_ih, b_hh, w_embed, b_embed,
-                                                                  start_input, hidden, in_features, kXPad, kKp,
-                                                                  packed);
+                                                                  start_input, hidden, in_features, kXPad, packed);
   return after_launch();
 }
 
@@ -332,37 +313,10 @@ int gnnpn_lstm_encode_f32(const float* inputs, int64_t n, int L, int in_features
     return tc_seq_encode(sa, st);
   }
   GNNPN_REQUIRE(enc_layout == GNNPN_ENC_ROWMAJOR, GNNPN_EUNSUPPORTED);
-  if (workspace) {
-    // ---- tcgen05 recurrence, one launch per step: [h|x] kept as hi/lo pairs in two ping-pong buffers
-    TcLstmPlan plan;
-    int rc = tc_lstm_plan(&plan, workspace, workspace_bytes, n, packed);
-    if (rc) return rc;
-    if ((rc = tc_lstm_reset(plan, inputs, (int64_t)L * in_features, 0, in_features, st))) return rc;
-    TcLstmStep s{};
-    s.use_x = 1; s.bias = packed + kOffBias; s.c = c_state; s.h_out_ld = (int64_t)L * kH;
-    s.x_next = inputs; s.x_inst_ld = (int64_t)L * in_features; s.F = in_features;
-    for (int t = 0; t < L; ++t) {
-      s.cur = t & 1; s.first = t == 0;
-      s.h_out = enc_out + (int64_t)t * kH;
-      s.x_row_next = t + 1 < L ? t + 1 : -1;
-      if ((rc = tc_lstm_step(plan, s, st))) return rc;
-    }
-    return GNNPN_OK;
-  }
-  LstmStepArgs a{};
-  a.x = inputs; a.x_inst_ld = (int64_t)L * in_features; a.F = in_features; a.use_x = 1; a.gather = nullptr;
-  a.P = packed; a.bias = packed + kOffBias;
-  a.c = c_state; a.M = (int)n;
-  a.h_in_ld = a.h_out_ld = (int64_t)L * kH;
-  for (int t = 0; t < L; ++t) {
-    a.first = t == 0;
-    a.h_in = t == 0 ? nullptr : enc_out + (int64_t)(t - 1) * kH;
-    a.h_out = enc_out + (int64_t)t * kH;
-    a.x_row = t;
-    int rc = launch_lstm_step(a, st);
-    if (rc) return rc;
-  }
-  return GNNPN_OK;
+  LstmRecurrence r;
+  int rc = lstm_recurrence_init(&r, packed, inputs, n, L, in_features, c_state, workspace, workspace_bytes);
+  for (int t = 0; t < L && !rc; ++t) rc = lstm_encoder_step(r, t, enc_out, nullptr, st);
+  return rc;
 }
 
 int gnnpn_pn_decode_greedy_f32(const float* inputs, const float* enc_out, float* c_state,
@@ -383,11 +337,7 @@ int gnnpn_pn_decode_greedy_f32(const float* inputs, const float* enc_out, float*
   GNNPN_REQUIRE(aligned16(enc_out) && aligned16(dec_h) && aligned16(c_state) && aligned16(packed), GNNPN_EALIGN);   // NULL dec_h passes
   if (n == 0) return GNNPN_OK;
   cudaStream_t st = (cudaStream_t)stream;
-  const float* bias = packed + kOffBias;
-  const float* start = packed + kOffStart;
-  const unsigned att_blocks = (unsigned)ceil_div(n, 8);
-  const bool use_tc = workspace != nullptr;
-  if (use_tc && (seq_mode() & 2) && in_features <= 8) {
+  if (workspace && (seq_mode() & 2) && in_features <= 8) {
     GNNPN_REQUIRE((reinterpret_cast<uintptr_t>(enc_out) & 31u) == 0 && (reinterpret_cast<uintptr_t>(c_state) & 31u) == 0 &&
                       (reinterpret_cast<uintptr_t>(dec_h) & 31u) == 0, GNNPN_EALIGN);
     SeqDecodeArgs sa{inputs, enc_out, c_state, latent_win, alpha, packed, use_tanh, C, n, L, in_features, K, N,
@@ -400,49 +350,15 @@ int gnnpn_pn_decode_greedy_f32(const float* inputs, const float* enc_out, float*
     return tc_seq_decode(sa, st);
   }
   GNNPN_REQUIRE(enc_layout == GNNPN_ENC_ROWMAJOR, GNNPN_EUNSUPPORTED);
-  TcLstmPlan plan;
-  TcLstmStep ts{};
-  LstmStepArgs a{};
-  int rc;
-  if (use_tc) {
-    if ((rc = tc_lstm_plan(&plan, workspace, workspace_bytes, n, packed))) return rc;
-    // decoder state starts from the encoder's last hidden state (modelPN.py:191,205)
-    if ((rc = tc_lstm_load_h(plan, 0, enc_out + (int64_t)(L - 1) * kH, (int64_t)L * kH, st))) return rc;
-    if ((rc = tc_lstm_zero(plan, 1, st))) return rc;
-    ts.c = c_state; ts.h_out_ld = (int64_t)K * kH; ts.x_next = nullptr; ts.x_row_next = -1;
-    ts.F = in_features; ts.first = 0;
-  } else {
-    a.x = inputs; a.x_inst_ld = (int64_t)L * in_features; a.F = in_features; a.x_row = -1;
-    a.P = packed; a.c = c_state; a.M = (int)n; a.first = 0;
-    a.h_out_ld = (int64_t)K * kH;
-  }
+  LstmRecurrence r;
+  int rc = lstm_recurrence_init(&r, packed, inputs, n, L, in_features, c_state, workspace, workspace_bytes);
+  if (rc) return rc;
+  const PointerStepArgs pa = pointer_step_args(enc_out, latent_win, alpha, use_tanh, C, n, L, N, idx_out, win_logits,
+                                               win_probs, forced_idx, sample_uniform);
   for (int k = 0; k < K; ++k) {
-    const int32_t* fed_prev = k == 0 ? nullptr : (forced_idx ? forced_idx : idx_out) + (int64_t)(k - 1) * n;
-    if (use_tc) {
-      ts.cur = k & 1; ts.use_x = k != 0; ts.bias = k == 0 ? start : bias;
-      ts.h_out = dec_h + (int64_t)k * kH;
-      if ((rc = tc_lstm_step(plan, ts, st))) return rc;
-    } else {
-      if (k == 0) {
-        a.h_in = enc_out + (int64_t)(L - 1) * kH; a.h_in_ld = (int64_t)L * kH;
-        a.use_x = 0; a.bias = start; a.gather = nullptr;
-      } else {
-        a.h_in = dec_h + (int64_t)(k - 1) * kH; a.h_in_ld = (int64_t)K * kH;
-        a.use_x = 1; a.bias = bias; a.gather = fed_prev;
-      }
-      a.h_out = dec_h + (int64_t)k * kH;
-      if ((rc = launch_lstm_step(a, st))) return rc;
-    }
-    const int nxt = (k + 1) & 1;
-    PointerStepArgs pa;
-    pa.enc_out = enc_out; pa.enc_inst_ld = (int64_t)L * kH; pa.latent_win = latent_win; pa.alpha = alpha;
-    pa.use_tanh = use_tanh; pa.C = C; pa.n = n; pa.L = L; pa.N = N;
-    pa.idx_out = idx_out; pa.win_logits = win_logits; pa.win_probs = win_probs;
-    pa.forced = forced_idx; pa.uniform = sample_uniform;
-    pointer_step_dot_kernel<<<att_blocks, 256, 0, st>>>(
-        pa, k, dec_h + (int64_t)k * kH, (int64_t)K * kH, inputs, in_features,
-        use_tc ? plan.hi[nxt] : nullptr, use_tc ? plan.lo[nxt] : nullptr, use_tc ? (int64_t)plan.ld : 0,
-        use_tc ? plan.f16 : 0);
+    if ((rc = lstm_decoder_step(r, k, enc_out, dec_h, K, forced_idx ? forced_idx : idx_out, nullptr, st))) return rc;
+    pointer_step_dot_kernel<<<(unsigned)ceil_div(n, 8), 256, 0, st>>>(pa, k, dec_h + (int64_t)k * kH, (int64_t)K * kH,
+                                                                     inputs, in_features, lstm_decoder_x_slot(r, k));
     if ((rc = after_launch())) return rc;
   }
   return GNNPN_OK;
@@ -462,42 +378,21 @@ int gnnpn_pn_train_forward_f32(const float* inputs, const float* packed_enc, con
   GNNPN_REQUIRE(aligned16(enc_out) && aligned16(dec_h) && aligned16(gates_e) && aligned16(gates_d), GNNPN_EALIGN);
   if (n == 0) return GNNPN_OK;
   cudaStream_t st = (cudaStream_t)stream;
-  int rc;
-  LstmStepArgs a{};
-  a.x = inputs; a.x_inst_ld = (int64_t)L * in_features; a.F = in_features; a.use_x = 1; a.gather = nullptr;
-  a.P = packed_enc; a.bias = packed_enc + kOffBias; a.M = (int)n;
-  a.h_in_ld = a.h_out_ld = (int64_t)L * kH;
-  for (int t = 0; t < L; ++t) {
-    a.first = t == 0;
-    a.h_in = t == 0 ? nullptr : enc_out + (int64_t)(t - 1) * kH;
-    a.h_out = enc_out + (int64_t)t * kH;
-    a.x_row = t;
-    a.gates_out = gates_e + (size_t)t * n * kG;
-    a.c = c_e + (size_t)t * n * kH;                                  // this step's slot of the saved cell states
-    a.c_in = t == 0 ? nullptr : c_e + (size_t)(t - 1) * n * kH;
-    if ((rc = launch_lstm_step(a, st))) return rc;
+  const size_t nh = (size_t)n * kH;
+  LstmRecurrence r;
+  int rc = lstm_recurrence_init(&r, packed_enc, inputs, n, L, in_features, nullptr, nullptr, 0);
+  for (int t = 0; t < L && !rc; ++t) {
+    const LstmStepSaves sv{gates_e + t * n * kG, c_e + t * nh, t == 0 ? nullptr : c_e + (t - 1) * nh};
+    rc = lstm_encoder_step(r, t, enc_out, &sv, st);
   }
-  a.P = packed_dec; a.x_row = -1; a.first = 0; a.h_out_ld = (int64_t)K * kH;
+  if (rc || (rc = lstm_recurrence_init(&r, packed_dec, inputs, n, L, in_features, nullptr, nullptr, 0))) return rc;
+  const PointerStepArgs pa = pointer_step_args(enc_out, latent_win, alpha, use_tanh, C, n, L, N, idx_free, win_logits,
+                                               win_probs, idx, nullptr);
   for (int k = 0; k < K; ++k) {
-    if (k == 0) {
-      a.h_in = enc_out + (int64_t)(L - 1) * kH; a.h_in_ld = (int64_t)L * kH;
-      a.use_x = 0; a.bias = packed_dec + kOffStart; a.gather = nullptr;
-    } else {
-      a.h_in = dec_h + (int64_t)(k - 1) * kH; a.h_in_ld = (int64_t)K * kH;
-      a.use_x = 1; a.bias = packed_dec + kOffBias; a.gather = idx + (int64_t)(k - 1) * n;
-    }
-    a.h_out = dec_h + (int64_t)k * kH;
-    a.gates_out = gates_d + (size_t)k * n * kG;
-    a.c = c_d + (size_t)k * n * kH;
-    a.c_in = k == 0 ? c_e + (size_t)(L - 1) * n * kH : c_d + (size_t)(k - 1) * n * kH;
-    if ((rc = launch_lstm_step(a, st))) return rc;
-    PointerStepArgs pa;
-    pa.enc_out = enc_out; pa.enc_inst_ld = (int64_t)L * kH; pa.latent_win = latent_win; pa.alpha = alpha;
-    pa.use_tanh = use_tanh; pa.C = C; pa.n = n; pa.L = L; pa.N = N;
-    pa.idx_out = idx_free; pa.win_logits = win_logits; pa.win_probs = win_probs;
-    pa.forced = idx; pa.uniform = nullptr;
+    const LstmStepSaves sv{gates_d + k * n * kG, c_d + k * nh, k == 0 ? c_e + (L - 1) * nh : c_d + (k - 1) * nh};
+    if ((rc = lstm_decoder_step(r, k, enc_out, dec_h, K, idx, &sv, st))) return rc;
     pointer_step_dot_kernel<<<(unsigned)ceil_div(n, 8), 256, 0, st>>>(pa, k, dec_h + (int64_t)k * kH, (int64_t)K * kH,
-                                                                     inputs, in_features, nullptr, nullptr, 0, 0);
+                                                                     inputs, in_features, lstm_decoder_x_slot(r, k));
     if ((rc = after_launch())) return rc;
   }
   return GNNPN_OK;
@@ -514,14 +409,11 @@ int gnnpn_pn_attention_windows_f32(const float* enc_out, const float* dec_h, con
   GNNPN_REQUIRE(hidden == kH && K >= 1 && N >= 1 && N <= kMaxWindow && (int64_t)K * N == L && n >= 0, GNNPN_ESHAPE);
   GNNPN_REQUIRE(aligned16(enc_out) && aligned16(dec_h), GNNPN_EALIGN);
   if (n == 0) return GNNPN_OK;
-  PointerStepArgs pa;
-  pa.enc_out = enc_out; pa.enc_inst_ld = (int64_t)L * kH; pa.latent_win = latent_win; pa.alpha = alpha;
-  pa.use_tanh = use_tanh; pa.C = C; pa.n = n; pa.L = L; pa.N = N;
-  pa.idx_out = idx_out; pa.win_logits = win_logits; pa.win_probs = win_probs;
-  pa.forced = nullptr; pa.uniform = nullptr;
+  const PointerStepArgs pa = pointer_step_args(enc_out, latent_win, alpha, use_tanh, C, n, L, N, idx_out, win_logits,
+                                               win_probs, nullptr, nullptr);
   for (int k = 0; k < K; ++k) {
     pointer_step_dot_kernel<<<(unsigned)ceil_div(n, 8), 256, 0, (cudaStream_t)stream>>>(
-        pa, k, dec_h + (int64_t)k * kH, (int64_t)K * kH, nullptr, 0, nullptr, nullptr, 0, 0);
+        pa, k, dec_h + (int64_t)k * kH, (int64_t)K * kH, nullptr, 0, LstmXSlot{nullptr, nullptr, 0});
     const int rc = after_launch();
     if (rc) return rc;
   }

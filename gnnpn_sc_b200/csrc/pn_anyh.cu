@@ -7,11 +7,9 @@
 // W_ih . start), torch gate order (i, f, g, o) as row blocks of Wcat [4H, H + F].
 #include <math.h>
 #include "common.cuh"
+#include "internal.cuh"
 
 namespace gnnpn {
-int launch_gemm_ffma(const float* A, int64_t lda, const float* W, int64_t ldw, const float* bias,
-                     const float* scale, const float* shift, int act, float* C, int64_t ldc, int64_t M, int N,
-                     int K, cudaStream_t st);
 namespace {
 
 constexpr int kMaxWindowAnyH = 32;

@@ -13,6 +13,7 @@
 // traffic beyond what the per-step kernels wrote; the cluster barrier (release / acquire at cluster scope) orders it.
 // Same formulas as lstm_cell_bwd_kernel (pn_train.cu); strict fp32.
 #include <math.h>
+#include "internal.cuh"
 #include "lstm_step.cuh"
 #include "options.cuh"
 

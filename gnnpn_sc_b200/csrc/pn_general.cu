@@ -10,14 +10,12 @@
 // same as pointer_step_warp's (canonical dot, fmaf latent, sequential softmax sum) -> bit-identical picks / logits.
 #include <math.h>
 #include <cuda_fp16.h>
+#include "internal.cuh"
 #include "lstm_step.cuh"
 #include "tc_lstm.cuh"
 #include "pointer.cuh"
 
 namespace gnnpn {
-int launch_gemm_ffma(const float* A, int64_t lda, const float* W, int64_t ldw, const float* bias,
-                     const float* scale, const float* shift, int act, float* C, int64_t ldc, int64_t M, int N,
-                     int K, cudaStream_t st);
 namespace {
 
 constexpr int kAttThreads = 256, kAttWarps = kAttThreads / 32;
@@ -126,10 +124,7 @@ struct PointerGeneralArgs {
   const float* uniform;      // [K, n] or nullptr
   const float* inputs;       // [n, L, F]
   int F;
-  void* a_hi_next;           // tensor-core LSTM path: A operand of the next step (nullptr: FFMA path gathers by idx)
-  void* a_lo_next;
-  int64_t a_ld;
-  int a_f16;
+  LstmXSlot x_next;          // tensor-core LSTM path: where the fed row goes (hi == nullptr: the FFMA step gathers it)
 };
 
 template <bool BAHD>
@@ -224,19 +219,9 @@ __global__ void __launch_bounds__(kAttThreads) pointer_general_kernel(const Poin
     s_pick = p.forced ? p.forced[(int64_t)k * p.g.n + b] : k * N + bj;
   }
   __syncthreads();
-  if (p.a_hi_next && threadIdx.x < p.F) {
+  if (p.x_next.hi && threadIdx.x < p.F) {
     const int f = threadIdx.x;
-    const float v = __ldg(p.inputs + (b * p.g.L + s_pick) * (int64_t)p.F + f);
-    if (p.a_f16) {
-      const __half hi = __float2half_rn(v);
-      reinterpret_cast<__half*>(p.a_hi_next)[b * p.a_ld + kH + f] = hi;
-      reinterpret_cast<__half*>(p.a_lo_next)[b * p.a_ld + kH + f] = __float2half_rn(v - __half2float(hi));
-    } else {
-      uint32_t hb;
-      asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(v));
-      reinterpret_cast<float*>(p.a_hi_next)[b * p.a_ld + kH + f] = __uint_as_float(hb);
-      reinterpret_cast<float*>(p.a_lo_next)[b * p.a_ld + kH + f] = v - __uint_as_float(hb);
-    }
+    stage_x_f16(p.x_next.hi, p.x_next.lo, p.x_next.ld, b, f, __ldg(p.inputs + (b * p.g.L + s_pick) * (int64_t)p.F + f));
   }
 }
 
@@ -342,22 +327,9 @@ int gnnpn_pn_decode_general_f32(const float* inputs, const float* enc_out, float
         (rc = launch_gemm_ffma(enc_out, kH, att_g + kOffWr, kH, att_g + kOffBr, nullptr, nullptr, GNNPN_ACT_NONE, e_g,
                                kH, n * (int64_t)L, kH, kH, st))) return rc;
   }
-  const float* bias = packed + kOffBias;
-  const float* start = packed + kOffStart;
-  TcLstmPlan plan;
-  TcLstmStep ts{};
-  LstmStepArgs a{};
-  if (use_tc) {
-    if ((rc = tc_lstm_plan(&plan, ws + wsl.tc, tc_lstm_workspace_bytes(n), n, packed))) return rc;
-    if ((rc = tc_lstm_load_h(plan, 0, enc_out + (int64_t)(L - 1) * kH, (int64_t)L * kH, st))) return rc;
-    if ((rc = tc_lstm_zero(plan, 1, st))) return rc;
-    ts.c = c_state; ts.h_out_ld = (int64_t)K * kH; ts.x_next = nullptr; ts.x_row_next = -1;
-    ts.F = in_features; ts.first = 0;
-  } else {
-    a.x = inputs; a.x_inst_ld = (int64_t)L * in_features; a.F = in_features; a.x_row = -1;
-    a.P = packed; a.c = c_state; a.M = (int)n; a.first = 0;
-    a.h_out_ld = (int64_t)K * kH;
-  }
+  LstmRecurrence r;
+  if ((rc = lstm_recurrence_init(&r, packed, inputs, n, L, in_features, c_state, use_tc ? ws + wsl.tc : nullptr,
+                                 tc_lstm_workspace_bytes(n)))) return rc;
   const int32_t* fed_all = forced_idx ? forced_idx : idx_out;
   const size_t glimpse_smem = (size_t)((((L + 31) / 32) + 3) & ~3) * 4 + (size_t)kAttWarps * (4 + kH) * 4;
   const size_t ptr_smem = (size_t)N * 2 * sizeof(float);
@@ -371,21 +343,7 @@ int gnnpn_pn_decode_general_f32(const float* inputs, const float* enc_out, float
   }
   for (int k = 0; k < K; ++k) {
     // ---- decoder LSTM cell (modelPN.py:205)
-    if (use_tc) {
-      ts.cur = k & 1; ts.use_x = k != 0; ts.bias = k == 0 ? start : bias;
-      ts.h_out = dec_h + (int64_t)k * kH;
-      if ((rc = tc_lstm_step(plan, ts, st))) return rc;
-    } else {
-      if (k == 0) {
-        a.h_in = enc_out + (int64_t)(L - 1) * kH; a.h_in_ld = (int64_t)L * kH;
-        a.use_x = 0; a.bias = start; a.gather = nullptr;
-      } else {
-        a.h_in = dec_h + (int64_t)(k - 1) * kH; a.h_in_ld = (int64_t)K * kH;
-        a.use_x = 1; a.bias = bias; a.gather = fed_all + (int64_t)(k - 1) * n;
-      }
-      a.h_out = dec_h + (int64_t)k * kH;
-      if ((rc = launch_lstm_step(a, st))) return rc;
-    }
+    if ((rc = lstm_decoder_step(r, k, enc_out, dec_h, K, fed_all, nullptr, st))) return rc;
     // ---- glimpses (modelPN.py:208-211)
     const float* q_cur = dec_h + (int64_t)k * kH;
     for (int g = 0; g < n_glimpses; ++g) {
@@ -416,9 +374,7 @@ int gnnpn_pn_decode_general_f32(const float* inputs, const float* enc_out, float
     pa.latent_win = latent_win; pa.alpha = alpha; pa.use_tanh = use_tanh; pa.C = C; pa.N = N;
     pa.idx_out = idx_out; pa.win_logits = win_logits; pa.win_probs = win_probs;
     pa.forced = forced_idx; pa.uniform = sample_uniform; pa.inputs = inputs; pa.F = in_features;
-    const int nxt = (k + 1) & 1;
-    pa.a_hi_next = use_tc ? plan.hi[nxt] : nullptr; pa.a_lo_next = use_tc ? plan.lo[nxt] : nullptr;
-    pa.a_ld = use_tc ? plan.ld : 0; pa.a_f16 = use_tc ? plan.f16 : 0;
+    pa.x_next = lstm_decoder_x_slot(r, k);
     if (bahd) {
       float* qwp = qw_pointer + (int64_t)k * kH;                 // [n, K, kH]: kept for the dense-logits kernel
       if ((rc = launch_gemm_ffma(q_cur, (int64_t)K * kH, att_p + kOffWq, kH, att_p + kOffBq, nullptr, nullptr,

@@ -10,17 +10,12 @@
 // (M = the folded W_ih . W_embed input block), which the caller runs through gnnpn_gemm_f32_bias_act.
 // Dot attention, no glimpses, embedding_size = 0 (what every reference call site trains).
 #include <math.h>
+#include "internal.cuh"
 #include "lstm_step.cuh"
 #include "pointer.cuh"
 #include "options.cuh"
 
 namespace gnnpn {
-int launch_gemm_ffma(const float* A, int64_t lda, const float* W, int64_t ldw, const float* bias,
-                     const float* scale, const float* shift, int act, float* C, int64_t ldc, int64_t M, int N,
-                     int K, cudaStream_t st);
-int launch_bptt_scan(const float* gates, const float* c, const float* c_init, const float* dh_ext, int64_t dh_ld_m,
-                     const float* dh_init, const float* dc_init, const float* w_hh, float* dG_T, float* dh_out,
-                     float* dc_out, int64_t n, int T, cudaStream_t st);
 namespace {
 
 // split-K of dh(t-1) = dG(t) . W_hh (dh_splitk_kernel): 16 chunks of 64 gate rows

@@ -20,6 +20,7 @@
 #include <cuda_fp16.h>
 #include "tc_common.cuh"
 #include "common.cuh"
+#include "internal.cuh"
 #include "lstm_step.cuh"
 #include "tc_lstm.cuh"
 #include "tc_seq.cuh"
@@ -491,21 +492,6 @@ lstm_colsplit_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid
   tc_fence_before();
   cluster_sync_all();
   if (warp == 2) tmem_dealloc(tmem_base, LY::TMEM_COLS);
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult qr;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qr) == cudaSuccess &&
-        qr == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)ptr;
-  }
-  return fn;
 }
 
 }  // namespace cs

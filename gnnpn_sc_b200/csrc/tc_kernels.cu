@@ -3,7 +3,8 @@
 //                                                                lo.lo term is ~2^-22 relative)
 // accumulated in fp32 in TMEM.  One mainloop, two epilogues:
 //   * node transform   C = act((A.W^T + bias)*scale + shift)                     (modelML.py linears / GCNConv X.W)
-//   * LSTM step        gates = [h|x].P^T + bias -> c', h'  (+ tf32 split of h' for the next step's A operand)
+//   * LSTM step        gates = [h|x].P^T + bias -> c', h'  (+ fp16 split of h' for the next step's A operand); its
+//                      operands are fp16 hi/lo pairs (3xFP16, same three products), see Kind<true>
 //
 // CTA = one 128-row M tile; loops over `n_tiles` N tiles of BN <= 256 columns with two TMEM
 // accumulator buffers so the epilogue of tile j overlaps the MMAs of tile j+1.
@@ -12,12 +13,13 @@
 // sub-partition, which is what hides the global-memory latency of the per-row state loads/stores).
 // smem ring: STAGES x { A_hi, A_lo [128 x 32 f32], B_hi, B_lo [BN x 32 f32] }, 128B-swizzled K-major tiles
 // written by TMA and read by tcgen05.mma through UMMA descriptors.
-#include <stdlib.h>
 #include <algorithm>
 #include "tc_common.cuh"
 #include "common.cuh"
+#include "internal.cuh"
 #include "lstm_step.cuh"
 #include "tc_lstm.cuh"
+#include "tc_seq.cuh"
 
 namespace gnnpn {
 namespace tc {
@@ -46,8 +48,8 @@ struct LstmEpilogueParams {
   float* c;                 // [M,256] in/out
   float* h_out;             // exact fp32 h' rows, h_out_ld apart
   int64_t h_out_ld;
-  float* a_hi_next;         // [M, a_ld]  tf32 split of h' for the next step (+ x columns)
-  float* a_lo_next;
+  __half* a_hi_next;        // [M, a_ld]  fp16 split of h' for the next step (+ x columns)
+  __half* a_lo_next;
   int64_t a_ld;
   const float* x_next;      // raw inputs row of the NEXT step per instance (nullptr: none)
   int64_t x_inst_ld;
@@ -62,7 +64,6 @@ struct MainloopParams {
   int bn;                   // columns per N tile (multiple of 16, <= 256)
   int k_blocks;             // K / 32
   int last_block_ksteps;    // k-steps (of 8) actually non-zero in the last k block (1..4)
-  int dbg;                  // profiling experiments only (GNNPN_TC_DBG): 1 = hi.hi MMA only, 2 = epilogue skips math
   int kb_per_split;         // split-K: k blocks per blockIdx.y (>= k_blocks: no split)
 };
 
@@ -160,13 +161,9 @@ tc_mainloop_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
           for (int ks = 0; ks < ksteps; ++ks) {
             const uint64_t adv = (uint64_t)(ks * 2);            // +32 B per k-step inside the 128-byte swizzle row
             const uint32_t acc0 = ((kb - kb0) | ks) != 0;
-            if (mp.dbg != 1) {
-              Kind<F16>::mma(d, a_lo + adv, b_hi + adv, idesc, acc0);
-              Kind<F16>::mma(d, a_hi + adv, b_lo + adv, idesc, 1u);
-              Kind<F16>::mma(d, a_hi + adv, b_hi + adv, idesc, 1u);
-            } else {
-              Kind<F16>::mma(d, a_hi + adv, b_hi + adv, idesc, acc0);
-            }
+            Kind<F16>::mma(d, a_lo + adv, b_hi + adv, idesc, acc0);
+            Kind<F16>::mma(d, a_hi + adv, b_lo + adv, idesc, 1u);
+            Kind<F16>::mma(d, a_hi + adv, b_hi + adv, idesc, 1u);
           }
           mma_commit(empty_bar(s));                 // smem slot reusable once these MMAs retire
           if (kb == kb1 - 1) mma_commit(tmem_full_bar(buf));
@@ -203,7 +200,7 @@ tc_mainloop_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
           float v[32];
           tmem_ld_32x32_issue(t0 + (uint32_t)c0, v);
           tmem_ld_wait(v);
-          if (mp.dbg != 2) epi.chunk(i, nt * mp.bn + c0, min(32, mp.bn - c0), v);
+          epi.chunk(i, nt * mp.bn + c0, min(32, mp.bn - c0), v);
         }
       }
       tc_fence_before();
@@ -269,32 +266,18 @@ __device__ __forceinline__ void stg256(float* p, const float* v) {
                "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7]) : "memory");
 }
 
-template <bool F16>
-struct LstmEpilogueT {
+struct LstmEpilogue {
   const LstmEpilogueParams& p; int64_t row; bool ok;
   const float* sbias;            // the 1024 gate biases, staged once per CTA
   float c_pre[BN_MAX / (32 * EPI_GROUPS)][8];   // prefetched cell state: 8 hidden units per owned chunk
   __device__ static void stage_smem(const LstmEpilogueParams& p, float* smem, int tid, int nthreads) {
     for (int i = tid; i < kG; i += nthreads) smem[i] = __ldg(p.bias + i);
   }
-  __device__ LstmEpilogueT(const LstmEpilogueParams& p_, const float* smem, int row_, bool ok_, bool primary)
+  __device__ LstmEpilogue(const LstmEpilogueParams& p_, const float* smem, int row_, bool ok_, bool primary)
       : p(p_), row(row_), ok(ok_), sbias(smem) {
     if (ok && primary && p.x_next && p.x_row_next >= 0) {   // stage the next step's raw input as A columns 256..
       const float* x = p.x_next + row * p.x_inst_ld + (int64_t)p.x_row_next * p.F;
-      for (int f = 0; f < p.F; ++f) {
-        const float xv = __ldg(x + f);
-        if (F16) {
-          __half hi, lo;
-          split_f16(xv, hi, lo);
-          reinterpret_cast<__half*>(p.a_hi_next)[row * p.a_ld + kH + f] = hi;
-          reinterpret_cast<__half*>(p.a_lo_next)[row * p.a_ld + kH + f] = lo;
-        } else {
-          float hi, lo;
-          split_tf32(xv, hi, lo);
-          p.a_hi_next[row * p.a_ld + kH + f] = hi;
-          p.a_lo_next[row * p.a_ld + kH + f] = lo;
-        }
-      }
+      for (int f = 0; f < p.F; ++f) stage_x_f16(p.a_hi_next, p.a_lo_next, p.a_ld, row, f, __ldg(x + f));
     }
   }
   __device__ void prefetch(int slot, int col0) {
@@ -311,7 +294,7 @@ struct LstmEpilogueT {
     const int j0 = col0 >> 2;
     float hv[8], cv[8];
     const float4* bias4 = reinterpret_cast<const float4*>(sbias + col0);
-    constexpr float kAccScale = F16 ? 1.0f / kW16Scale : 1.0f;      // fp16 weights are stored pre-scaled
+    constexpr float kAccScale = 1.0f / kW16Scale;      // fp16 weights are stored pre-scaled
 #pragma unroll
     for (int u = 0; u < 8; ++u) {
       const float4 b = bias4[u];
@@ -323,25 +306,17 @@ struct LstmEpilogueT {
     }
     stg256(p.c + row * kH + j0, cv);
     stg256(p.h_out + row * p.h_out_ld + j0, hv);
-    if (F16) {
-      __half2 hh[4], hl[4];
+    __half2 hh[4], hl[4];
 #pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        __half a0, l0, a1, l1;
-        split_f16(hv[2 * u], a0, l0);
-        split_f16(hv[2 * u + 1], a1, l1);
-        hh[u] = __halves2half2(a0, a1);
-        hl[u] = __halves2half2(l0, l1);
-      }
-      *reinterpret_cast<uint4*>(reinterpret_cast<__half*>(p.a_hi_next) + row * p.a_ld + j0) = *reinterpret_cast<uint4*>(hh);
-      *reinterpret_cast<uint4*>(reinterpret_cast<__half*>(p.a_lo_next) + row * p.a_ld + j0) = *reinterpret_cast<uint4*>(hl);
-    } else {
-      float hh[8], hl[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) split_tf32(hv[u], hh[u], hl[u]);
-      stg256(p.a_hi_next + row * p.a_ld + j0, hh);
-      stg256(p.a_lo_next + row * p.a_ld + j0, hl);
+    for (int u = 0; u < 4; ++u) {
+      __half a0, l0, a1, l1;
+      split_f16(hv[2 * u], a0, l0);
+      split_f16(hv[2 * u + 1], a1, l1);
+      hh[u] = __halves2half2(a0, a1);
+      hl[u] = __halves2half2(l0, l1);
     }
+    *reinterpret_cast<uint4*>(p.a_hi_next + row * p.a_ld + j0) = *reinterpret_cast<uint4*>(hh);
+    *reinterpret_cast<uint4*>(p.a_lo_next + row * p.a_ld + j0) = *reinterpret_cast<uint4*>(hl);
   }
 };
 
@@ -363,11 +338,7 @@ __global__ void split_tf32_kernel(const float* __restrict__ src, int64_t ld, int
 
 // ------------------------------------------------------------------------------------------------
 // host side: tensor maps through the driver entry point (no link-time libcuda dependency)
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn encode_fn() {
+EncodeTiledFn encode_fn() {
   static EncodeTiledFn fn = nullptr;
   if (!fn) {
     void* p = nullptr;
@@ -379,10 +350,7 @@ static EncodeTiledFn encode_fn() {
   return fn;
 }
 
-// row-major [rows, cols] fp32 (or fp16) with leading dimension ld (elements); box = {128 bytes of columns,
-// box_rows}; 128B swizzle
-int make_map_2d(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows,
-                bool f16 = false) {
+int make_map_2d(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows, bool f16) {
   EncodeTiledFn fn = encode_fn();
   if (!fn) return GNNPN_EUNSUPPORTED;
   const int esz = f16 ? 2 : 4;
@@ -407,9 +375,7 @@ int launch_mainloop(const CUtensorMap maps[4], const MainloopParams& mp, const E
     configured = true;
   }
   const unsigned grid = (unsigned)ceil_div(mp.M, BM);
-  static const int dbg = getenv("GNNPN_TC_DBG") ? atoi(getenv("GNNPN_TC_DBG")) : 0;
   MainloopParams mpd = mp;
-  mpd.dbg = dbg;
   if (mpd.kb_per_split <= 0) mpd.kb_per_split = mpd.k_blocks;
   kern<<<dim3(grid, (unsigned)splits), THREADS, SMEM_BYTES, st>>>(maps[0], maps[1], maps[2], maps[3], mpd, ep);
   return after_launch();
@@ -486,41 +452,29 @@ int launch_gemm_tc(const float* A, int64_t lda, const float* W, int64_t ldw, con
     float* part = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(w_lo + (int64_t)N * Kp) + 255) & ~uintptr_t(255));
     const int kps = (int)ceil_div(Kp / BK, S);
     const int S_eff = (int)ceil_div(Kp / BK, kps);               // every split owns at least one k block (S_eff <= S)
-    MainloopParams mp{(int)M, n_tiles, bn, Kp / BK, BK / 8, 0, kps};
+    MainloopParams mp{(int)M, n_tiles, bn, Kp / BK, BK / 8, kps};
     GemmEpilogueParams ep{nullptr, nullptr, nullptr, GNNPN_ACT_NONE, part, N, N, (int64_t)M * N};
     if ((rc = launch_mainloop<GemmEpilogue, GemmEpilogueParams, false>(maps, mp, ep, st, S_eff))) return rc;
     splitk_reduce_kernel<<<(unsigned)ceil_div(M * (int64_t)N, 256), 256, 0, st>>>(part, S_eff, M, N, bias, scale, shift, act, C,
                                                                                ldc);
     return after_launch();
   }
-  MainloopParams mp{(int)M, n_tiles, bn, Kp / BK, BK / 8, 0, Kp / BK};
+  MainloopParams mp{(int)M, n_tiles, bn, Kp / BK, BK / 8, Kp / BK};
   GemmEpilogueParams ep{bias, scale, shift, act, C, ldc, N, 0};
   return launch_mainloop<GemmEpilogue, GemmEpilogueParams, false>(maps, mp, ep, st);
 }
 
 // ------------------------------------------------------------------------------------------------
-// LSTM recurrence on tcgen05
+// LSTM recurrence, one launch per step
 namespace {
 
-template <bool F16>
 __global__ void stage_x_kernel(const float* __restrict__ inputs, int64_t x_inst_ld, int row, int F, int64_t n,
-                               void* __restrict__ hi, void* __restrict__ lo, int ld) {
+                               __half* __restrict__ hi, __half* __restrict__ lo, int ld) {
   const int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (e >= n * F) return;
   const int64_t m = e / F;
   const int f = (int)(e % F);
-  const float v = inputs[m * x_inst_ld + (int64_t)row * F + f];
-  if (F16) {
-    __half h, l;
-    tc::split_f16(v, h, l);
-    reinterpret_cast<__half*>(hi)[m * ld + kH + f] = h;
-    reinterpret_cast<__half*>(lo)[m * ld + kH + f] = l;
-  } else {
-    float h, l;
-    tc::split_tf32(v, h, l);
-    reinterpret_cast<float*>(hi)[m * ld + kH + f] = h;
-    reinterpret_cast<float*>(lo)[m * ld + kH + f] = l;
-  }
+  stage_x_f16(hi, lo, ld, m, f, inputs[m * x_inst_ld + (int64_t)row * F + f]);
 }
 
 // rows of fp32 h (ld apart) -> fp16 hi/lo rows of kKp16 columns, padding zeroed
@@ -538,96 +492,121 @@ __global__ void split_f16_rows_kernel(const float* __restrict__ src, int64_t ld,
   }
 }
 
-}  // namespace
-
-int tc_lstm_default_f16() {
-  static const int f16 = [] {
-    const char* e = getenv("GNNPN_TC_KIND");
-    return (e && (e[0] == 't' || e[0] == 'T')) ? 0 : 1;
-  }();
-  return f16;
+int tc_zero(const TcLstmPlan& plan, int which, cudaStream_t st) {
+  // hi[which] and lo[which] are adjacent in the workspace
+  cudaError_t e = cudaMemsetAsync(plan.hi[which], 0, (size_t)2 * plan.n * kKp16 * sizeof(__half), st);
+  return e == cudaSuccess ? GNNPN_OK : (int)e;
 }
 
-// sized for the larger (tf32) layout so one query serves both operand kinds
-// (also covers the persistent kernels' blocked cell-state scratch, tc_seq_scratch_floats(n))
-size_t tc_colsplit_scratch_bytes(int64_t n);
+// one tcgen05 step on [h | x] (h only when !use_x) of buffer cur; the epilogue writes h' into buffer cur ^ 1
+int tc_step(const TcLstmPlan& plan, int cur, bool use_x, tc::LstmEpilogueParams ep, cudaStream_t st) {
+  using namespace tc;
+  const CUtensorMap maps[4] = {plan.a_hi[cur], plan.a_lo[cur], plan.b_hi, plan.b_lo};
+  MainloopParams mp;
+  mp.M = (int)plan.n;
+  mp.n_tiles = kG / BN_MAX;
+  mp.bn = BN_MAX;
+  mp.k_blocks = kH / 64 + (use_x ? 1 : 0);
+  mp.last_block_ksteps = use_x ? (ep.F + 15) / 16 : 4;
+  mp.kb_per_split = mp.k_blocks;
+  ep.a_hi_next = plan.hi[cur ^ 1]; ep.a_lo_next = plan.lo[cur ^ 1]; ep.a_ld = kKp16;
+  return launch_mainloop<LstmEpilogue, LstmEpilogueParams, true>(maps, mp, ep, st);
+}
+
+int ffma_step(LstmStepArgs& a, const LstmRecurrence& r, const LstmStepSaves* saves, cudaStream_t st) {
+  a.P = r.packed;
+  a.M = (int)r.n;
+  a.c = saves ? saves->c : r.c;
+  a.c_in = saves ? saves->c_in : nullptr;
+  a.gates_out = saves ? saves->gates : nullptr;
+  return launch_lstm_step(a, st);
+}
+
+}  // namespace
+
 size_t tc_lstm_workspace_bytes(int64_t n) {
-  const size_t step = (size_t)4 * n * kKp * sizeof(float) + 1024;
-  const size_t seq = (size_t)((n + 255) / 256) * 256 * kH * sizeof(float) + 1024;
+  const size_t step = (size_t)4 * n * kKp16 * sizeof(__half) + 1024;
+  const size_t seq = tc_seq_scratch_floats(n) * sizeof(float) + 1024;
   const size_t colsplit = tc_colsplit_scratch_bytes(n) + 1024;
   const size_t m = step > seq ? step : seq;
   return m > colsplit ? m : colsplit;
 }
 
-int tc_lstm_plan(TcLstmPlan* plan, void* workspace, size_t workspace_bytes, int64_t n, const float* packed) {
+int lstm_recurrence_init(LstmRecurrence* r, const float* packed, const float* inputs, int64_t n, int L, int F,
+                         float* c_state, void* workspace, size_t workspace_bytes) {
+  r->packed = packed; r->inputs = inputs; r->n = n; r->L = L; r->F = F; r->c = c_state;
+  r->tc = workspace != nullptr;
+  if (!r->tc) return GNNPN_OK;
   if (workspace_bytes < tc_lstm_workspace_bytes(n)) return GNNPN_EWORKSPACE;
-  char* ws = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(workspace) + 1023) & ~uintptr_t(1023));
-  const int f16 = tc_lstm_default_f16();
-  plan->n = n;
-  plan->f16 = f16;
-  plan->ld = f16 ? kKp16 : kKp;
-  const size_t one = (size_t)n * plan->ld * (f16 ? 2 : 4);       // multiple of 64 bytes
-  plan->hi[0] = ws; plan->lo[0] = ws + one; plan->hi[1] = ws + 2 * one; plan->lo[1] = ws + 3 * one;
+  // two ping-pong [n, kKp16] hi/lo pairs
+  TcLstmPlan& p = r->plan;
+  __half* ws = reinterpret_cast<__half*>((reinterpret_cast<uintptr_t>(workspace) + 1023) & ~uintptr_t(1023));
+  const size_t one = (size_t)n * kKp16;       // halfs, a multiple of 64 bytes
+  p.n = n;
+  p.hi[0] = ws; p.lo[0] = ws + one; p.hi[1] = ws + 2 * one; p.lo[1] = ws + 3 * one;
   int rc;
   for (int b = 0; b < 2; ++b) {
-    if ((rc = tc::make_map_2d(&plan->a_hi[b], plan->hi[b], n, plan->ld, plan->ld, tc::BM, f16))) return rc;
-    if ((rc = tc::make_map_2d(&plan->a_lo[b], plan->lo[b], n, plan->ld, plan->ld, tc::BM, f16))) return rc;
+    if ((rc = tc::make_map_2d(&p.a_hi[b], p.hi[b], n, kKp16, kKp16, tc::BM, true))) return rc;
+    if ((rc = tc::make_map_2d(&p.a_lo[b], p.lo[b], n, kKp16, kKp16, tc::BM, true))) return rc;
   }
-  const float* w_hi = packed + (f16 ? kOffTc16Hi : kOffTcHi);
-  const float* w_lo = packed + (f16 ? kOffTc16Lo : kOffTcLo);
-  if ((rc = tc::make_map_2d(&plan->b_hi, w_hi, kG, plan->ld, plan->ld, tc::BN_MAX, f16))) return rc;
-  if ((rc = tc::make_map_2d(&plan->b_lo, w_lo, kG, plan->ld, plan->ld, tc::BN_MAX, f16))) return rc;
-  return GNNPN_OK;
+  if ((rc = tc::make_map_2d(&p.b_hi, packed + kOffTc16Hi, kG, kKp16, kKp16, tc::BN_MAX, true))) return rc;
+  return tc::make_map_2d(&p.b_lo, packed + kOffTc16Lo, kG, kKp16, kKp16, tc::BN_MAX, true);
 }
 
-int tc_lstm_zero(const TcLstmPlan& plan, int which, cudaStream_t st) {
-  // hi[which] and lo[which] are adjacent in the workspace
-  const size_t bytes = (size_t)2 * plan.n * plan.ld * (plan.f16 ? 2 : 4);
-  cudaError_t e = cudaMemsetAsync(plan.hi[which], 0, bytes, st);
-  return e == cudaSuccess ? GNNPN_OK : (int)e;
+int lstm_encoder_step(const LstmRecurrence& r, int t, float* enc_out, const LstmStepSaves* saves, cudaStream_t st) {
+  const int64_t x_inst_ld = (int64_t)r.L * r.F, h_ld = (int64_t)r.L * kH;
+  float* h_out = enc_out + (int64_t)t * kH;
+  if (r.tc) {
+    if (saves) return GNNPN_EUNSUPPORTED;
+    int rc;
+    if (t == 0) {                // h = 0 and x = raw row 0 in buffer 0; zero padding in both buffers
+      if ((rc = tc_zero(r.plan, 0, st)) || (rc = tc_zero(r.plan, 1, st))) return rc;
+      stage_x_kernel<<<(unsigned)ceil_div(r.n * r.F, 256), 256, 0, st>>>(r.inputs, x_inst_ld, 0, r.F, r.n, r.plan.hi[0],
+                                                                          r.plan.lo[0], kKp16);
+      if ((rc = after_launch())) return rc;
+    }
+    tc::LstmEpilogueParams ep{};
+    ep.bias = r.packed + kOffBias; ep.c = r.c; ep.h_out = h_out; ep.h_out_ld = h_ld;
+    ep.x_next = r.inputs; ep.x_inst_ld = x_inst_ld; ep.x_row_next = t + 1 < r.L ? t + 1 : -1; ep.F = r.F;
+    ep.first = t == 0;
+    return tc_step(r.plan, t & 1, true, ep, st);
+  }
+  LstmStepArgs a{};
+  a.h_in = t == 0 ? nullptr : h_out - kH; a.h_in_ld = h_ld;
+  a.x = r.inputs; a.x_inst_ld = x_inst_ld; a.x_row = t; a.F = r.F; a.use_x = 1;
+  a.bias = r.packed + kOffBias; a.h_out = h_out; a.h_out_ld = h_ld; a.first = t == 0;
+  return ffma_step(a, r, saves, st);
 }
 
-int tc_lstm_reset(const TcLstmPlan& plan, const float* inputs, int64_t x_inst_ld, int row0, int F,
-                  cudaStream_t st) {
-  int rc;
-  if ((rc = tc_lstm_zero(plan, 0, st))) return rc;
-  if ((rc = tc_lstm_zero(plan, 1, st))) return rc;
-  const unsigned grid = (unsigned)ceil_div(plan.n * F, 256);
-  if (plan.f16)
-    stage_x_kernel<true><<<grid, 256, 0, st>>>(inputs, x_inst_ld, row0, F, plan.n, plan.hi[0], plan.lo[0], plan.ld);
-  else
-    stage_x_kernel<false><<<grid, 256, 0, st>>>(inputs, x_inst_ld, row0, F, plan.n, plan.hi[0], plan.lo[0], plan.ld);
-  return after_launch();
+int lstm_decoder_step(const LstmRecurrence& r, int k, const float* enc_out, float* dec_h, int K, const int32_t* fed,
+                      const LstmStepSaves* saves, cudaStream_t st) {
+  // the decoder state starts from the encoder's last hidden state (modelPN.py:191,205)
+  const float* h_last = enc_out + (int64_t)(r.L - 1) * kH;
+  const float* bias = r.packed + (k == 0 ? kOffStart : kOffBias);
+  const int64_t h_ld = (int64_t)K * kH;
+  float* h_out = dec_h + (int64_t)k * kH;
+  if (r.tc) {
+    if (saves) return GNNPN_EUNSUPPORTED;
+    int rc;
+    if (k == 0) {
+      split_f16_rows_kernel<<<kNumSMs * 4, 256, 0, st>>>(h_last, (int64_t)r.L * kH, r.n, kH, kKp16, r.plan.hi[0],
+                                                         r.plan.lo[0]);
+      if ((rc = after_launch()) || (rc = tc_zero(r.plan, 1, st))) return rc;
+    }
+    tc::LstmEpilogueParams ep{};
+    ep.bias = bias; ep.c = r.c; ep.h_out = h_out; ep.h_out_ld = h_ld; ep.x_row_next = -1; ep.F = r.F;
+    return tc_step(r.plan, k & 1, k != 0, ep, st);
+  }
+  LstmStepArgs a{};
+  a.h_in = k == 0 ? h_last : h_out - kH; a.h_in_ld = k == 0 ? (int64_t)r.L * kH : h_ld;
+  a.x = r.inputs; a.x_inst_ld = (int64_t)r.L * r.F; a.x_row = -1; a.gather = k == 0 ? nullptr : fed + (int64_t)(k - 1) * r.n;
+  a.F = r.F; a.use_x = k != 0; a.bias = bias; a.h_out = h_out; a.h_out_ld = h_ld; a.first = 0;
+  return ffma_step(a, r, saves, st);
 }
 
-int tc_lstm_load_h(const TcLstmPlan& plan, int dst, const float* h, int64_t ld, cudaStream_t st) {
-  if (plan.f16)
-    split_f16_rows_kernel<<<kNumSMs * 4, 256, 0, st>>>(h, ld, plan.n, kH, kKp16, (__half*)plan.hi[dst],
-                                                       (__half*)plan.lo[dst]);
-  else
-    tc::split_tf32_kernel<<<kNumSMs * 4, 256, 0, st>>>(h, ld, plan.n, kH, kKp, (float*)plan.hi[dst],
-                                                       (float*)plan.lo[dst]);
-  return after_launch();
-}
-
-int tc_lstm_step(const TcLstmPlan& plan, const TcLstmStep& s, cudaStream_t st) {
-  using namespace tc;
-  const CUtensorMap maps[4] = {plan.a_hi[s.cur], plan.a_lo[s.cur], plan.b_hi, plan.b_lo};
-  const int bke = plan.f16 ? 64 : 32;
-  MainloopParams mp;
-  mp.M = (int)plan.n;
-  mp.n_tiles = kG / BN_MAX;
-  mp.bn = BN_MAX;
-  mp.k_blocks = kH / bke + (s.use_x ? 1 : 0);
-  mp.last_block_ksteps = s.use_x ? (s.F + (bke / 4) - 1) / (bke / 4) : 4;
-  mp.dbg = 0;
-  mp.kb_per_split = mp.k_blocks;
-  LstmEpilogueParams ep;
-  ep.bias = s.bias; ep.c = s.c; ep.h_out = s.h_out; ep.h_out_ld = s.h_out_ld;
-  ep.a_hi_next = (float*)plan.hi[s.cur ^ 1]; ep.a_lo_next = (float*)plan.lo[s.cur ^ 1]; ep.a_ld = plan.ld;
-  ep.x_next = s.x_next; ep.x_inst_ld = s.x_inst_ld; ep.x_row_next = s.x_row_next; ep.F = s.F; ep.first = s.first;
-  if (plan.f16) return launch_mainloop<LstmEpilogueT<true>, LstmEpilogueParams, true>(maps, mp, ep, st);
-  return launch_mainloop<LstmEpilogueT<false>, LstmEpilogueParams, false>(maps, mp, ep, st);
+LstmXSlot lstm_decoder_x_slot(const LstmRecurrence& r, int k) {
+  if (!r.tc) return LstmXSlot{nullptr, nullptr, 0};
+  return LstmXSlot{r.plan.hi[(k + 1) & 1], r.plan.lo[(k + 1) & 1], kKp16};
 }
 
 }  // namespace gnnpn

@@ -1,56 +1,74 @@
-// Host-side interface of the tcgen05 LSTM recurrence (implemented in tc_kernels.cu).
+// Packed LSTM block layout and the per-step LSTM recurrence driver (implemented in tc_kernels.cu).
 #pragma once
 #include <cuda.h>
 #include "lstm_step.cuh"
+#include "tc_common.cuh"
 
 namespace gnnpn {
 
-constexpr int kKp = kH + 32;     // [h | x | zero pad] columns of the tensor-core A operand (9 k-blocks of 32)
-
-// float offsets inside one packed LSTM block (see gnnpn_pn_packed_lstm_floats)
+// float offsets inside one packed LSTM block (see gnnpn_pn_packed_lstm_floats): FFMA block [kH + kXPad][kG], bias,
+// start, then the fp16-split tensor-core operand blocks [4H][kKp16] halfs (hi, lo), weights pre-scaled by kW16Scale
 constexpr size_t kOffBias = (size_t)(kH + kXPad) * kG;
 constexpr size_t kOffStart = kOffBias + kG;
-constexpr size_t kOffTcHi = kOffStart + kG;
-constexpr size_t kOffTcLo = kOffTcHi + (size_t)kG * kKp;
-// fp16-split operand blocks (default recurrence path): [4H][kKp16] halfs, weights pre-scaled by kW16Scale
 constexpr int kKp16 = kH + 64;   // [h | x | zero pad] as 5 k-blocks of 64 halfs (128-byte swizzle rows)
 constexpr float kW16Scale = 16.0f;   // |w| <~ 0.06 would push the fp16 "lo" parts into subnormals; 2^4 is exact to undo
-constexpr size_t kOffTc16Hi = kOffTcLo + (size_t)kG * kKp;
+constexpr size_t kOffTc16Hi = kOffStart + kG;
 constexpr size_t kOffTc16Lo = kOffTc16Hi + (size_t)kG * kKp16 / 2;
 constexpr size_t kPackedFloats = kOffTc16Lo + (size_t)kG * kKp16 / 2;
 
+// Where a raw input row is staged for the tensor-core step: columns [kH, kH + F) of the fp16 hi/lo [h | x] operand
+// rows, ld halfs apart.  hi == nullptr: the FFMA step, which gathers its input row itself.
+struct LstmXSlot {
+  __half* hi;
+  __half* lo;
+  int64_t ld;
+};
+__device__ __forceinline__ void stage_x_f16(__half* hi, __half* lo, int64_t ld, int64_t m, int f, float v) {
+  __half h, l;
+  tc::split_f16(v, h, l);
+  hi[m * ld + kH + f] = h;
+  lo[m * ld + kH + f] = l;
+}
+
+// the tensor-core step's two ping-pong [n, kKp16] hi/lo operand buffers and their TMA descriptors
 struct TcLstmPlan {
   CUtensorMap a_hi[2], a_lo[2], b_hi, b_lo;
-  void* hi[2];          // [n, ld] tf32-in-fp32 or fp16
-  void* lo[2];
+  __half* hi[2];
+  __half* lo[2];
   int64_t n;
-  int f16;              // 1: fp16 split (kKp16 columns), 0: tf32 split (kKp columns)
-  int ld;               // elements per row
 };
-int tc_lstm_default_f16();     // GNNPN_TC_KIND=tf32 selects the tf32 split, anything else fp16
 
+// scratch of the tensor-core recurrences (per-step operands, persistent scans' cell state, column-split exchange)
 size_t tc_lstm_workspace_bytes(int64_t n);
-// carve the workspace into the two ping-pong [n, kKp] hi/lo pairs and build the TMA descriptors
-int tc_lstm_plan(TcLstmPlan* plan, void* workspace, size_t workspace_bytes, int64_t n, const float* packed);
-// zero both ping-pong buffers and stage h = 0, x = inputs[:, row0, :] into buffer 0 (encoder start)
-int tc_lstm_reset(const TcLstmPlan& plan, const float* inputs, int64_t x_inst_ld, int row0, int F, cudaStream_t st);
-// buffer `dst` <- tf32 split of fp32 rows h[m*ld .. +kH), padding columns zeroed (decoder start)
-int tc_lstm_load_h(const TcLstmPlan& plan, int dst, const float* h, int64_t ld, cudaStream_t st);
-int tc_lstm_zero(const TcLstmPlan& plan, int which, cudaStream_t st);
 
-struct TcLstmStep {
-  int cur;                 // ping-pong buffer holding this step's [h | x]; the epilogue writes buffer cur^1
-  int use_x;               // 0: contract over h only (decoder start token is folded into the bias)
-  const float* bias;       // [kG]
-  float* c;                // [n, kH]
-  float* h_out;            // exact fp32 h', rows h_out_ld apart
-  int64_t h_out_ld;
-  const float* x_next;     // raw rows for the NEXT step (encoder) or nullptr (decoder: pointer step stages them)
-  int64_t x_inst_ld;
-  int x_row_next;
-  int F;
-  int first;
+// One LSTM recurrence run one launch per step over n instances: the tcgen05 step kernel when a workspace is given
+// (3xFP16 split of [h | x] kept in the workspace between steps), else the strict-fp32 FFMA step kernel.
+struct LstmRecurrence {
+  const float* packed;     // packed LSTM block
+  const float* inputs;     // raw rows [n, L, F]
+  int64_t n;
+  int L, F;
+  float* c;                // [n, kH] cell state, updated in place
+  bool tc;
+  TcLstmPlan plan;         // tc only
 };
-int tc_lstm_step(const TcLstmPlan& plan, const TcLstmStep& s, cudaStream_t st);
+// training replay (FFMA only): the step writes its cell state to c and its post-activation gates to gates, and reads
+// the previous cell state from c_in
+struct LstmStepSaves {
+  float* gates;            // [n, kG]
+  float* c;                // [n, kH]
+  const float* c_in;       // [n, kH]
+};
+int lstm_recurrence_init(LstmRecurrence* r, const float* packed, const float* inputs, int64_t n, int L, int F,
+                         float* c_state, void* workspace, size_t workspace_bytes);
+// encoder step t (from h = c = 0 at t = 0) on raw row t: h -> enc_out[:, t, :] ([n, L, kH])
+int lstm_encoder_step(const LstmRecurrence& r, int t, float* enc_out, const LstmStepSaves* saves, cudaStream_t st);
+// decoder step k: k = 0 starts from h = enc_out[:, L-1, :] with the start-token bias and no input; k > 0 feeds the raw
+// row fed[(k-1) * n + m] (the FFMA step gathers it, the tensor-core step reads what the pointer step staged in
+// lstm_decoder_x_slot(r, k - 1)).  h -> dec_h[:, k, :] ([n, K, kH])
+int lstm_decoder_step(const LstmRecurrence& r, int k, const float* enc_out, float* dec_h, int K, const int32_t* fed,
+                      const LstmStepSaves* saves, cudaStream_t st);
+// where the pointer step after decoder step k stages the row it feeds to step k + 1
+LstmXSlot lstm_decoder_x_slot(const LstmRecurrence& r, int k);
 
 }  // namespace gnnpn

@@ -37,6 +37,7 @@
 #include <type_traits>
 #include "tc_common.cuh"
 #include "common.cuh"
+#include "internal.cuh"
 #include "lstm_step.cuh"
 #include "tc_lstm.cuh"
 #include "tc_seq.cuh"
@@ -45,9 +46,6 @@
 #include "options.cuh"
 
 namespace gnnpn {
-namespace tc {
-int make_map_2d(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows, bool f16);
-}
 namespace seq {
 
 using namespace tc;
@@ -815,21 +813,6 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
   tc_fence_before();
   if (CG == 2) cluster_sync_all(); else __syncthreads();
   if (warp == 2) { if (CG == 2) tmem_dealloc_cg2(tmem_base, TMEM_COLS); else tmem_dealloc(tmem_base, TMEM_COLS); }
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult qr;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qr) == cudaSuccess &&
-        qr == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)ptr;
-  }
-  return fn;
 }
 
 template <bool DEC, int CG, int NR>

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define GNNPN_ABI_VERSION 7
+#define GNNPN_ABI_VERSION 8
 
 #if defined(__GNUC__)
 #define GNNPN_API __attribute__((visibility("default")))
@@ -56,10 +56,13 @@ GNNPN_API uint64_t gnnpn_launch_count(void);
 
 /* Process-wide run-time options (dispatch overrides for tests / benches / profiling; defaults need no call):
  *   "scan"         -1 auto by batch size (default) | 0 CTA-pair scan | 1 column-split cluster scan
- *   "scan_groups"   0 auto | 1 | 2 instance groups per column-split cluster
+ *   "scan_groups"   0 auto | 1 | 2 | 3 instance groups per column-split encoder cluster
  *   "persistent"    bit 0: encoder, bit 1: decoder run as one persistent launch (default 3; 0 = one launch per step)
+ *   "bptt"          1: REINFORCE backward as two persistent cluster scans (default) | 0: two launches per step
+ *   "spmm_chunk"    edges per chunk of a split aggregation row (default 0 = auto)
  *   "prof"          1: in-kernel wait-cycle counters printed to stderr (debug; makes the call synchronous)
- * Initial values are taken once, at load time, from GNNPN_COLSPLIT / GNNPN_COLSPLIT_G / GNNPN_SEQ / GNNPN_SEQ_PROF.
+ * Initial values are taken once, at load time, from GNNPN_COLSPLIT / GNNPN_COLSPLIT_G / GNNPN_SEQ / GNNPN_BPTT /
+ * GNNPN_SEQ_PROF.
  * Unknown name -> GNNPN_EUNSUPPORTED. */
 GNNPN_API int gnnpn_set_option(const char* name, int value);
 GNNPN_API int gnnpn_get_option(const char* name, int* value);
@@ -69,11 +72,13 @@ GNNPN_API int gnnpn_get_option(const char* name, int* value);
  * ------------------------------------------------------------------------- */
 
 /* Size in floats of one packed LSTM ("[h | x] -> 4H gates") weight block for hidden size H and
- * `in_features` raw input columns.  Layout (Kp = H + 32):
+ * `in_features` raw input columns: 624,640 for H = 256.  Layout (Kp = H + 64):
  *   [ (H + 32) x 4H   k-major block for the strict-fp32 FFMA step kernel ]
  *   [ 4H bias ] [ 4H start ]
- *   [ 4H x Kp  tf32 "hi" part, gate-column-major (K contiguous) for the tcgen05 step kernel ]
- *   [ 4H x Kp  tf32 "lo" part ( = w - hi ) ] */
+ *   [ 4H x Kp  fp16 "hi" part of 16 w, gate-column-major (K contiguous), for the tcgen05 kernels ]
+ *   [ 4H x Kp  fp16 "lo" part ( = fp16(16 w - hi) ) ]   (each fp16 block is 4H * Kp / 2 floats long)
+ * ABI version 8 changed this layout (version 7 also held tf32 hi/lo blocks): re-pack blocks stored by older versions,
+ * e.g. the host copies passed to gnnpn_pn_greedy_low_high_host. */
 GNNPN_API size_t gnnpn_pn_packed_lstm_floats(int hidden, int in_features);
 
 /* Fold nn.Linear(F,H) `embedding2` (modelPN.py:155,190) into an nn.LSTM's input weights
@@ -123,9 +128,10 @@ GNNPN_API int gnnpn_lstm_encode_f32(const float* inputs, int64_t n, int L, int i
                           const float* packed_encoder, float* enc_out, float* c_state,
                           void* workspace, size_t workspace_bytes, int enc_layout, void* stream);
 
-/* Scratch for the tensor-core (tcgen05, 3xTF32) recurrence: the tf32 hi/lo split of [h | x] of the
- * current and next step, 4 * n * (H + 32) floats.  Passing workspace == NULL to encode/decode selects
- * the strict-fp32 FFMA step kernel instead (same results to ~1e-6, ~5x slower). */
+/* Scratch for the tensor-core (tcgen05, 3xFP16) recurrences: at least the fp16 hi/lo split of [h | x] of the
+ * current and next step, 4 * n * (H + 64) halfs, and the persistent scans' cell-state and exchange buffers.  Passing
+ * workspace == NULL to encode/decode selects the strict-fp32 FFMA step kernel instead (same results to ~1e-6, ~5x
+ * slower). */
 GNNPN_API size_t gnnpn_pn_workspace_bytes(int64_t n, int hidden);
 
 /* Fused greedy pointer decode: K x { decoder LSTM cell -> pointer logits on window k ->
@@ -135,7 +141,8 @@ GNNPN_API size_t gnnpn_pn_workspace_bytes(int64_t n, int hidden);
  *   c_state      fp32 [n, H]        in: encoder final cell state; out: decoder final cell state
  *   latent_win   fp32 [n, L] or NULL   PNLow's step-(l/N) logit at position l (only the window
  *                                   slice of latent[k] can influence a pick, SURVEY 3.4)
- *   att_params   NULL for Dot; for Bahdanau a packed block, see gnnpn_pn_pack_bahdanau_f32
+ *   att_params   unused: Dot attention only (Bahdanau runs through gnnpn_pn_decode_general_f32 with a block of
+ *                                   gnnpn_pn_att_block_floats() floats, as ops.att_block lays it out)
  *   dec_h        fp32 [n, K, H]     out: decoder hidden state (= attention query) of every step; may be NULL with
  *                                   enc_layout = GNNPN_ENC_BLOCKED128 (the fused decoder does not need it in memory)
  *   idx_out      int32 [K, n]       out: selected position in [k*N, (k+1)*N)

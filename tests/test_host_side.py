@@ -22,7 +22,7 @@ def test_library_exports_every_declared_symbol():
         version = int(re.search(r"#define GNNPN_ABI_VERSION (\d+)", f.read()).group(1))
     assert L.gnnpn_abi_version() == version
     assert L.gnnpn_error_string(-2) == b"unsupported shape"
-    assert L.gnnpn_pn_packed_lstm_floats(256, 8) == (256 + 32 + 2) * 1024 + 2 * 1024 * 288 + 1024 * 320   # FFMA block, tf32 hi/lo, fp16 hi/lo (halfs)
+    assert L.gnnpn_pn_packed_lstm_floats(256, 8) == (256 + 32 + 2) * 1024 + 1024 * 320   # FFMA block, bias, start, fp16 hi/lo (halfs)
     # argument errors are detected before any CUDA call, so they are testable on a CPU box
     assert L.gnnpn_lstm_encode_f32(None, 1, 1, 8, 256, None, None, None, None, 0, 0, None) == -1
 

@@ -22,18 +22,17 @@ CUDA_CASES = ["qws_b4", "normal_b2", "small_b16", "sharp_b4", "notanh_b3", "bahd
 
 # "tc": tcgen05 recurrence as dispatched by default -- at these batch sizes the column-split cluster scan
 # (tc_colsplit.cu); "tc_pair": the same with option scan=0, i.e. the CTA-pair persistent scan (tc_seq.cu: blocked
-# encodings, pointer dots fused into the decoder's cell epilogue) that large batches use; "ffma": the strict-fp32 kernels.
-IMPLS = ["tc", "tc_pair", "ffma"]
+# encodings, pointer dots fused into the decoder's cell epilogue) that large batches use; "tc_step": option
+# persistent=0, the one-launch-per-step tcgen05 recurrence (tc_kernels.cu); "ffma": the strict-fp32 kernels.
+IMPLS = ["tc", "tc_pair", "tc_step", "ffma"]
 
 
 def _select(impl):
-    """Set the scan-kernel option for `impl` (gnnpn_set_option) and return the module-level impl."""
+    """Set the scan-kernel options for `impl` (gnnpn_set_option) and return the module-level impl."""
     from gnnpn_sc_b200 import ops
-    if impl == "tc_pair":
-        ops.set_option("scan", 0)
-        return "tc"
-    ops.set_option("scan", -1)
-    return impl
+    ops.set_option("scan", 0 if impl == "tc_pair" else -1)
+    ops.set_option("persistent", 0 if impl == "tc_step" else 3)
+    return "tc" if impl in ("tc_pair", "tc_step") else impl
 
 
 @pytest.fixture(autouse=True)
@@ -42,6 +41,7 @@ def _reset_scan_knob():
     from gnnpn_sc_b200 import ops
     ops.set_option("scan", -1)
     ops.set_option("scan_groups", 0)
+    ops.set_option("persistent", 3)
 
 
 
@@ -61,7 +61,7 @@ def _models(name, device="cuda", impl=None):
     return cfg, x, out[0], out[1]
 
 
-STRESS_FLOOR = {"ffma": 2.0, "tc": 4.0, "tc_pair": 4.0, None: 4.0}   # multiples of the reference's own fp32 noise, stress cases only
+STRESS_FLOOR = {"ffma": 2.0, "tc": 4.0, "tc_pair": 4.0, "tc_step": 4.0, None: 4.0}   # multiples of the reference's own fp32 noise, stress cases only
 
 
 def _close(a, b, tol=LOGIT_TOL, floor=0.0):
@@ -288,11 +288,11 @@ def test_host_batch_pipeline_matches_direct_calls():
         assert torch.equal(r_host, R.cpu())
 
 
-@pytest.mark.parametrize("impl", ["ffma"])
+@pytest.mark.parametrize("impl", ["ffma", "tc_step"])
 def test_general_kernels_equal_fused_path_bitwise(impl):
     """Dot / no glimpse / N <= 32 through the general (one-CTA-per-instance) kernels == the fused path, bit for bit
     (same LSTM kernel on both sides: with impl="tc" the fused path runs the persistent scan, whose cell epilogue rounds
-    differently from the per-step tcgen05 kernel the general path uses)."""
+    differently from the per-step tcgen05 kernel the general path uses; "tc_step" runs that per-step kernel on both)."""
     from gnnpn_sc_b200.synth import pn_instances
     cfg, _, low, high = _models("qws_b4", impl=impl)
     x = pn_instances(200, cfg.s_category, cfg.s_number, seed=31).cuda()
