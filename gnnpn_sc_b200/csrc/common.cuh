@@ -16,8 +16,15 @@ inline int after_launch() {
 }
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+inline bool aligned32(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 31u) == 0; }
 inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 inline int round_up(int a, int b) { return (a + b - 1) / b * b; }
+// A workspace is used from its first 1024-byte boundary (TMA and swizzled operand alignment); the *_workspace_bytes
+// sizes include that slack.
+template <class T = uint8_t>
+inline T* align_ws(void* workspace) {
+  return reinterpret_cast<T*>((reinterpret_cast<uintptr_t>(workspace) + 1023) & ~uintptr_t(1023));
+}
 
 constexpr int kNumSMs = 148;  // B200: 2 dies x 74 SMs
 

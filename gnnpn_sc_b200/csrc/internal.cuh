@@ -39,9 +39,10 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 EncodeTiledFn encode_fn();
-// row-major [rows, cols] fp32 (or fp16) with leading dimension ld (elements); box = {128 bytes of columns, box_rows};
-// 128B swizzle
-int make_map_2d(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows, bool f16 = false);
+// row-major [rows, cols] fp32 (or fp16) with leading dimension ld (elements); box = {box_cols (default: 128 bytes of
+// columns), box_rows}; 128B swizzle, or 32B for 32-byte box rows
+int make_map_2d(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows, bool f16 = false,
+                int box_cols = 0);
 }  // namespace tc
 
 }  // namespace gnnpn

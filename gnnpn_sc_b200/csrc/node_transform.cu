@@ -344,7 +344,7 @@ int launch_node_transform(const float* A, int64_t lda, const float* W, int64_t l
   using namespace nt;
   if ((lda & 3) || (reinterpret_cast<uintptr_t>(A) & 15u)) return GNNPN_EALIGN;
   const int Kp = round_up(K, KB);
-  __half* w_hi = reinterpret_cast<__half*>((reinterpret_cast<uintptr_t>(workspace) + 1023) & ~uintptr_t(1023));
+  __half* w_hi = align_ws<__half>(workspace);
   __half* w_lo = w_hi + (size_t)N * Kp;
   float2* st_tab = reinterpret_cast<float2*>(w_lo + (size_t)N * Kp);            // 16-byte aligned: N * Kp * 2 is a multiple of 2 KB
   int* status = reinterpret_cast<int*>(st_tab + MAX_N);

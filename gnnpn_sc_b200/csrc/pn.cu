@@ -6,7 +6,6 @@
 #include "tc_lstm.cuh"
 #include "tc_seq.cuh"
 #include "pointer.cuh"
-#include "options.cuh"
 
 namespace gnnpn {
 namespace {
@@ -90,12 +89,19 @@ __global__ void __launch_bounds__(256) pointer_step_dot_kernel(
     stage_x_f16(x_next.hi, x_next.lo, x_next.ld, b, lane, __ldg(inputs + (b * pa.L + fed) * (int64_t)F + lane));
 }
 
-// argument block of the pointer steps over row-major encodings [n, L, kH]
-PointerStepArgs pointer_step_args(const float* enc_out, const float* latent_win, float alpha, int use_tanh, float C,
-                                  int64_t n, int L, int N, int32_t* idx_out, float* win_logits, float* win_probs,
-                                  const int32_t* forced, const float* uniform) {
-  return PointerStepArgs{enc_out, (int64_t)L * kH, latent_win, alpha, use_tanh, C, n, L, N, idx_out, win_logits,
-                         win_probs, forced, uniform};
+// The K steps of a per-step decode: before_step(k) (the decoder's LSTM step, or nothing), then the pointer step on the
+// query dec_h[:, k].  With a tensor-core recurrence r the pointer step stages the fed row as r's next input.
+template <class BeforeStep>
+int launch_pointer_steps(const PointerStepArgs& pa, int K, const float* dec_h, const float* inputs, int F,
+                         const LstmRecurrence* r, cudaStream_t st, BeforeStep before_step) {
+  for (int k = 0; k < K; ++k) {
+    int rc = before_step(k);
+    if (rc) return rc;
+    pointer_step_dot_kernel<<<(unsigned)ceil_div(pa.n, 8), 256, 0, st>>>(
+        pa, k, dec_h + (int64_t)k * kH, (int64_t)K * kH, inputs, F, r ? lstm_decoder_x_slot(*r, k) : LstmXSlot{nullptr, nullptr, 0});
+    if ((rc = after_launch())) return rc;
+  }
+  return GNNPN_OK;
 }
 
 // ---------------------------------------------------------------------------
@@ -204,10 +210,6 @@ __global__ void reward_kernel(const float* __restrict__ inputs, const int32_t* _
   }
 }
 
-// option "persistent": bit 0 = persistent encoder scan, bit 1 = persistent fused decode (default 3); 0 selects the
-// one-launch-per-step kernels (kept for inputs wider than 8 columns and as the A/B reference)
-int seq_mode() { return options().persistent.load(std::memory_order_relaxed); }
-
 // raw input range check: *flag |= 1 if any value is NaN / inf or has |x| >= limit
 __global__ void check_inputs_kernel(const float* __restrict__ x, int64_t count, float limit, int32_t* __restrict__ flag) {
   bool bad = false;
@@ -270,10 +272,7 @@ int gnnpn_pn_check_inputs_f32(const float* inputs, int64_t count, int32_t* flag,
 
 int gnnpn_pn_enc_layout(int64_t n, int L, int in_features, int K, int N, int has_workspace) {
   (void)L; (void)K;
-  if (!has_workspace || seq_mode() != 3 || in_features < 1 || in_features > 8) return GNNPN_ENC_ROWMAJOR;
-  if (!tc_seq_fused_decode_supported(N)) return GNNPN_ENC_ROWMAJOR;
-  if (tc_colsplit_wanted(n) || tc_colsplit_wanted_encode(n)) return GNNPN_ENC_ROWMAJOR;   // small batch: cluster scan
-  return GNNPN_ENC_BLOCKED128;
+  return plan_scans(n, in_features, N, GNNPN_ENC_ROWMAJOR, has_workspace != 0).layout;
 }
 
 size_t gnnpn_pn_enc_out_floats(int64_t n, int L, int hidden, int layout) {
@@ -301,22 +300,20 @@ int gnnpn_lstm_encode_f32(const float* inputs, int64_t n, int L, int in_features
   GNNPN_REQUIRE(aligned16(enc_out) && aligned16(c_state) && aligned16(packed), GNNPN_EALIGN);
   if (n == 0) return GNNPN_OK;
   cudaStream_t st = (cudaStream_t)stream;
-  if (workspace && (seq_mode() & 1) && in_features <= 8) {
-    // ---- persistent tcgen05 scan: one launch for all L steps, h resident in shared memory
-    GNNPN_REQUIRE((reinterpret_cast<uintptr_t>(enc_out) & 31u) == 0 && (reinterpret_cast<uintptr_t>(c_state) & 31u) == 0,
-                  GNNPN_EALIGN);
-    GNNPN_REQUIRE(workspace_bytes >= tc_lstm_workspace_bytes(n), GNNPN_EWORKSPACE);
-    float* scr = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(workspace) + 1023) & ~uintptr_t(1023));
-    SeqEncodeArgs sa{inputs, n, L, in_features, packed, enc_out, c_state, scr, enc_layout};
-    if (enc_layout == GNNPN_ENC_BLOCKED128) return tc_seq_encode(sa, st);         // the CTA-pair scan owns this layout
-    if (tc_colsplit_wanted_encode(n)) return tc_colsplit_encode(sa, scr, st);     // small batch: column-split cluster scan
-    return tc_seq_encode(sa, st);
+  const ScanChoice scan = plan_scans(n, in_features, /*N: no window*/ 0, enc_layout, workspace != nullptr).enc;
+  if (scan.kind == ScanKind::kStep) {
+    GNNPN_REQUIRE(enc_layout == GNNPN_ENC_ROWMAJOR, GNNPN_EUNSUPPORTED);
+    LstmRecurrence r;
+    int rc = lstm_recurrence_init(&r, packed, inputs, n, L, in_features, c_state, workspace, workspace_bytes);
+    for (int t = 0; t < L && !rc; ++t) rc = lstm_encoder_step(r, t, enc_out, nullptr, st);
+    return rc;
   }
-  GNNPN_REQUIRE(enc_layout == GNNPN_ENC_ROWMAJOR, GNNPN_EUNSUPPORTED);
-  LstmRecurrence r;
-  int rc = lstm_recurrence_init(&r, packed, inputs, n, L, in_features, c_state, workspace, workspace_bytes);
-  for (int t = 0; t < L && !rc; ++t) rc = lstm_encoder_step(r, t, enc_out, nullptr, st);
-  return rc;
+  // ---- persistent tcgen05 scan: one launch for all L steps
+  GNNPN_REQUIRE(aligned32(enc_out) && aligned32(c_state), GNNPN_EALIGN);
+  GNNPN_REQUIRE(workspace_bytes >= tc_lstm_workspace_bytes(n), GNNPN_EWORKSPACE);
+  SeqEncodeArgs sa{inputs, n, L, in_features, packed, enc_out, c_state, align_ws<float>(workspace)};
+  if (scan.kind == ScanKind::kColsplit) return tc_colsplit_encode(sa, scan.variant, st);
+  return tc_seq_encode(sa, scan.variant, st);
 }
 
 int gnnpn_pn_decode_greedy_f32(const float* inputs, const float* enc_out, float* c_state,
@@ -337,31 +334,24 @@ int gnnpn_pn_decode_greedy_f32(const float* inputs, const float* enc_out, float*
   GNNPN_REQUIRE(aligned16(enc_out) && aligned16(dec_h) && aligned16(c_state) && aligned16(packed), GNNPN_EALIGN);   // NULL dec_h passes
   if (n == 0) return GNNPN_OK;
   cudaStream_t st = (cudaStream_t)stream;
-  if (workspace && (seq_mode() & 2) && in_features <= 8) {
-    GNNPN_REQUIRE((reinterpret_cast<uintptr_t>(enc_out) & 31u) == 0 && (reinterpret_cast<uintptr_t>(c_state) & 31u) == 0 &&
-                      (reinterpret_cast<uintptr_t>(dec_h) & 31u) == 0, GNNPN_EALIGN);
-    SeqDecodeArgs sa{inputs, enc_out, c_state, latent_win, alpha, packed, use_tanh, C, n, L, in_features, K, N,
-                     dec_h, idx_out, win_logits, win_probs, forced_idx, sample_uniform,
-                     reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(workspace) + 1023) & ~uintptr_t(1023)),
-                     enc_layout};
-    GNNPN_REQUIRE(workspace_bytes >= tc_lstm_workspace_bytes(n), GNNPN_EWORKSPACE);
-    if (enc_layout == GNNPN_ENC_BLOCKED128) return tc_seq_decode(sa, st);          // fused pointer dots (CTA-pair scan)
-    if (tc_colsplit_wanted(n)) return tc_colsplit_decode(sa, sa.c_scratch, st);    // small batch: column-split cluster scan
-    return tc_seq_decode(sa, st);
+  const ScanChoice scan = plan_scans(n, in_features, N, enc_layout, workspace != nullptr).dec;
+  if (scan.kind == ScanKind::kStep) {
+    GNNPN_REQUIRE(enc_layout == GNNPN_ENC_ROWMAJOR, GNNPN_EUNSUPPORTED);
+    LstmRecurrence r;
+    const int rc = lstm_recurrence_init(&r, packed, inputs, n, L, in_features, c_state, workspace, workspace_bytes);
+    if (rc) return rc;
+    const PointerStepArgs pa = pointer_step_args(enc_out, latent_win, alpha, use_tanh, C, n, L, N, idx_out, win_logits,
+                                                 win_probs, forced_idx, sample_uniform);
+    return launch_pointer_steps(pa, K, dec_h, inputs, in_features, &r, st, [&](int k) {
+      return lstm_decoder_step(r, k, enc_out, dec_h, K, forced_idx ? forced_idx : idx_out, nullptr, st);
+    });
   }
-  GNNPN_REQUIRE(enc_layout == GNNPN_ENC_ROWMAJOR, GNNPN_EUNSUPPORTED);
-  LstmRecurrence r;
-  int rc = lstm_recurrence_init(&r, packed, inputs, n, L, in_features, c_state, workspace, workspace_bytes);
-  if (rc) return rc;
-  const PointerStepArgs pa = pointer_step_args(enc_out, latent_win, alpha, use_tanh, C, n, L, N, idx_out, win_logits,
-                                               win_probs, forced_idx, sample_uniform);
-  for (int k = 0; k < K; ++k) {
-    if ((rc = lstm_decoder_step(r, k, enc_out, dec_h, K, forced_idx ? forced_idx : idx_out, nullptr, st))) return rc;
-    pointer_step_dot_kernel<<<(unsigned)ceil_div(n, 8), 256, 0, st>>>(pa, k, dec_h + (int64_t)k * kH, (int64_t)K * kH,
-                                                                     inputs, in_features, lstm_decoder_x_slot(r, k));
-    if ((rc = after_launch())) return rc;
-  }
-  return GNNPN_OK;
+  GNNPN_REQUIRE(aligned32(enc_out) && aligned32(c_state) && aligned32(dec_h), GNNPN_EALIGN);
+  GNNPN_REQUIRE(workspace_bytes >= tc_lstm_workspace_bytes(n), GNNPN_EWORKSPACE);
+  SeqDecodeArgs sa{inputs, enc_out, c_state, latent_win, alpha, packed, use_tanh, C, n, L, in_features, K, N,
+                   dec_h, idx_out, win_logits, win_probs, forced_idx, sample_uniform, align_ws<float>(workspace)};
+  if (scan.kind == ScanKind::kColsplit) return tc_colsplit_decode(sa, scan.variant, st);
+  return scan.kind == ScanKind::kPair ? tc_seq_decode(sa, scan.variant, st) : GNNPN_EUNSUPPORTED;
 }
 
 // Differentiable replay, forward half (see pn_train.cu): strict-fp32 FFMA LSTM steps + pointer steps, teacher-forced on
@@ -388,14 +378,10 @@ int gnnpn_pn_train_forward_f32(const float* inputs, const float* packed_enc, con
   if (rc || (rc = lstm_recurrence_init(&r, packed_dec, inputs, n, L, in_features, nullptr, nullptr, 0))) return rc;
   const PointerStepArgs pa = pointer_step_args(enc_out, latent_win, alpha, use_tanh, C, n, L, N, idx_free, win_logits,
                                                win_probs, idx, nullptr);
-  for (int k = 0; k < K; ++k) {
+  return launch_pointer_steps(pa, K, dec_h, inputs, in_features, &r, st, [&](int k) {
     const LstmStepSaves sv{gates_d + k * n * kG, c_d + k * nh, k == 0 ? c_e + (L - 1) * nh : c_d + (k - 1) * nh};
-    if ((rc = lstm_decoder_step(r, k, enc_out, dec_h, K, idx, &sv, st))) return rc;
-    pointer_step_dot_kernel<<<(unsigned)ceil_div(n, 8), 256, 0, st>>>(pa, k, dec_h + (int64_t)k * kH, (int64_t)K * kH,
-                                                                     inputs, in_features, lstm_decoder_x_slot(r, k));
-    if ((rc = after_launch())) return rc;
-  }
-  return GNNPN_OK;
+    return lstm_decoder_step(r, k, enc_out, dec_h, K, idx, &sv, st);
+  });
 }
 
 // The attention of the decode loop alone (modelPN.py:213-228 restricted to the windows): for given decoder states
@@ -411,13 +397,7 @@ int gnnpn_pn_attention_windows_f32(const float* enc_out, const float* dec_h, con
   if (n == 0) return GNNPN_OK;
   const PointerStepArgs pa = pointer_step_args(enc_out, latent_win, alpha, use_tanh, C, n, L, N, idx_out, win_logits,
                                                win_probs, nullptr, nullptr);
-  for (int k = 0; k < K; ++k) {
-    pointer_step_dot_kernel<<<(unsigned)ceil_div(n, 8), 256, 0, (cudaStream_t)stream>>>(
-        pa, k, dec_h + (int64_t)k * kH, (int64_t)K * kH, nullptr, 0, LstmXSlot{nullptr, nullptr, 0});
-    const int rc = after_launch();
-    if (rc) return rc;
-  }
-  return GNNPN_OK;
+  return launch_pointer_steps(pa, K, dec_h, nullptr, 0, nullptr, (cudaStream_t)stream, [](int) { return GNNPN_OK; });
 }
 
 int gnnpn_pn_train_forward_tc_f32(const float* inputs, const float* packed_enc, const float* packed_dec,
@@ -433,24 +413,26 @@ int gnnpn_pn_train_forward_tc_f32(const float* inputs, const float* packed_enc, 
   GNNPN_REQUIRE(aligned16(enc_out) && aligned16(dec_h) && aligned16(gates_e) && aligned16(gates_d) && aligned16(c_e) &&
                     aligned16(c_d), GNNPN_EALIGN);
   GNNPN_REQUIRE(workspace_bytes >= tc_lstm_workspace_bytes(n), GNNPN_EWORKSPACE);
-  // the column-split cluster scan only (training batches: the reference's is 128); larger batches use the FFMA replay
-  GNNPN_REQUIRE(tc_colsplit_wanted(n) && tc_colsplit_wanted_encode(n), GNNPN_EUNSUPPORTED);
+  // the saves exist in the column-split scan only, whatever the "persistent" option says; larger batches use the FFMA
+  // replay (training batches: the reference's is 128)
+  const ScanPlan plan = plan_scans(n, in_features, N, GNNPN_ENC_ROWMAJOR, true, 3);
+  GNNPN_REQUIRE(plan.enc.kind == ScanKind::kColsplit, GNNPN_EUNSUPPORTED);
   if (n == 0) return GNNPN_OK;
   cudaStream_t st = (cudaStream_t)stream;
-  float* scr = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(workspace) + 1023) & ~uintptr_t(1023));
+  float* scr = align_ws<float>(workspace);
   const size_t nh = (size_t)n * kH;
   float* c_last_e = c_e + (size_t)(L - 1) * nh;          // the encoder's final cell state = its last save
   float* c_last_d = c_d + (size_t)(K - 1) * nh;          // decoder: in (copy of c_last_e) / out (= its last save)
-  SeqEncodeArgs ea{inputs, n, L, in_features, packed_enc, enc_out, c_last_e, scr, GNNPN_ENC_ROWMAJOR};
+  SeqEncodeArgs ea{inputs, n, L, in_features, packed_enc, enc_out, c_last_e, scr};
   ea.save_gates = gates_e; ea.save_c = c_e;
-  int rc = tc_colsplit_encode(ea, scr, st);
+  int rc = tc_colsplit_encode(ea, plan.enc.variant, st);
   if (rc) return rc;
   cudaError_t ce = cudaMemcpyAsync(c_last_d, c_last_e, nh * sizeof(float), cudaMemcpyDeviceToDevice, st);
   if (ce != cudaSuccess) return (int)ce;
   SeqDecodeArgs da{inputs, enc_out, c_last_d, latent_win, alpha, packed_dec, use_tanh, C, n, L, in_features, K, N, dec_h,
-                   idx_out, win_logits, win_probs, forced_idx, sample_uniform, scr, GNNPN_ENC_ROWMAJOR};
+                   idx_out, win_logits, win_probs, forced_idx, sample_uniform, scr};
   da.save_gates = gates_d; da.save_c = c_d;
-  return tc_colsplit_decode(da, scr, st);
+  return tc_colsplit_decode(da, plan.dec.variant, st);
 }
 
 int gnnpn_pn_full_logits_f32(const float* enc_out, const float* dec_h, const int32_t* idx,

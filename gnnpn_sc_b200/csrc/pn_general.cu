@@ -312,7 +312,7 @@ int gnnpn_pn_decode_general_f32(const float* inputs, const float* enc_out, float
   cudaStream_t st = (cudaStream_t)stream;
   const GeneralWs wsl = general_ws(n, L, K, attention, n_glimpses, use_tc);
   GNNPN_REQUIRE(workspace_bytes >= wsl.total, GNNPN_EWORKSPACE);
-  uint8_t* ws = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(workspace) + 1023) & ~uintptr_t(1023));
+  uint8_t* ws = align_ws(workspace);
   float* e_p = reinterpret_cast<float*>(ws + wsl.e_p);
   float* e_g = reinterpret_cast<float*>(ws + wsl.e_g);
   float* qw = reinterpret_cast<float*>(ws + wsl.qw);

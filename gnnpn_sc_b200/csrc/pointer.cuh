@@ -33,6 +33,14 @@ struct PointerStepArgs {
 };
 // The decode step k is passed separately so that the argument block itself can stay in constant memory.
 
+// argument block of the pointer steps over row-major encodings [n, L, kH]
+inline PointerStepArgs pointer_step_args(const float* enc_out, const float* latent_win, float alpha, int use_tanh, float C,
+                                         int64_t n, int L, int N, int32_t* idx_out, float* win_logits, float* win_probs,
+                                         const int32_t* forced, const float* uniform) {
+  return PointerStepArgs{enc_out, (int64_t)L * kH, latent_win, alpha, use_tanh, C, n, L, N, idx_out, win_logits,
+                         win_probs, forced, uniform};
+}
+
 // ---- canonical pointer-logit dot product ------------------------------------------------------------------
 // Every kernel that forms a Dot pointer logit <row, q> rounds in THIS order, so window logits == the same entries of
 // the dense logits == the fused decoders' values, bit for bit, whichever kernel a batch is dispatched to:

@@ -16,7 +16,6 @@
 // Reference semantics: nn.LSTM cell, gate order i,f,g,o (modelPN.py:157,191); same packed weights, same cell
 // epilogue (lstm_cell8) as tc_seq.cu.
 #include <stdio.h>
-#include <stdlib.h>
 #include <cuda_fp16.h>
 #include "tc_common.cuh"
 #include "common.cuh"
@@ -25,7 +24,6 @@
 #include "tc_lstm.cuh"
 #include "tc_seq.cuh"
 #include "tc_seq_dev.cuh"
-#include "options.cuh"
 #include "pointer.cuh"
 
 namespace gnnpn {
@@ -502,145 +500,64 @@ size_t tc_colsplit_scratch_bytes(int64_t n) {
 }
 
 // how many 8-CTA clusters of this kernel the device can hold at once (GPC packing decides; measured, not assumed)
-static int max_active_clusters() {
+int tc_colsplit_max_active_clusters() {
   static const int v = [] {
     using namespace cs;
-    auto kern = lstm_colsplit_kernel<false, 1>;
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Layout<1>::SMEM_BYTES) != cudaSuccess) return 0;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(CL * 64); cfg.blockDim = dim3(THREADS); cfg.dynamicSmemBytes = Layout<1>::SMEM_BYTES;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
+    constexpr auto kern = lstm_colsplit_kernel<false, 1>;
+    cudaLaunchConfig_t cfg;
+    cudaLaunchAttribute attr;
+    if (cluster_config<kern>(&cfg, &attr, CL * 64, CL, THREADS, Layout<1>::SMEM_BYTES, nullptr)) return 0;
     int nc = 0;
     if (cudaOccupancyMaxActiveClusters(&nc, kern, &cfg) != cudaSuccess) { cudaGetLastError(); return 0; }
     return nc;
   }();
   return v;
 }
-int tc_colsplit_max_active_clusters() { return max_active_clusters(); }
-
-// GNNPN_COLSPLIT: -1 (default) = automatic, 0 = never, 1 = always; GNNPN_COLSPLIT_G = 1 / 2 / 3 forces the groups per cluster of
-// the encoder (default: 2 as soon as one-group clusters would need a second wave; 3 is chosen by pipeline.low_high for
-// 16..21 groups so that PNLow's and PNHigh's encoders -- 7 clusters each -- run side by side on the 15 cluster slots).  Automatic (measured on a B200 with 15
-// co-resident clusters, profiles/r01_colsplit_timing.jsonl, r01_pn_batch_sweep.jsonl): a step of the column-split scan
-// costs ~6.6 us per wave (~7 us with two groups per cluster) against ~16.7 us (encoder) / ~37 us (fused decoder) for
-// the CTA-pair scan at any batch up to 18,944.  Encoder: one-group clusters up to 15 groups of 128, two-group clusters up to
-// 30 groups (one wave; two waves of them are slower than the pair scan); decoder: one-group clusters up to two waves.
-static int colsplit_mode() { return options().scan.load(std::memory_order_relaxed); }   // gnnpn_set_option("scan", ..)
-bool tc_colsplit_wanted(int64_t n) {                     // fused decoder
-  const int mode = colsplit_mode();
-  if (mode == 0) return false;
-  if (mode == 1) return true;
-  return ceil_div(n, cs::BM) <= 2 * (int64_t)max_active_clusters();
-}
-bool tc_colsplit_wanted_encode(int64_t n) {
-  const int mode = colsplit_mode();
-  if (mode == 0) return false;
-  if (mode == 1) return true;
-  return ceil_div(n, cs::BM) <= 2 * (int64_t)max_active_clusters();
-}
-static int colsplit_groups_per_cluster(int64_t n) {
-  const int g = options().scan_groups.load(std::memory_order_relaxed);
-  if (g >= 1 && g <= 3) return g;
-  return ceil_div(n, cs::BM) > (int64_t)max_active_clusters() ? 2 : 1;
-}
 
 namespace cs {
 
 template <bool DEC, int G>
-static int launch(const float* packed, Params p, void* scratch, cudaStream_t st) {
-  EncodeTiledFn fn = encode_fn();
-  if (!fn) return GNNPN_EUNSUPPORTED;
+static int launch(const float* packed, Params p, cudaStream_t st) {
   const int64_t clusters = ceil_div(ceil_div(p.n, BM), G);
   CUtensorMap maps[5];
-  const float* w_hi = packed + kOffTc16Hi;
-  const float* w_lo = packed + kOffTc16Lo;
-  for (int i = 0; i < 4; ++i) {
-    cuuint64_t dims[2] = {(cuuint64_t)kKp16, (cuuint64_t)kG};
-    cuuint64_t strides[1] = {(cuuint64_t)kKp16 * 2};
-    cuuint32_t box[2] = {i < 2 ? 64u : 16u, (cuuint32_t)TILE_N};
-    cuuint32_t estr[2] = {1, 1};
-    if (fn(&maps[i], CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, (void*)((i & 1) ? w_lo : w_hi), dims, strides, box, estr,
-           CU_TENSOR_MAP_INTERLEAVE_NONE, i < 2 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_32B,
-           CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-      return GNNPN_ESHAPE;
-  }
-  {
-    // exchange scratch as one 2-D fp16 tensor {kH, groups * 2 parities * (hi|lo) * 128 rows}; box = one k-block
-    cuuint64_t dims[2] = {(cuuint64_t)kH, (cuuint64_t)(clusters * G * 4 * BM)};
-    cuuint64_t strides[1] = {(cuuint64_t)kH * 2};
-    cuuint32_t box[2] = {64u, (cuuint32_t)BM};
-    cuuint32_t estr[2] = {1, 1};
-    if (fn(&maps[4], CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, scratch, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-           CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-      return GNNPN_ESHAPE;
-  }
-  p.scratch = reinterpret_cast<__half*>(scratch);
-  auto kern = lstm_colsplit_kernel<DEC, G>;
-  constexpr int SMEM = Layout<G>::SMEM_BYTES;
-  static bool configured = false;
-  if (!configured) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM);
-    if (e != cudaSuccess) return (int)e;
-    configured = true;
-  }
-  const int do_prof = options().prof.load(std::memory_order_relaxed);
+  int rc = make_weight_maps(maps, packed, TILE_N);
+  // exchange scratch as one 2-D fp16 tensor [groups * 2 parities * (hi|lo) * 128 rows, kH]; box = one k-block
+  if (rc || (rc = make_map_2d(&maps[4], p.scratch, clusters * G * 4 * BM, kH, kH, BM, true))) return rc;
   const unsigned grid = (unsigned)(clusters * CL);
-  unsigned long long* prof = nullptr;
-  if (do_prof) {
-    if (cudaMalloc(&prof, (size_t)grid * 8 * 8) != cudaSuccess) return GNNPN_EUNSUPPORTED;
-    cudaMemsetAsync(prof, 0, (size_t)grid * 8 * 8, st);
-  }
-  p.prof = prof;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(THREADS); cfg.dynamicSmemBytes = SMEM; cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  cudaError_t le = cudaLaunchKernelEx(&cfg, kern, maps[0], maps[1], maps[2], maps[3], maps[4], p);
-  if (le != cudaSuccess) { cudaGetLastError(); return (int)le; }
-  const int rc = after_launch();
-  if (do_prof) {
-    unsigned long long* h = (unsigned long long*)malloc((size_t)grid * 8 * 8);
-    cudaStreamSynchronize(st);
-    cudaMemcpy(h, prof, (size_t)grid * 8 * 8, cudaMemcpyDeviceToHost);
-    double acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    for (unsigned c = 0; c < grid; ++c)
-      for (int i = 0; i < 8; ++i) acc[i] += (double)h[c * 8 + i];
+  if ((rc = prof_alloc(grid, 8, st, &p.prof))) return rc;
+  rc = launch_cluster<lstm_colsplit_kernel<DEC, G>>(grid, CL, THREADS, Layout<G>::SMEM_BYTES, st, maps[0], maps[1], maps[2],
+                                                    maps[3], maps[4], p);
+  if (p.prof) {
+    double acc[8];
+    prof_collect(p.prof, grid, 8, st, acc);
     const double d = (double)grid * p.steps;
     fprintf(stderr, "[colsplit prof %s G=%d steps=%d grid=%u max_active_clusters=%d] per-step cycles: mma total %.0f (wait A full %.0f) | "
             "tma wait a_rdy %.0f | epi (group 0) wait tmem_full %.0f, tmem ld + cell %.0f, publish %.0f, %s %.0f\n", DEC ? "dec" : "enc", G,
-            p.steps, grid, max_active_clusters(), acc[1] / d, acc[2] / d, acc[0] / d, acc[3] / d, acc[5] / d, acc[6] / d,
+            p.steps, grid, tc_colsplit_max_active_clusters(), acc[1] / d, acc[2] / d, acc[0] / d, acc[3] / d, acc[5] / d, acc[6] / d,
             DEC ? "pointer phase" : "h store", acc[7] / d);
-    free(h);
-    cudaFree(prof);
   }
   return rc;
 }
 
 }  // namespace cs
 
-int tc_colsplit_encode(const SeqEncodeArgs& a, void* scratch, cudaStream_t st) {
-  if (a.F < 1 || a.F > 8 || a.L < 1) return GNNPN_EUNSUPPORTED;
+int tc_colsplit_encode(const SeqEncodeArgs& a, int groups, cudaStream_t st) {
   cs::Params p{};
   p.n = a.n; p.steps = a.L; p.F = a.F; p.L = a.L;
   p.inputs = a.inputs; p.x_inst_ld = (int64_t)a.L * a.F;
   p.bias0 = p.bias = a.packed + kOffBias;
   p.c = a.c_state;
   p.h_out = a.enc_out; p.h_out_inst_ld = (int64_t)a.L * kH;
+  p.scratch = reinterpret_cast<__half*>(a.c_scratch);
   p.save_gates = a.save_gates; p.save_c = a.save_c;
-  switch (colsplit_groups_per_cluster(a.n)) {
-    case 3: return cs::launch<false, 3>(a.packed, p, scratch, st);
-    case 2: return cs::launch<false, 2>(a.packed, p, scratch, st);
-    default: return cs::launch<false, 1>(a.packed, p, scratch, st);
+  switch (groups) {
+    case 3: return cs::launch<false, 3>(a.packed, p, st);
+    case 2: return cs::launch<false, 2>(a.packed, p, st);
+    default: return cs::launch<false, 1>(a.packed, p, st);
   }
 }
 
-int tc_colsplit_decode(const SeqDecodeArgs& a, void* scratch, cudaStream_t st) {
-  if (a.F < 1 || a.F > 8 || a.K < 1 || a.N < 1 || a.N > kMaxWindow) return GNNPN_EUNSUPPORTED;
+int tc_colsplit_decode(const SeqDecodeArgs& a, int groups, cudaStream_t st) {
   cs::Params p{};
   p.n = a.n; p.steps = a.K; p.F = a.F; p.L = a.L;
   p.inputs = a.inputs; p.x_inst_ld = (int64_t)a.L * a.F;
@@ -648,14 +565,11 @@ int tc_colsplit_decode(const SeqDecodeArgs& a, void* scratch, cudaStream_t st) {
   p.c = a.c_state;
   p.h0 = a.enc_out + (int64_t)(a.L - 1) * kH; p.h0_ld = (int64_t)a.L * kH;
   p.h_out = a.dec_h; p.h_out_inst_ld = (int64_t)a.K * kH;
-  p.pa.enc_out = a.enc_out; p.pa.enc_inst_ld = (int64_t)a.L * kH; p.pa.latent_win = a.latent_win;
-  p.pa.alpha = a.alpha; p.pa.use_tanh = a.use_tanh; p.pa.C = a.C; p.pa.n = a.n; p.pa.L = a.L;
-  p.pa.N = a.N; p.pa.idx_out = a.idx_out; p.pa.win_logits = a.win_logits; p.pa.win_probs = a.win_probs;
-  p.pa.forced = a.forced_idx; p.pa.uniform = a.sample_uniform;
+  p.scratch = reinterpret_cast<__half*>(a.c_scratch);
+  p.pa = pointer_step_args(a.enc_out, a.latent_win, a.alpha, a.use_tanh, a.C, a.n, a.L, a.N, a.idx_out, a.win_logits,
+                           a.win_probs, a.forced_idx, a.sample_uniform);
   p.save_gates = a.save_gates; p.save_c = a.save_c;
-  // two groups per cluster as soon as one-group clusters would need a second wave (16..30 groups): one wave of 8..15 clusters
-  return colsplit_groups_per_cluster(a.n) >= 2 ? cs::launch<true, 2>(a.packed, p, scratch, st)
-                                                : cs::launch<true, 1>(a.packed, p, scratch, st);
+  return groups == 2 ? cs::launch<true, 2>(a.packed, p, st) : cs::launch<true, 1>(a.packed, p, st);
 }
 
 }  // namespace gnnpn

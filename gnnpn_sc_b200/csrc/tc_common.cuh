@@ -40,6 +40,18 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
       "}" ::"r"(bar), "r"(parity) : "memory");
 }
 
+// ----------------------------------------------------------------- 256-bit global accesses
+// sm_100: one full 32-byte sector per thread per instruction
+__device__ __forceinline__ void ldg256(const float* p, float* v) {
+  asm volatile("ld.global.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+               : "=f"(v[0]), "=f"(v[1]), "=f"(v[2]), "=f"(v[3]), "=f"(v[4]), "=f"(v[5]), "=f"(v[6]), "=f"(v[7])
+               : "l"(p));
+}
+__device__ __forceinline__ void stg256(float* p, const float* v) {
+  asm volatile("st.global.v8.f32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(p), "f"(v[0]), "f"(v[1]), "f"(v[2]),
+               "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7]) : "memory");
+}
+
 // ----------------------------------------------------------------- TMA
 __device__ __forceinline__ void tma_load_2d(uint32_t smem_dst, const CUtensorMap* map, uint32_t bar, int c0,
                                             int c1) {

@@ -255,17 +255,6 @@ struct GemmEpilogue {
   }
 };
 
-// 256-bit global accesses (sm_100): one full 32-byte sector per thread per instruction
-__device__ __forceinline__ void ldg256(const float* p, float* v) {
-  asm volatile("ld.global.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=f"(v[0]), "=f"(v[1]), "=f"(v[2]), "=f"(v[3]), "=f"(v[4]), "=f"(v[5]), "=f"(v[6]), "=f"(v[7])
-               : "l"(p));
-}
-__device__ __forceinline__ void stg256(float* p, const float* v) {
-  asm volatile("st.global.v8.f32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(p), "f"(v[0]), "f"(v[1]), "f"(v[2]),
-               "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7]) : "memory");
-}
-
 struct LstmEpilogue {
   const LstmEpilogueParams& p; int64_t row; bool ok;
   const float* sbias;            // the 1024 gate biases, staged once per CTA
@@ -350,18 +339,20 @@ EncodeTiledFn encode_fn() {
   return fn;
 }
 
-int make_map_2d(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows, bool f16) {
+int make_map_2d(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows, bool f16,
+                int box_cols) {
   EncodeTiledFn fn = encode_fn();
   if (!fn) return GNNPN_EUNSUPPORTED;
   const int esz = f16 ? 2 : 4;
+  if (!box_cols) box_cols = 128 / esz;
   cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
   cuuint64_t strides[1] = {(cuuint64_t)ld * esz};
-  cuuint32_t box[2] = {(cuuint32_t)(128 / esz), (cuuint32_t)box_rows};
+  cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
   cuuint32_t estr[2] = {1, 1};
   CUresult r = fn(m, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)base, dims,
-                  strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                  strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                  box_cols * esz == 32 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_128B,
+                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return r == CUDA_SUCCESS ? GNNPN_OK : GNNPN_ESHAPE;
 }
 
@@ -540,7 +531,7 @@ int lstm_recurrence_init(LstmRecurrence* r, const float* packed, const float* in
   if (workspace_bytes < tc_lstm_workspace_bytes(n)) return GNNPN_EWORKSPACE;
   // two ping-pong [n, kKp16] hi/lo pairs
   TcLstmPlan& p = r->plan;
-  __half* ws = reinterpret_cast<__half*>((reinterpret_cast<uintptr_t>(workspace) + 1023) & ~uintptr_t(1023));
+  __half* ws = align_ws<__half>(workspace);
   const size_t one = (size_t)n * kKp16;       // halfs, a multiple of 64 bytes
   p.n = n;
   p.hi[0] = ws; p.lo[0] = ws + one; p.hi[1] = ws + 2 * one; p.lo[1] = ws + 3 * one;

@@ -33,6 +33,7 @@
 // Cross-CTA mbarrier arrives use .release.cta semantics on purpose (see mbar_arrive_cluster).
 #include <stdio.h>
 #include <stdlib.h>
+#include <algorithm>
 #include <cuda_fp16.h>
 #include <type_traits>
 #include "tc_common.cuh"
@@ -816,24 +817,10 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
 }
 
 template <bool DEC, int CG, int NR>
-int launch_seq_cg(const float* packed, const SeqParams& p, cudaStream_t st) {
-  EncodeTiledFn fn = encode_fn();
-  if (!fn) return GNNPN_EUNSUPPORTED;
+int launch_seq_cg(const float* packed, SeqParams p, cudaStream_t st) {
   CUtensorMap maps[4];
-  const float* w_hi = packed + kOffTc16Hi;
-  const float* w_lo = packed + kOffTc16Lo;
-  const cuuint32_t box_rows = TILE_N / CG;
-  for (int i = 0; i < 4; ++i) {
-    // i<2: h part, 64 halfs (128 bytes) per gate column, 128B swizzle; i>=2: x part, 16 halfs, 32B swizzle
-    cuuint64_t dims[2] = {(cuuint64_t)kKp16, (cuuint64_t)kG};
-    cuuint64_t strides[1] = {(cuuint64_t)kKp16 * 2};
-    cuuint32_t box[2] = {i < 2 ? 64u : 16u, box_rows};
-    cuuint32_t estr[2] = {1, 1};
-    if (fn(&maps[i], CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, (void*)((i & 1) ? w_lo : w_hi), dims, strides, box, estr,
-           CU_TENSOR_MAP_INTERLEAVE_NONE, i < 2 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_32B,
-           CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-      return GNNPN_ESHAPE;
-  }
+  int rc = make_weight_maps(maps, packed, TILE_N / CG);
+  if (rc) return rc;
   CUtensorMap map_h = maps[0];                         // only the row-major encoder stores through it
   if (!DEC && NR == 0) {
     // h_out as a 3-D tensor {unit, step, instance}; box = 32 units x 1 step x 128 instances, 128B swizzle
@@ -842,62 +829,31 @@ int launch_seq_cg(const float* packed, const SeqParams& p, cudaStream_t st) {
     cuuint64_t strides[2] = {(cuuint64_t)kH * 4, (cuuint64_t)p.h_out_inst_ld * 4};
     cuuint32_t box[3] = {32, 1, (cuuint32_t)BM};
     cuuint32_t estr[3] = {1, 1, 1};
-    if (fn(&map_h, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, (void*)p.h_out, dims, strides, box, estr,
-           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+    if (encode_fn()(&map_h, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, (void*)p.h_out, dims, strides, box, estr,
+                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
       return GNNPN_ESHAPE;
   }
-  SeqParams pp = p;
-  auto kern = lstm_seq_kernel<DEC, CG, NR>;
-  static bool configured = false;
-  if (!configured) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e != cudaSuccess) return (int)e;
-    configured = true;
-  }
   const unsigned grid = (unsigned)(ceil_div(p.n, BM * CG) * CG);
-  const int do_prof = options().prof.load(std::memory_order_relaxed);
-  unsigned long long* prof = nullptr;
-  if (do_prof) {                                       // debug only: synchronous, allocates
-    if (cudaMalloc(&prof, (size_t)grid * 16 * 8) != cudaSuccess) return GNNPN_EUNSUPPORTED;
-    cudaMemsetAsync(prof, 0, (size_t)grid * 16 * 8, st);
-  }
-  pp.prof = prof;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(THREADS); cfg.dynamicSmemBytes = SMEM_BYTES; cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CG; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  cudaError_t le = cudaLaunchKernelEx(&cfg, kern, maps[0], maps[1], maps[2], maps[3], map_h, pp);
-  if (le != cudaSuccess) { cudaGetLastError(); return (int)le; }
-  const int rc_launch = after_launch();
-  if (do_prof) {
-    unsigned long long* hbuf = (unsigned long long*)malloc((size_t)grid * 16 * 8);
-    cudaStreamSynchronize(st);
-    cudaMemcpy(hbuf, prof, (size_t)grid * 16 * 8, cudaMemcpyDeviceToHost);
-    double acc[8] = {0};
-    unsigned leaders = 0;
-    for (unsigned c = 0; c < grid; ++c) {
-      if (hbuf[c * 16]) ++leaders;
-      for (int i = 0; i < 8; ++i) acc[i] += (double)hbuf[c * 16 + i];
-    }
+  if ((rc = prof_alloc(grid, 16, st, &p.prof))) return rc;
+  rc = launch_cluster<lstm_seq_kernel<DEC, CG, NR>>(grid, CG, THREADS, SMEM_BYTES, st, maps[0], maps[1], maps[2], maps[3],
+                                                    map_h, p);
+  if (p.prof) {
+    double acc[8];
+    unsigned leaders = prof_collect(p.prof, grid, 16, st, acc);     // the MMA-issuing CTAs write counter 0
     if (!leaders) leaders = 1;
     fprintf(stderr, "[seq prof %s cg=%d nr=%d steps=%d grid=%u] per-step cycles: mma total %.0f (wait a_ready %.0f, tmem_empty %.0f, "
             "B full %.0f) | epi total %.0f (wait tmem_full %.0f, h buf %.0f, pointer %.0f)\n", DEC ? "dec" : "enc", CG, NR,
             p.steps, grid, acc[0] / leaders / p.steps, acc[1] / leaders / p.steps, acc[2] / leaders / p.steps,
             acc[3] / leaders / p.steps, acc[4] / grid / p.steps, acc[5] / grid / p.steps, acc[6] / grid / p.steps,
             acc[7] / grid / p.steps);
-    free(hbuf);
-    cudaFree(prof);
   }
-  return rc_launch;
+  return rc;
 }
 
 }  // namespace seq
 
-int tc_seq_encode(const SeqEncodeArgs& a, cudaStream_t st) {
-  if (a.F < 1 || a.F > 8 || a.L < 1) return GNNPN_EUNSUPPORTED;
+int tc_seq_encode(const SeqEncodeArgs& a, int nr, cudaStream_t st) {
   seq::SeqParams p{};
   p.n = a.n; p.steps = a.L; p.L = a.L; p.F = a.F;
   p.inputs = a.inputs; p.x_inst_ld = (int64_t)a.L * a.F;
@@ -906,37 +862,114 @@ int tc_seq_encode(const SeqEncodeArgs& a, cudaStream_t st) {
   p.h0 = nullptr; p.h0_ld = 0;
   p.h_out = a.enc_out; p.h_out_inst_ld = (int64_t)a.L * kH;
   p.c_scr = a.c_scratch;
-  p.enc_layout = a.enc_layout;
-  if (a.enc_layout == GNNPN_ENC_BLOCKED128) return seq::launch_seq_cg<false, 2, 1>(a.packed, p, st);
-  return seq::launch_seq_cg<false, 2, 0>(a.packed, p, st);
+  p.enc_layout = nr ? GNNPN_ENC_BLOCKED128 : GNNPN_ENC_ROWMAJOR;
+  return nr ? seq::launch_seq_cg<false, 2, 1>(a.packed, p, st) : seq::launch_seq_cg<false, 2, 0>(a.packed, p, st);
 }
 
-bool tc_seq_fused_decode_supported(int N) { return N >= 1 && N <= 10; }
-
-int tc_seq_decode(const SeqDecodeArgs& a, cudaStream_t st) {
-  if (a.F < 1 || a.F > 8 || a.K < 1 || a.N < 1 || a.N > kMaxWindow) return GNNPN_EUNSUPPORTED;
+int tc_seq_decode(const SeqDecodeArgs& a, int nr, cudaStream_t st) {
   seq::SeqParams p{};
   p.n = a.n; p.steps = a.K; p.L = a.L; p.F = a.F;
   p.inputs = a.inputs; p.x_inst_ld = (int64_t)a.L * a.F;
   p.bias0 = a.packed + kOffStart; p.bias = a.packed + kOffBias;
   p.c = a.c_state; p.c_zero_init = 0;
   p.h_out = a.dec_h; p.h_out_inst_ld = (int64_t)a.K * kH;
-  p.pa.enc_out = a.enc_out; p.pa.enc_inst_ld = (int64_t)a.L * kH; p.pa.latent_win = a.latent_win;
-  p.pa.alpha = a.alpha; p.pa.use_tanh = a.use_tanh; p.pa.C = a.C; p.pa.n = a.n; p.pa.L = a.L;
-  p.pa.N = a.N; p.pa.idx_out = a.idx_out; p.pa.win_logits = a.win_logits; p.pa.win_probs = a.win_probs;
-  p.pa.forced = a.forced_idx; p.pa.uniform = a.sample_uniform;
+  p.pa = pointer_step_args(a.enc_out, a.latent_win, a.alpha, a.use_tanh, a.C, a.n, a.L, a.N, a.idx_out, a.win_logits,
+                           a.win_probs, a.forced_idx, a.sample_uniform);
   p.c_scr = a.c_scratch;
-  p.enc_layout = a.enc_layout;
-  if (a.enc_layout == GNNPN_ENC_BLOCKED128) {
-    // blocked encodings: the pointer dots ride in the cell epilogue (row capacity 5 / 8 / 10 of the window)
-    if (!tc_seq_fused_decode_supported(a.N)) return GNNPN_EUNSUPPORTED;
-    p.h0 = nullptr; p.h0_ld = 0;                         // read from the block's position L-1 inside the kernel
-    if (a.N == 5) return seq::launch_seq_cg<true, 2, 5>(a.packed, p, st);
-    if (a.N <= 8) return seq::launch_seq_cg<true, 2, 8>(a.packed, p, st);
-    return seq::launch_seq_cg<true, 2, 10>(a.packed, p, st);
+  p.enc_layout = nr ? GNNPN_ENC_BLOCKED128 : GNNPN_ENC_ROWMAJOR;
+  // blocked encodings (nr > 0): the pointer dots ride in the cell epilogue, and h0 is read from the block's position
+  // L-1 inside the kernel
+  if (nr == 0) { p.h0 = a.enc_out + (int64_t)(a.L - 1) * kH; p.h0_ld = (int64_t)a.L * kH; }
+  switch (nr) {
+    case 5: return seq::launch_seq_cg<true, 2, 5>(a.packed, p, st);
+    case 8: return seq::launch_seq_cg<true, 2, 8>(a.packed, p, st);
+    case 10: return seq::launch_seq_cg<true, 2, 10>(a.packed, p, st);
+    default: return seq::launch_seq_cg<true, 2, 0>(a.packed, p, st);
   }
-  p.h0 = a.enc_out + (int64_t)(a.L - 1) * kH; p.h0_ld = (int64_t)a.L * kH;
-  return seq::launch_seq_cg<true, 2, 0>(a.packed, p, st);
+}
+
+// ================================================================================================================
+// Host side shared by both scans (this file and tc_colsplit.cu): which kernel runs a batch, and their launch code.
+namespace {
+
+// Column-split groups of 128 instances per encoder cluster for a batch of n, or 0 when the CTA-pair scan runs it.
+// Option "scan": -1 automatic, 0 CTA-pair, 1 column-split.  Automatic (measured on a B200 with 15 co-resident clusters,
+// profiles/r01_colsplit_timing.jsonl, r01_pn_batch_sweep.jsonl): a column-split step costs ~6.6 us per wave (~7 us with
+// two groups per cluster) against ~16.7 us (encoder) / ~37 us (fused decoder) for the CTA-pair scan at any batch up to
+// 18,944.  So the column-split scan takes up to two waves of groups: one-group clusters up to one wave, two-group
+// clusters up to 30 groups (one wave; two waves of them are slower than the pair scan).  Option "scan_groups": 0
+// automatic, 1 / 2 / 3 forced; pipeline.low_high picks 3 for 15..21 groups so that PNLow's and PNHigh's encoders --
+// 7 clusters each -- run side by side on the 15 cluster slots.  The decoder runs two groups per cluster whenever the
+// encoder runs two or three (one wave of 8..15 clusters for 16..30 groups).
+int colsplit_groups(int64_t n) {
+  const int scan = options().scan.load(std::memory_order_relaxed);
+  if (scan == 0) return 0;
+  const int64_t groups = ceil_div(n, 128);
+  if (scan != 1 && groups > 2 * (int64_t)tc_colsplit_max_active_clusters()) return 0;
+  const int g = options().scan_groups.load(std::memory_order_relaxed);
+  if (g >= 1 && g <= 3) return g;
+  return groups > tc_colsplit_max_active_clusters() ? 2 : 1;
+}
+
+}  // namespace
+
+// Option "persistent": bit 0 runs the encoder, bit 1 the decoder as one persistent launch (default 3); without its bit
+// a recurrence runs one launch per step (kept for inputs wider than 8 columns, runs without a workspace and as the
+// A/B reference).  The blocked encodings layout exists for the CTA-pair scan's fused decoder, so it is asked for only
+// when both scans are persistent, the batch is not the column-split scan's, and the window fits the fused decoder's
+// row capacity (N <= 10).  Encodings that are already blocked go to the CTA-pair scan before the column-split test.
+ScanPlan plan_scans(int64_t n, int F, int N, int layout, bool has_workspace, int persistent) {
+  ScanPlan p{{ScanKind::kStep, 0}, {ScanKind::kStep, 0}, GNNPN_ENC_ROWMAJOR};
+  if (!has_workspace || F < 1 || F > 8) return p;
+  if (persistent < 0) persistent = options().persistent.load(std::memory_order_relaxed);
+  const bool blocked = layout == GNNPN_ENC_BLOCKED128;
+  const int g = colsplit_groups(n);
+  if (persistent == 3 && N >= 1 && N <= 10 && g == 0) p.layout = GNNPN_ENC_BLOCKED128;
+  if (persistent & 1) {
+    if (blocked) p.enc = {ScanKind::kPair, 1};
+    else if (g) p.enc = {ScanKind::kColsplit, g};
+    else p.enc = {ScanKind::kPair, 0};
+  }
+  if (persistent & 2) {
+    if (blocked && N > 10) p.dec = {ScanKind::kUnsupported, 0};
+    else if (blocked) p.dec = {ScanKind::kPair, N == 5 ? 5 : (N <= 8 ? 8 : 10)};
+    else if (g) p.dec = {ScanKind::kColsplit, std::min(g, 2)};
+    else p.dec = {ScanKind::kPair, 0};
+  }
+  return p;
+}
+
+int make_weight_maps(CUtensorMap maps[4], const float* packed, int box_rows) {
+  int rc = GNNPN_OK;
+  for (int i = 0; i < 4 && !rc; ++i)           // i < 2: h part, 64 halfs per gate column; i >= 2: x part, 16 halfs
+    rc = tc::make_map_2d(&maps[i], packed + ((i & 1) ? kOffTc16Lo : kOffTc16Hi), kG, kKp16, kKp16, box_rows, true,
+                         i < 2 ? 64 : 16);
+  return rc;
+}
+
+int prof_alloc(unsigned ctas, int per_cta, cudaStream_t st, unsigned long long** counters) {
+  *counters = nullptr;
+  if (!options().prof.load(std::memory_order_relaxed)) return GNNPN_OK;
+  const size_t bytes = (size_t)ctas * per_cta * sizeof(unsigned long long);
+  if (cudaMalloc(counters, bytes) != cudaSuccess) return GNNPN_EUNSUPPORTED;
+  cudaMemsetAsync(*counters, 0, bytes, st);
+  return GNNPN_OK;
+}
+
+unsigned prof_collect(unsigned long long* counters, unsigned ctas, int per_cta, cudaStream_t st, double sums[8]) {
+  const size_t bytes = (size_t)ctas * per_cta * sizeof(unsigned long long);
+  unsigned long long* h = (unsigned long long*)malloc(bytes);
+  cudaStreamSynchronize(st);
+  cudaMemcpy(h, counters, bytes, cudaMemcpyDeviceToHost);
+  cudaFree(counters);
+  unsigned wrote = 0;
+  for (int i = 0; i < 8; ++i) sums[i] = 0;
+  for (unsigned c = 0; c < ctas; ++c) {
+    if (h[(size_t)c * per_cta]) ++wrote;
+    for (int i = 0; i < 8; ++i) sums[i] += (double)h[(size_t)c * per_cta + i];
+  }
+  free(h);
+  return wrote;
 }
 
 }  // namespace gnnpn

@@ -1,4 +1,5 @@
-// Host-side interface of the persistent tcgen05 LSTM sequence kernels (implemented in tc_seq.cu).
+// Host-side interface of the persistent tcgen05 LSTM sequence kernels: the CTA-pair scan (tc_seq.cu), the column-split
+// cluster scan (tc_colsplit.cu) and which of them runs a batch (tc_seq.cu).
 //
 // One launch runs a whole LSTM scan (encoder: L steps; decoder: K steps with the pointer step fused
 // between them).  A CTA owns 128 composition instances for the whole scan; the recurrence is CTA-local
@@ -10,6 +11,65 @@
 
 namespace gnnpn {
 
+// ---- which kernel runs a recurrence (tc_seq.cu) -------------------------------------------------------------------
+enum class ScanKind {
+  kStep,          // one launch per step (lstm_recurrence_*)
+  kPair,          // CTA-pair scan lstm_seq_kernel<DEC, 2, NR>
+  kColsplit,      // column-split cluster scan lstm_colsplit_kernel<DEC, G>
+  kUnsupported,   // blocked encodings with a window the fused decoder cannot hold (N > 10)
+};
+struct ScanChoice {
+  ScanKind kind;
+  int variant;    // kPair: NR (encoder 0 row-major / 1 blocked; decoder 0 / 5 / 8 / 10); kColsplit: G (1 / 2 / 3)
+};
+struct ScanPlan {
+  ScanChoice enc, dec;
+  int layout;     // the encodings layout gnnpn_pn_enc_layout reports for the batch
+};
+// Encoder and decoder choice for n instances with F input columns and windows of N candidates, whose encodings are in
+// `layout`, under the current "scan" and "scan_groups" options and the "persistent" bits (-1: the option).  A step
+// choice with blocked encodings is GNNPN_EUNSUPPORTED for the caller.
+ScanPlan plan_scans(int64_t n, int F, int N, int layout, bool has_workspace, int persistent = -1);
+
+// ---- host launch code shared by the two scans (tc_seq.cu) ---------------------------------------------------------
+// The packed block's fp16 hi/lo weights as TMA maps, boxes of `box_rows` gate columns: {h hi, h lo} (64 halfs,
+// 128B swizzle) and {x hi, x lo} (16 halfs, 32B swizzle)
+int make_weight_maps(CUtensorMap maps[4], const float* packed, int box_rows);
+// "prof" option: `ctas * per_cta` zeroed device counters that the kernel adds clock64() cycles to, or nullptr when
+// the option is off
+int prof_alloc(unsigned ctas, int per_cta, cudaStream_t st, unsigned long long** counters);
+// waits for the stream, copies the counters back and frees them (debug only); sums[i] = counter i (< 8) summed over the
+// CTAs.  Returns how many CTAs wrote counter 0.
+unsigned prof_collect(unsigned long long* counters, unsigned ctas, int per_cta, cudaStream_t st, double sums[8]);
+
+// Launch configuration of `Kern` for a 1-D grid of 1-D clusters of `cluster` CTAs, setting the kernel's dynamic
+// shared-memory limit on first use.  `attr` receives the cluster-dimension attribute `cfg` points at.
+template <auto Kern>
+int cluster_config(cudaLaunchConfig_t* cfg, cudaLaunchAttribute* attr, unsigned grid, unsigned cluster, int threads,
+                   int smem, cudaStream_t st) {
+  static bool configured = false;
+  if (!configured) {
+    cudaError_t e = cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (e != cudaSuccess) return (int)e;
+    configured = true;
+  }
+  attr->id = cudaLaunchAttributeClusterDimension;
+  attr->val.clusterDim = {cluster, 1, 1};
+  *cfg = cudaLaunchConfig_t{dim3(grid), dim3(threads), (size_t)smem, st, attr, 1};
+  return GNNPN_OK;
+}
+template <auto Kern, class... Args>
+int launch_cluster(unsigned grid, unsigned cluster, int threads, int smem, cudaStream_t st, const Args&... args) {
+  cudaLaunchConfig_t cfg;
+  cudaLaunchAttribute attr;
+  const int rc = cluster_config<Kern>(&cfg, &attr, grid, cluster, threads, smem, st);
+  if (rc) return rc;
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, Kern, args...);
+  if (e != cudaSuccess) { cudaGetLastError(); return (int)e; }
+  return after_launch();
+}
+
+// ---- the scans -----------------------------------------------------------------------------------------------------
 // cell-state scratch of the persistent kernels: 128 x kH floats per CTA (blocked layout), CTAs launched in pairs
 inline size_t tc_seq_scratch_floats(int64_t n) { return (size_t)((n + 255) / 256) * 256 * kH; }
 
@@ -19,30 +79,28 @@ struct SeqEncodeArgs {
   int L;
   int F;                   // <= 8
   const float* packed;     // packed LSTM block (uses the bias and the fp16 hi/lo operand blocks)
-  float* enc_out;          // [n, L, kH], or the blocked layout (gnnpn_pn_enc_out_floats) when enc_layout says so
+  float* enc_out;          // [n, L, kH], or the blocked layout (gnnpn_pn_enc_out_floats) for tc_seq_encode's nr = 1
   float* c_state;          // [n, kH] out
-  float* c_scratch;        // tc_seq_scratch_floats(n) floats
-  int enc_layout;          // GNNPN_ENC_ROWMAJOR / GNNPN_ENC_BLOCKED128 (CTA-pair scan only)
+  float* c_scratch;        // the 1024-byte aligned workspace: cell-state scratch of the CTA-pair scan
+                           // (tc_seq_scratch_floats(n) floats), h' exchange of the column-split scan (tc_colsplit_scratch_bytes(n))
   // training (column-split scan only): per-step saves for the BPTT, or nullptr
   float* save_gates;       // [L, n, 4H] post-activation gates, columns 4j + {i,f,g,o}
   float* save_c;           // [L, n, H] cell state after every step
 };
-// returns GNNPN_EUNSUPPORTED when the shape is outside what the persistent kernel covers
-int tc_seq_encode(const SeqEncodeArgs& a, cudaStream_t st);
+// nr: 0 row-major, 1 blocked encodings
+int tc_seq_encode(const SeqEncodeArgs& a, int nr, cudaStream_t st);
 
-// Small-batch (latency) variant, tc_colsplit.cu: a cluster of 8 CTAs shares 128 instances and splits the gate
-// columns; `scratch` = tc_colsplit_scratch_bytes(n) bytes (1024-byte aligned) for the h' exchange.
-bool tc_colsplit_wanted(int64_t n);          // fused decoder
-bool tc_colsplit_wanted_encode(int64_t n);
+// Small-batch (latency) variant, tc_colsplit.cu: a cluster of 8 CTAs shares G groups of 128 instances and splits the
+// gate columns.
 int tc_colsplit_max_active_clusters();
 size_t tc_colsplit_scratch_bytes(int64_t n);
-int tc_colsplit_encode(const SeqEncodeArgs& a, void* scratch, cudaStream_t st);
+int tc_colsplit_encode(const SeqEncodeArgs& a, int groups, cudaStream_t st);
 struct SeqDecodeArgs;
-int tc_colsplit_decode(const SeqDecodeArgs& a, void* scratch, cudaStream_t st);
+int tc_colsplit_decode(const SeqDecodeArgs& a, int groups, cudaStream_t st);
 
 struct SeqDecodeArgs {
   const float* inputs;     // [n, L, F]
-  const float* enc_out;    // [n, L, kH]
+  const float* enc_out;    // [n, L, kH], or blocked for tc_seq_decode's nr > 0
   float* c_state;          // [n, kH] in/out
   const float* latent_win; // [n, L] or nullptr
   float alpha;
@@ -57,12 +115,11 @@ struct SeqDecodeArgs {
   float* win_probs;        // [n, L]
   const int32_t* forced_idx;     // [K, n] or nullptr
   const float* sample_uniform;   // [K, n] or nullptr
-  float* c_scratch;              // tc_seq_scratch_floats(n) floats
-  int enc_layout;                // layout of enc_out
+  float* c_scratch;              // as SeqEncodeArgs::c_scratch
   float* save_gates;             // training (column-split scan only): [K, n, 4H] post-activation gates, or nullptr
   float* save_c;                 // [K, n, H] cell state after every step, or nullptr
 };
-bool tc_seq_fused_decode_supported(int N);     // blocked-layout decoder (pointer dots fused into the cell epilogue)
-int tc_seq_decode(const SeqDecodeArgs& a, cudaStream_t st);
+// nr: 0 row-major encodings; 5 / 8 / 10 blocked encodings, window row capacity of the fused decoder (N <= nr)
+int tc_seq_decode(const SeqDecodeArgs& a, int nr, cudaStream_t st);
 
 }  // namespace gnnpn

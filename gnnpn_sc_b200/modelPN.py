@@ -263,6 +263,13 @@ class PointerNet(nn.Module):
         return (not self.force_general and self.embedding_size == 0 and self.n_glimpses == 0
                 and self.pointer.name == "Dot" and self.serNumber <= 32 and F <= 8 and not self._anyh())
 
+    def enc_layout(self, n: int, F: int) -> int:
+        """Layout of the encodings ``encode`` writes for n rows of F kernel input columns (``ops.pn_enc_layout``)."""
+        if not self._fast_path(F):
+            return ops.ENC_ROWMAJOR
+        has_ws = (self.impl or ops.DEFAULT_IMPL) == "tc"      # ops.pn_workspace: the tensor-core kernels' scratch
+        return ops.pn_enc_layout(n, self.seq_len, F, self.serCategory, self.serNumber, has_ws)
+
     def encode(self, inputs):
         """The encoder half of ``forward`` (modelPN.py:183-191: embedding + encoder LSTM), enqueued on the CURRENT stream.
         Returns an opaque handle for ``forward(..., encoded=handle)``.  The two networks of the ML+2PN decode read the
@@ -289,9 +296,7 @@ class PointerNet(nn.Module):
         enc_w, _ = self._packed_weights()
         with torch.no_grad():
             ws = ops.pn_workspace(B, self.hidden_size, x.device, self.impl)
-            # batches the CTA-pair scan takes keep their encodings in the blocked layout (pointer dots fused into the
-            # decoder's cell epilogue); ``self.last["enc_out"]`` / the dense logits convert lazily
-            layout = ops.pn_enc_layout(B, L, x.shape[2], K, N, ws is not None) if fast else ops.ENC_ROWMAJOR
+            layout = self.enc_layout(B, x.shape[2])
             buf = None
             if self.enc_buffer is not None:
                 # a caller-owned buffer (e.g. shared by PNLow and PNHigh at the scale-up size, where one network's
@@ -308,17 +313,16 @@ class PointerNet(nn.Module):
     def _train_forward(self, inputs, lat, uniform, use_tanh, C):
         """Free-running decode (greedy, or sampled with ``uniform``) on ``gnnpn_pn_train_forward_tc_f32``: the picks plus
         every per-step save of the BPTT.  Returns (saves, encode-handle) or (None, None) when the batch does not fit the
-        column-split cluster scan."""
+        column-split cluster scan; any other failure raises."""
         x = self._kernel_inputs(inputs)
         range_flag = ops.pn_check_inputs(x) if self.check_inputs else None
         enc_w, dec_w = self._packed_weights()
         K, N = self.serCategory, self.serNumber
         with torch.no_grad():
-            try:
-                sv = ops.pn_train_forward(x, enc_w, dec_w, None, K, N, latent_win=lat, alpha=float(self.alpha),
-                                          use_tanh=use_tanh, C=C, hidden=self.hidden_size, impl="tc", sample_uniform=uniform)
-            except ops.GnnpnError:
-                return None, None
+            sv = ops.pn_train_forward(x, enc_w, dec_w, None, K, N, latent_win=lat, alpha=float(self.alpha),
+                                      use_tanh=use_tanh, C=C, hidden=self.hidden_size, impl="tc", sample_uniform=uniform)
+        if sv is None:
+            return None, None
         return sv, {"x": x, "ws": None, "layout": ops.ENC_ROWMAJOR, "enc_out": sv["enc_out"], "c": None,
                     "range_flag": range_flag, "fast": True, "stream": torch.cuda.current_stream(x.device)}
 

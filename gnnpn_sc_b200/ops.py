@@ -226,7 +226,7 @@ def pn_train_forward(inputs, packed_enc, packed_dec, idx, K: int, N: int, latent
     ``impl="tc"`` (default when the batch fits the column-split cluster scan): ``gnnpn_pn_train_forward_tc_f32`` -- the
     tensor-core kernels of the small-batch inference path with saves enabled; with ``idx=None`` and ``sample_uniform``
     it IS the sampled decode (no replay needed).  ``impl="ffma"`` / larger batches: ``gnnpn_pn_train_forward_f32``
-    (strict-fp32 per-step kernels, teacher-forced on ``idx``)."""
+    (strict-fp32 per-step kernels, teacher-forced on ``idx``); with ``idx=None`` they return None: decode first."""
     x = _f32(inputs, "inputs")
     n, L, F = x.shape
     dev, H = x.device, hidden
@@ -252,7 +252,7 @@ def pn_train_forward(inputs, packed_enc, packed_dec, idx, K: int, N: int, latent
         if rc != EUNSUPPORTED:
             check(rc, "pn_train_forward_tc")
     if idx is None:
-        raise GnnpnError("pn_train_forward: this batch is outside the column-split scan; decode first and pass idx")
+        return None
     check(lib().gnnpn_pn_train_forward_f32(
         x.data_ptr(), packed_enc.data_ptr(), packed_dec.data_ptr(), sv["idx"].data_ptr(), _ptr(lat), float(alpha),
         int(bool(use_tanh)), float(C), n, L, F, H, K, N, sv["enc_out"].data_ptr(), sv["gates_e"].data_ptr(),

@@ -97,11 +97,9 @@ def _own_enc_buffer(actor, n: int, L: int, F: int, device):
     at n = 18,944 that would otherwise go through the caching allocator -- per stream, with deferred frees for buffers
     that crossed streams -- on every call).  A caller-set larger buffer is left alone."""
     from . import ops
-    K, N, H = actor.serCategory, actor.serNumber, actor.hidden_size
     if actor.embedding_size != 0 or actor.impl == "ffma" or actor._anyh():
         return
-    layout = ops.pn_enc_layout(n, L, F, K, N, True) if actor._fast_path(F) else ops.ENC_ROWMAJOR
-    need = ops.enc_out_floats(n, L, H, layout)
+    need = ops.enc_out_floats(n, L, actor.hidden_size, actor.enc_layout(n, F))
     if actor.enc_buffer is None or actor.enc_buffer.numel() < need:
         actor.enc_buffer = None                           # release the old block before asking for the larger one
         actor.enc_buffer = torch.empty(need, device=device, dtype=torch.float32)
