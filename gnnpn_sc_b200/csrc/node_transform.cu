@@ -356,7 +356,7 @@ int launch_node_transform(const float* A, int64_t lda, const float* W, int64_t l
   if ((rc = tc::make_map_2d(&maps[1], w_lo, N, Kp, Kp, N / 2, true))) return rc;
   Params p{};
   p.A = A; p.lda = lda; p.C = C; p.ldc = ldc; p.bias = bias; p.scale = scale; p.shift = shift; p.act = act;
-  p.M = M; p.N = N; p.K = K; p.nkb = Kp / KB; p.n_tiles = ceil_div(M, 2 * BM);
+  p.M = M; p.N = N; p.K = K; p.nkb = Kp / KB; p.n_tiles = ceil_div(M, 2 * nt::BM);
   const uintptr_t ca = reinterpret_cast<uintptr_t>(C);
   p.c_vec = ((ldc & 7) == 0 && (ca & 31u) == 0) ? 8 : ((ldc & 3) == 0 && (ca & 15u) == 0) ? 4 : 1;
   p.st_tab = st_tab;
@@ -385,7 +385,7 @@ int launch_node_transform(const float* A, int64_t lda, const float* W, int64_t l
   }
   const int64_t pairs = p.n_tiles < kNumSMs / 2 ? p.n_tiles : kNumSMs / 2;
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(2 * pairs)); cfg.blockDim = dim3(THREADS); cfg.dynamicSmemBytes = SMEM_BYTES; cfg.stream = st;
+  cfg.gridDim = dim3((unsigned)(2 * pairs)); cfg.blockDim = dim3(nt::THREADS); cfg.dynamicSmemBytes = SMEM_BYTES; cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
   attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;

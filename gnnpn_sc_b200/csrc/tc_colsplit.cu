@@ -33,13 +33,8 @@ using namespace tc;
 using namespace seq;
 
 constexpr int CL = 8;                      // CTAs per cluster = column slices
-constexpr int BM = 128;                    // instances per cluster = UMMA M
 constexpr int TILE_N = kG / CL;            // 128 gate columns per CTA
 constexpr int UNITS = kH / CL;             // 32 hidden units per CTA
-constexpr int KB_H = kH / 64;              // 4 k-blocks of 64 halfs
-constexpr int BLK_BYTES = 128 * 128;       // [128 rows x 64 halfs]
-constexpr int EPI_WARPS = 16;
-constexpr int THREADS = 128 + 32 * EPI_WARPS;
 
 // G = instance groups of 128 per cluster.  G = 1: lowest latency.  G = 2 (encoder only): two independent groups share the
 // resident weights and are software-pipelined against each other -- while one group's h' is in flight through the exchange
@@ -150,38 +145,13 @@ lstm_colsplit_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid
     sbias[i] = b * ((col & 3) == 2 ? -2.0f * kLog2e : -kLog2e);
   }
 
-  auto write_x_rows = [&](int g, const float (*xv)[8]) {
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int r = lane + 32 * i;
-      uint32_t hi[4], lo[4];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        hi[j] = pack_h2(xv[i][2 * j], xv[i][2 * j + 1]);
-        const float2 bk = unpack_h2(hi[j]);
-        lo[j] = pack_h2(xv[i][2 * j] - bk.x, xv[i][2 * j + 1] - bk.y);
-      }
-      const uint32_t o = (uint32_t)r * XROW_BYTES;
-      st_shared_v4(ax_hi_off(g) + o, hi[0], hi[1], hi[2], hi[3]);
-      st_shared_v4(ax_hi_off(g) + o + 16, hi[0], hi[1], hi[2], hi[3]);
-      st_shared_v4(ax_lo_off(g) + o, lo[0], lo[1], lo[2], lo[3]);
-      st_shared_v4(ax_lo_off(g) + o + 16, lo[0], lo[1], lo[2], lo[3]);
-    }
-  };
-  auto load_x_rows = [&](int g, int t, float (*xv)[8]) {
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int64_t m = (group0 + g) * BM + lane + 32 * i;
-#pragma unroll
-      for (int f = 0; f < 8; ++f)
-        xv[i][f] = (m < p.n && f < p.F) ? __ldg(p.inputs + m * p.x_inst_ld + (int64_t)t * p.F + f) : 0.f;
-    }
-  };
+  // load_x_rows is called through this lambda, as in tc_seq.cu: calling it directly changes the generated code
+  auto load_inputs = [&](int g, int t, float (*xv)[8]) { load_x_rows(p, (group0 + g) * BM, t, lane, xv); };
   if (!DEC && warp == 3) {
     for (int g = 0; g < G; ++g) {
       float xv[4][8];
-      load_x_rows(g, 0, xv);
-      write_x_rows(g, xv);
+      load_inputs(g, 0, xv);
+      write_x_rows(ax_hi_off(g), ax_lo_off(g), lane, xv);
     }
   }
   fence_proxy_async_smem();
@@ -309,9 +279,9 @@ lstm_colsplit_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid
       for (int t = 0; t + 1 < p.steps; ++t) {
         for (int g = 0; g < G; ++g) {
           float xv[4][8];
-          load_x_rows(g, t + 1, xv);
+          load_inputs(g, t + 1, xv);
           mbar_wait(tfull(g), (uint32_t)t & 1u);          // the MMAs of step t no longer read the x block
-          write_x_rows(g, xv);
+          write_x_rows(ax_hi_off(g), ax_lo_off(g), lane, xv);
           fence_proxy_async_smem();
           __syncwarp();
           if (lane == 0) mbar_arrive(x_rdy(g));
@@ -333,12 +303,7 @@ lstm_colsplit_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid
     // split 8 fp32 values to fp16 hi/lo and store them to scratch parity (j & 1) of group g
     auto stage = [&](int g, const float* hv, int j) {
       uint32_t pk[8];
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        pk[i] = pack_h2(hv[2 * i], hv[2 * i + 1]);
-        const float2 bk = unpack_h2(pk[i]);
-        pk[4 + i] = pack_h2(hv[2 * i] - bk.x, hv[2 * i + 1] - bk.y);
-      }
+      split_f16x8(hv, pk, pk + 4);
       __half* dst = p.scratch + (size_t)(group0 + g) * (2 * 2 * BM * kH) + (size_t)(j & 1) * (2 * BM * kH) + (size_t)r * kH + u0;
       stg128_u(dst, pk[0], pk[1], pk[2], pk[3]);                    // hi rows
       stg128_u(dst + BM * kH, pk[4], pk[5], pk[6], pk[7]);          // lo rows
@@ -400,7 +365,7 @@ lstm_colsplit_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid
         if (lane == 0) mbar_arrive(tempty(g));                         // accumulator is in registers
         float cn[8], hn[8];
         // training forward: v becomes the post-activation gates; they are stored AFTER the publish (off the step's critical path)
-        if (p.save_gates) lstm_cell8_gates(v, bias4, c[g], cn, hn, v);
+        if (p.save_gates) lstm_cell8(v, bias4, c[g], cn, hn, v);
         else lstm_cell8(v, bias4, c[g], cn, hn);
         auto save_step = [&]() {
           // the BPTT's saves (gnnpn_pn_train_backward_f32): 128 + 32 contiguous bytes per thread
@@ -443,12 +408,7 @@ lstm_colsplit_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid
               for (int f = 0; f < 8; ++f)
                 xv[f] = (b < p.n && f < p.F) ? __ldg(p.inputs + (b * p.L + fed) * (int64_t)p.F + f) : 0.f;
               uint32_t hi[4], lo[4];
-#pragma unroll
-              for (int i = 0; i < 4; ++i) {
-                hi[i] = pack_h2(xv[2 * i], xv[2 * i + 1]);
-                const float2 bk = unpack_h2(hi[i]);
-                lo[i] = pack_h2(xv[2 * i] - bk.x, xv[2 * i + 1] - bk.y);
-              }
+              split_f16x8(xv, hi, lo);
               const uint32_t o = (uint32_t)prow * XROW_BYTES;
               const uint32_t dhi = mapa_rank(ax_hi_off(g) + o, (uint32_t)lane);
               const uint32_t dlo = mapa_rank(ax_lo_off(g) + o, (uint32_t)lane);

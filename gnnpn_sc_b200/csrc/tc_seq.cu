@@ -7,7 +7,7 @@
 //     a.w ~= a_lo.w_hi + a_hi.w_hi + a_hi.w_lo) in the 128B-swizzled K-major UMMA layout; the epilogue of step t
 //     writes h'(t) there directly -- h never goes through global memory between steps;
 //   * B operand (the 4H x (H+F) folded weights, fp16 hi/lo, 1.1 MB, L2-resident) is streamed by TMA through a
-//     ring of 16 KB slots, one (N tile, k block, hi|lo) box per slot;
+//     ring of 8 slots; a slot holds one (N tile, k block, hi|lo) box, each CTA of the pair 8 KB = half its gate columns;
 //   * accumulators: two 128-column TMEM buffers (N tile = 128 gate columns = 32 hidden units), so the
 //     epilogue of tile j overlaps the MMAs of tile j+1;
 //   * h'(t) of tiles 0..6 cannot be written over A while the MMAs of step t still read it: it is staged in the
@@ -15,7 +15,7 @@
 // Warp roles: 0 = TMA producer, 1 = MMA issuer, 2 = TMEM allocator, 3 = x producer (encoder inputs),
 // 4..19 = epilogue (TMEM lane quarter = warp & 3, column group = (warp - 4) / 4).
 //
-// Encodings layout (template parameter NR, SeqParams::enc_layout):
+// Encodings layout (template parameter NR):
 //   NR == 0  row-major enc_out [n, L, H] (GNNPN_ENC_ROWMAJOR).  Encoder: h' tiles leave by TMA store.  Decoder: a
 //            separate pointer phase after each step's cell epilogue (each epilogue warp owns 8 instances, window rows
 //            streamed per instance, pointer.cuh::pointer_steps_batched) -- the step is MMA phase + pointer phase.
@@ -51,15 +51,12 @@ namespace seq {
 
 using namespace tc;
 
-constexpr int BM = 128;                    // instances per CTA = UMMA M = TMEM lanes
 constexpr int TILE_N = 128;                // gate columns per accumulator tile
 constexpr int N_TILES = kG / TILE_N;       // 8
-constexpr int KB_H = kH / 64;              // 4 k-blocks of 64 halfs (128-byte swizzle rows)
-constexpr int BLK_BYTES = 128 * 128;       // one [128 rows x 64 halfs] block
-constexpr int RING_BYTES = 4 * BLK_BYTES;  // weight ring: 4 slots of 16 KB (1 CTA) / 8 slots of 8 KB (CTA pair)
-constexpr int MAX_RING = 8;
-constexpr int EPI_WARPS = 16;
-constexpr int THREADS = 128 + 32 * EPI_WARPS;
+constexpr int RING = 8;                    // weight ring slots
+constexpr int SLOT_ROWS = TILE_N / 2;      // each CTA of the pair loads half of a tile's gate columns
+constexpr int SLOT_BYTES = BLK_BYTES / 2;  // [64 gate columns x 64 halfs]
+constexpr int RING_BYTES = RING * SLOT_BYTES;
 constexpr int TMEM_COLS = 512;             // [0,256): 2 accumulator buffers; [256,512): h' staging
 constexpr int STAGE_COL0 = 256;
 
@@ -88,7 +85,6 @@ struct SeqParams {
   const float* h0; int64_t h0_ld;          // initial hidden rows or nullptr (zeros)
   float* h_out; int64_t h_out_inst_ld;     // step t of instance m at h_out + m*ld + t*kH
   PointerStepArgs pa;      // decoder only
-  int enc_layout;          // GNNPN_ENC_ROWMAJOR / GNNPN_ENC_BLOCKED128 of h_out (encoder) or pa.enc_out (decoder)
   unsigned long long* prof; // debug (GNNPN_SEQ_PROF): per-CTA wait-cycle counters, 16 per CTA, or nullptr
   float* c_scr;            // blocked cell-state scratch, 128*kH floats per CTA (coalesced 128-bit accesses)
 };
@@ -253,28 +249,19 @@ __device__ __forceinline__ void pointer_finish_thread(const SeqParams& p, int k,
 #pragma unroll
     for (int f = 0; f < 8; ++f) xv[f] = (ok && f < p.F) ? __ldg(p.inputs + (b * p.L + fed) * (int64_t)p.F + f) : 0.f;
     uint32_t hi[4], lo[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      hi[j] = pack_h2(xv[2 * j], xv[2 * j + 1]);
-      const float2 bk = unpack_h2(hi[j]);
-      lo[j] = pack_h2(xv[2 * j] - bk.x, xv[2 * j + 1] - bk.y);
-    }
+    split_f16x8(xv, hi, lo);
     const uint32_t o = (uint32_t)rr * XROW_BYTES;
-    st_shared_v4(sbase + OFF_AX_HI + o, hi[0], hi[1], hi[2], hi[3]);
-    st_shared_v4(sbase + OFF_AX_HI + o + 16, hi[0], hi[1], hi[2], hi[3]);
-    st_shared_v4(sbase + OFF_AX_LO + o, lo[0], lo[1], lo[2], lo[3]);
-    st_shared_v4(sbase + OFF_AX_LO + o + 16, lo[0], lo[1], lo[2], lo[3]);
+    st_x_row(sbase + OFF_AX_HI + o, sbase + OFF_AX_LO + o, hi, lo);
   }
 }
 
 
 // ------------------------------------------------------------------------------------------------
-// CG = 1: one CTA per 128 instances, cta_group::1 MMAs (M=128, N=128).
-// CG = 2: CTA pair (cluster of 2 = one TPC), cta_group::2 MMAs (M=256: 128 instances per CTA, N=128): each CTA
-//         streams only HALF of every weight tile (64 of the 128 gate columns) and the tensor cores read the
-//         other half from the peer -- half the L2->SM weight traffic, half the B-operand shared-memory reads,
-//         twice the ring depth.  CTA rank 0 issues the MMAs for the pair; both CTAs run producer / epilogue.
-template <bool DEC, int CG, int NR>
+// CTA pair (cluster of 2 = one TPC), cta_group::2 MMAs (M=256: 128 instances per CTA, N=128): each CTA streams only
+// HALF of every weight tile (64 of the 128 gate columns) and the tensor cores read the other half from the peer --
+// half the L2->SM weight traffic and B-operand shared-memory reads a lone CTA would need, and twice the ring depth.
+// CTA rank 0 issues the MMAs for the pair; both CTAs run producer / epilogue.
+template <bool DEC, int NR>
 __global__ void __launch_bounds__(THREADS, 1)
 lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_constant__ CUtensorMap map_wh_lo,
                 const __grid_constant__ CUtensorMap map_wx_hi, const __grid_constant__ CUtensorMap map_wx_lo,
@@ -282,27 +269,21 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
   extern __shared__ uint8_t smem_raw[];
   const uint32_t sbase = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* sgen = smem_raw + (sbase - smem_u32(smem_raw));          // generic pointer to the aligned base
-  constexpr int RING = 4 * CG;                          // slots
-  constexpr int SLOT_BYTES = BLK_BYTES / CG;            // [128/CG gate columns x 64 halfs]
-  constexpr int SLOT_ROWS = TILE_N / CG;
   const uint32_t bar0 = sbase + OFF_BAR;
   auto full_bar = [&](int s) { return bar0 + 8u * s; };
-  auto empty_bar = [&](int s) { return bar0 + 8u * (MAX_RING + s); };
-  auto tfull_bar = [&](int b) { return bar0 + 8u * (2 * MAX_RING + b); };
-  auto tempty_bar = [&](int b) { return bar0 + 8u * (2 * MAX_RING + 2 + b); };
-  const uint32_t a_ready_bar = bar0 + 8u * (2 * MAX_RING + 4);
-  const uint32_t mma_done_bar = bar0 + 8u * (2 * MAX_RING + 5);
-  const uint32_t hfull_bar = bar0 + 8u * (2 * MAX_RING + 6);
-  const uint32_t hempty_bar = bar0 + 8u * (2 * MAX_RING + 7);
-  const uint32_t tmem_slot = bar0 + 8u * (2 * MAX_RING + 8);
-  const uint32_t h_ready_bar = bar0 + 8u * (2 * MAX_RING + 9);   // decoder: h'(t) is in the A tiles (the pointer phase follows)
-  const uint32_t rank = CG == 2 ? cluster_ctarank() : 0u;
+  auto empty_bar = [&](int s) { return bar0 + 8u * (RING + s); };
+  auto tfull_bar = [&](int b) { return bar0 + 8u * (2 * RING + b); };
+  auto tempty_bar = [&](int b) { return bar0 + 8u * (2 * RING + 2 + b); };
+  const uint32_t a_ready_bar = bar0 + 8u * (2 * RING + 4);
+  const uint32_t mma_done_bar = bar0 + 8u * (2 * RING + 5);
+  const uint32_t hfull_bar = bar0 + 8u * (2 * RING + 6);
+  const uint32_t hempty_bar = bar0 + 8u * (2 * RING + 7);
+  const uint32_t tmem_slot = bar0 + 8u * (2 * RING + 8);
+  const uint32_t h_ready_bar = bar0 + 8u * (2 * RING + 9);   // decoder: h'(t) is in the A tiles (the pointer phase follows)
+  const uint32_t rank = cluster_ctarank();
   // barriers the MMA issuer (rank 0) waits on collect arrivals from both CTAs of the pair
-  const uint32_t a_ready_remote = CG == 2 ? mapa_rank(a_ready_bar, 0) : a_ready_bar;
-  const uint32_t h_ready_remote = CG == 2 ? mapa_rank(h_ready_bar, 0) : h_ready_bar;
-  auto arrive_leader = [&](uint32_t local_bar) {
-    if (CG == 2) mbar_arrive_cluster(mapa_rank(local_bar, 0)); else mbar_arrive(local_bar);
-  };
+  const uint32_t a_ready_remote = mapa_rank(a_ready_bar, 0);
+  const uint32_t h_ready_remote = mapa_rank(h_ready_bar, 0);
   float* sbias = reinterpret_cast<float*>(sgen + OFF_BIAS);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -318,15 +299,15 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
   }
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < RING; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
-    for (int b = 0; b < 2; ++b) { mbar_init(tfull_bar(b), 1); mbar_init(tempty_bar(b), CG * EPI_WARPS); }
-    mbar_init(a_ready_bar, CG * (EPI_WARPS + (DEC ? 0 : 1)));
-    mbar_init(h_ready_bar, CG * EPI_WARPS);
+    for (int b = 0; b < 2; ++b) { mbar_init(tfull_bar(b), 1); mbar_init(tempty_bar(b), 2 * EPI_WARPS); }
+    mbar_init(a_ready_bar, 2 * (EPI_WARPS + (DEC ? 0 : 1)));
+    mbar_init(h_ready_bar, 2 * EPI_WARPS);
     mbar_init(mma_done_bar, 1);
     mbar_init(hfull_bar, EPI_WARPS);
     mbar_init(hempty_bar, 1);
     fence_mbar_init();
   }
-  if (warp == 2) { if (CG == 2) tmem_alloc_cg2(tmem_slot, TMEM_COLS); else tmem_alloc(tmem_slot, TMEM_COLS); }
+  if (warp == 2) tmem_alloc_cg2(tmem_slot, TMEM_COLS);
 
   // ---- initial A operand: h(-1) split to fp16 hi/lo (zeros for the encoder), x block of step 0
   {
@@ -341,12 +322,7 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
         } else {
           ldg256(p.h0 + (m0 + r) * p.h0_ld + ch * 8, hv);
         }
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          hi[j] = pack_h2(hv[2 * j], hv[2 * j + 1]);
-          const float2 bk = unpack_h2(hi[j]);
-          lo[j] = pack_h2(hv[2 * j] - bk.x, hv[2 * j + 1] - bk.y);
-        }
+        split_f16x8(hv, hi, lo);
       }
       const uint32_t off = (uint32_t)(ch >> 3) * BLK_BYTES + sw128_off(r, ch & 7);
       st_shared_v4(sbase + OFF_A_HI + off, hi[0], hi[1], hi[2], hi[3]);
@@ -360,35 +336,9 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
     }
   }
 
-  // x block writer (warp 3): row r -> 16 halfs = [x hi (8) | same again]; the weight block has zeros in
-  // halfs 8..15, so the duplicate makes the 32B swizzle pattern irrelevant on the A side.
-  auto write_x_rows = [&](const float (*xv)[8]) {
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int r = lane + 32 * i;
-      uint32_t hi[4], lo[4];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        hi[j] = pack_h2(xv[i][2 * j], xv[i][2 * j + 1]);
-        const float2 bk = unpack_h2(hi[j]);
-        lo[j] = pack_h2(xv[i][2 * j] - bk.x, xv[i][2 * j + 1] - bk.y);
-      }
-      const uint32_t o = (uint32_t)r * XROW_BYTES;
-      st_shared_v4(sbase + OFF_AX_HI + o, hi[0], hi[1], hi[2], hi[3]);
-      st_shared_v4(sbase + OFF_AX_HI + o + 16, hi[0], hi[1], hi[2], hi[3]);
-      st_shared_v4(sbase + OFF_AX_LO + o, lo[0], lo[1], lo[2], lo[3]);
-      st_shared_v4(sbase + OFF_AX_LO + o + 16, lo[0], lo[1], lo[2], lo[3]);
-    }
-  };
-  auto load_x_rows = [&](int t, float (*xv)[8]) {
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int64_t m = m0 + lane + 32 * i;
-#pragma unroll
-      for (int f = 0; f < 8; ++f)
-        xv[i][f] = (m < p.n && f < p.F) ? __ldg(p.inputs + m * p.x_inst_ld + (int64_t)t * p.F + f) : 0.f;
-    }
-  };
+  // load_x_rows is called through this lambda: calling it directly at the two sites changes the register allocation
+  // of the encoder kernels' TMA producer
+  auto load_inputs = [&](int t, float (*xv)[8]) { load_x_rows(p, m0, t, lane, xv); };
   if (warp == 3) {
     float xv[4][8];
     if (DEC) {
@@ -397,13 +347,13 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
 #pragma unroll
         for (int f = 0; f < 8; ++f) xv[i][f] = 0.f;
     } else {
-      load_x_rows(0, xv);
+      load_inputs(0, xv);
     }
-    write_x_rows(xv);
+    write_x_rows(sbase + OFF_AX_HI, sbase + OFF_AX_LO, lane, xv);
   }
   fence_proxy_async_smem();
   tc_fence_before();
-  if (CG == 2) cluster_sync_all(); else __syncthreads();     // barrier inits / TMEM / A operand visible pair-wide
+  cluster_sync_all();                                       // barrier inits / TMEM / A operand visible pair-wide
   tc_fence_after();
   uint32_t tmem_base;
   asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
@@ -423,14 +373,9 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
           for (int part = 0; part < 2; ++part) {
             mbar_wait(empty_bar(s), ph ^ 1u);
             const uint32_t dst = sbase + OFF_RING + s * SLOT_BYTES;
-            if (CG == 2) {
-              if (rank == 0) mbar_arrive_expect_tx(full_bar(s), 2 * SLOT_BYTES);
-              tma_load_2d_cg2(dst, part ? &map_wh_lo : &map_wh_hi, mapa_rank(full_bar(s), 0), kb * 64,
-                              nt * TILE_N + row_off);
-            } else {
-              mbar_arrive_expect_tx(full_bar(s), SLOT_BYTES);
-              tma_load_2d(dst, part ? &map_wh_lo : &map_wh_hi, full_bar(s), kb * 64, nt * TILE_N);
-            }
+            if (rank == 0) mbar_arrive_expect_tx(full_bar(s), 2 * SLOT_BYTES);
+            tma_load_2d_cg2(dst, part ? &map_wh_lo : &map_wh_hi, mapa_rank(full_bar(s), 0), kb * 64,
+                            nt * TILE_N + row_off);
             if (++s == RING) { s = 0; ph ^= 1u; }
           }
         }
@@ -439,16 +384,10 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
         const int nt = it;
         mbar_wait(empty_bar(s), ph ^ 1u);
         const uint32_t dst = sbase + OFF_RING + s * SLOT_BYTES;
-        if (CG == 2) {
-          if (rank == 0) mbar_arrive_expect_tx(full_bar(s), 2 * 2 * SLOT_ROWS * XROW_BYTES);
-          const uint32_t fb = mapa_rank(full_bar(s), 0);
-          tma_load_2d_cg2(dst, &map_wx_hi, fb, kH, nt * TILE_N + row_off);
-          tma_load_2d_cg2(dst + SLOT_ROWS * XROW_BYTES, &map_wx_lo, fb, kH, nt * TILE_N + row_off);
-        } else {
-          mbar_arrive_expect_tx(full_bar(s), 2 * TILE_N * XROW_BYTES);
-          tma_load_2d(dst, &map_wx_hi, full_bar(s), kH, nt * TILE_N);
-          tma_load_2d(dst + TILE_N * XROW_BYTES, &map_wx_lo, full_bar(s), kH, nt * TILE_N);
-        }
+        if (rank == 0) mbar_arrive_expect_tx(full_bar(s), 2 * 2 * SLOT_ROWS * XROW_BYTES);
+        const uint32_t fb = mapa_rank(full_bar(s), 0);
+        tma_load_2d_cg2(dst, &map_wx_hi, fb, kH, nt * TILE_N + row_off);
+        tma_load_2d_cg2(dst + SLOT_ROWS * XROW_BYTES, &map_wx_lo, fb, kH, nt * TILE_N + row_off);
         if (++s == RING) { s = 0; ph ^= 1u; }
       };
       for (int t = 0; t < p.steps; ++t) {
@@ -463,11 +402,8 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
     // in uniform registers); one elected lane issues tcgen05.mma / tcgen05.commit =================
     if (rank == 0) {
       const uint32_t leader = elect_one();
-      const uint32_t idesc = idesc_f16(CG * BM, TILE_N);
-      auto mma = [&](uint32_t d, uint64_t a, uint64_t b, uint32_t acc) {
-        if (CG == 2) mma_f16_ss_cg2(d, a, b, idesc, acc); else mma_f16_ss(d, a, b, idesc, acc);
-      };
-      auto commit = [&](uint32_t bar) { if (CG == 2) mma_commit_cg2(bar); else mma_commit(bar); };
+      const uint32_t idesc = idesc_f16(2 * BM, TILE_N);
+      auto mma = [&](uint32_t d, uint64_t a, uint64_t b, uint32_t acc) { mma_f16_ss_cg2(d, a, b, idesc, acc); };
       const uint64_t ax_hi = smem_desc_k_sw32(sbase + OFF_AX_HI), ax_lo = smem_desc_k_sw32(sbase + OFF_AX_LO);
       int s = 0; uint32_t ph = 0;
       uint32_t uses = 0;                                   // per-buffer use count = uses >> 1 (tiles alternate)
@@ -488,7 +424,7 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
 #pragma unroll
             for (int ks = 0; ks < 4; ++ks)
               mma(d, a_hi + (uint64_t)(ks * 2), b_hi + (uint64_t)(ks * 2), 1u);
-            commit(empty_bar(s));
+            mma_commit_cg2(empty_bar(s));
           }
           __syncwarp();
           if (++s == RING) { s = 0; ph ^= 1u; }
@@ -499,7 +435,7 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
 #pragma unroll
             for (int ks = 0; ks < 4; ++ks)
               mma(d, a_hi + (uint64_t)(ks * 2), b_lo + (uint64_t)(ks * 2), 1u);
-            commit(empty_bar(s));
+            mma_commit_cg2(empty_bar(s));
           }
           __syncwarp();
           if (++s == RING) { s = 0; ph ^= 1u; }
@@ -514,9 +450,9 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
           mma(d, ax_lo, bx_hi, 1u);
           mma(d, ax_hi, bx_hi, 1u);
           mma(d, ax_hi, bx_lo, 1u);
-          commit(empty_bar(s));
-          commit(tfull_bar(buf));
-          if (last) commit(mma_done_bar);
+          mma_commit_cg2(empty_bar(s));
+          mma_commit_cg2(tfull_bar(buf));
+          if (last) mma_commit_cg2(mma_done_bar);
         }
         __syncwarp();
         if (++s == RING) { s = 0; ph ^= 1u; }
@@ -528,28 +464,28 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
           // tiles 0 and 1 (96 of the step's 408 MMAs) are issued as soon as h'(t-1) is in the A tiles, i.e. while the
           // pointer phase of step t-1 still runs; their x parts follow once the picked rows are in the x block.
           if (t > 0) {
-            mbar_wait_t<CG == 2>(h_ready_bar, (uint32_t)(t - 1) & 1u, prof, w_aready);
+            mbar_wait_t<true>(h_ready_bar, (uint32_t)(t - 1) & 1u, prof, w_aready);
             tc_fence_after();
           }
           for (int b = 0; b < 2; ++b) {
-            mbar_wait_t<CG == 2>(tempty_bar(b), (((uses + b) >> 1) & 1u) ^ 1u, prof, w_tempty);
+            mbar_wait_t<true>(tempty_bar(b), (((uses + b) >> 1) & 1u) ^ 1u, prof, w_tempty);
             tc_fence_after();
             mma_h(tmem_base + (uint32_t)(b * TILE_N));
           }
           if (t > 0) {
-            mbar_wait_t<CG == 2>(a_ready_bar, (uint32_t)(t - 1) & 1u, prof, w_aready);   // x(t) is in the x block
+            mbar_wait_t<true>(a_ready_bar, (uint32_t)(t - 1) & 1u, prof, w_aready);   // x(t) is in the x block
             tc_fence_after();
           }
           for (int b = 0; b < 2; ++b) mma_x(tmem_base + (uint32_t)(b * TILE_N), b, false);
           uses += 2;
           nt0 = 2;
         } else if (t > 0) {
-          mbar_wait_t<CG == 2>(a_ready_bar, (uint32_t)(t - 1) & 1u, prof, w_aready);  // h'(t-1), x(t) are in smem
+          mbar_wait_t<true>(a_ready_bar, (uint32_t)(t - 1) & 1u, prof, w_aready);  // h'(t-1), x(t) are in smem
           tc_fence_after();
         }
         for (int nt = nt0; nt < N_TILES; ++nt, ++uses) {
           const int buf = nt & 1;
-          mbar_wait_t<CG == 2>(tempty_bar(buf), ((uses >> 1) & 1u) ^ 1u, prof, w_tempty);
+          mbar_wait_t<true>(tempty_bar(buf), ((uses >> 1) & 1u) ^ 1u, prof, w_tempty);
           tc_fence_after();
           const uint32_t d = tmem_base + (uint32_t)(buf * TILE_N);
           mma_h(d);
@@ -607,12 +543,12 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
     if (!DEC) {
       for (int t = 0; t + 1 < p.steps; ++t) {
         float xv[4][8];
-        load_x_rows(t + 1, xv);
+        load_inputs(t + 1, xv);
         mbar_wait(mma_done_bar, (uint32_t)t & 1u);        // the MMAs of step t no longer read the x block
-        write_x_rows(xv);
+        write_x_rows(sbase + OFF_AX_HI, sbase + OFF_AX_LO, lane, xv);
         fence_proxy_async_smem();
         __syncwarp();
-        if (lane == 0) { if (CG == 2) mbar_arrive_cluster(a_ready_remote); else mbar_arrive(a_ready_bar); }
+        if (lane == 0) mbar_arrive_cluster(a_ready_remote);
       }
     }
   }
@@ -684,7 +620,8 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
         tmem_ld_wait(v);
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) arrive_leader(tempty_bar(buf));  // accumulators are in registers: MMA may reuse the buffer
+        // accumulators are in registers: MMA may reuse the buffer
+        if (lane == 0) mbar_arrive_cluster(mapa_rank(tempty_bar(buf), 0));
         float cn[8], hn[8];
         lstm_cell8(v, bias4 + u0, c_old, cn, hn);
         if (!last && keep_c) {
@@ -714,12 +651,7 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
           if (lane == 0) mbar_arrive(hfull_bar);
         }
         uint32_t pk[8];                                  // {hi01, hi23, hi45, hi67, lo01, lo23, lo45, lo67}
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          pk[j] = pack_h2(hn[2 * j], hn[2 * j + 1]);
-          const float2 bk = unpack_h2(pk[j]);
-          pk[4 + j] = pack_h2(hn[2 * j] - bk.x, hn[2 * j + 1] - bk.y);
-        }
+        split_f16x8(hn, pk, pk + 4);
         if (it < N_TILES - 1) {
           tmem_st_32x32_x8(t_lane + (uint32_t)(STAGE_COL0 + nt * 32 + grp * 8), pk);
         } else {
@@ -743,7 +675,7 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
             fence_proxy_async_smem();
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) { if (CG == 2) mbar_arrive_cluster(h_ready_remote); else mbar_arrive(h_ready_bar); }
+            if (lane == 0) mbar_arrive_cluster(h_ready_remote);
           }
         }
         if (do_dot) {
@@ -804,7 +736,7 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
       fence_proxy_async_smem();
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) { if (CG == 2) mbar_arrive_cluster(a_ready_remote); else mbar_arrive(a_ready_bar); }
+      if (lane == 0) mbar_arrive_cluster(a_ready_remote);
     }
     if (prof && warp == 4 && lane == 0) {
       unsigned long long* o = p.prof + (size_t)blockIdx.x * 16;
@@ -812,14 +744,14 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
     }
   }
   tc_fence_before();
-  if (CG == 2) cluster_sync_all(); else __syncthreads();
-  if (warp == 2) { if (CG == 2) tmem_dealloc_cg2(tmem_base, TMEM_COLS); else tmem_dealloc(tmem_base, TMEM_COLS); }
+  cluster_sync_all();
+  if (warp == 2) tmem_dealloc_cg2(tmem_base, TMEM_COLS);
 }
 
-template <bool DEC, int CG, int NR>
-int launch_seq_cg(const float* packed, SeqParams p, cudaStream_t st) {
+template <bool DEC, int NR>
+int launch_seq(const float* packed, SeqParams p, cudaStream_t st) {
   CUtensorMap maps[4];
-  int rc = make_weight_maps(maps, packed, TILE_N / CG);
+  int rc = make_weight_maps(maps, packed, SLOT_ROWS);
   if (rc) return rc;
   CUtensorMap map_h = maps[0];                         // only the row-major encoder stores through it
   if (!DEC && NR == 0) {
@@ -834,16 +766,16 @@ int launch_seq_cg(const float* packed, SeqParams p, cudaStream_t st) {
                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
       return GNNPN_ESHAPE;
   }
-  const unsigned grid = (unsigned)(ceil_div(p.n, BM * CG) * CG);
+  const unsigned grid = (unsigned)(ceil_div(p.n, 2 * BM) * 2);
   if ((rc = prof_alloc(grid, 16, st, &p.prof))) return rc;
-  rc = launch_cluster<lstm_seq_kernel<DEC, CG, NR>>(grid, CG, THREADS, SMEM_BYTES, st, maps[0], maps[1], maps[2], maps[3],
-                                                    map_h, p);
+  rc = launch_cluster<lstm_seq_kernel<DEC, NR>>(grid, 2, THREADS, SMEM_BYTES, st, maps[0], maps[1], maps[2], maps[3], map_h,
+                                                p);
   if (p.prof) {
     double acc[8];
     unsigned leaders = prof_collect(p.prof, grid, 16, st, acc);     // the MMA-issuing CTAs write counter 0
     if (!leaders) leaders = 1;
-    fprintf(stderr, "[seq prof %s cg=%d nr=%d steps=%d grid=%u] per-step cycles: mma total %.0f (wait a_ready %.0f, tmem_empty %.0f, "
-            "B full %.0f) | epi total %.0f (wait tmem_full %.0f, h buf %.0f, pointer %.0f)\n", DEC ? "dec" : "enc", CG, NR,
+    fprintf(stderr, "[seq prof %s nr=%d steps=%d grid=%u] per-step cycles: mma total %.0f (wait a_ready %.0f, tmem_empty %.0f, "
+            "B full %.0f) | epi total %.0f (wait tmem_full %.0f, h buf %.0f, pointer %.0f)\n", DEC ? "dec" : "enc", NR,
             p.steps, grid, acc[0] / leaders / p.steps, acc[1] / leaders / p.steps, acc[2] / leaders / p.steps,
             acc[3] / leaders / p.steps, acc[4] / grid / p.steps, acc[5] / grid / p.steps, acc[6] / grid / p.steps,
             acc[7] / grid / p.steps);
@@ -862,8 +794,7 @@ int tc_seq_encode(const SeqEncodeArgs& a, int nr, cudaStream_t st) {
   p.h0 = nullptr; p.h0_ld = 0;
   p.h_out = a.enc_out; p.h_out_inst_ld = (int64_t)a.L * kH;
   p.c_scr = a.c_scratch;
-  p.enc_layout = nr ? GNNPN_ENC_BLOCKED128 : GNNPN_ENC_ROWMAJOR;
-  return nr ? seq::launch_seq_cg<false, 2, 1>(a.packed, p, st) : seq::launch_seq_cg<false, 2, 0>(a.packed, p, st);
+  return nr ? seq::launch_seq<false, 1>(a.packed, p, st) : seq::launch_seq<false, 0>(a.packed, p, st);
 }
 
 int tc_seq_decode(const SeqDecodeArgs& a, int nr, cudaStream_t st) {
@@ -876,15 +807,14 @@ int tc_seq_decode(const SeqDecodeArgs& a, int nr, cudaStream_t st) {
   p.pa = pointer_step_args(a.enc_out, a.latent_win, a.alpha, a.use_tanh, a.C, a.n, a.L, a.N, a.idx_out, a.win_logits,
                            a.win_probs, a.forced_idx, a.sample_uniform);
   p.c_scr = a.c_scratch;
-  p.enc_layout = nr ? GNNPN_ENC_BLOCKED128 : GNNPN_ENC_ROWMAJOR;
   // blocked encodings (nr > 0): the pointer dots ride in the cell epilogue, and h0 is read from the block's position
   // L-1 inside the kernel
   if (nr == 0) { p.h0 = a.enc_out + (int64_t)(a.L - 1) * kH; p.h0_ld = (int64_t)a.L * kH; }
   switch (nr) {
-    case 5: return seq::launch_seq_cg<true, 2, 5>(a.packed, p, st);
-    case 8: return seq::launch_seq_cg<true, 2, 8>(a.packed, p, st);
-    case 10: return seq::launch_seq_cg<true, 2, 10>(a.packed, p, st);
-    default: return seq::launch_seq_cg<true, 2, 0>(a.packed, p, st);
+    case 5: return seq::launch_seq<true, 5>(a.packed, p, st);
+    case 8: return seq::launch_seq<true, 8>(a.packed, p, st);
+    case 10: return seq::launch_seq<true, 10>(a.packed, p, st);
+    default: return seq::launch_seq<true, 0>(a.packed, p, st);
   }
 }
 

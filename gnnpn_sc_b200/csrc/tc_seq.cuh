@@ -14,7 +14,7 @@ namespace gnnpn {
 // ---- which kernel runs a recurrence (tc_seq.cu) -------------------------------------------------------------------
 enum class ScanKind {
   kStep,          // one launch per step (lstm_recurrence_*)
-  kPair,          // CTA-pair scan lstm_seq_kernel<DEC, 2, NR>
+  kPair,          // CTA-pair scan lstm_seq_kernel<DEC, NR>
   kColsplit,      // column-split cluster scan lstm_colsplit_kernel<DEC, G>
   kUnsupported,   // blocked encodings with a window the fused decoder cannot hold (N > 10)
 };

@@ -1,5 +1,5 @@
-// Device-side helpers shared by the persistent tcgen05 LSTM scan kernels (tc_seq.cu: one CTA / CTA pair per 128
-// instances; tc_colsplit.cu: the gate columns of 128 instances split over a cluster of 8 CTAs).
+// Device-side helpers shared by the persistent tcgen05 LSTM scan kernels (tc_seq.cu: a CTA pair, 128 instances per
+// CTA; tc_colsplit.cu: the gate columns of 128 instances split over a cluster of 8 CTAs).
 #pragma once
 #include <cuda_fp16.h>
 #include "tc_common.cuh"
@@ -13,6 +13,11 @@ using namespace tc;
 constexpr float kLog2e = 1.4426950408889634f;
 constexpr float kClampT = 30.0f;           // exponentials are clamped to 2^30 so products of three stay finite
 constexpr int XROW_BYTES = 32;             // x block: 16 halfs per row, 32-byte swizzle layout
+constexpr int BM = 128;                    // instances per CTA (column-split: per cluster) = UMMA M = TMEM lanes
+constexpr int KB_H = kH / 64;              // 4 k-blocks of 64 halfs (128-byte swizzle rows)
+constexpr int BLK_BYTES = 128 * 128;       // one [128 rows x 64 halfs] block
+constexpr int EPI_WARPS = 16;
+constexpr int THREADS = 128 + 32 * EPI_WARPS;
 
 // K-major operand block with 32-byte rows (16 halfs), 32B swizzle, 8-row groups 256 B apart
 __device__ __forceinline__ uint64_t smem_desc_k_sw32(uint32_t smem_addr) {
@@ -138,6 +143,48 @@ __device__ __forceinline__ float2 unpack_h2(uint32_t u) {
   return __half22float2(*reinterpret_cast<const __half2*>(&u));
 }
 
+// fp16 hi/lo split of 8 floats: hi[j] = fp16 pair (v[2j], v[2j+1]), lo[j] = the pair's rounding remainders
+__device__ __forceinline__ void split_f16x8(const float* v, uint32_t* hi, uint32_t* lo) {
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    hi[j] = pack_h2(v[2 * j], v[2 * j + 1]);
+    const float2 bk = unpack_h2(hi[j]);
+    lo[j] = pack_h2(v[2 * j] - bk.x, v[2 * j + 1] - bk.y);
+  }
+}
+
+// One 32-byte x-block row in shared memory: [x hi (8 halfs) | same again] at hi_addr, the same for lo at lo_addr.  The
+// weight block has zeros in halfs 8..15, so the duplicate makes the 32B swizzle pattern irrelevant on the A side.
+__device__ __forceinline__ void st_x_row(uint32_t hi_addr, uint32_t lo_addr, const uint32_t* hi, const uint32_t* lo) {
+  st_shared_v4(hi_addr, hi[0], hi[1], hi[2], hi[3]);
+  st_shared_v4(hi_addr + 16, hi[0], hi[1], hi[2], hi[3]);
+  st_shared_v4(lo_addr, lo[0], lo[1], lo[2], lo[3]);
+  st_shared_v4(lo_addr + 16, lo[0], lo[1], lo[2], lo[3]);
+}
+
+// Encoder x block of step t for the 128 instances from m_first (rows lane + 32i, i < 4 of the calling warp): the raw
+// input rows, zeros past n and past F.  P: either scan's parameter struct.
+template <class P>
+__device__ __forceinline__ void load_x_rows(const P& p, int64_t m_first, int t, int lane, float (*xv)[8]) {
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int64_t m = m_first + lane + 32 * i;
+#pragma unroll
+    for (int f = 0; f < 8; ++f)
+      xv[i][f] = (m < p.n && f < p.F) ? __ldg(p.inputs + m * p.x_inst_ld + (int64_t)t * p.F + f) : 0.f;
+  }
+}
+// xv from load_x_rows as fp16 hi/lo rows lane + 32i of the x block at ax_hi / ax_lo
+__device__ __forceinline__ void write_x_rows(uint32_t ax_hi, uint32_t ax_lo, int lane, const float (*xv)[8]) {
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const uint32_t o = (uint32_t)(lane + 32 * i) * XROW_BYTES;
+    uint32_t hi[4], lo[4];
+    split_f16x8(xv[i], hi, lo);
+    st_x_row(ax_hi + o, ax_lo + o, hi, lo);
+  }
+}
+
 // byte offset of the 16-byte chunk holding halfs [8*c16, 8*c16+8) of row r inside a 128B-swizzled block
 __device__ __forceinline__ uint32_t sw128_off(int r, int c16) {
   return (uint32_t)((r >> 3) * 1024 + (r & 7) * 128 + ((c16 ^ (r & 7)) << 4));
@@ -148,31 +195,12 @@ __device__ __forceinline__ uint32_t sw128_off(int r, int c16) {
 // One reciprocal serves sigm(f), sigm(i) and tanh(g); a second one sigm(o) and tanh(c'):
 //   c' = [c(1+Ei)(1+Eg) + (1-Eg)(1+Ef)] / [(1+Ei)(1+Ef)(1+Eg)],   h' = (1-Ec) / [(1+Eo)(1+Ec)]
 // with Ex = 2^min(t_x, 30) = e^-x (e^-2x for the tanh arguments).  MUFU.EX2 / MUFU.RCP + one Newton step.
-__device__ __forceinline__ void lstm_cell8(const float* v, const float4* bias4, const float* c_old, float* c_new,
-                                           float* h_new) {
-  constexpr float S1 = -kLog2e / kW16Scale, S2 = -2.0f * kLog2e / kW16Scale;
-#pragma unroll
-  for (int u = 0; u < 8; ++u) {
-    const float4 b = bias4[u];
-    const float Ei = ex2_approx(fminf(fmaf(v[4 * u + 0], S1, b.x), kClampT));
-    const float Ef = ex2_approx(fminf(fmaf(v[4 * u + 1], S1, b.y), kClampT));
-    const float Eg = ex2_approx(fminf(fmaf(v[4 * u + 2], S2, b.z), kClampT));
-    const float Eo = ex2_approx(fminf(fmaf(v[4 * u + 3], S1, b.w), kClampT));
-    const float a = 1.0f + Ei, d = 1.0f + Ef, g = 1.0f + Eg;
-    const float ag = a * g;
-    const float r = rcp_refined(ag * d);
-    const float cn = fmaf(1.0f - Eg, d, c_old[u] * ag) * r;
-    const float Ec = ex2_approx(fminf(cn * (-2.0f * kLog2e), kClampT));
-    const float r2 = rcp_refined((1.0f + Eo) * (1.0f + Ec));
-    c_new[u] = cn;
-    h_new[u] = (1.0f - Ec) * r2;
-  }
-}
-
-// Same cell, also returning the post-activation gates (training saves: the BPTT reads sigm(i), sigm(f), tanh(g), sigm(o)):
+// `gates`, if not null, receives the post-activation gates (training saves: the BPTT reads sigm(i), sigm(f), tanh(g),
+// sigm(o)):
 //   sigm(i) = d g r, sigm(f) = a g r, tanh(g) = (1 - Eg) a d r, sigm(o) = (1 + Ec) r2     (r, r2 as above)
-__device__ __forceinline__ void lstm_cell8_gates(const float* v, const float4* bias4, const float* c_old, float* c_new,
-                                                 float* h_new, float* gates) {
+// It may be v itself: gates 4u..4u+3 are written after v[4u..4u+3] is read.
+__device__ __forceinline__ void lstm_cell8(const float* v, const float4* bias4, const float* c_old, float* c_new,
+                                           float* h_new, float* gates = nullptr) {
   constexpr float S1 = -kLog2e / kW16Scale, S2 = -2.0f * kLog2e / kW16Scale;
 #pragma unroll
   for (int u = 0; u < 8; ++u) {
@@ -189,10 +217,12 @@ __device__ __forceinline__ void lstm_cell8_gates(const float* v, const float4* b
     const float r2 = rcp_refined((1.0f + Eo) * (1.0f + Ec));
     c_new[u] = cn;
     h_new[u] = (1.0f - Ec) * r2;
-    gates[4 * u + 0] = d * g * r;
-    gates[4 * u + 1] = ag * r;
-    gates[4 * u + 2] = (1.0f - Eg) * (a * d) * r;
-    gates[4 * u + 3] = (1.0f + Ec) * r2;
+    if (gates) {
+      gates[4 * u + 0] = d * g * r;
+      gates[4 * u + 1] = ag * r;
+      gates[4 * u + 2] = (1.0f - Eg) * (a * d) * r;
+      gates[4 * u + 3] = (1.0f + Ec) * r2;
+    }
   }
 }
 
