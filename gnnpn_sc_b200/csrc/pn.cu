@@ -1,5 +1,5 @@
-// Pointer-network entry points: weight packing, encoder scan, fused greedy decode,
-// interface-faithful logits materialisation, composition objective / reward.
+// Pointer-network entry points: weight packing, encoder scan, fused greedy decode, composition objective / reward
+// (the dense logits are in pn_general.cu).
 #include <math.h>
 #include <cuda_fp16.h>
 #include "lstm_step.cuh"
@@ -68,13 +68,7 @@ __global__ void pack_lstm_kernel(const float* __restrict__ w_ih, const float* __
 }
 
 // ---------------------------------------------------------------------------
-// pointer step (Dot attention): one warp per instance
-//   u_j   = <enc_out[b, kN+j, :], q[b,:]>            j in [0,N)
-//   l_j   = use_tanh ? C*tanh(u_j) : u_j            -> win_logits[b, kN+j]
-//   w_j   = l_j + alpha*latent[b, kN+j]
-//   p     = softmax_j(w)  (exp(w-max)/sum, fp32)    -> win_probs[b, kN+j]
-//   pick  = first j with maximal p                  -> idx_out[b] = kN + j
-// Positions outside the window carry -inf after modelPN.py:220-222 and contribute exp(-inf)=0.
+// pointer step (Dot attention, pointer.cuh): one warp per instance
 // ---------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) pointer_step_dot_kernel(
     const PointerStepArgs pa, int k, const float* __restrict__ q, int64_t q_ld, const float* __restrict__ inputs, int F,
@@ -102,39 +96,6 @@ int launch_pointer_steps(const PointerStepArgs& pa, int K, const float* dec_h, c
     if ((rc = after_launch())) return rc;
   }
   return GNNPN_OK;
-}
-
-// ---------------------------------------------------------------------------
-// full logits: one CTA per (instance, 32-row slab of L); queries of the instance in smem
-// ---------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) full_logits_dot_kernel(
-    const float* __restrict__ enc_out, const float* __restrict__ dec_h, const int32_t* __restrict__ idx,
-    int use_tanh, float C, int64_t n, int L, int K, float* __restrict__ out) {
-  extern __shared__ float sq[];                // [K][kH]
-  const int64_t b = blockIdx.x;
-  const int l0 = blockIdx.y * 32;
-  const float4* qsrc = reinterpret_cast<const float4*>(dec_h + b * (int64_t)K * kH);
-  for (int i = threadIdx.x; i < K * kH / 4; i += blockDim.x) reinterpret_cast<float4*>(sq)[i] = __ldg(qsrc + i);
-  __syncthreads();
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  for (int l = l0 + warp; l < min(L, l0 + 32); l += 8) {
-    const float4* rp = reinterpret_cast<const float4*>(enc_out + (b * L + l) * (int64_t)kH);
-    const float4 r0 = __ldg(rp + 2 * lane), r1 = __ldg(rp + 2 * lane + 1);   // canonical dot: lane owns floats [8*lane, +8)
-    for (int k = 0; k < K; ++k) {
-      const float4 a0 = reinterpret_cast<const float4*>(sq + k * kH)[2 * lane];
-      const float4 a1 = reinterpret_cast<const float4*>(sq + k * kH)[2 * lane + 1];
-      const float d = dot_reduce(dot8(r0, r1, a0, a1), lane);
-      if (lane == 0) out[((int64_t)k * n + b) * L + l] = use_tanh ? C * tanhf(d) : d;
-    }
-  }
-  // cumulative visited mask: step k sees -inf at the picks of steps 0..k-1 (modelPN.py:165-173)
-  __syncthreads();
-  for (int pair = threadIdx.x; pair < K * K; pair += blockDim.x) {
-    const int k = pair / K, jprev = pair % K;
-    if (jprev >= k) continue;
-    const int pos = idx[(int64_t)jprev * n + b];
-    if (pos >= l0 && pos < l0 + 32 && pos < L) out[((int64_t)k * n + b) * L + pos] = -INFINITY;
-  }
 }
 
 // ---------------------------------------------------------------------------
@@ -433,26 +394,6 @@ int gnnpn_pn_train_forward_tc_f32(const float* inputs, const float* packed_enc, 
                    idx_out, win_logits, win_probs, forced_idx, sample_uniform, scr};
   da.save_gates = gates_d; da.save_c = c_d;
   return tc_colsplit_decode(da, plan.dec.variant, st);
-}
-
-int gnnpn_pn_full_logits_f32(const float* enc_out, const float* dec_h, const int32_t* idx,
-                             int attention, const float* att_params, int use_tanh, float C,
-                             int64_t n, int L, int hidden, int K, float* logits_full, void* stream) {
-  GNNPN_REQUIRE(enc_out && dec_h && idx && logits_full, GNNPN_ENULL);
-  GNNPN_REQUIRE(hidden == kH && K >= 1 && L >= 1, GNNPN_ESHAPE);
-  GNNPN_REQUIRE(attention == GNNPN_ATT_DOT, GNNPN_EUNSUPPORTED);
-  (void)att_params;
-  const size_t smem = (size_t)K * kH * sizeof(float);
-  GNNPN_REQUIRE(smem <= 200 * 1024, GNNPN_ESHAPE);
-  GNNPN_REQUIRE(n < 65536ll * 32768ll, GNNPN_ERANGE);
-  if (n == 0) return GNNPN_OK;
-  cudaError_t e = cudaFuncSetAttribute(full_logits_dot_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)smem);
-  if (e != cudaSuccess) return (int)e;
-  dim3 grid((unsigned)n, (unsigned)ceil_div(L, 32));
-  full_logits_dot_kernel<<<grid, 256, smem, (cudaStream_t)stream>>>(enc_out, dec_h, idx, use_tanh, C, n, L, K,
-                                                                  logits_full);
-  return after_launch();
 }
 
 int gnnpn_pn_reward_f32(const float* inputs, const int32_t* idx, int64_t n, int L, int in_features,

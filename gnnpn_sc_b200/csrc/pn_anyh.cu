@@ -8,11 +8,10 @@
 #include <math.h>
 #include "common.cuh"
 #include "internal.cuh"
+#include "pointer.cuh"
 
 namespace gnnpn {
 namespace {
-
-constexpr int kMaxWindowAnyH = 32;
 
 inline unsigned init_grid(int64_t elems) {
   const int64_t b = ceil_div(elems, 256);
@@ -57,61 +56,28 @@ __global__ void anyh_cell_kernel(const float* __restrict__ gates, float* __restr
   if (next_row >= 0 && j < F) a_cat[m * (H + F) + H + j] = inputs[m * x_inst_ld + (int64_t)next_row * F + j];
 }
 
-// Pointer step k for one instance per warp (N <= 32: lane j finishes candidate j).
-__global__ void __launch_bounds__(256) anyh_pointer_kernel(
-    const float* __restrict__ enc_out, const float* __restrict__ q, int64_t q_ld, const float* __restrict__ latent_win,
-    float alpha, int use_tanh, float C, int64_t n, int L, int H, int N, int k, int32_t* __restrict__ idx_out,
-    float* __restrict__ win_logits, float* __restrict__ win_probs, const int32_t* __restrict__ forced,
-    const float* __restrict__ uniform, const float* __restrict__ inputs, int F, float* __restrict__ a_cat, int feed_next) {
+// Pointer step k for one instance per warp (N <= 32, a.enc_inst_ld = L * H): lane j forms d_j with the H-generic dot
+// and pointer_finish_lanes finishes candidate j.
+__global__ void __launch_bounds__(256) anyh_pointer_kernel(const PointerStepArgs a, int k, int H, const float* __restrict__ q,
+                                                           int64_t q_ld, const float* __restrict__ inputs, int F,
+                                                           float* __restrict__ a_cat, int feed_next) {
   const int lane = threadIdx.x & 31;
   const int64_t b = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  if (b >= n) return;
+  if (b >= a.n) return;
+  const int N = a.N;
   const float* qb = q + b * q_ld;
-  const int64_t wpos = b * L + (int64_t)k * N;
-  float mine = -INFINITY;                               // work logit of candidate `lane`
+  const float* rows = a.enc_out + b * a.enc_inst_ld + (int64_t)k * N * H;
+  float d = 0.f;
   for (int j = 0; j < N; ++j) {
-    const float* row = enc_out + (wpos + j) * (int64_t)H;
+    const float* row = rows + (int64_t)j * H;
     float s = 0.f;
     for (int u = lane; u < H; u += 32) s = fmaf(row[u], qb[u], s);
     s = warp_sum(s);                                    // xor butterfly: every lane holds the same sum
-    const float l = use_tanh ? C * tanhf(s) : s;
-    if (lane == 0) win_logits[wpos + j] = l;
-    const float w = latent_win ? fmaf(alpha, latent_win[wpos + j], l) : l;
-    if (lane == j) mine = w;
+    if (lane == j) d = s;
   }
-  float mx = mine;
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-  const float ex = lane < N ? expf(mine - mx) : 0.f;
-  float sum = 0.f;                                      // sequential in candidate order, identical in every lane
-  for (int j = 0; j < N; ++j) sum += __shfl_sync(0xffffffffu, ex, j);
-  const float p = ex / sum;
-  if (lane < N) win_probs[wpos + lane] = p;
-  // first maximal probability (torch.max tie rule, modelPN.py:225-226) or inverse-CDF draw (modelPN.py:227-228)
-  int pick = 0;
-  if (uniform) {
-    const float uu = uniform[(int64_t)k * n + b];
-    float cum = 0.f;
-    int chosen = -1, last_pos = 0;
-    for (int j = 0; j < N; ++j) {
-      const float pj = __shfl_sync(0xffffffffu, p, j);
-      cum += pj;
-      if (pj > 0.f) last_pos = j;
-      if (chosen < 0 && uu < cum) chosen = j;
-    }
-    pick = chosen < 0 ? last_pos : chosen;
-  } else {
-    float best = -1.f;
-    for (int j = 0; j < N; ++j) {
-      const float pj = __shfl_sync(0xffffffffu, p, j);
-      if (pj > best) { best = pj; pick = j; }
-    }
-  }
-  if (lane == 0) idx_out[(int64_t)k * n + b] = k * N + pick;
-  if (feed_next) {
-    const int fed = forced ? forced[(int64_t)k * n + b] : k * N + pick;
-    if (lane < F) a_cat[b * (H + F) + H + lane] = inputs[(b * L + fed) * (int64_t)F + lane];
-  }
+  const float lat = a.latent_win && lane < N ? a.latent_win[b * a.L + (int64_t)k * N + lane] : 0.f;
+  const int fed = pointer_finish_lanes<32>(a, k, b, true, d, lat, lane, N <= 8 ? 4 : 16);
+  if (feed_next && lane < F) a_cat[b * (H + F) + H + lane] = inputs[(b * a.L + fed) * (int64_t)F + lane];
 }
 
 // prev_logits materialised (modelPN.py:213-214,239): warp = (instance b, position l), loop over the K steps
@@ -183,7 +149,7 @@ int gnnpn_pn_decode_anyh_f32(const float* inputs, const float* enc_out, float* c
                              const float* sample_uniform, float* workspace, size_t workspace_floats, void* stream) {
   GNNPN_REQUIRE(inputs && enc_out && c_state && w_cat && bias && bias0 && dec_h && idx_out && win_logits && win_probs &&
                     workspace, GNNPN_ENULL);
-  GNNPN_REQUIRE(hidden >= 1 && in_features >= 1 && in_features <= 32 && K >= 1 && N >= 1 && N <= kMaxWindowAnyH &&
+  GNNPN_REQUIRE(hidden >= 1 && in_features >= 1 && in_features <= 32 && K >= 1 && N >= 1 && N <= kMaxWindow &&
                     (int64_t)K * N == L && n >= 0, GNNPN_ESHAPE);
   GNNPN_REQUIRE(workspace_floats >= gnnpn_pn_anyh_workspace_floats(n, hidden, in_features), GNNPN_EWORKSPACE);
   if (n == 0) return GNNPN_OK;
@@ -196,6 +162,8 @@ int gnnpn_pn_decode_anyh_f32(const float* inputs, const float* enc_out, float* c
   anyh_init_kernel<<<init_grid(n * W), 256, 0, st>>>(
       a_cat, n, H, F, enc_out + (int64_t)(L - 1) * H, (int64_t)L * H, nullptr, 0, -1);
   if ((rc = after_launch())) return rc;
+  const PointerStepArgs pa{enc_out, (int64_t)L * H, latent_win, alpha, use_tanh, C, n, L, N, idx_out, win_logits,
+                          win_probs, forced_idx, sample_uniform};
   for (int k = 0; k < K; ++k) {
     if ((rc = launch_gemm_ffma(a_cat, W, w_cat, W, k == 0 ? bias0 : bias, nullptr, nullptr, GNNPN_ACT_NONE, gates,
                                4 * (int64_t)H, n, 4 * H, W, st)))
@@ -203,9 +171,8 @@ int gnnpn_pn_decode_anyh_f32(const float* inputs, const float* enc_out, float* c
     anyh_cell_kernel<<<(unsigned)ceil_div(n * H, 256), 256, 0, st>>>(gates, c_state, 0, dec_h + (int64_t)k * H,
                                                                      (int64_t)K * H, a_cat, n, H, F, nullptr, 0, -1);
     if ((rc = after_launch())) return rc;
-    anyh_pointer_kernel<<<(unsigned)ceil_div(n, 8), 256, 0, st>>>(
-        enc_out, dec_h + (int64_t)k * H, (int64_t)K * H, latent_win, alpha, use_tanh, C, n, L, H, N, k, idx_out, win_logits,
-        win_probs, forced_idx, sample_uniform, inputs, F, a_cat, k + 1 < K);
+    anyh_pointer_kernel<<<(unsigned)ceil_div(n, 8), 256, 0, st>>>(pa, k, H, dec_h + (int64_t)k * H, (int64_t)K * H, inputs,
+                                                                  F, a_cat, k + 1 < K);
     if ((rc = after_launch())) return rc;
   }
   return GNNPN_OK;

@@ -7,7 +7,7 @@
 //   * any window width N (scale-up: N = 1000) and up to 32 raw input columns (embedding_size = 20).
 // One launch per piece and per step (LSTM cell, [query GEMM, glimpse] x n_glimpses, query GEMM, pointer); one CTA
 // per composition instance in the attention kernels.  For Dot / no glimpse / N <= 32 the pointer arithmetic is the
-// same as pointer_step_warp's (canonical dot, fmaf latent, sequential softmax sum) -> bit-identical picks / logits.
+// pointer.cuh's (canonical dot, then the shared logit / softmax / pick / draw rules) -> bit-identical picks / logits.
 #include <math.h>
 #include <cuda_fp16.h>
 #include "internal.cuh"
@@ -111,17 +111,11 @@ __global__ void __launch_bounds__(kAttThreads) glimpse_step_kernel(const General
 // pointer on window k, any N: one CTA per instance
 // ---------------------------------------------------------------------------------------------------------
 struct PointerGeneralArgs {
-  GeneralArgs g;
-  const float* latent_win;   // [n, L] or nullptr
-  float alpha;
-  int use_tanh;
-  float C;
-  int N;
-  int32_t* idx_out;          // [K, n]
-  float* win_logits;         // [n, L]
-  float* win_probs;          // [n, L]
-  const int32_t* forced;     // [K, n] or nullptr
-  const float* uniform;      // [K, n] or nullptr
+  PointerStepArgs s;         // s.enc_out: the rows the query scores, enc_out (Dot) or E (Bahdanau), [n, L, kH]
+  int k;
+  const float* q;            // [n] rows q_ld apart: the query (Dot) or W_query q + b_query (Bahdanau)
+  int64_t q_ld;
+  const float* V;            // [kH] (Bahdanau)
   const float* inputs;       // [n, L, F]
   int F;
   LstmXSlot x_next;          // tensor-core LSTM path: where the fed row goes (hi == nullptr: the FFMA step gathers it)
@@ -130,7 +124,8 @@ struct PointerGeneralArgs {
 template <bool BAHD>
 __global__ void __launch_bounds__(kAttThreads) pointer_general_kernel(const PointerGeneralArgs p) {
   extern __shared__ float smem_f[];
-  const int N = p.N, k = p.g.k;
+  const PointerStepArgs& a = p.s;
+  const int N = a.N, k = p.k;
   float* sw = smem_f;                  // [N] masked working logits
   float* se = smem_f + N;              // [N] exp(w - max)
   __shared__ float red_v[kAttWarps];
@@ -140,21 +135,21 @@ __global__ void __launch_bounds__(kAttThreads) pointer_general_kernel(const Poin
   const int64_t b = blockIdx.x;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   // Dot: canonical pointer dot (pointer.cuh), lane owns floats [8*lane, 8*lane+8); Bahdanau: float4 lane / 32+lane
-  const float4* qp = reinterpret_cast<const float4*>(p.g.q + b * p.g.q_ld);
+  const float4* qp = reinterpret_cast<const float4*>(p.q + b * p.q_ld);
   const int i0 = BAHD ? lane : 2 * lane, i1 = BAHD ? 32 + lane : 2 * lane + 1;
   const float4 q0 = qp[i0], q1 = qp[i1];
   float4 v0 = make_float4(0, 0, 0, 0), v1 = v0;
-  if (BAHD) { v0 = __ldg(reinterpret_cast<const float4*>(p.g.V) + lane); v1 = __ldg(reinterpret_cast<const float4*>(p.g.V) + 32 + lane); }
-  const float* base = p.g.rows + (b * (int64_t)p.g.L + (int64_t)k * N) * kH;
-  const int64_t wbase = b * (int64_t)p.g.L + (int64_t)k * N;
+  if (BAHD) { v0 = __ldg(reinterpret_cast<const float4*>(p.V) + lane); v1 = __ldg(reinterpret_cast<const float4*>(p.V) + 32 + lane); }
+  const int64_t wbase = b * (int64_t)a.L + (int64_t)k * N;
+  const float* base = a.enc_out + wbase * kH;                            // row-major rows: enc_inst_ld = L * kH
   for (int j = warp; j < N; j += kAttWarps) {
     const float4* rp = reinterpret_cast<const float4*>(base + (int64_t)j * kH);
     const float4 r0 = ldg_stream(rp + i0), r1 = ldg_stream(rp + i1);
     const float d = BAHD ? warp_sum(bahdanau8(r0, r1, q0, q1, v0, v1)) : dot_reduce(dot8(r0, r1, q0, q1), lane);
     if (lane == 0) {
-      const float l = p.use_tanh ? p.C * tanhf(d) : d;
-      p.win_logits[wbase + j] = l;
-      sw[j] = p.latent_win ? fmaf(p.alpha, __ldg(p.latent_win + wbase + j), l) : l;
+      const float l = window_logit(a.use_tanh, a.C, d);
+      a.win_logits[wbase + j] = l;
+      sw[j] = work_logit(a, l, a.latent_win ? __ldg(a.latent_win + wbase + j) : 0.f);
     }
   }
   __syncthreads();
@@ -181,72 +176,66 @@ __global__ void __launch_bounds__(kAttThreads) pointer_general_kernel(const Poin
   }
   __syncthreads();
   const float s = s_bcast[1];
-  // probabilities + first maximal probability (torch.max tie rule, modelPN.py:225-226)
-  float best = -1.f;
-  int best_j = 0x7fffffff;
+  // probabilities + first maximal probability: per thread, then per warp, then across the warps
+  FirstMax m{-1.f, 0x7fffffff};
   for (int j = threadIdx.x; j < N; j += kAttThreads) {
     const float pj = se[j] / s;
-    p.win_probs[wbase + j] = pj;
+    a.win_probs[wbase + j] = pj;
     se[j] = pj;
-    if (pj > best) { best = pj; best_j = j; }            // ascending j per thread: keeps the first maximum
+    m.add(j, pj);
   }
 #pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const float ob = __shfl_xor_sync(0xffffffffu, best, o);
-    const int oj = __shfl_xor_sync(0xffffffffu, best_j, o);
-    if (ob > best || (ob == best && oj < best_j)) { best = ob; best_j = oj; }
-  }
-  if (lane == 0) { red_v[warp] = best; red_i[warp] = best_j; }
+  for (int o = 16; o > 0; o >>= 1) m.merge(__shfl_xor_sync(0xffffffffu, m.best, o), __shfl_xor_sync(0xffffffffu, m.j, o));
+  if (lane == 0) { red_v[warp] = m.best; red_i[warp] = m.j; }
   __syncthreads();
   if (threadIdx.x == 0) {
-    float bv = red_v[0];
-    int bj = red_i[0];
-    for (int w = 1; w < kAttWarps; ++w)
-      if (red_v[w] > bv || (red_v[w] == bv && red_i[w] < bj)) { bv = red_v[w]; bj = red_i[w]; }
-    if (p.uniform) {                       // sample="sample": inverse-CDF draw (see pointer_finish_warp)
-      const float u = __ldg(p.uniform + (int64_t)k * p.g.n + b);
-      float cum = 0.f;
-      int pick = -1, last_pos = 0;
-      for (int j = 0; j < N; ++j) {
-        const float pj = se[j];
-        cum += pj;
-        if (pj > 0.f) last_pos = j;
-        if (pick < 0 && u < cum) pick = j;
-      }
-      bj = pick < 0 ? last_pos : pick;
+    FirstMax cta{red_v[0], red_i[0]};
+    for (int w = 1; w < kAttWarps; ++w) cta.merge(red_v[w], red_i[w]);
+    int pick = cta.j;
+    if (a.uniform) {
+      const float u = __ldg(a.uniform + (int64_t)k * a.n + b);
+      InverseCdf draw;
+      for (int j = 0; j < N; ++j) draw.add(j, se[j], u);
+      pick = draw.result();
     }
-    p.idx_out[(int64_t)k * p.g.n + b] = k * N + bj;
-    s_pick = p.forced ? p.forced[(int64_t)k * p.g.n + b] : k * N + bj;
+    s_pick = record_pick(a, k, b, pick, true, forced_pick(a, k, b));
   }
   __syncthreads();
   if (p.x_next.hi && threadIdx.x < p.F) {
     const int f = threadIdx.x;
-    stage_x_f16(p.x_next.hi, p.x_next.lo, p.x_next.ld, b, f, __ldg(p.inputs + (b * p.g.L + s_pick) * (int64_t)p.F + f));
+    stage_x_f16(p.x_next.hi, p.x_next.lo, p.x_next.ld, b, f, __ldg(p.inputs + (b * a.L + s_pick) * (int64_t)p.F + f));
   }
 }
 
-// dense logits for Bahdanau: out[k, b, l] = C*tanh( V . tanh(qw[b,k,:] + E[b,l,:]) ), -inf at the picks of steps < k
-__global__ void __launch_bounds__(256) full_logits_bahdanau_kernel(
-    const float* __restrict__ E, const float* __restrict__ qw, const float* __restrict__ V,
+// Dense logits (prev_logits, modelPN.py:213-214,239): out[k, b, l] = the window logit of row l against query k, -inf at
+// the picks of steps < k.  Dot: rows = enc_out, q = dec_h, canonical dot (pointer.cuh); Bahdanau: rows = E, q = qw,
+// V . tanh(qw + E).  One CTA per (instance, 32-row slab of L), the instance's K queries in shared memory.
+template <bool BAHD>
+__global__ void __launch_bounds__(256) full_logits_kernel(
+    const float* __restrict__ rows, const float* __restrict__ q, const float* __restrict__ V,
     const int32_t* __restrict__ idx, int use_tanh, float C, int64_t n, int L, int K, float* __restrict__ out) {
   extern __shared__ float sq[];                // [K][kH]
   const int64_t b = blockIdx.x;
   const int l0 = blockIdx.y * 32;
-  const float4* qsrc = reinterpret_cast<const float4*>(qw + b * (int64_t)K * kH);
+  const float4* qsrc = reinterpret_cast<const float4*>(q + b * (int64_t)K * kH);
   for (int i = threadIdx.x; i < K * kH / 4; i += blockDim.x) reinterpret_cast<float4*>(sq)[i] = __ldg(qsrc + i);
   __syncthreads();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const float4 v0 = __ldg(reinterpret_cast<const float4*>(V) + lane), v1 = __ldg(reinterpret_cast<const float4*>(V) + 32 + lane);
+  // Dot: lane owns floats [8*lane, 8*lane+8); Bahdanau: float4 lane / 32+lane
+  const int i0 = BAHD ? lane : 2 * lane, i1 = BAHD ? 32 + lane : 2 * lane + 1;
+  float4 v0 = make_float4(0, 0, 0, 0), v1 = v0;
+  if (BAHD) { v0 = __ldg(reinterpret_cast<const float4*>(V) + lane); v1 = __ldg(reinterpret_cast<const float4*>(V) + 32 + lane); }
   for (int l = l0 + warp; l < min(L, l0 + 32); l += 8) {
-    const float4* rp = reinterpret_cast<const float4*>(E + (b * L + l) * (int64_t)kH);
-    const float4 r0 = __ldg(rp + lane), r1 = __ldg(rp + 32 + lane);
+    const float4* rp = reinterpret_cast<const float4*>(rows + (b * L + l) * (int64_t)kH);
+    const float4 r0 = __ldg(rp + i0), r1 = __ldg(rp + i1);
     for (int k = 0; k < K; ++k) {
-      const float4 a0 = reinterpret_cast<const float4*>(sq + k * kH)[lane];
-      const float4 a1 = reinterpret_cast<const float4*>(sq + k * kH)[32 + lane];
-      const float d = warp_sum(bahdanau8(r0, r1, a0, a1, v0, v1));
-      if (lane == 0) out[((int64_t)k * n + b) * L + l] = use_tanh ? C * tanhf(d) : d;
+      const float4 a0 = reinterpret_cast<const float4*>(sq + k * kH)[i0];
+      const float4 a1 = reinterpret_cast<const float4*>(sq + k * kH)[i1];
+      const float d = BAHD ? warp_sum(bahdanau8(r0, r1, a0, a1, v0, v1)) : dot_reduce(dot8(r0, r1, a0, a1), lane);
+      if (lane == 0) out[((int64_t)k * n + b) * L + l] = window_logit(use_tanh, C, d);
     }
   }
+  // cumulative visited mask: step k sees -inf at the picks of steps 0..k-1 (modelPN.py:165-173)
   __syncthreads();
   for (int pair = threadIdx.x; pair < K * K; pair += blockDim.x) {
     const int k = pair / K, jprev = pair % K;
@@ -254,6 +243,20 @@ __global__ void __launch_bounds__(256) full_logits_bahdanau_kernel(
     const int pos = idx[(int64_t)jprev * n + b];
     if (pos >= l0 && pos < l0 + 32 && pos < L) out[((int64_t)k * n + b) * L + pos] = -INFINITY;
   }
+}
+
+template <bool BAHD>
+int launch_full_logits(const float* rows, const float* q, const float* V, const int32_t* idx, int use_tanh, float C,
+                       int64_t n, int L, int K, float* out, cudaStream_t st) {
+  const size_t smem = (size_t)K * kH * sizeof(float);
+  GNNPN_REQUIRE(smem <= 200 * 1024, GNNPN_ESHAPE);
+  GNNPN_REQUIRE(n < 65536ll * 32768ll, GNNPN_ERANGE);
+  if (n == 0) return GNNPN_OK;
+  cudaError_t e = cudaFuncSetAttribute(full_logits_kernel<BAHD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return (int)e;
+  dim3 grid((unsigned)n, (unsigned)ceil_div(L, 32));
+  full_logits_kernel<BAHD><<<grid, 256, smem, st>>>(rows, q, V, idx, use_tanh, C, n, L, K, out);
+  return after_launch();
 }
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
@@ -341,6 +344,13 @@ int gnnpn_pn_decode_general_f32(const float* inputs, const float* enc_out, float
     cudaFuncSetAttribute(pointer_general_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ptr_smem);
     cudaFuncSetAttribute(pointer_general_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ptr_smem);
   }
+  PointerGeneralArgs pa{};
+  pa.s = pointer_step_args(bahd ? e_p : enc_out, latent_win, alpha, use_tanh, C, n, L, N, idx_out, win_logits, win_probs,
+                           forced_idx, sample_uniform);
+  pa.q_ld = (int64_t)K * kH;
+  pa.V = bahd ? att_p + kOffV : nullptr;
+  pa.inputs = inputs;
+  pa.F = in_features;
   for (int k = 0; k < K; ++k) {
     // ---- decoder LSTM cell (modelPN.py:205)
     if ((rc = lstm_decoder_step(r, k, enc_out, dec_h, K, fed_all, nullptr, st))) return rc;
@@ -369,20 +379,16 @@ int gnnpn_pn_decode_general_f32(const float* inputs, const float* enc_out, float
         return (int)cudaGetLastError();
     }
     // ---- pointer on window k (modelPN.py:213-228)
-    PointerGeneralArgs pa{};
-    pa.g.fed = fed_all; pa.g.n = n; pa.g.L = L; pa.g.k = k;
-    pa.latent_win = latent_win; pa.alpha = alpha; pa.use_tanh = use_tanh; pa.C = C; pa.N = N;
-    pa.idx_out = idx_out; pa.win_logits = win_logits; pa.win_probs = win_probs;
-    pa.forced = forced_idx; pa.uniform = sample_uniform; pa.inputs = inputs; pa.F = in_features;
+    pa.k = k;
     pa.x_next = lstm_decoder_x_slot(r, k);
     if (bahd) {
       float* qwp = qw_pointer + (int64_t)k * kH;                 // [n, K, kH]: kept for the dense-logits kernel
       if ((rc = launch_gemm_ffma(q_cur, (int64_t)K * kH, att_p + kOffWq, kH, att_p + kOffBq, nullptr, nullptr,
                                  GNNPN_ACT_NONE, qwp, (int64_t)K * kH, n, kH, kH, st))) return rc;
-      pa.g.rows = e_p; pa.g.q = qwp; pa.g.q_ld = (int64_t)K * kH; pa.g.V = att_p + kOffV;
+      pa.q = qwp;
       pointer_general_kernel<true><<<(unsigned)n, kAttThreads, ptr_smem, st>>>(pa);
     } else {
-      pa.g.rows = enc_out; pa.g.q = q_cur; pa.g.q_ld = (int64_t)K * kH; pa.g.V = nullptr;
+      pa.q = q_cur;
       pointer_general_kernel<false><<<(unsigned)n, kAttThreads, ptr_smem, st>>>(pa);
     }
     if ((rc = after_launch())) return rc;
@@ -408,21 +414,23 @@ int gnnpn_pn_query_transform_f32(const float* q, int64_t q_ld, const float* att_
                           qw_ld, rows, kH, kH, (cudaStream_t)stream);
 }
 
+int gnnpn_pn_full_logits_f32(const float* enc_out, const float* dec_h, const int32_t* idx,
+                             int attention, const float* att_params, int use_tanh, float C,
+                             int64_t n, int L, int hidden, int K, float* logits_full, void* stream) {
+  GNNPN_REQUIRE(enc_out && dec_h && idx && logits_full, GNNPN_ENULL);
+  GNNPN_REQUIRE(hidden == kH && K >= 1 && L >= 1, GNNPN_ESHAPE);
+  GNNPN_REQUIRE(attention == GNNPN_ATT_DOT, GNNPN_EUNSUPPORTED);
+  (void)att_params;
+  return launch_full_logits<false>(enc_out, dec_h, nullptr, idx, use_tanh, C, n, L, K, logits_full, (cudaStream_t)stream);
+}
+
 int gnnpn_pn_full_logits_bahdanau_f32(const float* E, const float* qw, const float* att_block, const int32_t* idx,
                                       int use_tanh, float C, int64_t n, int L, int hidden, int K, float* logits_full,
                                       void* stream) {
   GNNPN_REQUIRE(E && qw && att_block && idx && logits_full, GNNPN_ENULL);
   GNNPN_REQUIRE(hidden == kH && K >= 1 && L >= 1, GNNPN_ESHAPE);
-  const size_t smem = (size_t)K * kH * sizeof(float);
-  GNNPN_REQUIRE(smem <= 200 * 1024, GNNPN_ESHAPE);
-  GNNPN_REQUIRE(n < 65536ll * 32768ll, GNNPN_ERANGE);
-  if (n == 0) return GNNPN_OK;
-  cudaError_t e = cudaFuncSetAttribute(full_logits_bahdanau_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return (int)e;
-  dim3 grid((unsigned)n, (unsigned)ceil_div(L, 32));
-  full_logits_bahdanau_kernel<<<grid, 256, smem, (cudaStream_t)stream>>>(E, qw, att_block + kOffV, idx, use_tanh, C, n, L,
-                                                                         K, logits_full);
-  return after_launch();
+  return launch_full_logits<true>(E, qw, att_block + kOffV, idx, use_tanh, C, n, L, K, logits_full,
+                                  (cudaStream_t)stream);
 }
 
 }  // extern "C"

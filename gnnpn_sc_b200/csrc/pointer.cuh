@@ -78,55 +78,135 @@ __device__ __forceinline__ void ld_row8(const float* row, int lane, float4& a, f
                : "l"(row + 8 * lane) : "memory");
 }
 
-// Second half of the pointer step, from the window logit pre-activations: lane j (< N) holds d_j = <row_j, q> in
-// `d` and (when a.latent_win != nullptr) latent[b, kN+j] in `lat`.  Writes win_logits / win_probs / idx_out and
-// returns, in every lane, the position fed to the next decoder step (the pick, or forced[b]).
-__device__ __forceinline__ int pointer_finish_warp(const PointerStepArgs& a, int k, int64_t b, float d, float lat, int lane) {
+// ---- the rest of the step, from the pre-activations d_j = <row_j, q> -----------------------------------------------
+// Each rule is written once, here.  The forms below (and the general kernels, pn_general.cu / pn_anyh.cu) only decide
+// which lane, thread or CTA handles which candidate, so their window logits, probabilities and picks are bit-identical.
+
+__device__ __forceinline__ float window_logit(int use_tanh, float C, float d) { return use_tanh ? C * tanhf(d) : d; }
+// working logit: the window logit plus PNHigh's latent term
+__device__ __forceinline__ float work_logit(const PointerStepArgs& a, float l, float lat) {
+  return a.latent_win ? fmaf(a.alpha, lat, l) : l;
+}
+
+// first maximal probability (torch.max tie rule, modelPN.py:225-226): `add` takes candidates in ascending order,
+// `merge` joins the result over another set of candidates
+struct FirstMax {
+  float best;
+  int j;
+  __device__ __forceinline__ void add(int c, float p) {
+    if (p > best) { best = p; j = c; }
+  }
+  __device__ __forceinline__ void merge(float ob, int oj) {
+    if (ob > best || (ob == best && oj < j)) { best = ob; j = oj; }
+  }
+};
+
+// sample="sample" (modelPN.py:227-228): inverse-CDF draw from the window distribution with a caller-supplied uniform
+// u in [0,1), candidates added in ascending order; falls back to the last candidate with non-zero probability when
+// round-off leaves the cumulative sum at or below u
+struct InverseCdf {
+  float cum = 0.f;
+  int pick = -1, last_pos = 0;
+  __device__ __forceinline__ void add(int c, float p, float u) {
+    cum += p;
+    if (p > 0.f) last_pos = c;
+    if (pick < 0 && u < cum) pick = c;
+  }
+  __device__ __forceinline__ int result() const { return pick < 0 ? last_pos : pick; }
+};
+
+// the teacher-forced position of step k for instance b, or -1
+__device__ __forceinline__ int forced_pick(const PointerStepArgs& a, int k, int64_t b) {
+  return a.forced ? a.forced[(int64_t)k * a.n + b] : -1;
+}
+// Records window candidate `pick` of step k (idx_out[k, b] = kN + pick, when `write`) and returns the position fed to
+// the next decoder step: `forced` (forced_pick) when teacher forcing, else kN + pick.
+__device__ __forceinline__ int record_pick(const PointerStepArgs& a, int k, int64_t b, int pick, bool write, int forced) {
+  if (write) a.idx_out[(int64_t)k * a.n + b] = k * a.N + pick;
+  return a.forced ? forced : k * a.N + pick;
+}
+
+// Lane form: one instance per segment of SEG lanes (8, 16 or 32).  Lane j (< N) of the segment holds d_j in `d` and,
+// with a latent, latent[b, kN+j] in `lat`; `inst` is false in a segment without an instance (b must still be a valid
+// index).  The butterflies start at offset `top`, a power of two with N <= 2 * top <= SEG: max and first maximum are
+// exact, so the depth changes no result.  Writes win_logits / win_probs / idx_out and returns, in every lane of the
+// segment, the position fed to the next decoder step.
+template <int SEG>
+__device__ __forceinline__ int pointer_finish_lanes(const PointerStepArgs& a, int k, int64_t b, bool inst, float d,
+                                                    float lat, int j, int top) {
   const int N = a.N;
-  const float my_l = a.use_tanh ? a.C * tanhf(d) : d;
-  float my_w = -INFINITY;
-  const int64_t wpos = b * a.L + (int64_t)k * N + lane;
-  if (lane < N) {
-    my_w = a.latent_win ? fmaf(a.alpha, lat, my_l) : my_l;
-    a.win_logits[wpos] = my_l;
+  const bool valid = inst && j < N;
+  const float l = window_logit(a.use_tanh, a.C, d);
+  const int64_t wpos = b * a.L + (int64_t)k * N + j;
+  float w = -INFINITY;
+  if (valid) {
+    w = work_logit(a, l, lat);
+    a.win_logits[wpos] = l;
   }
-  // windows of <= 8 candidates live in lanes 0..7: 3 butterfly levels instead of 5 (max / argmax are exact, so the
-  // result does not depend on the tree)
-  const int top = N <= 8 ? 4 : 16;
-  float mx = my_w;
+  float mx = w;
+#pragma unroll
   for (int o = top; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-  const float e = lane < N ? expf(my_w - mx) : 0.f;
-  // sequential sum in candidate order (deterministic, independent of warp shuffles' tree)
+  const float e = valid ? expf(w - mx) : 0.f;
   float s = 0.f;
-  for (int j = 0; j < N; ++j) s += __shfl_sync(0xffffffffu, e, j);
+  for (int c = 0; c < N; ++c) s += __shfl_sync(0xffffffffu, e, c, SEG);    // sequential, in candidate order
   const float p = e / s;
-  if (lane < N) a.win_probs[wpos] = p;
-  // first maximal probability (torch.max tie rule, modelPN.py:225-226)
-  float best = p;
-  int best_j = lane < N ? lane : 0x7fffffff;
-  if (lane >= N) best = -1.f;
-  for (int o = top; o > 0; o >>= 1) {
-    const float ob = __shfl_xor_sync(0xffffffffu, best, o);
-    const int oj = __shfl_xor_sync(0xffffffffu, best_j, o);
-    if (ob > best || (ob == best && oj < best_j)) { best = ob; best_j = oj; }
-  }
-  best_j = __shfl_sync(0xffffffffu, best_j, 0);
+  if (valid) a.win_probs[wpos] = p;
+  FirstMax m{valid ? p : -1.f, valid ? j : 0x7fffffff};
+#pragma unroll
+  for (int o = top; o > 0; o >>= 1) m.merge(__shfl_xor_sync(0xffffffffu, m.best, o), __shfl_xor_sync(0xffffffffu, m.j, o));
+  int pick = __shfl_sync(0xffffffffu, m.j, 0, SEG);   // lanes at or past 2 * top took no part in the butterflies
   if (a.uniform) {
-    // sample="sample" (modelPN.py:227-228): inverse-CDF draw from the window distribution with a caller-supplied
-    // uniform in [0,1); falls back to the last candidate with non-zero probability on round-off
     const float u = __ldg(a.uniform + (int64_t)k * a.n + b);
-    float cum = 0.f;
-    int pick = -1, last_pos = 0;
-    for (int j = 0; j < N; ++j) {
-      const float pj = __shfl_sync(0xffffffffu, p, j);
-      cum += pj;
-      if (pj > 0.f) last_pos = j;
-      if (pick < 0 && u < cum) pick = j;
-    }
-    best_j = pick < 0 ? last_pos : pick;
+    InverseCdf draw;
+    for (int c = 0; c < N; ++c) draw.add(c, __shfl_sync(0xffffffffu, p, c, SEG), u);
+    pick = draw.result();
   }
-  if (lane == 0) a.idx_out[(int64_t)k * a.n + b] = k * N + best_j;
-  return a.forced ? a.forced[(int64_t)k * a.n + b] : k * N + best_j;
+  return record_pick(a, k, b, pick, inst && j == 0, forced_pick(a, k, b));
+}
+
+// Serial form (the fused decoder, tc_seq.cu): ONE thread finishes the step of instance b from d[j] = d_j (j < N <= NR).
+// Threads without an instance (ok == false) run the same code on instance 0 without writing.  Returns the position fed
+// to the next decoder step.
+template <int NR>
+__device__ __forceinline__ int pointer_finish_thread(const PointerStepArgs& a, int k, int64_t b, bool ok,
+                                                     const float (&d)[NR]) {
+  const int N = a.N;
+  if (!ok) b = 0;
+  const int64_t wpos = b * a.L + (int64_t)k * N;
+  float w[NR];
+  float lat[NR];
+#pragma unroll
+  for (int j = 0; j < NR; ++j) lat[j] = (a.latent_win && j < N) ? __ldg(a.latent_win + wpos + j) : 0.f;
+  const float u = a.uniform ? __ldg(a.uniform + (int64_t)k * a.n + b) : 0.f;
+  const int forced = forced_pick(a, k, b);
+  float mx = -INFINITY;
+#pragma unroll
+  for (int j = 0; j < NR; ++j) {
+    w[j] = -INFINITY;
+    if (j < N) {
+      const float l = window_logit(a.use_tanh, a.C, d[j]);
+      if (ok) a.win_logits[wpos + j] = l;
+      w[j] = work_logit(a, l, lat[j]);
+      mx = fmaxf(mx, w[j]);
+    }
+  }
+  float s = 0.f;
+#pragma unroll
+  for (int j = 0; j < NR; ++j) {
+    if (j < N) { w[j] = expf(w[j] - mx); s += w[j]; }
+  }
+  InverseCdf draw;
+  FirstMax m{-1.f, 0};
+#pragma unroll
+  for (int j = 0; j < NR; ++j) {
+    if (j < N) {
+      const float pj = w[j] / s;
+      if (ok) a.win_probs[wpos + j] = pj;
+      m.add(j, pj);
+      draw.add(j, pj, u);
+    }
+  }
+  return record_pick(a, k, b, a.uniform ? draw.result() : m.j, ok, forced);
 }
 
 // q0/q1: the lane's 8 query elements (floats [8*lane, 8*lane+8) of the 256-float query).
@@ -155,7 +235,8 @@ __device__ __forceinline__ int pointer_step_warp(const PointerStepArgs& a, int k
   }
   float lat = 0.f;
   if (a.latent_win && lane < N) lat = __ldg(a.latent_win + b * a.L + (int64_t)k * N + lane);
-  return pointer_finish_warp(a, k, b, my_d, lat, lane);
+  // windows of <= 8 candidates live in lanes 0..7: 3 butterfly levels instead of 5
+  return pointer_finish_lanes<32>(a, k, b, true, my_d, lat, lane, N <= 8 ? 4 : 16);
 }
 
 // ---- form used by the fused decode kernel: one warp owns WI = 8 consecutive instances.
@@ -163,9 +244,7 @@ __device__ __forceinline__ int pointer_step_warp(const PointerStepArgs& a, int k
 // requested as soon as the dot products have consumed the current one, so the DRAM round trips of consecutive
 // instances overlap the butterfly reductions.  The logit pre-activations are parked lane-wise: instance i,
 // candidate j -> register i / IPP, lane (i % IPP) * SEG + j  (SEG = 8, 16 or 32 lanes per instance, IPP = 32 / SEG).
-// Phase 2 then runs tanh / latent / softmax / pick for IPP instances at once with SEG-wide segmented shuffles.
-// Per candidate the arithmetic is exactly that of pointer_step_warp (canonical dot, fmaf latent, sequential
-// softmax sum in candidate order) -> same bits.
+// Phase 2 then finishes IPP instances per pass with pointer_finish_lanes<SEG>.
 // `feed(i, b, fed, j)` is called by every lane of a pass with the position fed to the next step for ITS instance
 // (i = instance slot 0..7, j = lane index inside the segment); slots >= count must be ignored by the callee.
 constexpr int kWarpInstances = 8;
@@ -227,46 +306,8 @@ __device__ __forceinline__ void pointer_steps_batched(const PointerStepArgs& a, 
     const int si = r * IPP + seg_i;                // this lane's instance slot
     if (r * IPP >= count) break;                   // warp-uniform
     const bool inst_ok = si < count;
-    const bool valid = inst_ok && seg_j < N;
     const int64_t b = b0 + (inst_ok ? si : 0);
-    const float my_l = a.use_tanh ? a.C * tanhf(dv[r]) : dv[r];
-    const int64_t wpos = b * a.L + (int64_t)k * N + seg_j;
-    float my_w = -INFINITY;
-    if (valid) {
-      my_w = a.latent_win ? fmaf(a.alpha, lat[r], my_l) : my_l;
-      a.win_logits[wpos] = my_l;
-    }
-    float mx = my_w;
-#pragma unroll
-    for (int o = SEG / 2; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-    const float e = valid ? expf(my_w - mx) : 0.f;
-    float s = 0.f;
-    for (int j = 0; j < N; ++j) s += __shfl_sync(0xffffffffu, e, j, SEG);   // candidate order, per segment
-    const float p = e / s;
-    if (valid) a.win_probs[wpos] = p;
-    float best = valid ? p : -1.f;
-    int best_j = valid ? seg_j : 0x7fffffff;
-#pragma unroll
-    for (int o = SEG / 2; o > 0; o >>= 1) {
-      const float ob = __shfl_xor_sync(0xffffffffu, best, o);
-      const int oj = __shfl_xor_sync(0xffffffffu, best_j, o);
-      if (ob > best || (ob == best && oj < best_j)) { best = ob; best_j = oj; }
-    }
-    if (a.uniform) {                               // sample="sample": inverse-CDF draw, see pointer_finish_warp
-      const float uu = __ldg(a.uniform + (int64_t)k * a.n + b);
-      float cum = 0.f;
-      int pick = -1, last_pos = 0;
-      for (int j = 0; j < N; ++j) {
-        const float pj = __shfl_sync(0xffffffffu, p, j, SEG);
-        cum += pj;
-        if (pj > 0.f) last_pos = j;
-        if (pick < 0 && uu < cum) pick = j;
-      }
-      best_j = pick < 0 ? last_pos : pick;
-    }
-    if (inst_ok && seg_j == 0) a.idx_out[(int64_t)k * a.n + b] = k * N + best_j;
-    const int fed = a.forced ? a.forced[(int64_t)k * a.n + b] : k * N + best_j;
-    feed(si, b, fed, seg_j);
+    feed(si, b, pointer_finish_lanes<SEG>(a, k, b, inst_ok, dv[r], lat[r], seg_j, SEG / 2), seg_j);
   }
 }
 

@@ -195,66 +195,6 @@ __device__ __forceinline__ void named_bar_sync(int id, int threads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory");
 }
 
-// Last part of a fused decode step (NR >= 1), executed by ONE thread per instance (the group-0 epilogue thread of row
-// rr): d[j] = canonical dot <enc_out[b, kN+j], h'(k)>.  Same arithmetic, operation by operation, as
-// pointer_finish_warp (C*tanhf, fmaf latent, expf(w - max), sequential sum in candidate order, first maximal
-// probability, inverse-CDF draw) -- a thread-serial loop instead of warp shuffles.  Writes win_logits / win_probs /
-// idx_out and the x block row of the next step.
-template <int NR>
-__device__ __forceinline__ void pointer_finish_thread(const SeqParams& p, int k, int rr, int64_t b, bool ok,
-                                                      const float (&d)[NR], uint32_t sbase) {
-  const PointerStepArgs& a = p.pa;
-  const int N = a.N;
-  const int64_t wpos = (ok ? b : 0) * a.L + (int64_t)k * N;
-  float w[NR];
-  float lat[NR];
-#pragma unroll
-  for (int j = 0; j < NR; ++j) lat[j] = (a.latent_win && j < N) ? __ldg(a.latent_win + wpos + j) : 0.f;
-  const float uu = a.uniform ? __ldg(a.uniform + (int64_t)k * a.n + (ok ? b : 0)) : 0.f;
-  const int forced = a.forced ? a.forced[(int64_t)k * a.n + (ok ? b : 0)] : -1;
-  float mx = -INFINITY;
-#pragma unroll
-  for (int j = 0; j < NR; ++j) {
-    w[j] = -INFINITY;
-    if (j < N) {
-      const float l = a.use_tanh ? a.C * tanhf(d[j]) : d[j];
-      if (ok) a.win_logits[wpos + j] = l;
-      w[j] = a.latent_win ? fmaf(a.alpha, lat[j], l) : l;
-      mx = fmaxf(mx, w[j]);
-    }
-  }
-  float s = 0.f;
-#pragma unroll
-  for (int j = 0; j < NR; ++j) {
-    if (j < N) { w[j] = expf(w[j] - mx); s += w[j]; }
-  }
-  float best = -1.f, cum = 0.f;
-  int best_j = 0, pick = -1, last_pos = 0;
-#pragma unroll
-  for (int j = 0; j < NR; ++j) {
-    if (j < N) {
-      const float pj = w[j] / s;
-      if (ok) a.win_probs[wpos + j] = pj;
-      if (pj > best) { best = pj; best_j = j; }            // ascending j, strict >: first maximum (torch.max tie rule)
-      cum += pj;
-      if (pj > 0.f) last_pos = j;
-      if (pick < 0 && uu < cum) pick = j;
-    }
-  }
-  if (a.uniform) best_j = pick < 0 ? last_pos : pick;
-  if (ok) a.idx_out[(int64_t)k * a.n + b] = k * N + best_j;
-  if (k + 1 < p.steps) {
-    const int fed = a.forced ? forced : k * N + best_j;
-    float xv[8];
-#pragma unroll
-    for (int f = 0; f < 8; ++f) xv[f] = (ok && f < p.F) ? __ldg(p.inputs + (b * p.L + fed) * (int64_t)p.F + f) : 0.f;
-    uint32_t hi[4], lo[4];
-    split_f16x8(xv, hi, lo);
-    const uint32_t o = (uint32_t)rr * XROW_BYTES;
-    st_x_row(sbase + OFF_AX_HI + o, sbase + OFF_AX_LO + o, hi, lo);
-  }
-}
-
 
 // ------------------------------------------------------------------------------------------------
 // CTA pair (cluster of 2 = one TPC), cta_group::2 MMAs (M=256: 128 instances per CTA, N=128): each CTA streams only
@@ -729,7 +669,17 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
           for (int j = 0; j < NR; ++j)
             d[j] = j < N ? __fadd_rn(__fadd_rn(acc[j], part[(0 * NR + j) * BM + r]),
                                       __fadd_rn(part[(1 * NR + j) * BM + r], part[(2 * NR + j) * BM + r])) : 0.f;
-          pointer_finish_thread<NRA>(p, t, r, m, ok, d, sbase);
+          const int fed = pointer_finish_thread<NRA>(p.pa, t, m, ok, d);
+          if (t + 1 < p.steps) {                        // the fed row is the x block row of the next step
+            float xv[8];
+#pragma unroll
+            for (int f = 0; f < 8; ++f)
+              xv[f] = (ok && f < p.F) ? __ldg(p.inputs + (m * p.L + fed) * (int64_t)p.F + f) : 0.f;
+            uint32_t hi[4], lo[4];
+            split_f16x8(xv, hi, lo);
+            const uint32_t o = (uint32_t)r * XROW_BYTES;
+            st_x_row(sbase + OFF_AX_HI + o, sbase + OFF_AX_LO + o, hi, lo);
+          }
         }
         if (prof) w_ptr += clock64() - tp0;
       }

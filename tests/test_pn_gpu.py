@@ -393,6 +393,82 @@ def test_column_split_scan_equals_cta_pair_scan_bitwise(n, K, N):
             assert torch.equal(a, b), key
 
 
+def _sampled_decode(actor, x, lat, K, N, seed=5):
+    """A sample="sample" decode whose uniforms come from a fresh generator, so every kernel draws with the same ones.
+    Checks that every pick is the inverse CDF of the kernel's own window probabilities at the uniform PointerNet.forward
+    drew (sequential float32 cumulative sum; the last candidate with p > 0 when no candidate qualifies).  Returns
+    (picks [K, n], win_logits, win_probs, how many picks differ from the first maximal probability)."""
+    actor.generator = torch.Generator(device="cuda").manual_seed(seed)
+    with torch.no_grad():
+        _, idx, _ = actor(x, lat, sample="sample")
+    u = torch.rand(K, x.shape[0], device="cuda", generator=torch.Generator(device="cuda").manual_seed(seed))
+    idx = torch.stack(idx).cpu().numpy()
+    wl, wp = actor.last["win_logits"].clone(), actor.last["win_probs"].clone()
+    p = wp.view(-1, K, N).permute(1, 0, 2).cpu().numpy()                       # [K, n, N]
+    hit = u.cpu().numpy()[..., None] < np.cumsum(p, axis=2, dtype=np.float32)
+    last_pos = np.where(p > 0, np.arange(N), 0).max(axis=2)
+    base = np.arange(K)[:, None] * N
+    assert np.array_equal(idx, np.where(hit.any(axis=2), hit.argmax(axis=2), last_pos) + base)
+    return idx, wl, wp, int((idx != p.argmax(axis=2) + base).sum())
+
+
+def _high_net(n, K, N, H=256, seed=3):
+    from gnnpn_sc_b200 import modelPN as M
+    from gnnpn_sc_b200.synth import pn_instances
+    from gnnpn_sc_b200.weights import reference_shaped_state_dict
+    x = pn_instances(n, K, N, seed=seed).cuda()
+    m = M.CombinatorialRL(0, H, K * N, 0, 10, 1, M.reward, "Dot", N, K, level="High")
+    m.load_state_dict(reference_shaped_state_dict(H, 8, 78) if H == 256 else
+                      po.make_state_dict(po.PNConfig(hidden_size=H, seq_len=K * N, s_number=N, s_category=K), 11))
+    lat = [torch.randn(n, K * N, device="cuda", generator=torch.Generator(device="cuda").manual_seed(seed))] * K
+    return m.cuda().eval(), x, lat
+
+
+@pytest.mark.parametrize("N", [5, 10, 12, 32])
+def test_sampled_decode_column_split_equals_cta_pair_bitwise(N):
+    """Sampled decodes with a latent draw the same picks and write the same window logits / probabilities on the CTA-pair
+    scan (N <= 10: one thread finishes an instance; N > 10: lane segments) and on the column-split scan (one warp per
+    instance, one and two groups per cluster), and every draw is the inverse CDF of the window probabilities."""
+    from gnnpn_sc_b200 import ops
+    K, n = 6, 260
+    m, x, lat = _high_net(n, K, N)
+    outs = {}
+    for key, (mode, g) in {"pair": (0, 0), "cs1": (1, 1), "cs2": (1, 2)}.items():
+        ops.set_option("scan", mode)
+        ops.set_option("scan_groups", g)
+        *outs[key], differ = _sampled_decode(m.actor, x, lat, K, N)
+        assert differ > 0, key
+        assert m.actor.last["enc_layout"] == (ops.ENC_BLOCKED128 if key == "pair" and N <= 10 else ops.ENC_ROWMAJOR)
+    for key in ("cs1", "cs2"):
+        assert np.array_equal(outs[key][0], outs["pair"][0]), key
+        assert torch.equal(outs[key][1], outs["pair"][1]) and torch.equal(outs[key][2], outs["pair"][2]), key
+
+
+@pytest.mark.parametrize("impl", ["ffma", "tc_step"])
+@pytest.mark.parametrize("N", [5, 12])
+def test_sampled_decode_general_kernels_equal_per_step_path_bitwise(impl, N):
+    """Sampled decodes on the per-step path (one warp per instance) and through the general kernels (one CTA per
+    instance) draw the same picks and write the same window logits / probabilities; every draw is the inverse CDF."""
+    K, n = 6, 200
+    m, x, lat = _high_net(n, K, N)
+    m.actor.impl = _select(impl)
+    outs = []
+    for general in (False, True):
+        m.actor.force_general = general
+        *out, differ = _sampled_decode(m.actor, x, lat, K, N)
+        assert differ > 0
+        outs.append(out)
+    assert np.array_equal(outs[0][0], outs[1][0])
+    assert torch.equal(outs[0][1], outs[1][1]) and torch.equal(outs[0][2], outs[1][2])
+
+
+def test_sampled_decode_any_hidden_size_draws_the_inverse_cdf():
+    """The any-hidden-size pointer kernel draws the inverse CDF of its own window probabilities."""
+    K, N, n = 6, 7, 130
+    m, x, lat = _high_net(n, K, N, H=128)
+    assert _sampled_decode(m.actor, x, lat, K, N)[3] > 0
+
+
 @pytest.mark.parametrize("n,K,N,with_latent", [(300, 47, 5, False), (130, 12, 10, True), (5, 3, 32, True)])
 def test_attention_windows_entry_equals_the_decode(n, K, N, with_latent):
     """gnnpn_pn_attention_windows_f32 (the decode loop's attention alone, for given decoder states) reproduces the window
