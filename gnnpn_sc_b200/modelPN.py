@@ -22,6 +22,7 @@ No CPU fallback: CUDA tensors only, and a missing extension raises.
 from __future__ import annotations
 
 import math
+from dataclasses import dataclass
 from typing import Optional, Sequence
 
 import torch
@@ -92,6 +93,21 @@ class _Last(dict):
             dict.__setitem__(self, "dec_h", dec_h)
             dict.__setitem__(self, "dec_q", dec_h)
         return dict.__getitem__(self, key)
+
+
+@dataclass
+class _Encoded:
+    """The handle ``PointerNet.encode`` returns for ``forward(..., encoded=handle)``.  ``path`` is the decode path of the
+    batch (``PointerNet._path``), or "train" when the decode already ran with the BPTT's saves (``saves``)."""
+    path: str
+    x: torch.Tensor                         # the kernel input rows
+    ws: Optional[torch.Tensor]              # tensor-core scratch (None: FFMA kernels)
+    layout: int                             # ops.ENC_ROWMAJOR | ops.ENC_BLOCKED128
+    enc_out: torch.Tensor
+    c: Optional[torch.Tensor]               # encoder cell state, where the decoder starts
+    range_flag: Optional[torch.Tensor]
+    stream: torch.cuda.Stream               # the stream the encoder was enqueued on
+    saves: Optional[dict] = None            # path == "train": ops.pn_train_forward's saves
 
 
 def _window_of(latent, K: int, N: int) -> torch.Tensor:
@@ -201,8 +217,8 @@ class PointerNet(nn.Module):
         self.glimpse = Attention(hidden_size, use_tanh=False, name=attention, use_cuda=use_cuda)
         bound = 1.0 / math.sqrt(hidden_size)
         self.decoder_start_input = nn.Parameter(torch.empty(hidden_size).uniform_(-bound, bound))
-        self._pack_key = None
-        self._packed = None
+        self._weights_key = None
+        self._weights_cache = None
         self.last = None                          # device-side results of the most recent forward
         self.impl = None                          # None -> ops.DEFAULT_IMPL ("tc"); "ffma" = strict-fp32 kernels
         self.generator = None                     # optional torch.Generator (cuda) for sample="sample"
@@ -214,41 +230,34 @@ class PointerNet(nn.Module):
         self.replay_impl = "own"                  # REINFORCE gradient: "own" = library kernels (fast configuration), "torch"
         self._train_saves = None                  # (saves, inputs, latent window) of a training-mode forward, consumed by the replay
 
-    # -- packed weights are a cache over the parameters; rebuilt when any of them changes
-    def _packed_weights(self):
+    # -- the kernels' weights are a cache over the parameters; rebuilt when any of them changes
+    def _weights(self):
+        """(encoder, decoder) weights in the form the kernels of this hidden size take: the packed LSTM blocks
+        (``ops.pack_lstm``) for H = 256, else the folded ``(w_cat, bias, bias0)`` triples of the any-hidden-size kernels
+        (``ops.anyh_fold``; the encoder's bias0 is None)."""
         ps = [self.embedding2.weight, self.embedding2.bias, self.decoder_start_input]
         for rnn in (self.encoder, self.decoder):
             ps += [rnn.weight_ih_l0, rnn.weight_hh_l0, rnn.bias_ih_l0, rnn.bias_hh_l0]
         key = tuple((p.data_ptr(), p._version) for p in ps)
-        if key != self._pack_key:
+        if key != self._weights_key:
+            make = ops.pack_lstm if self.hidden_size == 256 else ops.anyh_fold
             with torch.no_grad():
                 e, d = self.encoder, self.decoder
                 we, be = self.embedding2.weight, self.embedding2.bias
-                enc = ops.pack_lstm(e.weight_ih_l0, e.weight_hh_l0, e.bias_ih_l0, e.bias_hh_l0, we, be, None)
-                dec = ops.pack_lstm(d.weight_ih_l0, d.weight_hh_l0, d.bias_ih_l0, d.bias_hh_l0, we, be,
-                                    self.decoder_start_input)
-            self._packed, self._pack_key = (enc, dec), key
-        return self._packed
+                enc = make(e.weight_ih_l0, e.weight_hh_l0, e.bias_ih_l0, e.bias_hh_l0, we, be, None)
+                dec = make(d.weight_ih_l0, d.weight_hh_l0, d.bias_ih_l0, d.bias_hh_l0, we, be, self.decoder_start_input)
+            self._weights_cache, self._weights_key = (enc, dec), key
+        return self._weights_cache
 
-    def _anyh(self) -> bool:
-        """hidden_size other than the shipped 256: the strict-fp32 any-hidden-size kernels (``gnnpn_*_anyh_f32``)."""
-        return self.hidden_size != 256
+    def _packed_weights(self):
+        """(encoder, decoder) packed LSTM blocks of the hidden_size = 256 kernels."""
+        assert self.hidden_size == 256, "packed LSTM blocks exist for hidden_size = 256 only"
+        return self._weights()
 
-    def _folded_weights(self):
-        """((w_cat, bias, None), (w_cat, bias, bias0)) of encoder / decoder for the any-hidden-size kernels (cached)."""
-        ps = [self.embedding2.weight, self.embedding2.bias, self.decoder_start_input]
-        for rnn in (self.encoder, self.decoder):
-            ps += [rnn.weight_ih_l0, rnn.weight_hh_l0, rnn.bias_ih_l0, rnn.bias_hh_l0]
-        key = ("anyh",) + tuple((p.data_ptr(), p._version) for p in ps)
-        if key != self._pack_key:
-            with torch.no_grad():
-                e, d = self.encoder, self.decoder
-                we, be = self.embedding2.weight, self.embedding2.bias
-                enc = ops.anyh_fold(e.weight_ih_l0, e.weight_hh_l0, e.bias_ih_l0, e.bias_hh_l0, we, be, None)
-                dec = ops.anyh_fold(d.weight_ih_l0, d.weight_hh_l0, d.bias_ih_l0, d.bias_hh_l0, we, be,
-                                    self.decoder_start_input)
-            self._packed, self._pack_key = (enc, dec), key
-        return self._packed
+    @property
+    def _impl(self) -> str:
+        """``impl`` resolved: "tc" (tensor-core recurrence, the default) or "ffma" (strict-fp32 kernels)."""
+        return self.impl or ops.DEFAULT_IMPL
 
     def _kernel_inputs(self, inputs):
         """Raw rows the LSTM kernels consume: with a category embedding (modelPN.py:183-188) column 0 is replaced by
@@ -259,72 +268,97 @@ class PointerNet(nn.Module):
         B, L, C = x.shape
         return ops.embed_concat(x.view(B * L, C), self.embedding1.weight.detach()).view(B, L, -1)
 
-    def _fast_path(self, F: int) -> bool:
-        return (not self.force_general and self.embedding_size == 0 and self.n_glimpses == 0
-                and self.pointer.name == "Dot" and self.serNumber <= 32 and F <= 8 and not self._anyh())
+    def _path(self, F: int) -> str:
+        """Decode path of a batch of F kernel input columns: "anyh" for a hidden size other than the shipped 256 (the
+        strict-fp32 any-hidden-size kernels, ``gnnpn_*_anyh_f32``), "fast" for the fused / scan kernels (Dot attention,
+        no glimpses, no category embedding, at most 32 candidates per window and 8 columns), else "general"
+        (``gnnpn_pn_decode_general_f32``; ``force_general`` sends a fast configuration there too)."""
+        if self.hidden_size != 256:
+            return "anyh"
+        if (not self.force_general and self.embedding_size == 0 and self.n_glimpses == 0 and self.pointer.name == "Dot"
+                and self.serNumber <= 32 and F <= 8):
+            return "fast"
+        return "general"
+
+    def _decodes_with_saves(self, inputs, forced) -> bool:
+        """A REINFORCE forward whose decode runs with the BPTT's saves enabled (``gnnpn_pn_train_forward_tc_f32``, the
+        tensor-core column-split scan), so ``replay_action_probs`` needs no second forward."""
+        return (forced is None and self.training and torch.is_grad_enabled() and self.replay_impl != "torch"
+                and self._impl != "ffma" and inputs.is_cuda and self._path(inputs.shape[2]) == "fast")
 
     def enc_layout(self, n: int, F: int) -> int:
         """Layout of the encodings ``encode`` writes for n rows of F kernel input columns (``ops.pn_enc_layout``)."""
-        if not self._fast_path(F):
+        if self._path(F) != "fast":
             return ops.ENC_ROWMAJOR
-        has_ws = (self.impl or ops.DEFAULT_IMPL) == "tc"      # ops.pn_workspace: the tensor-core kernels' scratch
+        has_ws = self._impl == "tc"                           # ops.pn_workspace: the tensor-core kernels' scratch
         return ops.pn_enc_layout(n, self.seq_len, F, self.serCategory, self.serNumber, has_ws)
+
+    def own_enc_buffer(self, x) -> None:
+        """Gives this network a persistent ``enc_buffer`` for batches shaped like the rows ``x`` (kept across calls: a
+        4.6 GB block per network at n = 18,944 that would otherwise go through the caching allocator -- per stream, with
+        deferred frees for buffers that crossed streams -- on every call).  A caller-set larger buffer is left alone.
+        Does nothing with a category embedding, the FFMA kernels or a hidden size other than 256."""
+        n, L, F = x.shape
+        if self.embedding_size != 0 or self._impl == "ffma" or self._path(F) == "anyh":
+            return
+        need = ops.enc_out_floats(n, L, self.hidden_size, self.enc_layout(n, F))
+        if self.enc_buffer is None or self.enc_buffer.numel() < need:
+            self.enc_buffer = None                            # release the old block before asking for the larger one
+            self.enc_buffer = torch.empty(need, device=x.device, dtype=torch.float32)
 
     def encode(self, inputs):
         """The encoder half of ``forward`` (modelPN.py:183-191: embedding + encoder LSTM), enqueued on the CURRENT stream.
         Returns an opaque handle for ``forward(..., encoded=handle)``.  The two networks of the ML+2PN decode read the
         same rows and their encoders are independent, so a caller can run them concurrently on two streams (batches
         that do not fill the machine finish in the time of one encoder; gnnpn_sc_b200.pipeline does)."""
+        return self._encode(inputs)
+
+    def _encode(self, inputs, train=None):
+        """``encode``.  With ``train = (latent window, uniforms)`` the decode runs as well, free-running (greedy, or sampled
+        with the uniforms) with every per-step save of the BPTT (``gnnpn_pn_train_forward_tc_f32``): path "train".  That
+        returns None when the batch does not fit the column-split cluster scan; any other failure raises."""
         B, L, _ = inputs.shape
         assert L == self.seq_len
         if not inputs.is_cuda:
             raise RuntimeError("PointerNet.forward needs CUDA tensors: the B200 path has no CPU fallback")
-        K, N = self.serCategory, self.serNumber
+        K, N, H = self.serCategory, self.serNumber, self.hidden_size
         x = self._kernel_inputs(inputs)
-        if self._anyh():
-            if self.n_glimpses != 0 or self.pointer.name != "Dot" or N > 32:
-                raise NotImplementedError(
-                    f"hidden_size = {self.hidden_size}: the any-hidden-size kernels cover Dot attention without glimpses and "
-                    "windows of at most 32 candidates (Bahdanau / glimpses / wider windows need hidden_size = 256)")
-            (w_cat, bias, _), _ = self._folded_weights()
-            with torch.no_grad():
-                enc_out, c = ops.lstm_encode_anyh(x, w_cat, bias, self.hidden_size)
-            return {"x": x, "ws": None, "layout": ops.ENC_ROWMAJOR, "enc_out": enc_out, "c": c, "range_flag": None,
-                    "fast": False, "anyh": True, "stream": torch.cuda.current_stream(x.device)}
-        range_flag = ops.pn_check_inputs(x) if (self.check_inputs and self.impl != "ffma") else None
-        fast = self._fast_path(x.shape[2])
-        enc_w, _ = self._packed_weights()
+        path = "train" if train is not None else self._path(x.shape[2])
+        if path == "anyh" and (self.n_glimpses != 0 or self.pointer.name != "Dot" or N > 32):
+            raise NotImplementedError(
+                f"hidden_size = {H}: the any-hidden-size kernels cover Dot attention without glimpses and "
+                "windows of at most 32 candidates (Bahdanau / glimpses / wider windows need hidden_size = 256)")
+        range_flag = None
+        if self.check_inputs and path != "anyh" and self._impl != "ffma":
+            range_flag = ops.pn_check_inputs(x)
+        enc_w, dec_w = self._weights()
+        ws, layout, c, saves = None, ops.ENC_ROWMAJOR, None, None
         with torch.no_grad():
-            ws = ops.pn_workspace(B, self.hidden_size, x.device, self.impl)
-            layout = self.enc_layout(B, x.shape[2])
-            buf = None
-            if self.enc_buffer is not None:
-                # a caller-owned buffer (e.g. shared by PNLow and PNHigh at the scale-up size, where one network's
-                # encodings are ~100 GB and the caching allocator would fragment)
-                need = ops.enc_out_floats(B, L, self.hidden_size, layout)
-                if self.enc_buffer.numel() >= need:
-                    buf = self.enc_buffer.view(-1)[:need]
-                    if layout == ops.ENC_ROWMAJOR:
-                        buf = buf.view(B, L, self.hidden_size)
-            enc_out, c = ops.lstm_encode(x, enc_w, self.hidden_size, enc_out=buf, workspace=ws, layout=layout)
-        return {"x": x, "ws": ws, "layout": layout, "enc_out": enc_out, "c": c, "range_flag": range_flag, "fast": fast,
-                "stream": torch.cuda.current_stream(x.device)}
-
-    def _train_forward(self, inputs, lat, uniform, use_tanh, C):
-        """Free-running decode (greedy, or sampled with ``uniform``) on ``gnnpn_pn_train_forward_tc_f32``: the picks plus
-        every per-step save of the BPTT.  Returns (saves, encode-handle) or (None, None) when the batch does not fit the
-        column-split cluster scan; any other failure raises."""
-        x = self._kernel_inputs(inputs)
-        range_flag = ops.pn_check_inputs(x) if self.check_inputs else None
-        enc_w, dec_w = self._packed_weights()
-        K, N = self.serCategory, self.serNumber
-        with torch.no_grad():
-            sv = ops.pn_train_forward(x, enc_w, dec_w, None, K, N, latent_win=lat, alpha=float(self.alpha),
-                                      use_tanh=use_tanh, C=C, hidden=self.hidden_size, impl="tc", sample_uniform=uniform)
-        if sv is None:
-            return None, None
-        return sv, {"x": x, "ws": None, "layout": ops.ENC_ROWMAJOR, "enc_out": sv["enc_out"], "c": None,
-                    "range_flag": range_flag, "fast": True, "stream": torch.cuda.current_stream(x.device)}
+            if path == "anyh":
+                w_cat, bias, _ = enc_w
+                enc_out, c = ops.lstm_encode_anyh(x, w_cat, bias, H)
+            elif path == "train":
+                lat, uniform = train
+                saves = ops.pn_train_forward(x, enc_w, dec_w, None, K, N, latent_win=lat, alpha=float(self.alpha),
+                                             use_tanh=bool(self.pointer.use_tanh), C=float(self.pointer.C), hidden=H,
+                                             impl="tc", sample_uniform=uniform)
+                if saves is None:
+                    return None
+                enc_out = saves["enc_out"]
+            else:
+                ws = ops.pn_workspace(B, H, x.device, self._impl)
+                layout = self.enc_layout(B, x.shape[2])
+                buf = None
+                if self.enc_buffer is not None:
+                    # a caller-owned buffer (e.g. shared by PNLow and PNHigh at the scale-up size, where one network's
+                    # encodings are ~100 GB and the caching allocator would fragment)
+                    need = ops.enc_out_floats(B, L, H, layout)
+                    if self.enc_buffer.numel() >= need:
+                        buf = self.enc_buffer.view(-1)[:need]
+                        if layout == ops.ENC_ROWMAJOR:
+                            buf = buf.view(B, L, H)
+                enc_out, c = ops.lstm_encode(x, enc_w, H, enc_out=buf, workspace=ws, layout=layout)
+        return _Encoded(path, x, ws, layout, enc_out, c, range_flag, torch.cuda.current_stream(x.device), saves)
 
     def forward(self, inputs, latent, sample="sample", forced_idxs=None, encoded=None):
         """inputs [B, L, F] -> (prev_probs, prev_idxs, prev_logits), K-long each (modelPN.py:241)."""
@@ -339,42 +373,38 @@ class PointerNet(nn.Module):
             forced = None if forced_idxs is None else torch.stack([t.to(torch.int32) for t in forced_idxs])
             # sample != "greedy": multinomial draw per step (modelPN.py:227-228) as an inverse-CDF pick in the kernel
             uniform = None if sample == "greedy" else torch.rand(K, B, device=inputs.device, generator=self.generator)
-        train_sv = None
         self._train_saves = None
         if encoded is None:
-            if (forced is None and self.training and torch.is_grad_enabled() and self.replay_impl != "torch"
-                    and self.impl != "ffma" and inputs.is_cuda and self._fast_path(inputs.shape[2])):
-                # REINFORCE: the decode itself runs with the BPTT's saves enabled (tensor-core column-split scan), so
-                # replay_action_probs needs no second forward; batches outside that scan decode normally and replay
-                train_sv, encoded = self._train_forward(inputs, lat, uniform, use_tanh, C)
+            if self._decodes_with_saves(inputs, forced):
+                # None: the batch does not fit the column-split scan; it decodes normally and replays teacher-forced
+                encoded = self._encode(inputs, train=(lat, uniform))
             if encoded is None:
                 encoded = self.encode(inputs)
         else:
             cur = torch.cuda.current_stream(inputs.device)
-            if encoded["stream"] != cur:                   # encoded on a side stream: order after it, keep its buffers alive
-                cur.wait_stream(encoded["stream"])
-                for t in (encoded["x"], encoded["ws"], encoded["enc_out"], encoded["c"]):
+            if encoded.stream != cur:                      # encoded on a side stream: order after it, keep its buffers alive
+                cur.wait_stream(encoded.stream)
+                for t in (encoded.x, encoded.ws, encoded.enc_out, encoded.c):
                     if t is not None:
                         t.record_stream(cur)
-        x, ws, layout, enc_out, c = (encoded[k] for k in ("x", "ws", "layout", "enc_out", "c"))
-        range_flag, fast = encoded["range_flag"], encoded["fast"]
-        anyh = bool(encoded.get("anyh"))
-        dec_w = None if anyh else self._packed_weights()[1]
+        path, x, ws, layout, enc_out, c = encoded.path, encoded.x, encoded.ws, encoded.layout, encoded.enc_out, encoded.c
+        _, dec_w = self._weights()
         att = self.pointer.name
         with torch.no_grad():
             ptr_blk = qw = None
             replay = None
-            if train_sv is not None:
-                dec_h = dec_q = train_sv["dec_h"]
-                idx, win_logits, win_probs = train_sv["idx"], train_sv["win_logits"], train_sv["win_probs"]
-                self._train_saves = (train_sv, inputs, lat)
-            elif anyh:
-                _, (w_cat, bias, bias0) = self._folded_weights()
+            if path == "train":
+                sv = encoded.saves
+                dec_h = dec_q = sv["dec_h"]
+                idx, win_logits, win_probs = sv["idx"], sv["win_logits"], sv["win_probs"]
+                self._train_saves = (sv, inputs, lat)
+            elif path == "anyh":
+                w_cat, bias, bias0 = dec_w
                 dec_h, idx, win_logits, win_probs = ops.pn_decode_anyh(
                     x, enc_out, c, w_cat, bias, bias0, K, N, latent_win=lat, alpha=float(self.alpha), use_tanh=use_tanh, C=C,
                     forced_idx=forced, sample_uniform=uniform)
                 dec_q = dec_h
-            elif fast:
+            elif path == "fast":
                 lazy_h = layout == ops.ENC_BLOCKED128          # fused decoder: hidden states stay on chip
                 c_enc = c.clone() if lazy_h else None
                 kw = dict(latent_win=lat, alpha=float(self.alpha), attention="Dot", use_tanh=use_tanh, C=C,
@@ -398,12 +428,12 @@ class PointerNet(nn.Module):
                     x, enc_out, c, dec_w, K, N, latent_win=lat, alpha=float(self.alpha), attention=att,
                     att_params=blocks, n_glimpses=self.n_glimpses, use_tanh=use_tanh, C=C, forced_idx=forced,
                     sample_uniform=uniform, use_tc=ws is not None)
-        if range_flag is not None and not self.defer_range_check:
-            self.raise_if_out_of_range(range_flag)
+        if not self.defer_range_check:
+            self.raise_if_out_of_range(encoded.range_flag)
         idx64 = idx.long()
         self.last = _Last({"idx": idx, "win_logits": win_logits, "win_probs": win_probs, "latent_win": lat,
                            "enc_buf": enc_out, "enc_layout": layout, "enc_shape": (B, L, self.hidden_size),
-                           "range_flag": range_flag})
+                           "range_flag": encoded.range_flag})
         if layout == ops.ENC_ROWMAJOR:
             self.last["enc_out"] = enc_out
         if dec_h is not None:
@@ -415,7 +445,7 @@ class PointerNet(nn.Module):
         fed = idx if forced is None else forced.contiguous()     # the picks the visited mask follows
 
         def dense_logits():
-            if anyh:
+            if path == "anyh":
                 return ops.pn_full_logits_anyh(last["enc_out"], last["dec_h"], fed, use_tanh, C)
             if att == "Dot":
                 return ops.pn_full_logits(last["enc_out"], last["dec_q"], fed, "Dot", None, use_tanh, C)
@@ -450,7 +480,7 @@ class PointerNet(nn.Module):
         (modelPN.py:220-224) -- so the gradient equals the reference's.  Encoder via nn.LSTM (cuDNN), K cell steps;
         glimpses (when configured) attend over all positions with the cumulative visited mask as in modelPN.py:208-211."""
         saves, self._train_saves = self._train_saves, None
-        if self.replay_impl != "torch" and self._fast_path(inputs.shape[2]):
+        if self.replay_impl != "torch" and self._path(inputs.shape[2]) == "fast":
             # the library's own forward-with-saves + BPTT kernels (Dot attention, no glimpse, embedding_size = 0).  When the
             # forward of THIS batch already ran with the saves enabled (same inputs / latent objects) they are used as is
             sv = saves[0] if (saves is not None and saves[1] is inputs and saves[2] is latent_win) else None
@@ -505,7 +535,7 @@ class _ReplayFn(torch.autograd.Function):
         if sv is None:                             # teacher-forced replay of the picks (no saves from the decode itself)
             enc_w, dec_w = actor._packed_weights()
             sv = ops.pn_train_forward(x, enc_w, dec_w, idx, K, N, latent_win=latent_win, alpha=float(actor.alpha),
-                                      use_tanh=use_tanh, C=C, hidden=actor.hidden_size, impl=actor.impl)
+                                      use_tanh=use_tanh, C=C, hidden=actor.hidden_size, impl=actor._impl)
         ctx.sv, ctx.x, ctx.cfg = sv, x, (K, N, use_tanh, C)
         ctx.save_for_backward(emb_w, emb_b, start, e_ih, e_hh, d_ih, d_hh)
         return sv["win_probs"].gather(1, idx.t().long()).t().contiguous()            # [K, B]

@@ -9,11 +9,9 @@ import torch
 
 from ._lib import GnnpnError, check, get_option, lib, set_option  # noqa: F401  (re-exported)
 
-import os
-
 ACT = {None: 0, "none": 0, "relu": 1, "sigmoid": 2}
 # "tc": tcgen05 3xTF32 recurrence / node transform (default);  "ffma": strict-fp32 CUDA-core kernels
-DEFAULT_IMPL = os.environ.get("GNNPN_IMPL", "tc")
+DEFAULT_IMPL = "tc"
 TC_GEMM_MIN_ROWS = 512          # below this the tile pipeline cannot fill; the FFMA kernel is used
 ATT = {"Dot": 0, "Bahdanau": 1}
 EUNSUPPORTED = -6               # GNNPN_EUNSUPPORTED (include/gnnpn_b200.h)
@@ -64,6 +62,27 @@ def pn_workspace(n: int, hidden: int = 256, device=None, impl: Optional[str] = N
 
 def _ws(ws):
     return (None, 0) if ws is None else (ws.data_ptr(), ws.numel())
+
+
+def _decode_inputs(n: int, L: int, K: int, latent_win, forced_idx, sample_uniform):
+    """The optional inputs of a decode as the kernels take them: ``latent_win`` fp32 [n, L], ``forced_idx`` int32 [K, n],
+    ``sample_uniform`` fp32 [K, n], contiguous (None stays None)."""
+    if latent_win is not None:
+        latent_win = _f32(latent_win, "latent_win")
+        assert latent_win.shape == (n, L)
+    if forced_idx is not None:
+        forced_idx = forced_idx.to(torch.int32).contiguous()
+        assert forced_idx.shape == (K, n)
+    if sample_uniform is not None:
+        sample_uniform = _f32(sample_uniform, "sample_uniform")
+        assert sample_uniform.shape == (K, n)
+    return latent_win, forced_idx, sample_uniform
+
+
+def _decode_outputs(n: int, L: int, K: int, device):
+    """(idx int32 [K, n], win_logits [n, L], win_probs [n, L]) of a decode."""
+    return (torch.empty(K, n, device=device, dtype=torch.int32), torch.empty(n, L, device=device, dtype=torch.float32),
+            torch.empty(n, L, device=device, dtype=torch.float32))
 
 
 def pn_check_inputs(inputs: torch.Tensor) -> torch.Tensor:
@@ -131,20 +150,10 @@ def pn_decode_greedy(inputs, enc_out, c_state, packed_dec, K: int, N: int, laten
     dev = x.device
     if out is None:
         dec_h = torch.empty(n, K, H, device=dev, dtype=torch.float32) if (want_dec_h or enc_layout == ENC_ROWMAJOR) else None
-        idx = torch.empty(K, n, device=dev, dtype=torch.int32)
-        wl = torch.empty(n, L, device=dev, dtype=torch.float32)
-        wp = torch.empty(n, L, device=dev, dtype=torch.float32)
+        idx, wl, wp = _decode_outputs(n, L, K, dev)
     else:
         dec_h, idx, wl, wp = out
-    if latent_win is not None:
-        latent_win = _f32(latent_win, "latent_win")
-        assert latent_win.shape == (n, L)
-    if forced_idx is not None:
-        forced_idx = forced_idx.to(torch.int32).contiguous()
-        assert forced_idx.shape == (K, n)
-    if sample_uniform is not None:
-        sample_uniform = _f32(sample_uniform, "sample_uniform")
-        assert sample_uniform.shape == (K, n)
+    latent_win, forced_idx, sample_uniform = _decode_inputs(n, L, K, latent_win, forced_idx, sample_uniform)
     check(lib().gnnpn_pn_decode_greedy_f32(
         x.data_ptr(), enc_out.data_ptr(), c_state.data_ptr(), _ptr(latent_win), float(alpha),
         packed_dec.data_ptr(), ATT[attention], _ptr(att_params), int(bool(use_tanh)), float(C),
@@ -188,16 +197,8 @@ def pn_decode_anyh(inputs, enc_out, c_state, w_cat, bias, bias0, K: int, N: int,
     H = enc_out.shape[2]
     dev = x.device
     dec_h = torch.empty(n, K, H, device=dev, dtype=torch.float32)
-    idx = torch.empty(K, n, device=dev, dtype=torch.int32)
-    wl = torch.empty(n, L, device=dev, dtype=torch.float32)
-    wp = torch.empty(n, L, device=dev, dtype=torch.float32)
-    if latent_win is not None:
-        latent_win = _f32(latent_win, "latent_win")
-        assert latent_win.shape == (n, L)
-    if forced_idx is not None:
-        forced_idx = forced_idx.to(torch.int32).contiguous()
-    if sample_uniform is not None:
-        sample_uniform = _f32(sample_uniform, "sample_uniform")
+    idx, wl, wp = _decode_outputs(n, L, K, dev)
+    latent_win, forced_idx, sample_uniform = _decode_inputs(n, L, K, latent_win, forced_idx, sample_uniform)
     ws = _anyh_ws(n, H, F, dev)
     check(lib().gnnpn_pn_decode_anyh_f32(x.data_ptr(), enc_out.data_ptr(), c_state.data_ptr(), _ptr(latent_win), float(alpha),
                                          w_cat.data_ptr(), bias.data_ptr(), bias0.data_ptr(), int(bool(use_tanh)), float(C),
@@ -230,15 +231,13 @@ def pn_train_forward(inputs, packed_enc, packed_dec, idx, K: int, N: int, latent
     x = _f32(inputs, "inputs")
     n, L, F = x.shape
     dev, H = x.device, hidden
+    lat, idx, uni = _decode_inputs(n, L, K, latent_win, idx, sample_uniform)
     f = lambda *shape: torch.empty(*shape, device=dev, dtype=torch.float32)
+    idx_free, wl, wp = _decode_outputs(n, L, K, dev)
     sv = {"enc_out": f(n, L, H), "gates_e": f(L, n, 4 * H), "c_e": f(L, n, H), "dec_h": f(n, K, H),
-          "gates_d": f(K, n, 4 * H), "c_d": f(K, n, H), "win_logits": f(n, L), "win_probs": f(n, L),
-          "idx": None if idx is None else idx.to(torch.int32).contiguous()}
-    idx_free = torch.empty(K, n, device=dev, dtype=torch.int32)
-    lat = None if latent_win is None else _f32(latent_win, "latent_win")
+          "gates_d": f(K, n, 4 * H), "c_d": f(K, n, H), "win_logits": wl, "win_probs": wp, "idx": idx}
     if (impl or DEFAULT_IMPL) == "tc":
         ws = pn_workspace(n, H, dev, "tc")
-        uni = None if sample_uniform is None else _f32(sample_uniform, "sample_uniform")
         rc = lib().gnnpn_pn_train_forward_tc_f32(
             x.data_ptr(), packed_enc.data_ptr(), packed_dec.data_ptr(), _ptr(sv["idx"]), _ptr(uni), _ptr(lat), float(alpha),
             int(bool(use_tanh)), float(C), n, L, F, H, K, N, sv["enc_out"].data_ptr(), sv["gates_e"].data_ptr(),
@@ -301,18 +300,8 @@ def pn_decode_general(inputs, enc_out, c_state, packed_dec, K: int, N: int, late
     dec_h = torch.empty(n, K, H, device=dev, dtype=torch.float32)
     dec_q = torch.empty(n, K, H, device=dev, dtype=torch.float32) if n_glimpses > 0 else dec_h
     qw = torch.empty(n, K, H, device=dev, dtype=torch.float32) if attention == "Bahdanau" else None
-    idx = torch.empty(K, n, device=dev, dtype=torch.int32)
-    wl = torch.empty(n, L, device=dev, dtype=torch.float32)
-    wp = torch.empty(n, L, device=dev, dtype=torch.float32)
-    if latent_win is not None:
-        latent_win = _f32(latent_win, "latent_win")
-        assert latent_win.shape == (n, L)
-    if forced_idx is not None:
-        forced_idx = forced_idx.to(torch.int32).contiguous()
-        assert forced_idx.shape == (K, n)
-    if sample_uniform is not None:
-        sample_uniform = _f32(sample_uniform, "sample_uniform")
-        assert sample_uniform.shape == (K, n)
+    idx, wl, wp = _decode_outputs(n, L, K, dev)
+    latent_win, forced_idx, sample_uniform = _decode_inputs(n, L, K, latent_win, forced_idx, sample_uniform)
     nbytes = int(lib().gnnpn_pn_decode_general_workspace_bytes(n, L, K, H, ATT[attention], n_glimpses, int(use_tc)))
     ws = torch.empty(nbytes, device=dev, dtype=torch.uint8)
     check(lib().gnnpn_pn_decode_general_f32(
@@ -370,10 +359,7 @@ def pn_attention_windows(enc_out, dec_h, N: int, latent_win=None, alpha: float =
     ``[n, L, H]``, ``dec_h [n, K, H]``): ``gnnpn_pn_attention_windows_f32``.  Returns (idx int32 [K, n], win_logits, win_probs)."""
     n, L, H = enc_out.shape
     K = dec_h.shape[1]
-    if out is None:
-        out = (torch.empty(K, n, device=enc_out.device, dtype=torch.int32), torch.empty(n, L, device=enc_out.device),
-               torch.empty(n, L, device=enc_out.device))
-    idx, wl, wp = out
+    idx, wl, wp = _decode_outputs(n, L, K, enc_out.device) if out is None else out
     lat = None if latent_win is None else _f32(latent_win, "latent_win")
     check(lib().gnnpn_pn_attention_windows_f32(enc_out.data_ptr(), dec_h.data_ptr(), _ptr(lat), float(alpha), int(bool(use_tanh)),
                                                float(C), n, L, H, K, N, idx.data_ptr(), wl.data_ptr(), wp.data_ptr(), _stream()),

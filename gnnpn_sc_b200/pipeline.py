@@ -16,6 +16,53 @@ import torch
 NUM_SMS = 148          # B200
 
 
+@torch.no_grad()
+def _one_batch_behind(host_batches, upload, enqueue, device) -> Iterator[Tuple[torch.Tensor, ...]]:
+    """Runs a pipeline over host batches with every batch's results read back one batch late.
+
+    ``upload(item, slot)`` starts the host->device copy of one batch (on a copy stream) and returns a handle for
+    ``enqueue(handle)``, which orders the current stream after that copy, enqueues the batch's kernels and returns
+    (device results, device range flag | None).  The upload of batch i+1 overlaps the kernels of batch i, and the kernels
+    of batch i+1 are enqueued before the host waits for the results of batch i (asynchronous device->host copies into
+    double-buffered pinned tensors + an event), so the GPU never idles while the host prepares the next launches.  The
+    input range flag travels with the results (no mid-batch sync).  Yields the results as cpu tensors, in order."""
+    from .modelPN import PointerNet
+    main = torch.cuda.current_stream(device)
+    pinned = [None, None]
+    pending = None                                        # (pinned results, pinned flag, event, handle) of the previous batch
+
+    def finish(p):
+        results, flag, ev, _ = p
+        ev.synchronize()
+        PointerNet.raise_if_out_of_range(flag)
+        return tuple(t.clone() for t in results)          # the pinned buffers are reused two batches later
+
+    it = iter(host_batches)
+    item = next(it, None)
+    handle = None if item is None else upload(item, 0)
+    slot = 0
+    while handle is not None:
+        item = next(it, None)
+        nxt = None if item is None else upload(item, slot ^ 1)   # overlaps this batch's kernels
+        results, flag = enqueue(handle)
+        if pinned[slot] is None or any(o.shape != r.shape for o, r in zip(pinned[slot][0], results)):
+            pinned[slot] = ([torch.empty(r.shape, dtype=r.dtype, pin_memory=True) for r in results],
+                            torch.zeros(1, dtype=torch.int32, pin_memory=True))
+        out, flag_pin = pinned[slot]
+        for o, r in zip(out, results):
+            o.copy_(r, non_blocking=True)
+        if flag is not None:
+            flag_pin.copy_(flag, non_blocking=True)
+        ev = torch.cuda.Event()
+        ev.record(main)
+        if pending is not None:
+            yield finish(pending)
+        pending = (out, flag_pin if flag is not None else None, ev, handle)    # the handle keeps the batch's inputs alive
+        handle, slot = nxt, slot ^ 1
+    if pending is not None:
+        yield finish(pending)
+
+
 class GreedyLowHigh:
     def __init__(self, low, high, device=None):
         self.low, self.high = low.eval(), high.eval()
@@ -28,9 +75,8 @@ class GreedyLowHigh:
         self._stage = [None, None]            # device staging buffers (double buffer)
         self._ready = [torch.cuda.Event(), torch.cuda.Event()]
         self._consumed = [None, None]
-        self._out = [None, None]              # pinned result buffers (double buffer)
 
-    def _upload(self, slot: int, x_host: torch.Tensor) -> None:
+    def _upload(self, x_host: torch.Tensor, slot: int) -> int:
         buf = self._stage[slot]
         if buf is None or buf.shape != x_host.shape:
             buf = self._stage[slot] = torch.empty(x_host.shape, device=self.device, dtype=torch.float32)
@@ -41,68 +87,20 @@ class GreedyLowHigh:
                 self._copy.wait_event(self._consumed[slot])
             buf.copy_(x_host, non_blocking=True)
             self._ready[slot].record(self._copy)
+        return slot
 
-    @torch.no_grad()
-    def run(self, host_batches: Iterable[torch.Tensor]) -> Iterator[Tuple[torch.Tensor, torch.Tensor]]:
-        """Yields ``(idx_high int32 [K, n] (cpu), reward fp32 [n] (cpu))`` per host batch ``fp32 [n, L, F]``, in order.
-        Software-pipelined by one batch: the kernels of batch i+1 are enqueued before the host waits for the results of
-        batch i (asynchronous device->host copies into pinned buffers + an event), so the GPU never idles while the host
-        prepares the next launches; the input range flag travels with the results (no mid-batch sync)."""
-        it = iter(host_batches)
-        nxt = next(it, None)
-        slot = 0
-        if nxt is not None:
-            self._upload(slot, nxt)
+    def _enqueue(self, slot: int):
         main = torch.cuda.current_stream(self.device)
-        pending = None                                    # (pinned idx, pinned reward, pinned flag, event) of the previous batch
+        main.wait_event(self._ready[slot])
+        latent, R, idx, flag = low_high(self.low, self.high, self._stage[slot], self._side, check="defer")
+        self._consumed[slot] = torch.cuda.Event()
+        self._consumed[slot].record(main)                 # after every kernel that reads the staging buffer
+        return (torch.stack(idx).to(torch.int32), R), flag
 
-        def finish(p):
-            idx_pin, r_pin, flag_pin, ev = p
-            ev.synchronize()
-            if flag_pin is not None and int(flag_pin[0]):
-                self.low.actor.raise_if_out_of_range(flag_pin)
-            return idx_pin.clone(), r_pin.clone()         # the pinned buffers are reused two batches later
-
-        while nxt is not None:
-            cur_slot = slot
-            nxt = next(it, None)
-            if nxt is not None:                           # upload of the next batch overlaps this batch's kernels
-                self._upload(cur_slot ^ 1, nxt)
-            main.wait_event(self._ready[cur_slot])
-            x = self._stage[cur_slot]
-            latent, R, idx, flag = low_high(self.low, self.high, x, self._side, check="defer")
-            idx32 = torch.stack(idx).to(torch.int32)
-            out = self._out[cur_slot]
-            if out is None or out[0].shape != idx32.shape:
-                out = self._out[cur_slot] = (torch.empty(idx32.shape, dtype=torch.int32).pin_memory(),
-                                             torch.empty(R.shape, dtype=torch.float32).pin_memory(),
-                                             torch.zeros(1, dtype=torch.int32).pin_memory())
-            out[0].copy_(idx32, non_blocking=True)
-            out[1].copy_(R, non_blocking=True)
-            if flag is not None:
-                out[2].copy_(flag, non_blocking=True)
-            ev = torch.cuda.Event()
-            ev.record(main)
-            self._consumed[cur_slot] = ev
-            if pending is not None:
-                yield finish(pending)
-            pending = (out[0], out[1], out[2] if flag is not None else None, ev)
-            slot = cur_slot ^ 1
-        if pending is not None:
-            yield finish(pending)
-
-
-def _own_enc_buffer(actor, n: int, L: int, F: int, device):
-    """Gives ``actor`` a persistent encodings buffer for batches of n rows (kept across calls: a 4.6 GB block per network
-    at n = 18,944 that would otherwise go through the caching allocator -- per stream, with deferred frees for buffers
-    that crossed streams -- on every call).  A caller-set larger buffer is left alone."""
-    from . import ops
-    if actor.embedding_size != 0 or actor.impl == "ffma" or actor._anyh():
-        return
-    need = ops.enc_out_floats(n, L, actor.hidden_size, actor.enc_layout(n, F))
-    if actor.enc_buffer is None or actor.enc_buffer.numel() < need:
-        actor.enc_buffer = None                           # release the old block before asking for the larger one
-        actor.enc_buffer = torch.empty(need, device=device, dtype=torch.float32)
+    def run(self, host_batches: Iterable[torch.Tensor]) -> Iterator[Tuple[torch.Tensor, torch.Tensor]]:
+        """Yields ``(idx_high int32 [K, n] (cpu), reward fp32 [n] (cpu))`` per host batch ``fp32 [n, L, F]``, in order,
+        software-pipelined by one batch; the host batches upload into two reused device staging buffers."""
+        return _one_batch_behind(host_batches, self._upload, self._enqueue, self.device)
 
 
 def low_high(low, high, x, side_stream, own_buffers: bool = True, check: str = "now"):
@@ -117,7 +115,7 @@ def low_high(low, high, x, side_stream, own_buffers: bool = True, check: str = "
     main = torch.cuda.current_stream(x.device)
     if own_buffers:
         for m in (low, high):
-            _own_enc_buffer(m.actor, x.shape[0], x.shape[1], x.shape[2], x.device)
+            m.actor.own_enc_buffer(x)
     # two streams only while both encoders fit on the machine together (one CTA per 128 rows, 148 SMs).  At a full wave
     # the second encoder's CTAs would interleave with PNLow's decoder and delay it: measured 15.5 ms against 14.5 ms
     # back to back at n = 18,944 (profiles/r02_pn_batch_sweep.jsonl)
@@ -213,15 +211,13 @@ class ML2PN:
         self._side = torch.cuda.Stream(self.device)
         self._copy = torch.cuda.Stream(self.device)                       # host->device uploads of run()
 
-    @torch.no_grad()
     def run(self, host_batches):
         """The pipeline from HOST batches: every item is ``(request_batch, local_bounds, used, global_bounds)`` with pinned
         host tensors (``trainML.collate_requests(..., pin=True)``, ``constraint_arrays``).  Yields, in order,
-        ``(services int32 [n, K] (cpu), objective fp32 [n] (cpu))``.  The upload of batch i+1 runs on a copy stream under the
-        kernels of batch i, and the results of batch i are waited for only after batch i+1 has been enqueued."""
-        main = torch.cuda.current_stream(self.device)
+        ``(services int32 [n, K] (cpu), objective fp32 [n] (cpu))``, software-pipelined by one batch; every batch is
+        uploaded into fresh device tensors."""
 
-        def upload(item):
+        def upload(item, slot):
             rb, lb, us, gb = item
             with torch.cuda.stream(self._copy):
                 dev = type(rb)(x=rb.x.to(self.device, non_blocking=True), edge_index=rb.edge_index.to(self.device, non_blocking=True),
@@ -231,42 +227,16 @@ class ML2PN:
                 ev.record(self._copy)
             return dev, cons, ev
 
-        def finish(p):
-            svc_pin, obj_pin, flag_pin, ev, keep = p
-            ev.synchronize()
-            if flag_pin is not None and int(flag_pin[0]):
-                self.low.actor.raise_if_out_of_range(flag_pin)
-            return svc_pin.clone(), obj_pin.clone()
-
-        it = iter(host_batches)
-        nxt = next(it, None)
-        up = upload(nxt) if nxt is not None else None
-        pending, out, slot = None, [None, None], 0
-        while up is not None:
+        def enqueue(up):
             dev, cons, ev_up = up
-            nxt = next(it, None)
-            up = upload(nxt) if nxt is not None else None    # next upload overlaps this batch's kernels
+            main = torch.cuda.current_stream(self.device)
             main.wait_event(ev_up)
             for t in (dev.x, dev.edge_index, dev.batch, *cons):
                 t.record_stream(main)                        # allocated on the copy stream, consumed on the main one
             r = self.compose(dev, *cons, defer_check=True)
-            svc, obj, flag = r["services"].to(torch.int32), r["objective"], r["range_flag"]
-            if out[slot] is None or out[slot][0].shape != svc.shape:
-                out[slot] = (torch.empty(svc.shape, dtype=torch.int32).pin_memory(),
-                             torch.empty(obj.shape, dtype=torch.float32).pin_memory(),
-                             torch.zeros(1, dtype=torch.int32).pin_memory())
-            out[slot][0].copy_(svc, non_blocking=True)
-            out[slot][1].copy_(obj, non_blocking=True)
-            if flag is not None:
-                out[slot][2].copy_(flag, non_blocking=True)
-            ev = torch.cuda.Event()
-            ev.record(main)
-            if pending is not None:
-                yield finish(pending)
-            pending = (out[slot][0], out[slot][1], out[slot][2] if flag is not None else None, ev, (dev, cons))
-            slot ^= 1
-        if pending is not None:
-            yield finish(pending)
+            return (r["services"].to(torch.int32), r["objective"]), r["range_flag"]
+
+        return _one_batch_behind(host_batches, upload, enqueue, self.device)
 
     @torch.no_grad()
     def compose(self, request_batch, local_bounds, used, global_bounds, stage_events=None, defer_check: bool = False):
