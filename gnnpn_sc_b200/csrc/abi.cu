@@ -77,9 +77,19 @@ const char* gnnpn_error_string(int code) {
   return "unknown gnnpn error";
 }
 
+// The kernel gnnpn_gemm_f32_bias_act runs.  A misaligned A of a node-transform shape runs the FFMA kernel, which needs
+// no workspace, so the workspace size, planned for an aligned A (nullptr, lda = K), holds for every A.
+enum class GemmKernel { kFfma, kNodeTransform, kTf32 };
+static GemmKernel plan_gemm(int64_t M, int N, int K, const float* A, int64_t lda, bool has_workspace) {
+  if (!has_workspace) return GemmKernel::kFfma;
+  if (!node_transform_supported(M, N, K)) return GemmKernel::kTf32;
+  return aligned16(A) && (lda & 3) == 0 ? GemmKernel::kNodeTransform : GemmKernel::kFfma;
+}
+
 size_t gnnpn_gemm_workspace_bytes(int64_t M, int N, int K) {
   if (M < 0 || N < 1 || K < 1) return 0;
-  return node_transform_supported(M, N, K) ? node_transform_workspace_bytes(N, K) : tc_gemm_workspace_bytes(M, N, K);
+  return plan_gemm(M, N, K, nullptr, K, true) == GemmKernel::kNodeTransform ? node_transform_workspace_bytes(N, K)
+                                                                            : tc_gemm_workspace_bytes(M, N, K);
 }
 
 int gnnpn_gemm_f32_bias_act(const float* A, int64_t lda, const float* W, int64_t ldw, const float* bias,
@@ -90,18 +100,19 @@ int gnnpn_gemm_f32_bias_act(const float* A, int64_t lda, const float* W, int64_t
   GNNPN_REQUIRE((scale == nullptr) == (shift == nullptr), GNNPN_ENULL);
   GNNPN_REQUIRE(M < (1ll << 31) * 64, GNNPN_ERANGE);
   if (M == 0) return GNNPN_OK;
-  if (workspace && node_transform_supported(M, N, K) && (lda & 3) == 0 && (reinterpret_cast<uintptr_t>(A) & 15u) == 0) {
-    GNNPN_REQUIRE(workspace_bytes >= node_transform_workspace_bytes(N, K), GNNPN_EWORKSPACE);
-    return launch_node_transform(A, lda, W, ldw, bias, scale, shift, act, C, ldc, M, N, K, workspace,
-                                 (cudaStream_t)stream);
+  const cudaStream_t st = (cudaStream_t)stream;
+  switch (plan_gemm(M, N, K, A, lda, workspace != nullptr)) {
+    case GemmKernel::kNodeTransform:
+      GNNPN_REQUIRE(workspace_bytes >= node_transform_workspace_bytes(N, K), GNNPN_EWORKSPACE);
+      return launch_node_transform(A, lda, W, ldw, bias, scale, shift, act, C, ldc, M, N, K, workspace, st);
+    case GemmKernel::kTf32:
+      GNNPN_REQUIRE(workspace_bytes >= tc_gemm_workspace_bytes(M, N, K), GNNPN_EWORKSPACE);
+      GNNPN_REQUIRE(M < (1ll << 31), GNNPN_ERANGE);
+      return launch_gemm_tc(A, lda, W, ldw, bias, scale, shift, act, C, ldc, M, N, K, workspace, st);
+    case GemmKernel::kFfma:
+      break;
   }
-  if (workspace) {
-    GNNPN_REQUIRE(workspace_bytes >= tc_gemm_workspace_bytes(M, N, K), GNNPN_EWORKSPACE);
-    GNNPN_REQUIRE(M < (1ll << 31), GNNPN_ERANGE);
-    return launch_gemm_tc(A, lda, W, ldw, bias, scale, shift, act, C, ldc, M, N, K, workspace,
-                          (cudaStream_t)stream);
-  }
-  return launch_gemm_ffma(A, lda, W, ldw, bias, scale, shift, act, C, ldc, M, N, K, (cudaStream_t)stream);
+  return launch_gemm_ffma(A, lda, W, ldw, bias, scale, shift, act, C, ldc, M, N, K, st);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -30,6 +30,35 @@ constexpr int kNumSMs = 148;  // B200: 2 dies x 74 SMs
 
 __device__ __forceinline__ float sigmoid_accurate(float x) { return 1.0f / (1.0f + expf(-x)); }
 
+// The fused tail of a GIN / GCN layer, act((r + b) * s + t): bias, eval-mode BatchNorm scale / shift, activation.  The
+// FFMA and 3xTF32 GEMMs, the split-K reduction and the aggregation all end a layer with this one copy, so the layer
+// gives the same bits whichever of them runs.  It updates N consecutive columns r[0..N) of a row in place.  Each kernel
+// keeps its own loads: load(p, v) puts the N columns of the per-column array p into v; it runs only for the arrays the
+// layer has, right before their use.  The add is __fadd_rn so that no call site can contract it into an FMA.
+template <int N, class Load>
+__device__ __forceinline__ void bias_bn_act(float* r, const float* bias, const float* scale, const float* shift, int act,
+                                            Load load) {
+  float v[N], w[N];
+  if (bias) {
+    load(bias, v);
+#pragma unroll
+    for (int i = 0; i < N; ++i) r[i] = __fadd_rn(r[i], v[i]);
+  }
+  if (scale) {
+    load(scale, v);
+    load(shift, w);
+#pragma unroll
+    for (int i = 0; i < N; ++i) r[i] = fmaf(r[i], v[i], w[i]);
+  }
+  if (act == GNNPN_ACT_RELU) {
+#pragma unroll
+    for (int i = 0; i < N; ++i) r[i] = fmaxf(r[i], 0.f);
+  } else if (act == GNNPN_ACT_SIGMOID) {
+#pragma unroll
+    for (int i = 0; i < N; ++i) r[i] = sigmoid_accurate(r[i]);
+  }
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

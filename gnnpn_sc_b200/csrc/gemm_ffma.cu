@@ -1,6 +1,7 @@
 // Strict-fp32 FFMA node transform:  C = act((A . W^T + bias) * scale + shift).
-// Parity anchor and small-shape path (request graphs have <= ~100 nodes per batch, K = 28/128/256);
-// the large service-side transforms go through the tcgen05 3xTF32 kernel in gemm_tc.cu.
+// Parity anchor and small-shape path (request graphs have <= ~100 nodes per batch, K = 28/128/256), and the range
+// guard of the node transform; the large service-side transforms go through the tcgen05 kernels in node_transform.cu
+// and tc_kernels.cu (gnnpn_gemm_f32_bias_act in abi.cu picks the kernel).
 #include "common.cuh"
 #include "internal.cuh"
 
@@ -60,10 +61,7 @@ __global__ void __launch_bounds__(TPB) gemm_ffma_kernel(
       const int nn = n0 + tx * 4 + j;
       if (nn >= N) continue;
       float v = acc[i][j];
-      if (bias) v += __ldg(bias + nn);
-      if (scale) v = fmaf(v, __ldg(scale + nn), __ldg(shift + nn));
-      if (act == GNNPN_ACT_RELU) v = fmaxf(v, 0.f);
-      else if (act == GNNPN_ACT_SIGMOID) v = sigmoid_accurate(v);
+      bias_bn_act<1>(&v, bias, scale, shift, act, [&](const float* p, float* x) { x[0] = __ldg(p + nn); });
       C[m * ldc + nn] = v;
     }
   }

@@ -201,21 +201,9 @@ __device__ __forceinline__ void spmm_finish_row(const float4 (&acc)[VPL], int64_
       r.x = __fdiv_rn(r.x, inv_cnt_den); r.y = __fdiv_rn(r.y, inv_cnt_den);
       r.z = __fdiv_rn(r.z, inv_cnt_den); r.w = __fdiv_rn(r.w, inv_cnt_den);
     }
-    if (ep.bias) {
-      const float4 b = __ldg(reinterpret_cast<const float4*>(ep.bias) + c4);
-      r.x = __fadd_rn(r.x, b.x); r.y = __fadd_rn(r.y, b.y); r.z = __fadd_rn(r.z, b.z); r.w = __fadd_rn(r.w, b.w);
-    }
-    if (ep.scale) {
-      const float4 s = __ldg(reinterpret_cast<const float4*>(ep.scale) + c4);
-      const float4 t = __ldg(reinterpret_cast<const float4*>(ep.shift) + c4);
-      r.x = fmaf(r.x, s.x, t.x); r.y = fmaf(r.y, s.y, t.y); r.z = fmaf(r.z, s.z, t.z); r.w = fmaf(r.w, s.w, t.w);
-    }
-    if (ep.act == GNNPN_ACT_RELU) {
-      r.x = fmaxf(r.x, 0.f); r.y = fmaxf(r.y, 0.f); r.z = fmaxf(r.z, 0.f); r.w = fmaxf(r.w, 0.f);
-    } else if (ep.act == GNNPN_ACT_SIGMOID) {
-      r.x = sigmoid_accurate(r.x); r.y = sigmoid_accurate(r.y);
-      r.z = sigmoid_accurate(r.z); r.w = sigmoid_accurate(r.w);
-    }
+    bias_bn_act<4>(reinterpret_cast<float*>(&r), ep.bias, ep.scale, ep.shift, ep.act, [&](const float* p, float* x) {
+      *reinterpret_cast<float4*>(x) = __ldg(reinterpret_cast<const float4*>(p) + c4);
+    });
     reinterpret_cast<float4*>(y + row * ldy)[c4] = r;
   }
 }

@@ -1,6 +1,6 @@
 // Host functions that one .cu file of the library defines and another calls, declared once so that a signature change
-// is a compile error instead of a silent mismatch at link time.  (The LSTM and scan kernels keep theirs with their
-// argument structs: lstm_step.cuh, tc_lstm.cuh, tc_seq.cuh.)
+// is a compile error instead of a silent mismatch at link time, and the host launch helpers they share.  (The LSTM and
+// scan kernels keep theirs with their argument structs: lstm_step.cuh, tc_lstm.cuh, tc_seq.cuh.)
 #pragma once
 #include <cuda.h>
 #include "common.cuh"
@@ -20,7 +20,8 @@ int launch_gemm_tc(const float* A, int64_t lda, const float* W, int64_t ldw, con
                    const float* shift, int act, float* C, int64_t ldc, int64_t M, int N, int K, void* workspace,
                    cudaStream_t st);
 
-// node_transform.cu: persistent fp16-split node transform: K <= 256, N <= 256, N % 16 == 0, K % 4 == 0
+// node_transform.cu: persistent fp16-split node transform: K <= 256, N <= 256, N % 16 == 0, K % 4 == 0; A 16-byte
+// aligned with lda % 4 == 0 (plan_gemm in abi.cu)
 bool node_transform_supported(int64_t M, int N, int K);
 size_t node_transform_workspace_bytes(int N, int K);
 int launch_node_transform(const float* A, int64_t lda, const float* W, int64_t ldw, const float* bias,
@@ -44,5 +45,32 @@ EncodeTiledFn encode_fn();
 int make_map_2d(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows, bool f16 = false,
                 int box_cols = 0);
 }  // namespace tc
+
+// Launch configuration of `Kern` for a 1-D grid of 1-D clusters of `cluster` CTAs, setting the kernel's dynamic
+// shared-memory limit on first use.  `attr` receives the cluster-dimension attribute `cfg` points at.
+template <auto Kern>
+int cluster_config(cudaLaunchConfig_t* cfg, cudaLaunchAttribute* attr, unsigned grid, unsigned cluster, int threads,
+                   int smem, cudaStream_t st) {
+  static bool configured = false;
+  if (!configured) {
+    cudaError_t e = cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (e != cudaSuccess) return (int)e;
+    configured = true;
+  }
+  attr->id = cudaLaunchAttributeClusterDimension;
+  attr->val.clusterDim = {cluster, 1, 1};
+  *cfg = cudaLaunchConfig_t{dim3(grid), dim3(threads), (size_t)smem, st, attr, 1};
+  return GNNPN_OK;
+}
+template <auto Kern, class... Args>
+int launch_cluster(unsigned grid, unsigned cluster, int threads, int smem, cudaStream_t st, const Args&... args) {
+  cudaLaunchConfig_t cfg;
+  cudaLaunchAttribute attr;
+  const int rc = cluster_config<Kern>(&cfg, &attr, grid, cluster, threads, smem, st);
+  if (rc) return rc;
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, Kern, args...);
+  if (e != cudaSuccess) { cudaGetLastError(); return (int)e; }
+  return after_launch();
+}
 
 }  // namespace gnnpn

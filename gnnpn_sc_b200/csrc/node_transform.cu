@@ -21,7 +21,8 @@
 // converters check every value they touch; when one is outside the range (or not finite) they raise a flag in the
 // workspace and launch_node_transform's guarded strict-fp32 FFMA pass (gemm_ffma.cu) recomputes C -- on the device,
 // no host round trip; it returns immediately when the flag is clear (the normal case).
-// Shapes outside (K > 256, N > 256, N % 16 != 0, K % 4 != 0) use the 3xTF32 mainloop in tc_kernels.cu.
+// The converters read A in 16-byte vectors, so plan_gemm (abi.cu) runs this kernel only for a 16-byte aligned A with
+// lda % 4 == 0; shapes outside (K or N > 256, N % 16 != 0, K % 4 != 0) use the 3xTF32 mainloop in tc_kernels.cu.
 #include <cuda_fp16.h>
 #include "tc_common.cuh"
 #include "common.cuh"
@@ -228,6 +229,8 @@ node_transform_kernel(const __grid_constant__ CUtensorMap map_w_hi, const __grid
     const int e = warp - (4 + CONV_WARPS);
     const int q = warp & 3, grp = e >> 2;
     // out = act((acc / 256 + bias) * scale + shift) = act(acc * s' + t'), {s', t'} per column from p.st_tab (L1-resident).
+    // The folded form, not bias_bn_act: one FMA per value where the epilogue warps were this kernel's measured
+    // bottleneck; it rounds differently from the unfolded form of the other GEMM kernels.
     // Results leave through a per-warp [32 rows x 32 columns] shared-memory tile and a TMA store: a direct row store
     // scatters every warp instruction over 32 rows (32 L1 tag cycles each), which made the L1/LSU the busiest unit.
     const uint32_t stage = sbase + OFF_STAGE + (uint32_t)e * 4096u + (uint32_t)lane * 128u;
@@ -342,7 +345,6 @@ int launch_node_transform(const float* A, int64_t lda, const float* W, int64_t l
                           const float* scale, const float* shift, int act, float* C, int64_t ldc, int64_t M, int N,
                           int K, void* workspace, cudaStream_t st) {
   using namespace nt;
-  if ((lda & 3) || (reinterpret_cast<uintptr_t>(A) & 15u)) return GNNPN_EALIGN;
   const int Kp = round_up(K, KB);
   __half* w_hi = align_ws<__half>(workspace);
   __half* w_lo = w_hi + (size_t)N * Kp;
@@ -364,35 +366,15 @@ int launch_node_transform(const float* A, int64_t lda, const float* W, int64_t l
   CUtensorMap map_c;
   if (p.c_vec >= 4) {
     // C as a 2-D fp32 tensor {N, M}; box = 32 columns x 32 rows, 128B swizzle (one epilogue warp's tile)
-    EncodeTiledFn fn = encode_fn();
-    if (!fn) return GNNPN_EUNSUPPORTED;
-    cuuint64_t dims[2] = {(cuuint64_t)N, (cuuint64_t)M};
-    cuuint64_t strides[1] = {(cuuint64_t)ldc * 4};
-    cuuint32_t box[2] = {32, 32};
-    cuuint32_t estr[2] = {1, 1};
-    if (fn(&map_c, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)C, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-           CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-      return GNNPN_ESHAPE;
+    if ((rc = tc::make_map_2d(&map_c, C, M, N, ldc, 32, false, 32))) return rc;
     p.c_vec = 0;
   } else {
     map_c = maps[0];                                       // unused by the direct-store path
   }
-  static bool configured = false;
-  if (!configured) {
-    cudaError_t e = cudaFuncSetAttribute(node_transform_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e != cudaSuccess) return (int)e;
-    configured = true;
-  }
   const int64_t pairs = p.n_tiles < kNumSMs / 2 ? p.n_tiles : kNumSMs / 2;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(2 * pairs)); cfg.blockDim = dim3(nt::THREADS); cfg.dynamicSmemBytes = SMEM_BYTES; cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  cudaError_t le = cudaLaunchKernelEx(&cfg, node_transform_kernel, maps[0], maps[1], map_c, p);
-  if (le != cudaSuccess) { cudaGetLastError(); return (int)le; }
-  if ((rc = after_launch())) return rc;
+  rc = launch_cluster<node_transform_kernel>((unsigned)(2 * pairs), 2, nt::THREADS, SMEM_BYTES, st, maps[0], maps[1],
+                                             map_c, p);
+  if (rc) return rc;
   // inputs outside the fp16-split range (|a| >= 4095, NaN, inf): the converters raised *status and the strict-fp32
   // pass below recomputes C; with the flag clear its grid returns immediately
   return launch_gemm_ffma_if(status, A, lda, W, ldw, bias, scale, shift, act, C, ldc, M, N, K, st);

@@ -2,7 +2,8 @@
 //     A.B^T  ~=  A_hi.B_hi^T + A_lo.B_hi^T + A_hi.B_lo^T       (hi = tf32(a), lo = a - hi; the dropped
 //                                                                lo.lo term is ~2^-22 relative)
 // accumulated in fp32 in TMEM.  One mainloop, two epilogues:
-//   * node transform   C = act((A.W^T + bias)*scale + shift)                     (modelML.py linears / GCNConv X.W)
+//   * GEMM             C = act((A.W^T + bias)*scale + shift) for the shapes node_transform.cu does not take (K or N
+//                      > 256, K % 4 != 0, N % 16 != 0), split-K for the long-K weight gradients
 //   * LSTM step        gates = [h|x].P^T + bias -> c', h'  (+ fp16 split of h' for the next step's A operand); its
 //                      operands are fp16 hi/lo pairs (3xFP16, same three products), see Kind<true>
 //
@@ -235,10 +236,7 @@ struct GemmEpilogue {
         const int n = col0 + j0 + j;
         float r = v[j0 + j];
         if (j0 + j < ncols && n < p.N) {
-          if (p.bias) r += __ldg(p.bias + n);
-          if (p.scale) r = fmaf(r, __ldg(p.scale + n), __ldg(p.shift + n));
-          if (p.act == GNNPN_ACT_RELU) r = fmaxf(r, 0.f);
-          else if (p.act == GNNPN_ACT_SIGMOID) r = sigmoid_accurate(r);
+          bias_bn_act<1>(&r, p.bias, p.scale, p.shift, p.act, [&](const float* a, float* x) { x[0] = __ldg(a + n); });
         }
         r8[j] = r;
       }
@@ -375,7 +373,7 @@ int launch_mainloop(const CUtensorMap maps[4], const MainloopParams& mp, const E
 }  // namespace tc
 
 // ------------------------------------------------------------------------------------------------
-// node transform through tcgen05.  Workspace holds the tf32 splits of A and W.
+// 3xTF32 GEMM through tcgen05.  Workspace holds the tf32 splits of A and W.
 // split-K factor of the GEMM: only when the output has few row tiles and K is long (weight gradients of the REINFORCE
 // replay: [4H, T*n] x [T*n, H+16] = 8 row tiles, 940 k blocks of 32).  Two reasons: (1) 8 CTAs on 148 SMs; (2) the tensor
 // cores' fp32 accumulation loses ~0.5 ulp per MMA, so one 11,000-MMA chain is 1e-4 off where the element-wise bound of
@@ -408,10 +406,7 @@ __global__ void splitk_reduce_kernel(const float* __restrict__ part, int S, int6
   const int n = (int)(e % N);
   float r = part[e];
   for (int s = 1; s < S; ++s) r += part[(int64_t)s * M * N + e];
-  if (bias) r += __ldg(bias + n);
-  if (scale) r = fmaf(r, __ldg(scale + n), __ldg(shift + n));
-  if (act == GNNPN_ACT_RELU) r = fmaxf(r, 0.f);
-  else if (act == GNNPN_ACT_SIGMOID) r = sigmoid_accurate(r);
+  bias_bn_act<1>(&r, bias, scale, shift, act, [&](const float* p, float* x) { x[0] = __ldg(p + n); });
   C[(e / N) * ldc + n] = r;
 }
 }  // namespace

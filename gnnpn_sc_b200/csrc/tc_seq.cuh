@@ -42,33 +42,6 @@ int prof_alloc(unsigned ctas, int per_cta, cudaStream_t st, unsigned long long**
 // CTAs.  Returns how many CTAs wrote counter 0.
 unsigned prof_collect(unsigned long long* counters, unsigned ctas, int per_cta, cudaStream_t st, double sums[8]);
 
-// Launch configuration of `Kern` for a 1-D grid of 1-D clusters of `cluster` CTAs, setting the kernel's dynamic
-// shared-memory limit on first use.  `attr` receives the cluster-dimension attribute `cfg` points at.
-template <auto Kern>
-int cluster_config(cudaLaunchConfig_t* cfg, cudaLaunchAttribute* attr, unsigned grid, unsigned cluster, int threads,
-                   int smem, cudaStream_t st) {
-  static bool configured = false;
-  if (!configured) {
-    cudaError_t e = cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (e != cudaSuccess) return (int)e;
-    configured = true;
-  }
-  attr->id = cudaLaunchAttributeClusterDimension;
-  attr->val.clusterDim = {cluster, 1, 1};
-  *cfg = cudaLaunchConfig_t{dim3(grid), dim3(threads), (size_t)smem, st, attr, 1};
-  return GNNPN_OK;
-}
-template <auto Kern, class... Args>
-int launch_cluster(unsigned grid, unsigned cluster, int threads, int smem, cudaStream_t st, const Args&... args) {
-  cudaLaunchConfig_t cfg;
-  cudaLaunchAttribute attr;
-  const int rc = cluster_config<Kern>(&cfg, &attr, grid, cluster, threads, smem, st);
-  if (rc) return rc;
-  const cudaError_t e = cudaLaunchKernelEx(&cfg, Kern, args...);
-  if (e != cudaSuccess) { cudaGetLastError(); return (int)e; }
-  return after_launch();
-}
-
 // ---- the scans -----------------------------------------------------------------------------------------------------
 // cell-state scratch of the persistent kernels: 128 x kH floats per CTA (blocked layout), CTAs launched in pairs
 inline size_t tc_seq_scratch_floats(int64_t n) { return (size_t)((n + 255) / 256) * 256 * kH; }

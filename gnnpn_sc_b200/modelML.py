@@ -57,13 +57,11 @@ class _Aggregate(torch.autograd.Function):
 
 
 def _gemm_nt(a: torch.Tensor, b: torch.Tensor, bias=None) -> torch.Tensor:
-    """a [M,K] @ b[N,K]^T (+ bias) through ``gnnpn_gemm_f32_bias_act``: the tcgen05 kernels when the shape allows (rows >=
-    512, K % 4 == 0, N % 16 == 0), the strict-fp32 FFMA kernel otherwise."""
+    """a [M,K] @ b[N,K]^T (+ bias) through ``ops.gemm_bias_act``, which picks the kernel from the shape.  Training keeps
+    K % 4 != 0 or N % 16 != 0 on the strict-fp32 FFMA kernel: a tensor-core kernel there would change the gradients' bits."""
     a, b = a.contiguous(), b.contiguous()
-    M, K = a.shape
-    N = b.shape[0]
-    tc_ok = M >= ops.TC_GEMM_MIN_ROWS and K % 4 == 0 and N % 16 == 0
-    return ops.gemm_bias_act(a, b, bias=bias, impl="tc" if tc_ok else "ffma")
+    K, N = a.shape[1], b.shape[0]
+    return ops.gemm_bias_act(a, b, bias=bias, impl=None if K % 4 == 0 and N % 16 == 0 else "ffma")
 
 
 class _MatmulNT(torch.autograd.Function):

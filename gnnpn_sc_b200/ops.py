@@ -10,7 +10,7 @@ import torch
 from ._lib import GnnpnError, check, get_option, lib, set_option  # noqa: F401  (re-exported)
 
 ACT = {None: 0, "none": 0, "relu": 1, "sigmoid": 2}
-# "tc": tcgen05 3xTF32 recurrence / node transform (default);  "ffma": strict-fp32 CUDA-core kernels
+# "tc": tcgen05 recurrence / node transform (default);  "ffma": strict-fp32 CUDA-core kernels
 DEFAULT_IMPL = "tc"
 TC_GEMM_MIN_ROWS = 512          # below this the tile pipeline cannot fill; the FFMA kernel is used
 ATT = {"Dot": 0, "Bahdanau": 1}
@@ -544,7 +544,10 @@ def gemm_bias_act(a, w, bias=None, scale=None, shift=None, act=None, out=None, i
                   pad_ld: bool = False) -> torch.Tensor:
     """``act((a @ w.T + bias) * scale + shift)`` with ``w`` in nn.Linear layout [N,K].
 
-    ``impl="tc"`` (default for M >= TC_GEMM_MIN_ROWS): tcgen05 3xTF32; ``"ffma"``: strict fp32 CUDA cores.
+    ``impl="tc"`` (default for M >= TC_GEMM_MIN_ROWS): the tensor-core kernels -- the persistent 3xFP16 node transform
+    for K, N <= 256 (K % 4 == 0, N % 16 == 0, a 16-byte aligned with a.stride(0) % 4 == 0; inputs outside its fp16 range
+    are recomputed in strict fp32), 3xTF32 for other shapes, and strict fp32 for a misaligned ``a`` of a node-transform
+    shape.  ``"ffma"``: strict fp32 CUDA cores.
     ``pad_ld``: allocate the result with rows padded to a multiple of 8 floats and return the ``[:, :N]`` view (row stride
     != N): the tensor-core epilogue then writes whole 32-byte sectors -- for wide outputs whose N is not a multiple of 8."""
     a = _f32(a, "a")

@@ -409,9 +409,14 @@ GNNPN_API int gnnpn_bn_train_backward_f32(const float* y, int64_t ldy, const flo
 
 /* Node transform: C[M,N] = act( (A[M,K] . W[N,K]^T + bias[N]) * scale[N] + shift[N] )
  * (nn.Linear / GCNConv's X.W, modelML.py:77-93,98-106,164-165; bias/scale/shift may be NULL).
- * fp32 in/out.  With a workspace of gnnpn_gemm_workspace_bytes() the contraction runs on tcgen05
- * as error-compensated 3xTF32 (fp32 accumulate in TMEM); with workspace == NULL it runs as strict
- * fp32 FFMA (the small request-graph shapes). */
+ * fp32 in/out.  One of three kernels runs:
+ *   - workspace == NULL: strict fp32 FFMA (the small request-graph shapes);
+ *   - K, N <= 256, K % 4 == 0, N % 16 == 0, A 16-byte aligned and lda % 4 == 0: the persistent tcgen05 node transform,
+ *     error-compensated 3xFP16 with fp32 accumulate in TMEM; when an input is outside its fp16 range (|a| >= 4095, or
+ *     not finite) a strict fp32 FFMA pass recomputes C on the device;
+ *   - any other shape: tcgen05 error-compensated 3xTF32, split over K when the output has few row tiles and K is long.
+ * A node-transform shape whose A is misaligned runs the FFMA kernel, which needs no workspace: the size
+ * gnnpn_gemm_workspace_bytes(M, N, K) returns is enough for every A. */
 GNNPN_API size_t gnnpn_gemm_workspace_bytes(int64_t M, int N, int K);
 GNNPN_API int gnnpn_gemm_f32_bias_act(const float* A, int64_t lda, const float* W, int64_t ldw,
                             const float* bias, const float* scale, const float* shift, int act,

@@ -215,6 +215,21 @@ def test_node_transform_strided_output():
         assert torch.all(buf[:, N:] == 7.0)
 
 
+def test_node_transform_shape_with_misaligned_a_runs_ffma():
+    """A node-transform shape whose A is not 16-byte aligned (a contiguous view at a one-float storage offset) runs the
+    strict-fp32 FFMA kernel inside the workspace that gnnpn_gemm_workspace_bytes sized: the same bits as impl="ffma"."""
+    from gnnpn_sc_b200 import ops
+    g = torch.Generator().manual_seed(13)
+    M, N, K = 5014, 256, 24
+    a = torch.randn(M * K + 1, generator=g).cuda()[1:].view(M, K)
+    w, b = torch.randn(N, K, generator=g).cuda() / K ** 0.5, torch.randn(N, generator=g).cuda()
+    scale, shift = torch.rand(N, generator=g).cuda() + 0.5, torch.randn(N, generator=g).cuda()
+    assert a.is_contiguous() and a.data_ptr() % 16 != 0
+    y = ops.gemm_bias_act(a, w, bias=b, scale=scale, shift=shift, act="relu", impl="tc")
+    ref = ops.gemm_bias_act(a.clone(), w, bias=b, scale=scale, shift=shift, act="relu", impl="ffma")
+    assert torch.equal(y, ref)
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # hand-derived known-answer tests (tests/ml_kats.py) through the CUDA kernels
 # ---------------------------------------------------------------------------------------------------------------------
