@@ -39,9 +39,9 @@ SIGNATURES = {
     "gnnpn_pn_workspace_bytes": (C.c_size_t, [_i64, _i]),
     "gnnpn_pn_decode_greedy_f32": (_i, [_p, _p, _p, _p, _f, _p, _i, _p, _i, _f, _i64, _i, _i, _i, _i, _i,
                                         _p, _p, _p, _p, _p, _p, _p, C.c_size_t, _i, _p]),
-    "gnnpn_pn_train_forward_f32": (_i, [_p, _p, _p, _p, _p, _f, _i, _f, _i64, _i, _i, _i, _i, _i] + [_p] * 10),
-    "gnnpn_pn_train_forward_tc_f32": (_i, [_p, _p, _p, _p, _p, _p, _f, _i, _f, _i64, _i, _i, _i, _i, _i] + [_p] * 10 +
-                                      [C.c_size_t, _p]),
+    "gnnpn_pn_train_forward_workspace_bytes": (C.c_size_t, [_i64, _i, _i, _i, _i, _i]),
+    "gnnpn_pn_train_forward_f32": (_i, [_p, _p, _p, _p, _p, _p, _f, _i, _f, _i64, _i, _i, _i, _i, _i] + [_p] * 10 +
+                                   [C.c_size_t, _p]),
     "gnnpn_pn_train_backward_workspace_floats": (C.c_size_t, [_i64, _i, _i, _i]),
     "gnnpn_pn_train_backward_f32": (_i, [_p] * 12 + [_i, _f, _i64, _i, _i, _i, _i, _p, _p, _p, C.c_size_t, _p]),
     "gnnpn_pn_att_block_floats": (C.c_size_t, [_i]),
@@ -98,7 +98,7 @@ def lib():
                 fn = getattr(h, name)          # AttributeError if the ABI lost a symbol
                 fn.restype = res
                 fn.argtypes = args
-            if h.gnnpn_abi_version() != 8:
+            if h.gnnpn_abi_version() != 9:
                 raise GnnpnError("libgnnpn_b200.so ABI version mismatch")
             _lib = h
     return _lib

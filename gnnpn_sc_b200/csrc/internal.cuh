@@ -28,10 +28,11 @@ int launch_node_transform(const float* A, int64_t lda, const float* W, int64_t l
                           const float* scale, const float* shift, int act, float* C, int64_t ldc, int64_t M, int N,
                           int K, void* workspace, cudaStream_t st);
 
-// pn_bptt.cu: BPTT through one LSTM as one cluster scan
+// pn_bptt.cu: BPTT through one LSTM of T steps as one cluster scan (arguments: bptt::Args).  `scratch` is unused: the
+// signature is that of launch_bptt_steps (pn_train.cu), the per-step reference, so that a caller picks one of the two.
 int launch_bptt_scan(const float* gates, const float* c, const float* c_init, const float* dh_ext, int64_t dh_ld_m,
                      const float* dh_init, const float* dc_init, const float* w_hh, float* dG_T, float* dh_out,
-                     float* dc_out, int64_t n, int T, cudaStream_t st);
+                     float* dc_out, int64_t n, int T, float* scratch, cudaStream_t st);
 
 namespace tc {
 // cuTensorMapEncodeTiled through the runtime's driver entry point (no link-time libcuda dependency); nullptr when the

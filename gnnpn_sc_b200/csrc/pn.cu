@@ -193,6 +193,15 @@ __global__ void enc_unblock_kernel(const float* __restrict__ blk, int64_t n, int
   }
 }
 
+// The kernels of gnnpn_pn_train_forward_f32: of the scans only the column-split scan has the saves, whatever the
+// "persistent" option says; it runs when a workspace is given and it takes the batch (the reference trains with 128).
+// Otherwise forced picks are replayed on the strict-fp32 FFMA per-step kernels (kStep); free-running is kUnsupported.
+ScanPlan plan_train_forward(int64_t n, int F, int N, bool has_workspace, bool forced) {
+  ScanPlan p = plan_scans(n, F, N, GNNPN_ENC_ROWMAJOR, has_workspace, 3);
+  if (p.enc.kind != ScanKind::kColsplit) p.enc = p.dec = {forced ? ScanKind::kStep : ScanKind::kUnsupported, 0};
+  return p;
+}
+
 }  // namespace
 }  // namespace gnnpn
 
@@ -315,34 +324,65 @@ int gnnpn_pn_decode_greedy_f32(const float* inputs, const float* enc_out, float*
   return scan.kind == ScanKind::kPair ? tc_seq_decode(sa, scan.variant, st) : GNNPN_EUNSUPPORTED;
 }
 
-// Differentiable replay, forward half (see pn_train.cu): strict-fp32 FFMA LSTM steps + pointer steps, teacher-forced on
-// the picks `idx`, saving the post-activation gates and the cell state of every step for the backward pass.
-int gnnpn_pn_train_forward_f32(const float* inputs, const float* packed_enc, const float* packed_dec, const int32_t* idx,
-                               const float* latent_win, float alpha, int use_tanh, float C, int64_t n, int L,
-                               int in_features, int hidden, int K, int N, float* enc_out, float* gates_e, float* c_e,
-                               float* dec_h, float* gates_d, float* c_d, float* win_logits, float* win_probs,
-                               int32_t* idx_free, void* stream) {
-  GNNPN_REQUIRE(inputs && packed_enc && packed_dec && idx && enc_out && gates_e && c_e && dec_h && gates_d && c_d &&
-                    win_logits && win_probs && idx_free, GNNPN_ENULL);
+size_t gnnpn_pn_train_forward_workspace_bytes(int64_t n, int L, int in_features, int hidden, int K, int N) {
+  (void)L; (void)K;
+  if (hidden != kH || n < 0) return 0;
+  const ScanPlan plan = plan_train_forward(n, in_features, N, true, false);
+  return plan.enc.kind == ScanKind::kColsplit ? tc_lstm_workspace_bytes(n) : 0;
+}
+
+// Differentiable replay, forward half (see pn_train.cu): the decode, saving the post-activation gates and the cell state
+// of every step for the backward pass, on the kernels plan_train_forward picks.
+int gnnpn_pn_train_forward_f32(const float* inputs, const float* packed_enc, const float* packed_dec,
+                               const int32_t* forced_idx, const float* sample_uniform, const float* latent_win,
+                               float alpha, int use_tanh, float C, int64_t n, int L, int in_features, int hidden, int K,
+                               int N, float* enc_out, float* gates_e, float* c_e, float* dec_h, float* gates_d,
+                               float* c_d, float* win_logits, float* win_probs, int32_t* idx_out, void* workspace,
+                               size_t workspace_bytes, void* stream) {
+  GNNPN_REQUIRE(inputs && packed_enc && packed_dec && enc_out && gates_e && c_e && dec_h && gates_d && c_d && win_logits &&
+                    win_probs && idx_out, GNNPN_ENULL);
   GNNPN_REQUIRE(hidden == kH && in_features >= 1 && in_features <= 8 && K >= 1 && N >= 1 && N <= kMaxWindow &&
                     (int64_t)K * N == L && n >= 0 && n < (1ll << 31), GNNPN_ESHAPE);
   GNNPN_REQUIRE(aligned16(enc_out) && aligned16(dec_h) && aligned16(gates_e) && aligned16(gates_d), GNNPN_EALIGN);
+  const ScanPlan plan = plan_train_forward(n, in_features, N, workspace != nullptr, forced_idx != nullptr);
+  GNNPN_REQUIRE(plan.enc.kind != ScanKind::kUnsupported, GNNPN_EUNSUPPORTED);
+  if (plan.enc.kind == ScanKind::kColsplit) {
+    GNNPN_REQUIRE(aligned16(c_e) && aligned16(c_d), GNNPN_EALIGN);
+    GNNPN_REQUIRE(workspace_bytes >= tc_lstm_workspace_bytes(n), GNNPN_EWORKSPACE);
+  }
   if (n == 0) return GNNPN_OK;
   cudaStream_t st = (cudaStream_t)stream;
   const size_t nh = (size_t)n * kH;
-  LstmRecurrence r;
-  int rc = lstm_recurrence_init(&r, packed_enc, inputs, n, L, in_features, nullptr, nullptr, 0);
-  for (int t = 0; t < L && !rc; ++t) {
-    const LstmStepSaves sv{gates_e + t * n * kG, c_e + t * nh, t == 0 ? nullptr : c_e + (t - 1) * nh};
-    rc = lstm_encoder_step(r, t, enc_out, &sv, st);
+  if (plan.enc.kind == ScanKind::kStep) {
+    // strict-fp32 FFMA steps + pointer steps, teacher-forced on forced_idx
+    LstmRecurrence r;
+    int rc = lstm_recurrence_init(&r, packed_enc, inputs, n, L, in_features, nullptr, nullptr, 0);
+    for (int t = 0; t < L && !rc; ++t) {
+      const LstmStepSaves sv{gates_e + t * n * kG, c_e + t * nh, t == 0 ? nullptr : c_e + (t - 1) * nh};
+      rc = lstm_encoder_step(r, t, enc_out, &sv, st);
+    }
+    if (rc || (rc = lstm_recurrence_init(&r, packed_dec, inputs, n, L, in_features, nullptr, nullptr, 0))) return rc;
+    const PointerStepArgs pa = pointer_step_args(enc_out, latent_win, alpha, use_tanh, C, n, L, N, idx_out, win_logits,
+                                                 win_probs, forced_idx, nullptr);
+    return launch_pointer_steps(pa, K, dec_h, inputs, in_features, &r, st, [&](int k) {
+      const LstmStepSaves sv{gates_d + k * n * kG, c_d + k * nh, k == 0 ? c_e + (L - 1) * nh : c_d + (k - 1) * nh};
+      return lstm_decoder_step(r, k, enc_out, dec_h, K, forced_idx, &sv, st);
+    });
   }
-  if (rc || (rc = lstm_recurrence_init(&r, packed_dec, inputs, n, L, in_features, nullptr, nullptr, 0))) return rc;
-  const PointerStepArgs pa = pointer_step_args(enc_out, latent_win, alpha, use_tanh, C, n, L, N, idx_free, win_logits,
-                                               win_probs, idx, nullptr);
-  return launch_pointer_steps(pa, K, dec_h, inputs, in_features, &r, st, [&](int k) {
-    const LstmStepSaves sv{gates_d + k * n * kG, c_d + k * nh, k == 0 ? c_e + (L - 1) * nh : c_d + (k - 1) * nh};
-    return lstm_decoder_step(r, k, enc_out, dec_h, K, idx, &sv, st);
-  });
+  // column-split scans with saves, free-running or teacher-forced
+  float* scr = align_ws<float>(workspace);
+  float* c_last_e = c_e + (size_t)(L - 1) * nh;          // the encoder's final cell state = its last save
+  float* c_last_d = c_d + (size_t)(K - 1) * nh;          // decoder: in (copy of c_last_e) / out (= its last save)
+  SeqEncodeArgs ea{inputs, n, L, in_features, packed_enc, enc_out, c_last_e, scr};
+  ea.save_gates = gates_e; ea.save_c = c_e;
+  int rc = tc_colsplit_encode(ea, plan.enc.variant, st);
+  if (rc) return rc;
+  cudaError_t ce = cudaMemcpyAsync(c_last_d, c_last_e, nh * sizeof(float), cudaMemcpyDeviceToDevice, st);
+  if (ce != cudaSuccess) return (int)ce;
+  SeqDecodeArgs da{inputs, enc_out, c_last_d, latent_win, alpha, packed_dec, use_tanh, C, n, L, in_features, K, N, dec_h,
+                   idx_out, win_logits, win_probs, forced_idx, sample_uniform, scr};
+  da.save_gates = gates_d; da.save_c = c_d;
+  return tc_colsplit_decode(da, plan.dec.variant, st);
 }
 
 // The attention of the decode loop alone (modelPN.py:213-228 restricted to the windows): for given decoder states
@@ -359,41 +399,6 @@ int gnnpn_pn_attention_windows_f32(const float* enc_out, const float* dec_h, con
   const PointerStepArgs pa = pointer_step_args(enc_out, latent_win, alpha, use_tanh, C, n, L, N, idx_out, win_logits,
                                                win_probs, nullptr, nullptr);
   return launch_pointer_steps(pa, K, dec_h, nullptr, 0, nullptr, (cudaStream_t)stream, [](int) { return GNNPN_OK; });
-}
-
-int gnnpn_pn_train_forward_tc_f32(const float* inputs, const float* packed_enc, const float* packed_dec,
-                                  const int32_t* forced_idx, const float* sample_uniform, const float* latent_win,
-                                  float alpha, int use_tanh, float C, int64_t n, int L, int in_features, int hidden, int K,
-                                  int N, float* enc_out, float* gates_e, float* c_e, float* dec_h, float* gates_d,
-                                  float* c_d, float* win_logits, float* win_probs, int32_t* idx_out, void* workspace,
-                                  size_t workspace_bytes, void* stream) {
-  GNNPN_REQUIRE(inputs && packed_enc && packed_dec && enc_out && gates_e && c_e && dec_h && gates_d && c_d && win_logits &&
-                    win_probs && idx_out && workspace, GNNPN_ENULL);
-  GNNPN_REQUIRE(hidden == kH && in_features >= 1 && in_features <= 8 && K >= 1 && N >= 1 && N <= kMaxWindow &&
-                    (int64_t)K * N == L && n >= 0 && n < (1ll << 31), GNNPN_ESHAPE);
-  GNNPN_REQUIRE(aligned16(enc_out) && aligned16(dec_h) && aligned16(gates_e) && aligned16(gates_d) && aligned16(c_e) &&
-                    aligned16(c_d), GNNPN_EALIGN);
-  GNNPN_REQUIRE(workspace_bytes >= tc_lstm_workspace_bytes(n), GNNPN_EWORKSPACE);
-  // the saves exist in the column-split scan only, whatever the "persistent" option says; larger batches use the FFMA
-  // replay (training batches: the reference's is 128)
-  const ScanPlan plan = plan_scans(n, in_features, N, GNNPN_ENC_ROWMAJOR, true, 3);
-  GNNPN_REQUIRE(plan.enc.kind == ScanKind::kColsplit, GNNPN_EUNSUPPORTED);
-  if (n == 0) return GNNPN_OK;
-  cudaStream_t st = (cudaStream_t)stream;
-  float* scr = align_ws<float>(workspace);
-  const size_t nh = (size_t)n * kH;
-  float* c_last_e = c_e + (size_t)(L - 1) * nh;          // the encoder's final cell state = its last save
-  float* c_last_d = c_d + (size_t)(K - 1) * nh;          // decoder: in (copy of c_last_e) / out (= its last save)
-  SeqEncodeArgs ea{inputs, n, L, in_features, packed_enc, enc_out, c_last_e, scr};
-  ea.save_gates = gates_e; ea.save_c = c_e;
-  int rc = tc_colsplit_encode(ea, plan.enc.variant, st);
-  if (rc) return rc;
-  cudaError_t ce = cudaMemcpyAsync(c_last_d, c_last_e, nh * sizeof(float), cudaMemcpyDeviceToDevice, st);
-  if (ce != cudaSuccess) return (int)ce;
-  SeqDecodeArgs da{inputs, enc_out, c_last_d, latent_win, alpha, packed_dec, use_tanh, C, n, L, in_features, K, N, dec_h,
-                   idx_out, win_logits, win_probs, forced_idx, sample_uniform, scr};
-  da.save_gates = gates_d; da.save_c = c_d;
-  return tc_colsplit_decode(da, plan.dec.variant, st);
 }
 
 int gnnpn_pn_reward_f32(const float* inputs, const int32_t* idx, int64_t n, int L, int in_features,

@@ -211,26 +211,12 @@ __global__ void __launch_bounds__(THREADS, 1) lstm_bptt_cluster_kernel(const Arg
 // BPTT through one LSTM; see bptt::Args.  n_max_per_launch is unlimited (clusters are independent).
 int launch_bptt_scan(const float* gates, const float* c, const float* c_init, const float* dh_ext, int64_t dh_ld_m,
                      const float* dh_init, const float* dc_init, const float* w_hh, float* dG_T, float* dh_out,
-                     float* dc_out, int64_t n, int T, cudaStream_t st) {
+                     float* dc_out, int64_t n, int T, float* scratch, cudaStream_t st) {
   using namespace bptt;
+  (void)scratch;
   if (n <= 0 || T <= 0) return GNNPN_OK;
-  static bool configured = false;
-  if (!configured) {
-    cudaError_t e = cudaFuncSetAttribute(lstm_bptt_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
-    if (e != cudaSuccess) return (int)e;
-    configured = true;
-  }
-  Args a{gates, c, c_init, dh_ext, dh_ld_m, dh_init, dc_init, w_hh, dG_T, dh_out, dc_out, n, T};
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(ceil_div(n, BI) * CL)); cfg.blockDim = dim3(THREADS); cfg.dynamicSmemBytes = SMEM_BYTES;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  cudaError_t le = cudaLaunchKernelEx(&cfg, lstm_bptt_cluster_kernel, a);
-  if (le != cudaSuccess) { cudaGetLastError(); return (int)le; }
-  return after_launch();
+  const Args a{gates, c, c_init, dh_ext, dh_ld_m, dh_init, dc_init, w_hh, dG_T, dh_out, dc_out, n, T};
+  return launch_cluster<lstm_bptt_cluster_kernel>((unsigned)(ceil_div(n, BI) * CL), CL, THREADS, (int)SMEM_BYTES, st, a);
 }
 
 }  // namespace gnnpn

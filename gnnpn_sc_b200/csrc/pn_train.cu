@@ -1,11 +1,13 @@
 // REINFORCE backward of the pointer network (src/models/trainPNLow.py:77-106, trainPNHigh.py:77-112: the reference
 // back-propagates sum_k log p_k(a_k) through its K-step python graph with torch autograd).  Here the differentiable
 // replay of a sampled decode runs on this library's kernels:
-//   forward  (gnnpn_pn_train_forward_f32, pn.cu): the strict-fp32 FFMA LSTM steps + pointer steps, teacher-forced on the
-//            sampled picks, saving per step the post-activation gates and the cell state;
+//   forward  (gnnpn_pn_train_forward_f32, pn.cu): the sampled decode itself on the column-split scan, or a replay of the
+//            sampled picks on the strict-fp32 FFMA LSTM steps + pointer steps, saving per step the post-activation gates
+//            and the cell state;
 //   backward (this file): window-softmax / C*tanh / dot-attention backward in one launch, then BPTT through the decoder
-//            (K steps) and the encoder (L steps) -- per step one cell kernel (gate derivatives, written row-major for the
-//            recurrence and TRANSPOSED [4H, T*n] for the weight-gradient GEMMs) and one GEMM dh(t-1) = dG(t) . W_hh.
+//            (K steps) and the encoder (L steps): one persistent cluster scan per LSTM (pn_bptt.cu), or per step one cell
+//            kernel (gate derivatives, written row-major for the recurrence and TRANSPOSED [4H, T*n] for the
+//            weight-gradient GEMMs) and one GEMM dh(t-1) = dG(t) . W_hh (launch_bptt_steps below, option "bptt" = 0).
 // The weight gradients are then contractions over all (step, instance) pairs, dW_hh = dG^T . h(t-1), dM = dG^T . x(t)
 // (M = the folded W_ih . W_embed input block), which the caller runs through gnnpn_gemm_f32_bias_act.
 // Dot attention, no glimpses, embedding_size = 0 (what every reference call site trains).
@@ -73,6 +75,7 @@ struct CellBwdArgs {
   const float* c_prev;     // [n, H] cell state before this step, or nullptr (zeros)
   const float* dh_ext;     // external gradient w.r.t. h_t (attention), rows dh_ext_ld apart, or nullptr
   int64_t dh_ext_ld;
+  const float* dh_init;    // [n, H] gradient w.r.t. h_t from downstream (last step only), added after dh_ext, or nullptr
   const float* dh_rec;     // [SK_S][n, H] split-K partials of the gradient from step t+1 (dG(t+1) . W_hh), or nullptr
   const float* dc_next;    // [n, H] or nullptr
   float* dc_prev;          // [n, H]
@@ -102,6 +105,7 @@ __global__ void __launch_bounds__(256) lstm_cell_bwd_kernel(const CellBwdArgs a)
       const float tc = tanhf(a.c_t[m * kH + j]);
       float dh = 0.f;
       if (a.dh_ext) dh += a.dh_ext[m * a.dh_ext_ld + j];
+      if (a.dh_init) dh += a.dh_init[m * kH + j];
       if (a.dh_rec) {
         float rsum = a.dh_rec[m * kH + j];
 #pragma unroll
@@ -176,22 +180,50 @@ __global__ void __launch_bounds__(256) dh_splitk_kernel(const float* __restrict_
   }
 }
 
-// dst rows += sum of the SK_S split-K partials in src (chunk order)
-__global__ void add_rows_kernel(float* __restrict__ dst, int64_t dst_ld, const float* __restrict__ src, int64_t n) {
+// dst [n, H] = sum of the SK_S split-K partials in src (chunk order, as lstm_cell_bwd_kernel adds them)
+__global__ void sum_partials_kernel(float* __restrict__ dst, const float* __restrict__ src, int64_t n) {
   const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= n * kH) return;
   float s = src[e];
   for (int sidx = 1; sidx < SK_S; ++sidx) s += src[(int64_t)sidx * n * kH + e];
-  dst[(e / kH) * dst_ld + (e % kH)] += s;
+  dst[e] = s;
 }
 
-int dh_gemm(const float* dG, const float* w_hh, int64_t n, float* part, cudaStream_t st) {
-  dh_splitk_kernel<<<dim3(SK_S, kH / SK_COLS, (unsigned)ceil_div(n, SK_ROWS)), 256, 0, st>>>(dG, w_hh, n, part);
-  return after_launch();
-}
+// scratch of launch_bptt_steps: dG [n, 4H] + 2 x dh split-K partials [SK_S][n, H] + 2 x dc [n, H]
+size_t bptt_steps_scratch_floats(int64_t n) { return (size_t)n * kG + (2 * SK_S + 2) * (size_t)n * kH; }
 
-int cell_bwd(const CellBwdArgs& a, cudaStream_t st) {
-  lstm_cell_bwd_kernel<<<dim3((unsigned)ceil_div(a.n, 32), kH / 32), 256, 0, st>>>(a);
+// BPTT through one LSTM with two launches per step (the A/B reference of the cluster scan); the arguments of
+// launch_bptt_scan (internal.cuh) and bptt_steps_scratch_floats(n) floats of scratch.
+int launch_bptt_steps(const float* gates, const float* c, const float* c_init, const float* dh_ext, int64_t dh_ld_m,
+                      const float* dh_init, const float* dc_init, const float* w_hh, float* dG_T, float* dh_out,
+                      float* dc_out, int64_t n, int T, float* scratch, cudaStream_t st) {
+  if (n <= 0 || T <= 0) return GNNPN_OK;
+  const size_t nh = (size_t)n * kH;
+  float* dG = scratch;
+  float* dh_rec[2] = {dG + (size_t)n * kG, dG + (size_t)n * kG + SK_S * nh};
+  float* dc[2] = {dh_rec[1] + SK_S * nh, dh_rec[1] + SK_S * nh + nh};
+  int cur = 0, rc;
+  for (int t = T - 1; t >= 0; --t) {
+    CellBwdArgs a{};
+    a.gates = gates + (size_t)t * n * kG;
+    a.c_t = c + (size_t)t * nh;
+    a.c_prev = t > 0 ? c + (size_t)(t - 1) * nh : c_init;
+    a.dh_ext = dh_ext + (size_t)t * kH; a.dh_ext_ld = dh_ld_m;
+    a.dh_init = t == T - 1 ? dh_init : nullptr;
+    a.dh_rec = t == T - 1 ? nullptr : dh_rec[cur];
+    a.dc_next = t == T - 1 ? dc_init : dc[cur];
+    a.dc_prev = t == 0 && dc_out ? dc_out : dc[cur ^ 1];
+    a.dG = dG; a.dG_T = dG_T; a.t_off = (int64_t)t * n; a.Tn = (int64_t)T * n; a.n = n;
+    lstm_cell_bwd_kernel<<<dim3((unsigned)ceil_div(n, 32), kH / 32), 256, 0, st>>>(a);
+    if ((rc = after_launch())) return rc;
+    if (t > 0 || dh_out) {                                    // dh(t-1) = dG . W_hh (split-K partials)
+      dh_splitk_kernel<<<dim3(SK_S, kH / SK_COLS, (unsigned)ceil_div(n, SK_ROWS)), 256, 0, st>>>(dG, w_hh, n, dh_rec[cur ^ 1]);
+      if ((rc = after_launch())) return rc;
+    }
+    cur ^= 1;
+  }
+  if (!dh_out) return GNNPN_OK;
+  sum_partials_kernel<<<(unsigned)ceil_div(n * kH, 256), 256, 0, st>>>(dh_out, dh_rec[cur], n);
   return after_launch();
 }
 
@@ -204,8 +236,8 @@ extern "C" {
 
 size_t gnnpn_pn_train_backward_workspace_floats(int64_t n, int L, int K, int hidden) {
   if (hidden != kH || n < 0) return 0;
-  // dq [n,K,H] + d_enc [n,L,H] + dG [n,4H] + 2 x dh_rec split-K partials [16][n,H] + 2 x dc [n,H]
-  return (size_t)n * K * kH + (size_t)n * L * kH + (size_t)n * kG + (2 * 16 + 2) * (size_t)n * kH;
+  // dq [n,K,H] + d_enc [n,L,H] + the decoder's dh / dc w.r.t. its initial state [n,H] each + launch_bptt_steps' scratch
+  return (size_t)n * K * kH + (size_t)n * L * kH + 2 * (size_t)n * kH + bptt_steps_scratch_floats(n);
 }
 
 int gnnpn_pn_train_backward_f32(const float* enc_out, const float* gates_e, const float* c_e, const float* dec_h,
@@ -223,63 +255,21 @@ int gnnpn_pn_train_backward_f32(const float* enc_out, const float* gates_e, cons
   cudaStream_t st = (cudaStream_t)stream;
   float* dq = workspace;
   float* d_enc = dq + (size_t)n * K * kH;
-  float* dG = d_enc + (size_t)n * L * kH;
-  float* dh_rec[2] = {dG + (size_t)n * kG, dG + (size_t)n * kG + (size_t)SK_S * n * kH};
-  float* dc[2] = {dh_rec[1] + (size_t)SK_S * n * kH, dh_rec[1] + (size_t)SK_S * n * kH + (size_t)n * kH};
+  float* dh0 = d_enc + (size_t)n * L * kH;
+  float* dc0 = dh0 + (size_t)n * kH;
+  float* scratch = dc0 + (size_t)n * kH;
   int rc;
   attention_bwd_kernel<<<(unsigned)ceil_div(n * K, 8), 256, 0, st>>>(enc_out, dec_h, win_logits, win_probs, idx, grad_p,
                                                                     use_tanh, C, n, L, K, N, dq, d_enc);
   if ((rc = after_launch())) return rc;
-  if (options().bptt.load(std::memory_order_relaxed)) {
-    // ---- persistent cluster scans (pn_bptt.cu): one launch per LSTM instead of two per step.  The decoder started from the
-    // encoder's last state: its dh / dc w.r.t. that state enter the encoder scan at t = L-1
-    float* dh0 = dh_rec[0];
-    float* dc0 = dc[0];
-    if ((rc = launch_bptt_scan(gates_d, c_d, c_e + (size_t)(L - 1) * n * kH, dq, (int64_t)K * kH, nullptr, nullptr, w_hh_dec,
-                               dG_dec_T, dh0, dc0, n, K, st)))
-      return rc;
-    return launch_bptt_scan(gates_e, c_e, nullptr, d_enc, (int64_t)L * kH, dh0, dc0, w_hh_enc, dG_enc_T, nullptr, nullptr, n,
-                            L, st);
-  }
-  // ---- per-step kernels (option "bptt" = 0; kept as the A/B reference of the scan)
-  // ---- decoder BPTT, k = K-1 .. 0;  c_prev of step 0 is the encoder's final cell state c_e[L-1]
-  int cur = 0;
-  for (int k = K - 1; k >= 0; --k) {
-    CellBwdArgs a{};
-    a.gates = gates_d + (size_t)k * n * kG;
-    a.c_t = c_d + (size_t)k * n * kH;
-    a.c_prev = k > 0 ? c_d + (size_t)(k - 1) * n * kH : c_e + (size_t)(L - 1) * n * kH;
-    a.dh_ext = dq + (size_t)k * kH; a.dh_ext_ld = (int64_t)K * kH;
-    a.dh_rec = k == K - 1 ? nullptr : dh_rec[cur];
-    a.dc_next = k == K - 1 ? nullptr : dc[cur];
-    a.dc_prev = dc[cur ^ 1];
-    a.dG = dG; a.dG_T = dG_dec_T; a.t_off = (int64_t)k * n; a.Tn = (int64_t)K * n; a.n = n;
-    if ((rc = cell_bwd(a, st))) return rc;
-    if ((rc = dh_gemm(dG, w_hh_dec, n, dh_rec[cur ^ 1], st))) return rc;        // dh(k-1) = dG . W_hh (split-K partials)
-    cur ^= 1;
-  }
-  // the decoder started from the encoder's last state: its dh / dc enter the encoder at t = L-1
-  add_rows_kernel<<<(unsigned)ceil_div(n * kH, 256), 256, 0, st>>>(d_enc + (size_t)(L - 1) * kH, (int64_t)L * kH,
-                                                                  dh_rec[cur], n);
-  if ((rc = after_launch())) return rc;
-  // ---- encoder BPTT, t = L-1 .. 0
-  for (int t = L - 1; t >= 0; --t) {
-    CellBwdArgs a{};
-    a.gates = gates_e + (size_t)t * n * kG;
-    a.c_t = c_e + (size_t)t * n * kH;
-    a.c_prev = t > 0 ? c_e + (size_t)(t - 1) * n * kH : nullptr;
-    a.dh_ext = d_enc + (size_t)t * kH; a.dh_ext_ld = (int64_t)L * kH;
-    a.dh_rec = t == L - 1 ? nullptr : dh_rec[cur];
-    a.dc_next = dc[cur];                                   // at t = L-1: the decoder's dc w.r.t. its initial cell state
-    a.dc_prev = dc[cur ^ 1];
-    a.dG = dG; a.dG_T = dG_enc_T; a.t_off = (int64_t)t * n; a.Tn = (int64_t)L * n; a.n = n;
-    if ((rc = cell_bwd(a, st))) return rc;
-    if (t > 0) {
-      if ((rc = dh_gemm(dG, w_hh_enc, n, dh_rec[cur ^ 1], st))) return rc;
-    }
-    cur ^= 1;
-  }
-  return GNNPN_OK;
+  const auto bptt = options().bptt.load(std::memory_order_relaxed) ? launch_bptt_scan : launch_bptt_steps;
+  // the decoder started from the encoder's last state: its dh / dc w.r.t. that state enter the encoder at t = L-1
+  const float* c_last_e = c_e + (size_t)(L - 1) * n * kH;
+  if ((rc = bptt(gates_d, c_d, c_last_e, dq, (int64_t)K * kH, nullptr, nullptr, w_hh_dec, dG_dec_T, dh0, dc0, n, K,
+                 scratch, st)))
+    return rc;
+  return bptt(gates_e, c_e, nullptr, d_enc, (int64_t)L * kH, dh0, dc0, w_hh_enc, dG_enc_T, nullptr, nullptr, n, L, scratch,
+              st);
 }
 
 }  // extern "C"

@@ -16,7 +16,8 @@ enum class ScanKind {
   kStep,          // one launch per step (lstm_recurrence_*)
   kPair,          // CTA-pair scan lstm_seq_kernel<DEC, NR>
   kColsplit,      // column-split cluster scan lstm_colsplit_kernel<DEC, G>
-  kUnsupported,   // blocked encodings with a window the fused decoder cannot hold (N > 10)
+  kUnsupported,   // blocked encodings with a window the fused decoder cannot hold (N > 10); a free-running forward with
+                  // saves outside the column-split scan (pn.cu)
 };
 struct ScanChoice {
   ScanKind kind;

@@ -281,7 +281,7 @@ class PointerNet(nn.Module):
         return "general"
 
     def _decodes_with_saves(self, inputs, forced) -> bool:
-        """A REINFORCE forward whose decode runs with the BPTT's saves enabled (``gnnpn_pn_train_forward_tc_f32``, the
+        """A REINFORCE forward whose decode runs with the BPTT's saves enabled (``gnnpn_pn_train_forward_f32`` on the
         tensor-core column-split scan), so ``replay_action_probs`` needs no second forward."""
         return (forced is None and self.training and torch.is_grad_enabled() and self.replay_impl != "torch"
                 and self._impl != "ffma" and inputs.is_cuda and self._path(inputs.shape[2]) == "fast")
@@ -315,8 +315,8 @@ class PointerNet(nn.Module):
 
     def _encode(self, inputs, train=None):
         """``encode``.  With ``train = (latent window, uniforms)`` the decode runs as well, free-running (greedy, or sampled
-        with the uniforms) with every per-step save of the BPTT (``gnnpn_pn_train_forward_tc_f32``): path "train".  That
-        returns None when the batch does not fit the column-split cluster scan; any other failure raises."""
+        with the uniforms) with every per-step save of the BPTT (``gnnpn_pn_train_forward_f32`` on the column-split
+        cluster scan): path "train".  That returns None when the batch does not fit that scan; any other failure raises."""
         B, L, _ = inputs.shape
         assert L == self.seq_len
         if not inputs.is_cuda:

@@ -14,7 +14,6 @@ ACT = {None: 0, "none": 0, "relu": 1, "sigmoid": 2}
 DEFAULT_IMPL = "tc"
 TC_GEMM_MIN_ROWS = 512          # below this the tile pipeline cannot fill; the FFMA kernel is used
 ATT = {"Dot": 0, "Bahdanau": 1}
-EUNSUPPORTED = -6               # GNNPN_EUNSUPPORTED (include/gnnpn_b200.h)
 CSR_PLAIN, CSR_GCN_NORM = 0, 1
 ENC_ROWMAJOR, ENC_BLOCKED128 = 0, 1     # include/gnnpn_b200.h: layouts of the encoder -> decoder encodings buffer
 
@@ -221,43 +220,34 @@ def pn_full_logits_anyh(enc_out, dec_h, idx, use_tanh: bool = True, C: float = 1
 def pn_train_forward(inputs, packed_enc, packed_dec, idx, K: int, N: int, latent_win=None, alpha: float = 1.0,
                      use_tanh: bool = True, C: float = 10.0, hidden: int = 256, impl: Optional[str] = None,
                      sample_uniform=None):
-    """Forward half of the REINFORCE gradient: runs the network saving what the BPTT needs.  Returns the dict of saves
-    (``sv["idx"]``: the picks the steps were fed).
+    """Forward half of the REINFORCE gradient (``gnnpn_pn_train_forward_f32``): runs the network saving what the BPTT
+    needs.  Returns the dict of saves (``sv["idx"]``: the picks the steps were fed).
 
-    ``impl="tc"`` (default when the batch fits the column-split cluster scan): ``gnnpn_pn_train_forward_tc_f32`` -- the
-    tensor-core kernels of the small-batch inference path with saves enabled; with ``idx=None`` and ``sample_uniform``
-    it IS the sampled decode (no replay needed).  ``impl="ffma"`` / larger batches: ``gnnpn_pn_train_forward_f32``
-    (strict-fp32 per-step kernels, teacher-forced on ``idx``); with ``idx=None`` they return None: decode first."""
+    ``impl="tc"`` (default) runs the tensor-core column-split cluster scan when it takes the batch
+    (``gnnpn_pn_train_forward_workspace_bytes`` > 0): the kernels of the small-batch inference path with saves enabled;
+    with ``idx=None`` and ``sample_uniform`` it IS the sampled decode (no replay needed).  ``impl="ffma"`` and larger
+    batches replay the picks ``idx`` on the strict-fp32 per-step kernels; with ``idx=None`` they return None: decode
+    first."""
     x = _f32(inputs, "inputs")
     n, L, F = x.shape
     dev, H = x.device, hidden
     lat, idx, uni = _decode_inputs(n, L, K, latent_win, idx, sample_uniform)
+    ws = None
+    if (impl or DEFAULT_IMPL) == "tc":
+        nbytes = int(lib().gnnpn_pn_train_forward_workspace_bytes(n, L, F, H, K, N))
+        ws = torch.empty(nbytes, device=dev, dtype=torch.uint8) if nbytes else None
+    if idx is None and ws is None:
+        return None
     f = lambda *shape: torch.empty(*shape, device=dev, dtype=torch.float32)
     idx_free, wl, wp = _decode_outputs(n, L, K, dev)
     sv = {"enc_out": f(n, L, H), "gates_e": f(L, n, 4 * H), "c_e": f(L, n, H), "dec_h": f(n, K, H),
-          "gates_d": f(K, n, 4 * H), "c_d": f(K, n, H), "win_logits": wl, "win_probs": wp, "idx": idx}
-    if (impl or DEFAULT_IMPL) == "tc":
-        ws = pn_workspace(n, H, dev, "tc")
-        rc = lib().gnnpn_pn_train_forward_tc_f32(
-            x.data_ptr(), packed_enc.data_ptr(), packed_dec.data_ptr(), _ptr(sv["idx"]), _ptr(uni), _ptr(lat), float(alpha),
-            int(bool(use_tanh)), float(C), n, L, F, H, K, N, sv["enc_out"].data_ptr(), sv["gates_e"].data_ptr(),
-            sv["c_e"].data_ptr(), sv["dec_h"].data_ptr(), sv["gates_d"].data_ptr(), sv["c_d"].data_ptr(),
-            sv["win_logits"].data_ptr(), sv["win_probs"].data_ptr(), idx_free.data_ptr(), ws.data_ptr(), ws.numel(), _stream())
-        if rc == 0:
-            sv["impl"] = "tc"
-            if sv["idx"] is None:
-                sv["idx"] = idx_free                      # free-running (greedy / sampled): the picks ARE the fed picks
-            return sv
-        if rc != EUNSUPPORTED:
-            check(rc, "pn_train_forward_tc")
-    if idx is None:
-        return None
+          "gates_d": f(K, n, 4 * H), "c_d": f(K, n, H), "win_logits": wl, "win_probs": wp,
+          "idx": idx_free if idx is None else idx}        # free-running (greedy / sampled): the picks ARE the fed picks
     check(lib().gnnpn_pn_train_forward_f32(
-        x.data_ptr(), packed_enc.data_ptr(), packed_dec.data_ptr(), sv["idx"].data_ptr(), _ptr(lat), float(alpha),
+        x.data_ptr(), packed_enc.data_ptr(), packed_dec.data_ptr(), _ptr(idx), _ptr(uni), _ptr(lat), float(alpha),
         int(bool(use_tanh)), float(C), n, L, F, H, K, N, sv["enc_out"].data_ptr(), sv["gates_e"].data_ptr(),
         sv["c_e"].data_ptr(), sv["dec_h"].data_ptr(), sv["gates_d"].data_ptr(), sv["c_d"].data_ptr(),
-        sv["win_logits"].data_ptr(), sv["win_probs"].data_ptr(), idx_free.data_ptr(), _stream()), "pn_train_forward")
-    sv["impl"] = "ffma"
+        wl.data_ptr(), wp.data_ptr(), idx_free.data_ptr(), *_ws(ws), _stream()), "pn_train_forward")
     return sv
 
 

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define GNNPN_ABI_VERSION 8
+#define GNNPN_ABI_VERSION 9
 
 #if defined(__GNUC__)
 #define GNNPN_API __attribute__((visibility("default")))
@@ -167,32 +167,29 @@ GNNPN_API int gnnpn_pn_decode_greedy_f32(const float* inputs, const float* enc_o
  * trainPNHigh.py:77-112 back-propagate sum_k log p_k(a_k) with torch autograd through the K-step python graph).
  * Dot attention, no glimpses, embedding_size = 0, N <= 32 (what every reference call site trains).
  *
- * forward: strict-fp32 LSTM steps + pointer steps teacher-forced on the picks `idx` int32 [K, n], saving for the backward
+ * forward: the decode, free-running (greedy, or sampled with sample_uniform: modelPN.py:227-228) or teacher-forced on
+ *   forced_idx int32 [K, n], saving for the backward
  *   enc_out [n,L,H], gates_e [L,n,4H] (post-activation, columns 4j+{i,f,g,o}), c_e [L,n,H], dec_h [n,K,H],
- *   gates_d [K,n,4H], c_d [K,n,H], win_logits / win_probs [n,L]; idx_free int32 [K,n] scratch (the free choices).
+ *   gates_d [K,n,4H], c_d [K,n,H], win_logits / win_probs [n,L]; idx_out int32 [K,n] receives the free picks (the fed
+ *   picks when free-running, so a sampled decode needs no replay forward).  It runs on
+ *   - the tensor-core column-split cluster scan (tcgen05, 3xFP16 split: the kernels of the small-batch inference path
+ *     with the per-step saves enabled) when a workspace of gnnpn_pn_train_forward_workspace_bytes() bytes is given and
+ *     that size is not 0, i.e. the scan takes the batch (n <= ~3,840 on a B200; the reference trains with 128);
+ *   - else, with forced_idx, the strict-fp32 per-step kernels (FFMA LSTM steps + pointer steps; sample_uniform unused);
+ *   - else nothing: GNNPN_EUNSUPPORTED before any launch.
  * backward: grad_p fp32 [K,n] = dLoss/dp_k[idx_k] ->
  *   dG_enc_T [4H, L*n], dG_dec_T [4H, K*n]: gradients w.r.t. the gate pre-activations, TORCH gate order (row = gate*H +
  *   unit), column = step*n + instance.  The weight gradients are contractions of these with the step inputs
  *   (dW_hh = dG_T . h(t-1), d(W_ih.W_embed) = dG_T . x(t), db = row sums), run by the caller through
  *   gnnpn_gemm_f32_bias_act.  w_hh_* = weight_hh_l0 as torch stores it, fp32 [4H, H].
  *   workspace: gnnpn_pn_train_backward_workspace_floats(n, L, K, H) floats, 16-byte aligned. */
-GNNPN_API int gnnpn_pn_train_forward_f32(const float* inputs, const float* packed_enc, const float* packed_dec,
-                               const int32_t* idx, const float* latent_win, float alpha, int use_tanh, float C,
-                               int64_t n, int L, int in_features, int hidden, int K, int N, float* enc_out,
-                               float* gates_e, float* c_e, float* dec_h, float* gates_d, float* c_d,
-                               float* win_logits, float* win_probs, int32_t* idx_free, void* stream);
-/* The same forward on the tensor-core column-split cluster scan (tcgen05, 3xFP16 split: the kernels of the small-batch
- * inference path with the per-step saves enabled), for batches that scan takes (n <= ~3,840 on a B200; the reference trains
- * with 128) -- else GNNPN_EUNSUPPORTED and the caller uses gnnpn_pn_train_forward_f32.  forced_idx != NULL: teacher-forced
- * replay of those picks; forced_idx == NULL with sample_uniform: the SAMPLED decode itself (modelPN.py:227-228) saving what
- * the BPTT needs, so no replay forward is required at all; idx_out [K, n] receives the (free) picks.
- * workspace: gnnpn_pn_workspace_bytes(n, hidden). */
-GNNPN_API int gnnpn_pn_train_forward_tc_f32(const float* inputs, const float* packed_encoder, const float* packed_decoder,
-                                  const int32_t* forced_idx, const float* sample_uniform, const float* latent_win,
-                                  float alpha, int use_tanh, float C, int64_t n, int L, int in_features, int hidden,
-                                  int K, int N, float* enc_out, float* gates_e, float* c_e, float* dec_h, float* gates_d,
-                                  float* c_d, float* win_logits, float* win_probs, int32_t* idx_out, void* workspace,
-                                  size_t workspace_bytes, void* stream);
+GNNPN_API size_t gnnpn_pn_train_forward_workspace_bytes(int64_t n, int L, int in_features, int hidden, int K, int N);
+GNNPN_API int gnnpn_pn_train_forward_f32(const float* inputs, const float* packed_encoder, const float* packed_decoder,
+                               const int32_t* forced_idx, const float* sample_uniform, const float* latent_win,
+                               float alpha, int use_tanh, float C, int64_t n, int L, int in_features, int hidden,
+                               int K, int N, float* enc_out, float* gates_e, float* c_e, float* dec_h, float* gates_d,
+                               float* c_d, float* win_logits, float* win_probs, int32_t* idx_out, void* workspace,
+                               size_t workspace_bytes, void* stream);
 GNNPN_API size_t gnnpn_pn_train_backward_workspace_floats(int64_t n, int L, int K, int hidden);
 GNNPN_API int gnnpn_pn_train_backward_f32(const float* enc_out, const float* gates_e, const float* c_e, const float* dec_h,
                                 const float* gates_d, const float* c_d, const float* win_logits,

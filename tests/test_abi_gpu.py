@@ -107,8 +107,9 @@ def test_host_buffer_entry_point_equals_module_path():
     assert np.array_equal(rew, R.cpu().numpy(), equal_nan=True)
 
 
-def test_argument_errors_of_the_round_2_entry_points():
-    """Any-hidden-size kernels and the tensor-core training forward: negative codes before any launch, n = 0 is a no-op."""
+def test_argument_errors_of_the_anyh_and_training_forward_entry_points():
+    """Any-hidden-size kernels and the training forward with saves (its workspace query and the refusals of
+    gnnpn_pn_train_forward_f32): negative codes before any launch, n = 0 is a no-op."""
     from gnnpn_sc_b200 import _lib
     lib = _lib.lib()
     st = torch.cuda.current_stream().cuda_stream
@@ -142,16 +143,19 @@ def test_argument_errors_of_the_round_2_entry_points():
     assert dec_call(K=5) == -2                                   # K * N != L
     assert lib.gnnpn_pn_full_logits_anyh_f32(enc.data_ptr(), dec_h.data_ptr(), None, 1, C.c_float(10.0), n, L, Hh, K,
                                              wl.data_ptr(), st) == -1
-    # tensor-core training forward: a batch beyond the column-split scan is refused (the caller replays on the FFMA kernels)
+    # training forward: a batch beyond the column-split scan needs no workspace (the FFMA kernels replay forced picks);
+    # a free-running call outside that scan, or without a workspace, is refused
     big = 8192
+    assert lib.gnnpn_pn_train_forward_workspace_bytes(big, L, F, H, K, N) == 0
+    wsb = lib.gnnpn_pn_train_forward_workspace_bytes(64, L, F, H, K, N)
+    assert wsb > 0
     dummy = torch.empty(16, device="cuda")
-    wsb = lib.gnnpn_pn_workspace_bytes(big, H)
     p = dummy.data_ptr()
-    rc = lib.gnnpn_pn_train_forward_tc_f32(p, enc_p.data_ptr(), dec_p.data_ptr(), None, None, None, C.c_float(1.0), 1,
-                                           C.c_float(10.0), big, L, F, H, K, N, p, p, p, p, p, p, p, p, p, p, wsb, st)
-    assert rc == -6                                              # GNNPN_EUNSUPPORTED
-    rc = lib.gnnpn_pn_train_forward_tc_f32(p, enc_p.data_ptr(), dec_p.data_ptr(), None, None, None, C.c_float(1.0), 1,
-                                           C.c_float(10.0), 64, L, F, 128, K, N, p, p, p, p, p, p, p, p, p, p, wsb, st)
-    assert rc == -2                                              # hidden_size != 256
+    fwd = lambda n_, H_, ws_, wsb_: lib.gnnpn_pn_train_forward_f32(
+        p, enc_p.data_ptr(), dec_p.data_ptr(), None, None, None, C.c_float(1.0), 1, C.c_float(10.0), n_, L, F, H_, K, N,
+        p, p, p, p, p, p, p, p, p, ws_, wsb_, st)
+    assert fwd(big, H, p, lib.gnnpn_pn_workspace_bytes(big, H)) == -6    # GNNPN_EUNSUPPORTED
+    assert fwd(64, H, None, 0) == -6
+    assert fwd(64, 128, p, wsb) == -2                                     # hidden_size != 256
     assert lib.gnnpn_launch_count() == before
     torch.cuda.synchronize()
