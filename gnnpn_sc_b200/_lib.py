@@ -62,6 +62,8 @@ SIGNATURES = {
     "gnnpn_woa_fitness_f64": (_i, [_p, _i64, _p, _i64, _p, _p, _i64, _i, _p, _p, _p, _p]),
     "gnnpn_ml2pn_score_f64": (_i, [_p, _i64, _p, _i64, _p, _p, _i64, _i, _p, _p, _p, _p]),
     "gnnpn_woa_search_f64": (_i, [_p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _i, _i, _i, _p]),
+    "gnnpn_woa_prepare_f64": (_i, [_p, _p, _p, _i64, _i] + [_p] * 7 + [_i64, _i, C.c_double] + [_p] * 12),
+    "gnnpn_woa_prepare_rows": (_i64, [_i64, _i64, _i]),
     "gnnpn_pn_greedy_low_high_host": (_i, [_p, _i64, _i, _i, _i, _i, _i, _p, _p, _i, _f, _f, _p, _p, _p]),
     "gnnpn_select_candidates_f32": (_i, [_p, _i64, _p, _p, _i, _p, _p, _p, _i64, _i, _i, _i, _p, _p, _p]),
     "gnnpn_csr_build_workspace_bytes": (_i, [_i64, _i64, _i, C.POINTER(C.c_size_t)]),
@@ -98,7 +100,7 @@ def lib():
                 fn = getattr(h, name)          # AttributeError if the ABI lost a symbol
                 fn.restype = res
                 fn.argtypes = args
-            if h.gnnpn_abi_version() != 9:
+            if h.gnnpn_abi_version() != 10:
                 raise GnnpnError("libgnnpn_b200.so ABI version mismatch")
             _lib = h
     return _lib

@@ -425,6 +425,54 @@ def woa_search(qos, base, size, klen, bounds, pops, best_fit, best_ref, best_vec
                                      _stream()), "woa_search")
 
 
+# gnnpn_woa_prepare_f64's flags: the host path raises for all but 8, which is input the device stage does not take
+WOA_FLAGS = {1: "more seed rows than candidate lists", 2: "the reduct front replaces past the end of its list",
+             4: "no feasible candidate for any task",
+             8: "unsupported request: a category requested twice or outside the catalogue",
+             16: "fewer seed rows than candidate lists (a requested category with a neutral pick)"}
+
+
+def woa_prepare(svc_raw, svc_round, cat_ptr, req_cat, n_req, local_bounds, global_bounds, seed_rows, seed_ids, seeds,
+                popSize: int, reduct: float):
+    """Candidate lists, seed, initial population and best state of the ESWOA stage on the device
+    (``gnnpn_woa_prepare_f64``), in the layouts :func:`woa_search` takes.  Returns a dict of CUDA tensors: qos, ids,
+    base, size, klen, list_cat, pops, best_fit, best_ref, best_vec, flags (see the header)."""
+    n, K = req_cat.shape
+    for x, dt in ((svc_raw, torch.float64), (svc_round, torch.float64), (cat_ptr, torch.int32), (req_cat, torch.int32),
+                  (n_req, torch.int32), (local_bounds, torch.float64), (global_bounds, torch.float64),
+                  (seed_rows, torch.float32), (seed_ids, torch.int32), (seeds, torch.int64)):
+        if not (x.is_cuda and x.is_contiguous() and x.dtype == dt):
+            raise GnnpnError("woa_prepare needs contiguous CUDA tensors of the declared dtypes (no CPU fallback)")
+    assert cat_ptr.numel() == K + 1 and local_bounds.shape == (n, K, 4) and seed_rows.shape == (n, K, 4)
+    S = svc_raw.shape[0]
+    dev = req_cat.device
+    rows = int(lib().gnnpn_woa_prepare_rows(n, S, K))
+    i32 = lambda *s: torch.empty(s, device=dev, dtype=torch.int32)
+    o = {"qos": torch.empty(rows, 4, device=dev, dtype=torch.float64), "ids": i32(rows), "base": i32(n, K),
+           "size": i32(n, K), "klen": i32(n), "list_cat": i32(n, K), "pops": i32(n, popSize, K),
+           "best_fit": torch.empty(n, device=dev, dtype=torch.float64), "best_ref": i32(n), "best_vec": i32(n, K),
+           "flags": i32(n)}
+    check(lib().gnnpn_woa_prepare_f64(
+        svc_raw.data_ptr(), svc_round.data_ptr(), cat_ptr.data_ptr(), S, K, req_cat.data_ptr(), n_req.data_ptr(),
+        local_bounds.data_ptr(), global_bounds.data_ptr(), seed_rows.data_ptr(), seed_ids.data_ptr(), seeds.data_ptr(),
+        n, popSize, float(reduct), o["qos"].data_ptr(), o["ids"].data_ptr(), o["base"].data_ptr(), o["size"].data_ptr(),
+        o["klen"].data_ptr(), o["list_cat"].data_ptr(), o["pops"].data_ptr(), o["best_fit"].data_ptr(),
+        o["best_ref"].data_ptr(), o["best_vec"].data_ptr(), o["flags"].data_ptr(), _stream()), "woa_prepare")
+    return o
+
+
+def raise_if_woa_flagged(flags) -> None:
+    """Raises naming every instance whose ``woa_prepare`` flags are set: the host path raises for them too, or (flag 8)
+    the request is one the device stage does not take."""
+    import numpy as np
+    f = np.asarray(flags.cpu() if torch.is_tensor(flags) else flags)
+    bad = np.nonzero(f)[0]
+    if len(bad):
+        why = "; ".join(f"{msg}: instances {np.nonzero(f & bit)[0].tolist()}" for bit, msg in WOA_FLAGS.items()
+                        if (f & bit).any())
+        raise GnnpnError(f"ESWOA stage cannot run {len(bad)} instance(s) of the batch: {why}")
+
+
 def select_candidates(scores, svc_qos, cat_ptr, local_bounds, used, global_bounds, N: int, with_category: bool = False,
                       return_picked: bool = False, max_category_size: Optional[int] = None):
     """ML scores ``[n, S]`` -> PN input rows ``[n, K*N, 8(+1)]`` (see ``gnnpn_select_candidates_f32``).

@@ -45,7 +45,8 @@ def _one_batch_behind(host_batches, upload, enqueue, device) -> Iterator[Tuple[t
         item = next(it, None)
         nxt = None if item is None else upload(item, slot ^ 1)   # overlaps this batch's kernels
         results, flag = enqueue(handle)
-        if pinned[slot] is None or any(o.shape != r.shape for o, r in zip(pinned[slot][0], results)):
+        if (pinned[slot] is None or len(pinned[slot][0]) != len(results)
+                or any(o.shape != r.shape for o, r in zip(pinned[slot][0], results))):
             pinned[slot] = ([torch.empty(r.shape, dtype=r.dtype, pin_memory=True) for r in results],
                             torch.zeros(1, dtype=torch.int32, pin_memory=True))
         out, flag_pin = pinned[slot]
@@ -179,8 +180,39 @@ def constraint_arrays(nodefeatures, K: int):
     return local, used, glob
 
 
-def service_arrays(serviceFeature):
-    """``svc_qos [S,4]`` (last four attributes, loadData.py:40) and ``cat_ptr [K+1]`` in category-key order."""
+def woa_arrays(nodefeatures, K: int):
+    """What the ESWOA stage reads from the raw ``nodefeatures.data`` rows, parsed as ``loadDataOther`` parses them
+    (gnnpn_sc_b200/WOA.py:541-554), all float64 as the JSON values are:
+    ``req_cat int32 [n, K]`` = the category of every task node after the first node, in request-node order (-1 padded),
+    ``n_req int32 [n]``, ``local f64 [n, K, 4]`` = (lo_cost, hi_cost, lo_q, hi_q) of the last task node of each category,
+    ``glob f64 [n, 4]`` = (lo1, hi1, lo2, hi2) of the last global-constraint node.  A global node after the first node, or
+    more tasks than categories (a category requested twice), raise ``ValueError``: ``loadDataOther`` accepts them, but the
+    device stage does not take them (``gnnpn_woa_prepare_f64`` flag 8)."""
+    import numpy as np
+    n = len(nodefeatures)
+    req = np.full((n, K), -1, dtype=np.int32)
+    n_req = np.zeros(n, dtype=np.int32)
+    local = np.zeros((n, K, 4), dtype=np.float64)
+    glob = np.zeros((n, 4), dtype=np.float64)
+    for b, inst in enumerate(nodefeatures):
+        kinds = [node[:-6].index(1) for node in inst]
+        for node, kind in zip(inst, kinds):
+            vals = node[-5:-3] + node[-2:]
+            if node[0] == 1:
+                glob[b] = vals
+            else:
+                local[b, kind - 1] = vals
+        tasks = [kind - 1 for kind in kinds[1:]]
+        if min(tasks, default=0) < 0 or len(tasks) > K:
+            raise ValueError(f"instance {b}: a global node after the first node, or more tasks than categories")
+        req[b, :len(tasks)] = tasks
+        n_req[b] = len(tasks)
+    return req, n_req, local, glob
+
+
+def service_arrays(serviceFeature, dtype=None):
+    """``svc_qos [S,4]`` (last four attributes, loadData.py:40; float32, or ``dtype``) and ``cat_ptr [K+1]`` in
+    category-key order."""
     import numpy as np
     keys = sorted(int(k) for k in serviceFeature.keys())
     qos, ptr = [], [0]
@@ -188,16 +220,20 @@ def service_arrays(serviceFeature):
         rows = np.asarray(serviceFeature[str(k)], dtype=np.float64)[:, -4:]
         qos.append(rows)
         ptr.append(ptr[-1] + len(rows))
-    return np.concatenate(qos).astype(np.float32), np.asarray(ptr, dtype=np.int32)
+    return np.concatenate(qos).astype(dtype or np.float32), np.asarray(ptr, dtype=np.int32)
 
 
 class ML2PN:
     """The whole inference pipeline of ``main.py <ds> ML+2PN`` on one device, batched over request instances:
     ``Net`` scores (modelML.py:131-176) -> per-category top-N feasible candidates (loadDataPN, loadData.py:99-150,
     ranking order) -> PNLow greedy -> PNHigh greedy (trainPNHigh.py:131-144) -> objective (ML2PN.py:6-12).
-    Nothing leaves the GPU between the stages."""
+    Nothing leaves the GPU between the stages.
 
-    def __init__(self, net, low, high, service_sample, serviceFeature, device=None):
+    ``woa``: optional ESWOA fine-tuning stage after the objective (the third stage of ``ML2PNWOATest``,
+    gnnpn_sc_b200/WOA.py), a dict with ``popSize``, ``MAX_Iter`` and ``reduct`` (0, or 0.55 in the Normal ini
+    sections).  PNHigh's picks seed it, as ``WOA.start`` seeds it from ``allActions`` files."""
+
+    def __init__(self, net, low, high, service_sample, serviceFeature, device=None, woa=None):
         self.device = torch.device(device if device is not None else "cuda")
         self.net, self.low, self.high = net.eval(), low.eval(), high.eval()
         self.high.actor.check_inputs = False      # same rows as PNLow
@@ -210,40 +246,73 @@ class ML2PN:
         self.service_enc = net.service_encodings(service_sample)          # static: encoded once
         self._side = torch.cuda.Stream(self.device)
         self._copy = torch.cuda.Stream(self.device)                       # host->device uploads of run()
+        self.woa = None
+        if woa is not None:
+            import numpy as np
+            from .WOA import _round5
+            self.woa = {"popSize": int(woa["popSize"]), "MAX_Iter": int(woa["MAX_Iter"]),
+                        "reduct": float(woa.get("reduct") or 0.0)}
+            if not (1 <= self.woa["popSize"] <= 128 and self.K <= 128 and self.woa["MAX_Iter"] >= 0):
+                raise ValueError("the device ESWOA stage takes popSize <= 128 and at most 128 categories")
+            raw, _ = service_arrays(serviceFeature, dtype=np.float64)
+            self.svc_raw = torch.from_numpy(raw).to(self.device)                       # the JSON values
+            self.svc_round = torch.from_numpy(_round5(raw)).to(self.device)            # Python round(x, 5)
 
     def run(self, host_batches):
         """The pipeline from HOST batches: every item is ``(request_batch, local_bounds, used, global_bounds)`` with pinned
-        host tensors (``trainML.collate_requests(..., pin=True)``, ``constraint_arrays``).  Yields, in order,
-        ``(services int32 [n, K] (cpu), objective fp32 [n] (cpu))``, software-pipelined by one batch; every batch is
-        uploaded into fresh device tensors."""
+        host tensors (``trainML.collate_requests(..., pin=True)``, ``constraint_arrays``), optionally followed by the
+        ESWOA stage's ``(req_cat, n_req, local, glob, instance_ids)`` (``woa_arrays``; see ``compose``).  Yields, in order,
+        ``(services int32 [n, K] (cpu), objective fp32 [n] (cpu))`` -- plus ``woa_fitness``, ``woa_services`` and
+        ``woa_traj`` for items with the ESWOA arrays -- software-pipelined by one batch; every batch is uploaded into fresh
+        device tensors.  Instances the ESWOA stage cannot run raise after their batch."""
+        from . import ops
 
         def upload(item, slot):
-            rb, lb, us, gb = item
+            rb, lb, us, gb = item[:4]
             with torch.cuda.stream(self._copy):
                 dev = type(rb)(x=rb.x.to(self.device, non_blocking=True), edge_index=rb.edge_index.to(self.device, non_blocking=True),
                                batch=rb.batch.to(self.device, non_blocking=True), num_graphs=rb.num_graphs)
                 cons = [t.to(self.device, non_blocking=True) for t in (lb, us, gb)]
+                woa = [t.to(self.device, non_blocking=True) for t in item[4]] if len(item) > 4 else None
                 ev = torch.cuda.Event()
                 ev.record(self._copy)
-            return dev, cons, ev
+            return dev, cons, woa, ev
 
         def enqueue(up):
-            dev, cons, ev_up = up
+            dev, cons, woa, ev_up = up
             main = torch.cuda.current_stream(self.device)
             main.wait_event(ev_up)
-            for t in (dev.x, dev.edge_index, dev.batch, *cons):
+            for t in (dev.x, dev.edge_index, dev.batch, *cons, *(woa or ())):
                 t.record_stream(main)                        # allocated on the copy stream, consumed on the main one
-            r = self.compose(dev, *cons, defer_check=True)
-            return (r["services"].to(torch.int32), r["objective"]), r["range_flag"]
+            r = self.compose(dev, *cons, defer_check=True, woa=woa)
+            res = (r["services"].to(torch.int32), r["objective"])
+            if woa is not None:
+                res += (r["woa_fitness"], r["woa_services"], r["woa_traj"], r["woa_flags"])
+            return res, r["range_flag"]
 
-        return _one_batch_behind(host_batches, upload, enqueue, self.device)
+        def checked(results):
+            for res in results:
+                if len(res) > 2:
+                    ops.raise_if_woa_flagged(res[-1])
+                    res = res[:-1]
+                yield res
+
+        return checked(_one_batch_behind(host_batches, upload, enqueue, self.device))
 
     @torch.no_grad()
-    def compose(self, request_batch, local_bounds, used, global_bounds, stage_events=None, defer_check: bool = False):
+    def compose(self, request_batch, local_bounds, used, global_bounds, stage_events=None, defer_check: bool = False,
+                woa=None):
         """``request_batch``: collated request graphs (x, edge_index, batch) on the device; constraint tensors from
         ``constraint_arrays``.  Returns scores, PN rows, picked service ids per row, PNHigh picks and objective.
         ``stage_events``: optional list that receives five CUDA events recorded on the current stream at the stage
-        boundaries (start, scores, candidates, PNLow+PNHigh, objective) -- bench.py's per-stage times."""
+        boundaries (start, scores, candidates, PNLow+PNHigh, objective) -- bench.py's per-stage times -- and two more with
+        ``woa`` (ESWOA prepare, search).
+        ``woa``: ``(req_cat, n_req, local, glob, instance_ids int64 [n])`` on the device (``woa_arrays`` + the instances'
+        numbers, the Philox seed of each, as ``WOA.start`` seeds instance k with k) runs the ESWOA stage after the
+        objective (the constructor's ``woa`` configuration) and adds ``woa_fitness f64 [n]``, ``woa_services int32 [n, K]``
+        (best composition as service ids by category, -1 where unused), ``woa_traj f64 [n, MAX_Iter]`` and
+        ``woa_flags int32 [n]``; instances the stage cannot run raise here, or with ``defer_check`` are left to the
+        caller in ``woa_flags`` (``ops.raise_if_woa_flagged``)."""
         from . import ops
 
         def mark():
@@ -268,5 +337,37 @@ class ML2PN:
         mark()
         viol, obj, _ = ops.pn_reward(rows, idx.to(torch.int32))
         mark()
-        return {"scores": scores, "rows": rows, "picked": picked, "idx_high": idx, "services": services,
-                "reward": R, "violations": viol, "objective": obj, "range_flag": flag}
+        out = {"scores": scores, "rows": rows, "picked": picked, "idx_high": idx, "services": services,
+               "reward": R, "violations": viol, "objective": obj, "range_flag": flag}
+        if woa is not None:
+            out.update(self._woa(rows, idx, services, woa, mark))
+            if not defer_check:
+                ops.raise_if_woa_flagged(out["woa_flags"])
+        return out
+
+    def _woa(self, rows, idx, services, woa, mark):
+        """ESWOA stage: candidate lists + seed + initial population on the device, then the unchanged search."""
+        from . import ops
+        if self.woa is None:
+            raise ValueError("ML2PN was built without a woa configuration")
+        req_cat, n_req, local, glob, inst = woa
+        B, K, P = rows.shape[0], self.K, self.woa["popSize"]
+        pick = idx.t().long()                                                                  # [B, K]
+        seed_rows = rows.gather(1, pick[..., None].expand(B, K, rows.shape[2]))[..., :4].contiguous()
+        seeds = (inst.to(torch.int64) & 0x7FFFFFFFFFFFFFFF).contiguous()
+        p = ops.woa_prepare(self.svc_raw, self.svc_round, self.cat_ptr, req_cat.to(torch.int32).contiguous(),
+                            n_req.to(torch.int32).contiguous(), local.contiguous(), glob.contiguous(), seed_rows,
+                            services.to(torch.int32).contiguous(), seeds, P, self.woa["reduct"])
+        mark()
+        traj = torch.empty(B, self.woa["MAX_Iter"], device=rows.device, dtype=torch.float64)
+        ops.woa_search(p["qos"], p["base"], p["size"], p["klen"], glob.contiguous(), p["pops"], p["best_fit"],
+                       p["best_ref"], p["best_vec"], seeds, traj)
+        mark()
+        # best position (local index per list, Python semantics) -> service ids by category
+        valid = torch.arange(K, device=rows.device)[None, :] < p["klen"][:, None]
+        pos = p["best_vec"].long().remainder(p["size"].long())
+        svc = torch.where(valid, p["ids"][p["base"].long() + pos], -1)
+        by_cat = torch.full((B, K + 1), -1, device=rows.device, dtype=torch.int32)
+        by_cat.scatter_(1, torch.where(valid, p["list_cat"].long(), K), svc)
+        return {"woa_fitness": p["best_fit"], "woa_services": by_cat[:, :K].contiguous(), "woa_traj": traj,
+                "woa_flags": p["flags"]}

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define GNNPN_ABI_VERSION 9
+#define GNNPN_ABI_VERSION 10
 
 #if defined(__GNUC__)
 #define GNNPN_API __attribute__((visibility("default")))
@@ -312,6 +312,48 @@ GNNPN_API int gnnpn_woa_search_f64(const double* qos, int64_t n_services, const 
                          const int32_t* klen, const double* bounds, int32_t* pops, double* best_fit,
                          int32_t* best_ref, int32_t* best_vec, const uint64_t* seeds, double* traj,
                          int64_t n_instances, int popSize, int Kmax, int iters, void* stream);
+
+/* Everything gnnpn_woa_search_f64 needs, built on the device from request data and PNHigh's picks, exactly as the host
+ * path computes it before its search (gnnpn_sc_b200/WOA.py: loadDataOther + _add_s, the seed rows of WOA.start,
+ * _Instance.__init__, _Engine._init_population).  One CTA per instance.
+ *  Candidate lists: for every requested task in request order, the services of its category in position order with
+ *   lo_cost <= q2 <= hi_cost and lo_q <= q3 <= hi_q (float64); with reduct != 0 thinned by _add_s's running front
+ *   (sentinel entry, index bookkeeping and protected seed rows included).  Empty lists are dropped.
+ *  Seed: the picks whose float64 sum ((q0+q1)+q2)+q3 is not 3, in category order.  With at least one, every candidate row
+ *   is rounded to 5 decimals (svc_round), the seed rows too, six of them patched as the reference does; seed row l is
+ *   looked up in list l (first exact match) or appended to it.  Without one the rows stay unrounded and the best
+ *   fitness starts at 3.
+ *  Population: pops[i, k] = floor(u * size_before_append[k]), u = Philox(seeds[I]) at (slot k, whale i, phase 3, t 0);
+ *   the seed is evaluated first, then whales 0..popSize-1, accepted on a strictly lower fitness.
+ *   svc_raw, svc_round f64 [n_services, 4]  q0..q3 of every service (JSON values) and the same rounded (Python round)
+ *   cat_ptr      int32 [K+1]          service range of every category (category-major service ids), K <= 128
+ *   req_cat      int32 [I, K]         category (0-based) of task j in request-node order, j < n_req[I]
+ *   n_req        int32 [I]
+ *   local_bounds f64 [I, K, 4]        lo_cost, hi_cost, lo_q, hi_q of the task node of every category
+ *   global_bounds f64 [I, 4]          lo1, hi1, lo2, hi2 of the global-constraint node (the search's `bounds`)
+ *   seed_rows    fp32 [I, K, 4]       q0..q3 of PNHigh's pick per category; seed_ids int32 [I, K] its service id
+ *   seeds        uint64 [I]           Philox key of every instance (the search takes the same array)
+ *   reduct       0 (plain lists) or the _add_s threshold (0.55 in the Normal ini sections)
+ * Outputs, in the layouts gnnpn_woa_search_f64 takes with Kmax = K:
+ *   qos f64 [gnnpn_woa_prepare_rows(I, n_services, K), 4] candidate rows; ids int32 [same rows] service id of every row
+ *   base, size int32 [I, K] (size after the seed appends; base 0, size 1 past klen); klen int32 [I] number of lists
+ *   list_cat int32 [I, K]             category of every list (-1 past klen)
+ *   pops int32 [I, popSize, K], best_fit f64 [I], best_ref int32 [I], best_vec int32 [I, K]
+ *   flags int32 [I]   0, or why the instance has no result.  The host path raises for bits 0, 1, 2 and 4: bit 0 more
+ *                     seed rows than lists, bit 1 the front replaces past the end of its list, bit 2 no list at all,
+ *                     bit 4 fewer seed rows than lists.  Bit 3 is input this entry does not take: a category outside
+ *                     [0, K), or one requested twice (the host path gives both tasks the same list object, so a seed
+ *                     row appended to one shows in the other).  Results of a flagged instance are meaningless.
+ * popSize <= 128; GNNPN_ESHAPE when I * (n_services + K) reaches 2^31 rows. */
+GNNPN_API int gnnpn_woa_prepare_f64(const double* svc_raw, const double* svc_round, const int32_t* cat_ptr,
+                          int64_t n_services, int K, const int32_t* req_cat, const int32_t* n_req,
+                          const double* local_bounds, const double* global_bounds, const float* seed_rows,
+                          const int32_t* seed_ids, const uint64_t* seeds, int64_t n_instances, int popSize,
+                          double reduct, double* qos, int32_t* ids, int32_t* base, int32_t* size, int32_t* klen,
+                          int32_t* list_cat, int32_t* pops, double* best_fit, int32_t* best_ref, int32_t* best_vec,
+                          int32_t* flags, void* stream);
+/* rows of gnnpn_woa_prepare_f64's qos / ids: n_instances * (n_services + K), one slot of (size + 1) rows per category */
+GNNPN_API int64_t gnnpn_woa_prepare_rows(int64_t n_instances, int64_t n_services, int K);
 
 /* Host-buffer convenience for non-torch callers: PNLow greedy -> latent -> PNHigh greedy
  * (src/models/trainPNHigh.py:131-144) on pageable or pinned HOST memory; allocates its own device
