@@ -18,9 +18,17 @@ namespace {
 
 // numpy's pairwise summation for contiguous float64 (numpy/core/src/umath/loops_utils.h.src, pairwise_sum_DOUBLE):
 // < 8 elements sequential, <= 128 elements eight running accumulators, above that a recursive split at
-// n/2 rounded down to a multiple of 8.  The recursion is unrolled at compile time (depth 3 covers n <= 512: the
-// pieces are <= 263, <= 135, <= 71 elements), so the kernel needs no device call stack.
-__device__ __forceinline__ double numpy_block_sum_f64(const double* a, int n) {
+// n/2 rounded down to a multiple of 8.  The recursion is unrolled at compile time for n <= NMAX (a piece of n holds
+// at most ceil(n/2) + 7 elements; NMAX = 512 unrolls three levels), so the kernel needs no device call stack.
+template <int NMAX>
+__device__ __forceinline__ double numpy_sum_f64(const double* a, int n) {
+  if constexpr (NMAX > 128) {
+    if (n > 128) {
+      int n2 = n / 2;
+      n2 -= n2 % 8;
+      return __dadd_rn(numpy_sum_f64<NMAX / 2 + 8>(a, n2), numpy_sum_f64<NMAX / 2 + 8>(a + n2, n - n2));
+    }
+  }
   if (n < 8) {
     double res = 0.0;
     for (int i = 0; i < n; ++i) res = __dadd_rn(res, a[i]);
@@ -36,19 +44,46 @@ __device__ __forceinline__ double numpy_block_sum_f64(const double* a, int n) {
   for (; i < n; ++i) res = __dadd_rn(res, a[i]);
   return res;
 }
-template <int DEPTH>
-__device__ __forceinline__ double numpy_sum_f64(const double* a, int n) {
-  if (n <= 128) return numpy_block_sum_f64(a, n);
-  int n2 = n / 2;
-  n2 -= n2 % 8;
-  return __dadd_rn(numpy_sum_f64<DEPTH - 1>(a, n2), numpy_sum_f64<DEPTH - 1>(a + n2, n - n2));
+
+// The fitness (violate + objFunc) of one composition of K <= KMAX picks, b the (lo, hi) pair of each product; violate
+// and objFunc also go to viol_out and obj_out when given.  Pick k is row pos[k] of qos (kRow), or entry pos[k] of the
+// task's list of size[k] rows from row base[k], a negative pos[k] counting from its end as in Python (kLocal).
+// MEAN_ALL: `np.average(qos[0])` over all K picks (src/ML2PN.py:6-12, `ML2PN.calc`) instead of sum / #{q0 > 0}.
+enum class WoaPick { kRow, kLocal };
+template <int KMAX, bool MEAN_ALL, WoaPick PICK>
+__device__ __forceinline__ double woa_fitness(const double* __restrict__ qos, const int32_t* pos, const int32_t* base,
+                                              const int32_t* size, int K, const double* b, int* viol_out = nullptr,
+                                              double* obj_out = nullptr) {
+  double q0s[KMAX];
+  double prod[2] = {1.0, 1.0};
+  double min_q1 = INFINITY;
+  int used = 0;
+  for (int k = 0; k < K; ++k) {
+    int r = pos[k];
+    if constexpr (PICK == WoaPick::kLocal) {
+      int v = r % size[k];
+      if (v < 0) v += size[k];
+      r = base[k] + v;
+    }
+    const double* row = qos + (int64_t)r * 4;
+    q0s[k] = row[0];
+    used += row[0] > 0.0;
+    min_q1 = fmin(min_q1, row[1]);
+    prod[0] = k == 0 ? row[2] : __dmul_rn(prod[0], row[2]);
+    prod[1] = k == 0 ? row[3] : __dmul_rn(prod[1], row[3]);
+  }
+  int viol = 0;
+  for (int i = 0; i < 2; ++i) viol += (prod[i] < b[2 * i] || prod[i] > b[2 * i + 1]) ? 1 : 0;
+  double obj = __ddiv_rn(numpy_sum_f64<KMAX>(q0s, K), (double)(MEAN_ALL ? K : used));
+  obj = __dadd_rn(obj, 1.0);
+  obj = __dsub_rn(obj, min_q1);
+  obj = __ddiv_rn(obj, 2.0);
+  if (viol_out) *viol_out = viol;
+  if (obj_out) *obj_out = obj;
+  return __dadd_rn((double)viol, obj);
 }
-template <>
-__device__ __forceinline__ double numpy_sum_f64<0>(const double* a, int n) { return numpy_block_sum_f64(a, n); }
 
-constexpr int kMaxTasksWoa = 512;
-
-// MEAN_ALL: `np.average(qos[0])` over all K picks (src/ML2PN.py:6-12, `ML2PN.calc`) instead of sum / #{q0 > 0}
+constexpr int kMaxTasksWoa = 512;     // picks per composition in woa_fitness_kernel
 template <bool MEAN_ALL>
 __global__ void woa_fitness_kernel(const double* __restrict__ qos, const int32_t* __restrict__ idx, int64_t idx_ld,
                                    const int32_t* __restrict__ klen, const double* __restrict__ bounds, int64_t P,
@@ -57,29 +92,10 @@ __global__ void woa_fitness_kernel(const double* __restrict__ qos, const int32_t
   const int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (p >= P) return;
   const int K = klen ? klen[p] : Kmax;
-  double q0s[kMaxTasksWoa];
-  double prod[2] = {1.0, 1.0};
-  double min_q1 = INFINITY;
-  int used = 0;
-  for (int k = 0; k < K; ++k) {
-    const double* row = qos + (int64_t)idx[p * idx_ld + k] * 4;
-    const double q0 = row[0], q1 = row[1];
-    q0s[k] = q0;
-    used += q0 > 0.0;
-    min_q1 = fmin(min_q1, q1);
-    prod[0] = k == 0 ? row[2] : __dmul_rn(prod[0], row[2]);
-    prod[1] = k == 0 ? row[3] : __dmul_rn(prod[1], row[3]);
-  }
-  const double* b = bounds + p * 4;
-  int viol = 0;
-  for (int i = 0; i < 2; ++i) viol += (prod[i] < b[2 * i] || prod[i] > b[2 * i + 1]) ? 1 : 0;
-  double obj = __ddiv_rn(numpy_sum_f64<3>(q0s, K), (double)(MEAN_ALL ? K : used));
-  obj = __dadd_rn(obj, 1.0);
-  obj = __dsub_rn(obj, min_q1);
-  obj = __ddiv_rn(obj, 2.0);
-  if (viol_out) viol_out[p] = viol;
-  if (obj_out) obj_out[p] = obj;
-  if (fit_out) fit_out[p] = __dadd_rn((double)viol, obj);
+  const double fit = woa_fitness<kMaxTasksWoa, MEAN_ALL, WoaPick::kRow>(
+      qos, idx + p * idx_ld, nullptr, nullptr, K, bounds + p * 4, viol_out ? viol_out + p : nullptr,
+      obj_out ? obj_out + p : nullptr);
+  if (fit_out) fit_out[p] = fit;
 }
 
 
@@ -104,6 +120,8 @@ __device__ __forceinline__ double philox_uniform(uint64_t seed, uint32_t slot, u
   for (int r = 0; r < 10; ++r) philox_round(c, k);
   return __dmul_rn(__dadd_rn(__dmul_rn((double)(c[0] >> 5), 67108864.0), (double)(c[1] >> 6)), 1.0 / 9007199254740992.0);
 }
+// one of n choices drawn with u = philox_uniform(...): floor(u * n) (host mirror: PhiloxRng.randint, .choice and .block)
+__device__ __forceinline__ int philox_index(double u, int n) { return (int)__dmul_rn(u, (double)n); }
 
 constexpr int kWoaMaxK = 128;       // tasks per instance in the device search
 constexpr int kWoaThreads = 128;    // whales per instance (popSize <= 128)
@@ -123,30 +141,12 @@ struct WoaSearchArgs {
   int P, Kmax, iters;
 };
 
-// fitness of one position given as local indices (Python semantics for negatives) into the instance's candidate lists
-__device__ double woa_fitness_local(const double* __restrict__ qos, const int32_t* pos, const int32_t* base, const int32_t* size,
-                                    int K, const double* b) {
-  double q0s[kWoaMaxK];
-  double prod[2] = {1.0, 1.0};
-  double min_q1 = INFINITY;
-  int used = 0;
-  for (int k = 0; k < K; ++k) {
-    int v = pos[k] % size[k];
-    if (v < 0) v += size[k];
-    const double* row = qos + (int64_t)(base[k] + v) * 4;
-    q0s[k] = row[0];
-    used += row[0] > 0.0;
-    min_q1 = fmin(min_q1, row[1]);
-    prod[0] = k == 0 ? row[2] : __dmul_rn(prod[0], row[2]);
-    prod[1] = k == 0 ? row[3] : __dmul_rn(prod[1], row[3]);
-  }
-  int viol = 0;
-  for (int i = 0; i < 2; ++i) viol += (prod[i] < b[2 * i] || prod[i] > b[2 * i + 1]) ? 1 : 0;
-  double obj = __ddiv_rn(numpy_sum_f64<0>(q0s, K), (double)used);
-  obj = __dadd_rn(obj, 1.0);
-  obj = __dsub_rn(obj, min_q1);
-  obj = __ddiv_rn(obj, 2.0);
-  return __dadd_rn((double)viol, obj);
+// one thread's best-so-far scan in whale order (`if bestFitness > fitness`, WOA.py:78-81,119-122); 1 if the best moved
+__device__ __forceinline__ int scan_best(const double* fit, int P, double& best, int& ref) {
+  int changed = 0;
+  for (int w = 0; w < P; ++w)
+    if (best > fit[w]) { best = fit[w]; ref = w; changed = 1; }
+  return changed;
 }
 
 __global__ void __launch_bounds__(kWoaThreads) woa_search_kernel(const WoaSearchArgs a) {
@@ -178,18 +178,17 @@ __global__ void __launch_bounds__(kWoaThreads) woa_search_kernel(const WoaSearch
     const double prob = __dmul_rn(0.2, __dsub_rn(1.0, __ddiv_rn((double)t, (double)a.iters)));
     double f = INFINITY;
     if (whale && philox_uniform(seed, 0, i, 0, t) < prob) {
-      const int rand = (int)(philox_uniform(seed, 1, i, 0, t) * K);
-      const int randi = (int)(philox_uniform(seed, 2, i, 0, t) * sz[rand]);
+      const int rand = philox_index(philox_uniform(seed, 1, i, 0, t), K);
+      const int randi = philox_index(philox_uniform(seed, 2, i, 0, t), sz[rand]);
       pos[i * KM + rand] = randi;
       if (s_ref == i) bestv[rand] = randi;                 // the best IS this whale's row: it moves with it
-      f = woa_fitness_local(a.qos, pos + i * KM, bs, sz, K, bnd);
+      f = woa_fitness<kWoaMaxK, false, WoaPick::kLocal>(a.qos, pos + i * KM, bs, sz, K, bnd);
     }
     if (whale) fit[i] = f;
     __syncthreads();
     if (i == 0) {
-      int ref = s_ref; double best = s_best; int changed = 0;
-      for (int w = 0; w < P; ++w)
-        if (best > fit[w]) { best = fit[w]; ref = w; changed = 1; }
+      int ref = s_ref; double best = s_best;
+      const int changed = scan_best(fit, P, best, ref);
       s_best = best; s_ref = ref; s_star = changed;
       s_skip = 0.2 > philox_uniform(seed, 0, 0, 1, t);        // exploration skip (WOA.py:124-128)
     }
@@ -228,7 +227,7 @@ __global__ void __launch_bounds__(kWoaThreads) woa_search_kernel(const WoaSearch
               if (abs(q) >= sz[k]) { q %= sz[k]; if (q < 0) q += sz[k]; }
               newp[i * KM + k] = q;
             }
-            f = woa_fitness_local(a.qos, newp + i * KM, bs, sz, K, bnd);
+            f = woa_fitness<kWoaMaxK, false, WoaPick::kLocal>(a.qos, newp + i * KM, bs, sz, K, bnd);
           }
           fit[i] = f;
         }
@@ -267,7 +266,8 @@ __global__ void __launch_bounds__(kWoaThreads) woa_search_kernel(const WoaSearch
 
 // ------------------------------------------------------------------------------------------------------------------
 // What the host does before the search starts (gnnpn_sc_b200/WOA.py: loadDataOther + _add_s, the seed preparation of
-// WOA.start, _Instance.__init__, _Engine._init_population), one CTA per instance, for gnnpn_woa_search_f64.
+// WOA.start, _Instance.__init__ and _Engine._init_population, whose draws, fitness and best-so-far scan are
+// philox_index, woa_fitness and scan_best as in the search), one CTA per instance, for gnnpn_woa_search_f64.
 struct WoaPrepareArgs {
   const double* svc_raw;     // [S, 4] JSON values
   const double* svc_round;   // [S, 4] the same rounded to 5 decimals (Python `round`)
@@ -472,16 +472,15 @@ __global__ void __launch_bounds__(kWoaThreads) woa_prepare_kernel(const WoaPrepa
   if (tid < P) {
     int32_t* row = a.pops + ((int64_t)I * P + tid) * K;
     for (int k = 0; k < K; ++k)
-      row[k] = k < kl ? (int)__dmul_rn(philox_uniform(seed, k, tid, 3, 0), (double)s_size0[k]) : 0;
-    s_fit[tid] = kl > 0 ? woa_fitness_local(a.qos, row, s_base, s_size, kl, bnd) : INFINITY;
+      row[k] = k < kl ? philox_index(philox_uniform(seed, k, tid, 3, 0), s_size0[k]) : 0;
+    s_fit[tid] = kl > 0 ? woa_fitness<kWoaMaxK, false, WoaPick::kLocal>(a.qos, row, s_base, s_size, kl, bnd) : INFINITY;
   }
   __syncthreads();
   if (tid == 0) {
     double best = 3.0;
     int ref = -1;
-    if (seeded && ns == kl) best = woa_fitness_local(a.qos, s_own, s_base, s_size, kl, bnd);
-    for (int w = 0; w < P; ++w)
-      if (best > s_fit[w]) { best = s_fit[w]; ref = w; }
+    if (seeded && ns == kl) best = woa_fitness<kWoaMaxK, false, WoaPick::kLocal>(a.qos, s_own, s_base, s_size, kl, bnd);
+    scan_best(s_fit, P, best, ref);
     s_ref = ref;
     a.best_fit[I] = best;
     a.best_ref[I] = ref;
