@@ -19,8 +19,8 @@ from .loadData import loadDataPN
 
 def composition_scores(allActions, serCategory: int, constraints: np.ndarray) -> np.ndarray:
     """Score per instance exactly as ``ML2PN.calc`` (ML2PN.py:6-12) does it, float64 in numpy's operation order:
-    ``0.5*(np.average(q0) + 1 - np.min(q1)) + #violated global constraints`` over the REAL picks of the instance
-    (rows whose python ``sum`` is not 3 -- the neutral ``[0,1,1,1]`` of absent categories, ML2PN.py:42).
+    ``0.5*(np.average(q0) + 1 - np.min(q1))``, then 1 added per violated global constraint, over the REAL picks of
+    the instance (rows whose python ``sum`` is not 3 -- the neutral ``[0,1,1,1]`` of absent categories, ML2PN.py:42).
     ``allActions`` = K lists of [n_test][F] chosen rows; ``constraints`` [n_test, 4] = (lo1, hi1, lo2, hi2).
     One launch of ``gnnpn_ml2pn_score_f64`` for all instances."""
     acts = np.asarray([a for a in allActions[:serCategory]], dtype=np.float64)      # [K, n, F]

@@ -59,6 +59,38 @@ __device__ __forceinline__ void bias_bn_act(float* r, const float* bias, const f
   }
 }
 
+__device__ __forceinline__ float add_rn(float a, float b) { return __fadd_rn(a, b); }
+__device__ __forceinline__ double add_rn(double a, double b) { return __dadd_rn(a, b); }
+
+// np.sum of a contiguous float32 / float64 vector, in numpy's order (pairwise_sum in
+// numpy/core/src/umath/loops_utils.h.src): < 8 elements sequential, <= 128 elements eight running accumulators, above
+// that a recursive split at n/2 rounded down to a multiple of 8.  The recursion is unrolled at compile time for
+// n <= NMAX (a piece of n holds at most ceil(n/2) + 7 elements; NMAX = 512 unrolls three levels), so the kernel needs
+// no device call stack.
+template <int NMAX, class T>
+__device__ __forceinline__ T numpy_sum(const T* a, int n) {
+  if constexpr (NMAX > 128) {
+    if (n > 128) {
+      int n2 = n / 2;
+      n2 -= n2 % 8;
+      return add_rn(numpy_sum<NMAX / 2 + 8>(a, n2), numpy_sum<NMAX / 2 + 8>(a + n2, n - n2));
+    }
+  }
+  if (n < 8) {
+    T res = 0;
+    for (int i = 0; i < n; ++i) res = add_rn(res, a[i]);
+    return res;
+  }
+  T r[8];
+  for (int j = 0; j < 8; ++j) r[j] = a[j];
+  int i;
+  for (i = 8; i < n - (n % 8); i += 8)
+    for (int j = 0; j < 8; ++j) r[j] = add_rn(r[j], a[i + j]);
+  T res = add_rn(add_rn(add_rn(r[0], r[1]), add_rn(r[2], r[3])), add_rn(add_rn(r[4], r[5]), add_rn(r[6], r[7])));
+  for (; i < n; ++i) res = add_rn(res, a[i]);
+  return res;
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

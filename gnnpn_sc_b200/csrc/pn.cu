@@ -102,38 +102,6 @@ int launch_pointer_steps(const PointerStepArgs& pa, int K, const float* dec_h, c
 // composition objective (calc / reward): one thread per instance, fp32 sequential products
 // and numpy's float32 pairwise-sum order for sum(q0) so results are bit-identical to the CPU path
 // ---------------------------------------------------------------------------
-__device__ float numpy_pairwise_sum_f32(const float* v, int n) {
-  // numpy pairwise_sum for n < 128 (PW_BLOCKSIZE): 8 accumulators, then the tail in order.
-  if (n < 8) {
-    float r = 0.f;
-    for (int i = 0; i < n; ++i) r = __fadd_rn(r, v[i]);
-    return r;
-  }
-  float r[8];
-  for (int j = 0; j < 8; ++j) r[j] = v[j];
-  int i = 8;
-  for (; i < n - (n % 8); i += 8)
-    for (int j = 0; j < 8; ++j) r[j] = __fadd_rn(r[j], v[i + j]);
-  float res = __fadd_rn(__fadd_rn(__fadd_rn(r[0], r[1]), __fadd_rn(r[2], r[3])),
-                        __fadd_rn(__fadd_rn(r[4], r[5]), __fadd_rn(r[6], r[7])));
-  for (; i < n; ++i) res = __fadd_rn(res, v[i]);
-  return res;
-}
-
-// numpy splits n > 128 as (n/2 rounded down to a multiple of 8) + rest, recursively; unrolled by
-// template depth (3 levels cover n <= 1024) because device recursion has no static stack bound.
-template <int DEPTH>
-__device__ float numpy_sum_f32(const float* v, int n) {
-  if (n <= 128) return numpy_pairwise_sum_f32(v, n);
-  if constexpr (DEPTH == 0) {
-    return numpy_pairwise_sum_f32(v, n);   // unreachable for n <= kMaxTasks
-  } else {
-    int n2 = n / 2;
-    n2 -= n2 % 8;
-    return __fadd_rn(numpy_sum_f32<DEPTH - 1>(v, n2), numpy_sum_f32<DEPTH - 1>(v + n2, n - n2));
-  }
-}
-
 constexpr int kMaxTasks = 512;
 
 __global__ void reward_kernel(const float* __restrict__ inputs, const int32_t* __restrict__ idx, int64_t n,
@@ -158,7 +126,7 @@ __global__ void reward_kernel(const float* __restrict__ inputs, const int32_t* _
   }
   int viol = 0;
   for (int i = 0; i < 2; ++i) viol += (prod[i] < lo[i] || prod[i] > hi[i]) ? 1 : 0;
-  const float s = numpy_sum_f32<2>(q0s, K);
+  const float s = numpy_sum<kMaxTasks>(q0s, K);
   float obj = __fdiv_rn(s, (float)used);
   obj = __fadd_rn(obj, 1.0f);
   obj = __fsub_rn(obj, min_q1);

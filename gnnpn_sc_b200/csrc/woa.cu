@@ -16,39 +16,12 @@
 namespace gnnpn {
 namespace {
 
-// numpy's pairwise summation for contiguous float64 (numpy/core/src/umath/loops_utils.h.src, pairwise_sum_DOUBLE):
-// < 8 elements sequential, <= 128 elements eight running accumulators, above that a recursive split at
-// n/2 rounded down to a multiple of 8.  The recursion is unrolled at compile time for n <= NMAX (a piece of n holds
-// at most ceil(n/2) + 7 elements; NMAX = 512 unrolls three levels), so the kernel needs no device call stack.
-template <int NMAX>
-__device__ __forceinline__ double numpy_sum_f64(const double* a, int n) {
-  if constexpr (NMAX > 128) {
-    if (n > 128) {
-      int n2 = n / 2;
-      n2 -= n2 % 8;
-      return __dadd_rn(numpy_sum_f64<NMAX / 2 + 8>(a, n2), numpy_sum_f64<NMAX / 2 + 8>(a + n2, n - n2));
-    }
-  }
-  if (n < 8) {
-    double res = 0.0;
-    for (int i = 0; i < n; ++i) res = __dadd_rn(res, a[i]);
-    return res;
-  }
-  double r[8];
-  for (int j = 0; j < 8; ++j) r[j] = a[j];
-  int i;
-  for (i = 8; i < n - (n % 8); i += 8)
-    for (int j = 0; j < 8; ++j) r[j] = __dadd_rn(r[j], a[i + j]);
-  double res = __dadd_rn(__dadd_rn(__dadd_rn(r[0], r[1]), __dadd_rn(r[2], r[3])),
-                         __dadd_rn(__dadd_rn(r[4], r[5]), __dadd_rn(r[6], r[7])));
-  for (; i < n; ++i) res = __dadd_rn(res, a[i]);
-  return res;
-}
-
 // The fitness (violate + objFunc) of one composition of K <= KMAX picks, b the (lo, hi) pair of each product; violate
 // and objFunc also go to viol_out and obj_out when given.  Pick k is row pos[k] of qos (kRow), or entry pos[k] of the
 // task's list of size[k] rows from row base[k], a negative pos[k] counting from its end as in Python (kLocal).
-// MEAN_ALL: `np.average(qos[0])` over all K picks (src/ML2PN.py:6-12, `ML2PN.calc`) instead of sum / #{q0 > 0}.
+// MEAN_ALL: `ML2PN.calc` (src/ML2PN.py:6-12): `np.average(qos[0])` over all K picks instead of sum / #{q0 > 0}, and
+// 1.0 added to the objective once per violated constraint, in constraint order, instead of `violate + objFunc` in one
+// add (with both violated, (obj + 1) + 1 and obj + 2 can round apart).
 enum class WoaPick { kRow, kLocal };
 template <int KMAX, bool MEAN_ALL, WoaPick PICK>
 __device__ __forceinline__ double woa_fitness(const double* __restrict__ qos, const int32_t* pos, const int32_t* base,
@@ -74,12 +47,18 @@ __device__ __forceinline__ double woa_fitness(const double* __restrict__ qos, co
   }
   int viol = 0;
   for (int i = 0; i < 2; ++i) viol += (prod[i] < b[2 * i] || prod[i] > b[2 * i + 1]) ? 1 : 0;
-  double obj = __ddiv_rn(numpy_sum_f64<KMAX>(q0s, K), (double)(MEAN_ALL ? K : used));
+  double obj = __ddiv_rn(numpy_sum<KMAX>(q0s, K), (double)(MEAN_ALL ? K : used));
   obj = __dadd_rn(obj, 1.0);
   obj = __dsub_rn(obj, min_q1);
   obj = __ddiv_rn(obj, 2.0);
   if (viol_out) *viol_out = viol;
   if (obj_out) *obj_out = obj;
+  if constexpr (MEAN_ALL) {
+    double score = obj;
+    for (int i = 0; i < 2; ++i)
+      if (prod[i] < b[2 * i] || prod[i] > b[2 * i + 1]) score = __dadd_rn(score, 1.0);
+    return score;
+  }
   return __dadd_rn((double)viol, obj);
 }
 

@@ -395,7 +395,8 @@ def woa_fitness(qos: torch.Tensor, idx: torch.Tensor, bounds: torch.Tensor, klen
 
 def ml2pn_score(qos: torch.Tensor, idx: torch.Tensor, bounds: torch.Tensor, klen: torch.Tensor):
     """``ML2PN.calc`` (ML2PN.py:6-12) for a batch of compositions, float64: same layout as :func:`woa_fitness`, the
-    mean of q0 runs over all ``klen[p]`` picks.  -> (viol int32 [P], obj f64 [P], obj + viol f64 [P])."""
+    mean of q0 runs over all ``klen[p]`` picks.  -> (viol int32 [P], obj f64 [P], score f64 [P]): the score is obj
+    with 1.0 added once per violated constraint, one add at a time as ``ML2PN.calc`` does."""
     if not (qos.is_cuda and idx.is_cuda and bounds.is_cuda and klen.is_cuda):
         raise GnnpnError("ml2pn_score needs CUDA tensors (no CPU fallback)")
     assert qos.dtype == torch.float64 and bounds.dtype == torch.float64

@@ -292,7 +292,9 @@ GNNPN_API int gnnpn_woa_fitness_f64(const double* qos, int64_t n_services, const
 
 /* `ML2PN.calc` (src/ML2PN.py:6-12) for a batch of compositions, float64 in numpy's operation order: same layout as
  * gnnpn_woa_fitness_f64, but the objective is 0.5*(np.average(q0) + 1 - np.min(q1)) -- the mean runs over ALL klen[p]
- * picks, not over those with q0 > 0 -- and score = obj + #violated global constraints. */
+ * picks, not over those with q0 > 0 -- and score = obj with 1.0 added once per violated global constraint, constraint 1
+ * first (as `obj += 1` in ML2PN.calc; with both violated, (obj + 1) + 1 can differ from obj + 2 in the last bit).
+ * obj_out is the objective before the violations. */
 GNNPN_API int gnnpn_ml2pn_score_f64(const double* qos, int64_t n_rows, const int32_t* idx, int64_t idx_ld,
                           const int32_t* klen, const double* bounds, int64_t P, int Kmax,
                           int32_t* viol_out, double* obj_out, double* score_out, void* stream);
