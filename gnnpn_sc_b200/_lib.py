@@ -69,10 +69,9 @@ SIGNATURES = {
     "gnnpn_csr_build_workspace_bytes": (_i, [_i64, _i64, _i, C.POINTER(C.c_size_t)]),
     "gnnpn_csr_build": (_i, [_p, _p, _i64, _i64, _i, _p, _p, _p, _p, _p, C.c_size_t, _p]),
     "gnnpn_embed_concat_f32": (_i, [_p, _i64, _i, _p, _i, _i, _p, _i64, _p]),
-    "gnnpn_spmm_csr_f32": (_i, [_p, _p, _p, _p, _i64, _p, _i64, _i64, _i, _f, _i, _p, _p, _p, _i, _p]),
-    "gnnpn_spmm_csr_split_workspace_bytes": (C.c_size_t, [_i64, _i, _i64]),
-    "gnnpn_spmm_csr_split_f32": (_i, [_p, _p, _p, _p, _i64, _p, _i64, _i64, _i64, _i, _f, _i, _p, _p, _p, _i, _i64, _p,
-                                      C.c_size_t, _p]),
+    "gnnpn_spmm_csr_workspace_bytes": (C.c_size_t, [_i64, _i, _i64]),
+    "gnnpn_spmm_csr_f32": (_i, [_p, _p, _p, _p, _i64, _p, _i64, _i64, _i64, _i, _f, _i, _p, _p, _p, _i, _i64, _p,
+                                C.c_size_t, _p]),
     "gnnpn_bn_train_forward_f32": (_i, [_p, _i64, _i64, _i, _p, _p, _f, _f, _i, _p, _i64, _p, _p, _p, _p, _p]),
     "gnnpn_bn_train_backward_f32": (_i, [_p, _i64, _p, _i64, _p, _i64, _i64, _i, _p, _p, _p, _i, _p, _i64, _p, _p, _p]),
     "gnnpn_gemm_workspace_bytes": (C.c_size_t, [_i64, _i, _i]),
@@ -100,7 +99,7 @@ def lib():
                 fn = getattr(h, name)          # AttributeError if the ABI lost a symbol
                 fn.restype = res
                 fn.argtypes = args
-            if h.gnnpn_abi_version() != 10:
+            if h.gnnpn_abi_version() != 11:
                 raise GnnpnError("libgnnpn_b200.so ABI version mismatch")
             _lib = h
     return _lib
@@ -114,7 +113,7 @@ def check(rc: int, what: str = "") -> None:
 
 def set_option(name: str, value: int) -> None:
     """``gnnpn_set_option``: "scan" (-1 auto / 0 CTA-pair / 1 column-split), "scan_groups", "persistent", "prof",
-    "bptt" (0: per-step BPTT kernels), "spmm_chunk" (aggregation tuning)."""
+    "bptt" (0: per-step BPTT kernels)."""
     check(lib().gnnpn_set_option(name.encode(), int(value)), f"set_option({name})")
 
 

@@ -35,7 +35,6 @@ static std::atomic<int>* option_slot(const char* name) {
   if (!strcmp(name, "persistent")) return &o.persistent;
   if (!strcmp(name, "prof")) return &o.prof;
   if (!strcmp(name, "bptt")) return &o.bptt;
-  if (!strcmp(name, "spmm_chunk")) return &o.spmm_chunk;
   return nullptr;
 }
 }  // namespace gnnpn

@@ -1,7 +1,6 @@
 // ML stage graph kernels: edge_index -> CSR (+ gcn_norm), CSR segment-reduce aggregation.
 #include <cub/device/device_radix_sort.cuh>
 #include "common.cuh"
-#include "options.cuh"
 
 namespace gnnpn {
 namespace {
@@ -102,13 +101,14 @@ int key_bits(int64_t Nn) {
   return b;
 }
 
+inline size_t al(size_t x) { return (x + 255) & ~size_t(255); }      // workspace arrays start at 256-byte offsets
+
 struct CsrWorkspace {
   size_t keys_in, keys_out, pay_in, pay_out, loop_eid, dis, cub, total;
 };
 
 CsrWorkspace csr_layout(int64_t Nn, int64_t E, int mode) {
   const int64_t total = E + (mode == GNNPN_CSR_GCN_NORM ? Nn : 0);
-  auto al = [](size_t x) { return (x + 255) & ~size_t(255); };
   CsrWorkspace w{};
   size_t off = 0;
   w.keys_in = off;  off += al(total * 4);
@@ -235,7 +235,7 @@ __global__ void __launch_bounds__(256) spmm_csr_kernel(
 }
 
 // ---- long-row splitting (hub destinations: a service used by 10^5 compositions would otherwise be ONE group's
-// sequential walk).  Rows with more than T edges are cut into chunks of Tc = T / 8 consecutive edges; every chunk is summed
+// sequential walk).  Rows with more than T edges are cut into chunks of Tc = chunk_len(T) consecutive edges; every chunk is summed
 // by one group exactly like a short row (sequential in CSR order), the chunk sums are then added in chunk order.
 // Deterministic (fixed order, no atomics in the arithmetic); rows of <= T edges stay bit-identical to index_add_ order,
 // split rows differ from the strictly sequential sum by re-association only (~1e-7 relative; tests bound it by 1e-5).
@@ -373,8 +373,6 @@ __global__ void embed_concat_kernel(const float* __restrict__ x, int64_t n, int 
 }
 
 inline int64_t chunk_len(int64_t T) {                                       // edges per chunk of a split row
-  const int o = options().spmm_chunk.load(std::memory_order_relaxed);
-  if (o >= 32) return o / 32 * 32;
   // 256 edges = 8 staging rounds: amortises the chunk's dependent look-ups (slot -> row -> rowptr).  Chunks of 32 made the
   // chunk pass 3x slower per edge than the short-row kernel (scripts/agg_threshold_probe.py)
   return T / 8 < 256 ? 256 : T / 8;
@@ -412,6 +410,53 @@ int launch_spmm(const int64_t* rowptr, const int32_t* col, const float* val, con
   if ((rc = after_launch())) return rc;
   spmm_combine_kernel<GROUP, VPL><<<kNumSMs, 256, 0, st>>>(rowptr, x, ldx, y, ldy, F4, chunk_len(T), ep, *plan);
   return after_launch();
+}
+
+template <int G, int V, int U>
+struct SpmmShape { static constexpr int GROUP = G, VPL = V, UNROLL = U; };
+
+// The lane-group table: calls fn with the SpmmShape whose kernels aggregate F4 float4 columns (32 / GROUP rows per warp)
+template <class Fn>
+auto with_spmm_shape(int F4, Fn&& fn) {
+  if (F4 <= 8) return fn(SpmmShape<8, 1, 8>{});
+  if (F4 <= 16) return fn(SpmmShape<16, 1, 8>{});
+  if (F4 <= 32) return fn(SpmmShape<32, 1, 8>{});
+  if (F4 <= 64) return fn(SpmmShape<32, 2, 4>{});
+  if (F4 <= 128) return fn(SpmmShape<32, 4, 2>{});
+  return fn(SpmmShape<32, 8, 1>{});
+}
+
+// The long-row threshold a call runs with (0: no split): `requested` when it is >= 0, else the library's choice.
+// - Below 2^22 edges nothing is split: there the split path's three extra (tiny) launches cost more than a hub row.
+// - Where the lane group is narrower than a warp, 4 or 2 rows share a warp and a 10^3-edge row idles its warp mates, so
+//   rows of more than 256 edges are split (in-degree-Zipf sweep, F = 32: 0.53 -> 0.59 of the HBM peak, F = 64: 0.68 ->
+//   0.72).
+// - Otherwise rows of more than 2048 edges are split.  The QWS co-usage graph's largest row has 1,378 edges: never split,
+//   bit-identical to index_add_.
+int64_t resolve_long_row_threshold(int64_t nnz, int F, int64_t requested) {
+  if (requested >= 0) return requested;
+  if (nnz < (int64_t(1) << 22)) return 0;
+  return with_spmm_shape(F / 4, [](auto s) -> int64_t { return decltype(s)::GROUP < 32 ? 256 : 2048; });
+}
+
+// Workspace of the long-row plan of nnz edges, F columns and threshold T: the LongRowPlan arrays and their capacities
+struct LongRowLayout {
+  int64_t max_long, max_chunks;
+  size_t counters, row, chunk_base, chunk_slot, partial, total;
+};
+
+LongRowLayout long_row_layout(int64_t nnz, int F, int64_t T) {
+  LongRowLayout w{};
+  w.max_long = nnz / (T + 1) + 1;                           // a long row has at least T + 1 edges
+  w.max_chunks = nnz / chunk_len(T) + w.max_long + 1;       // sum of ceil(d / Tc) over the long rows
+  size_t off = 0;
+  w.counters = off;   off += al(2 * sizeof(int));
+  w.row = off;        off += al(w.max_long * sizeof(int64_t));
+  w.chunk_base = off; off += al(w.max_long * sizeof(int));
+  w.chunk_slot = off; off += al(w.max_chunks * sizeof(int));
+  w.partial = off;    off += al(w.max_chunks * F * sizeof(float));     // read and written as float4
+  w.total = off;
+  return w;
 }
 
 }  // namespace
@@ -492,71 +537,46 @@ int gnnpn_embed_concat_f32(const float* x, int64_t n, int n_cols, const float* t
   return after_launch();
 }
 
-static int spmm_dispatch(const int64_t* rowptr, const int32_t* col, const float* val, const float* x, int64_t ldx, float* y,
-                         int64_t ldy, int64_t n_rows, int F, const SpmmEpilogue& ep, int64_t T, const LongRowPlan* plan,
-                         cudaStream_t st) {
-  const int F4 = F / 4;
-#define GNNPN_SPMM(G, V, U) return launch_spmm<G, V, U>(rowptr, col, val, x, ldx, y, ldy, n_rows, F4, ep, T, plan, st)
-  if (F4 <= 8) GNNPN_SPMM(8, 1, 8);
-  if (F4 <= 16) GNNPN_SPMM(16, 1, 8);
-  if (F4 <= 32) GNNPN_SPMM(32, 1, 8);
-  if (F4 <= 64) GNNPN_SPMM(32, 2, 4);
-  if (F4 <= 128) GNNPN_SPMM(32, 4, 2);
-  GNNPN_SPMM(32, 8, 1);
-#undef GNNPN_SPMM
+size_t gnnpn_spmm_csr_workspace_bytes(int64_t nnz, int F, int64_t long_row_threshold) {
+  if (nnz < 0 || F < 4 || (long_row_threshold > 0 && long_row_threshold < 32)) return 0;
+  const int64_t T = resolve_long_row_threshold(nnz, F, long_row_threshold);
+  return T ? long_row_layout(nnz, F, T).total : 0;
 }
 
-#define GNNPN_SPMM_CHECKS                                                                                        \
-  GNNPN_REQUIRE(rowptr && (col || n_rows == 0) && x && y, GNNPN_ENULL);                                            \
-  GNNPN_REQUIRE(F >= 4 && F % 4 == 0 && F <= 1024 && ldx % 4 == 0 && ldy % 4 == 0 && ldx >= F && ldy >= F,         \
-                GNNPN_ESHAPE);                                                                                     \
-  GNNPN_REQUIRE((scale == nullptr) == (shift == nullptr), GNNPN_ENULL);                                            \
-  GNNPN_REQUIRE(aligned16(x) && aligned16(y) && aligned16(bias) && aligned16(scale) && aligned16(shift), GNNPN_EALIGN)
-
-int gnnpn_spmm_csr_f32(const int64_t* rowptr, const int32_t* col, const float* val, const float* x,
-                       int64_t ldx, float* y, int64_t ldy, int64_t n_rows, int F, float self_scale, int mean,
-                       const float* bias, const float* scale, const float* shift, int act, void* stream) {
-  GNNPN_SPMM_CHECKS;
-  if (n_rows == 0) return GNNPN_OK;
-  const SpmmEpilogue ep{self_scale, mean, bias, scale, shift, act};
-  return spmm_dispatch(rowptr, col, val, x, ldx, y, ldy, n_rows, F, ep, 0, nullptr, (cudaStream_t)stream);
-}
-
-static void split_bounds(int64_t nnz, int64_t T, int64_t* max_long, int64_t* max_chunks) {
-  *max_long = nnz / (T + 1) + 1;                 // a long row has at least T + 1 edges
-  *max_chunks = nnz / chunk_len(T) + *max_long + 1;      // sum of ceil(d / Tc) over the long rows
-}
-
-size_t gnnpn_spmm_csr_split_workspace_bytes(int64_t nnz, int F, int64_t long_row_threshold) {
-  if (nnz < 0 || F < 4 || long_row_threshold < 32) return 0;
-  int64_t ml, mc;
-  split_bounds(nnz, long_row_threshold, &ml, &mc);
-  return 256 + (size_t)ml * 16 + (size_t)mc * 4 + 256 + (size_t)mc * F * 4;
-}
-
-int gnnpn_spmm_csr_split_f32(const int64_t* rowptr, const int32_t* col, const float* val, const float* x,
-                             int64_t ldx, float* y, int64_t ldy, int64_t n_rows, int64_t nnz, int F, float self_scale,
-                             int mean, const float* bias, const float* scale, const float* shift, int act,
-                             int64_t long_row_threshold, void* workspace, size_t workspace_bytes, void* stream) {
-  GNNPN_SPMM_CHECKS;
-  GNNPN_REQUIRE(workspace, GNNPN_ENULL);
-  GNNPN_REQUIRE(long_row_threshold >= 32 && nnz >= 0, GNNPN_ESHAPE);
-  GNNPN_REQUIRE(nnz < (1ll << 31) * (int64_t)32, GNNPN_ERANGE);
-  GNNPN_REQUIRE(workspace_bytes >= gnnpn_spmm_csr_split_workspace_bytes(nnz, F, long_row_threshold), GNNPN_EWORKSPACE);
-  GNNPN_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, GNNPN_EALIGN);
-  if (n_rows == 0) return GNNPN_OK;
-  int64_t ml, mc;
-  split_bounds(nnz, long_row_threshold, &ml, &mc);
-  uint8_t* w = static_cast<uint8_t*>(workspace);
+int gnnpn_spmm_csr_f32(const int64_t* rowptr, const int32_t* col, const float* val, const float* x, int64_t ldx,
+                       float* y, int64_t ldy, int64_t n_rows, int64_t nnz, int F, float self_scale, int mean,
+                       const float* bias, const float* scale, const float* shift, int act, int64_t long_row_threshold,
+                       void* workspace, size_t workspace_bytes, void* stream) {
+  GNNPN_REQUIRE(rowptr && (col || n_rows == 0) && x && y, GNNPN_ENULL);
+  GNNPN_REQUIRE(F >= 4 && F % 4 == 0 && F <= 1024 && ldx % 4 == 0 && ldy % 4 == 0 && ldx >= F && ldy >= F && nnz >= 0 &&
+                    (long_row_threshold <= 0 || long_row_threshold >= 32),
+                GNNPN_ESHAPE);
+  GNNPN_REQUIRE((scale == nullptr) == (shift == nullptr), GNNPN_ENULL);
+  GNNPN_REQUIRE(aligned16(x) && aligned16(y) && aligned16(bias) && aligned16(scale) && aligned16(shift), GNNPN_EALIGN);
+  const int64_t T = resolve_long_row_threshold(nnz, F, long_row_threshold);
   LongRowPlan plan{};
-  plan.counters = reinterpret_cast<int*>(w);            w += 256;
-  plan.row = reinterpret_cast<int64_t*>(w);             w += (size_t)ml * 8;
-  plan.chunk_base = reinterpret_cast<int*>(w);          w += (size_t)ml * 8;     // keeps the next array 8-byte aligned
-  plan.chunk_slot = reinterpret_cast<int*>(w);          w += ((size_t)mc * 4 + 255) & ~size_t(255);
-  plan.partial = reinterpret_cast<float*>(w);
-  plan.max_long = (int)ml; plan.max_chunks = (int)mc;
+  if (T) {
+    GNNPN_REQUIRE(workspace, GNNPN_ENULL);
+    GNNPN_REQUIRE(nnz < (1ll << 31) * (int64_t)32, GNNPN_ERANGE);
+    const LongRowLayout w = long_row_layout(nnz, F, T);
+    GNNPN_REQUIRE(workspace_bytes >= w.total, GNNPN_EWORKSPACE);
+    GNNPN_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, GNNPN_EALIGN);
+    uint8_t* ws = static_cast<uint8_t*>(workspace);
+    plan.counters = reinterpret_cast<int*>(ws + w.counters);
+    plan.row = reinterpret_cast<int64_t*>(ws + w.row);
+    plan.chunk_base = reinterpret_cast<int*>(ws + w.chunk_base);
+    plan.chunk_slot = reinterpret_cast<int*>(ws + w.chunk_slot);
+    plan.partial = reinterpret_cast<float*>(ws + w.partial);
+    plan.max_long = (int)w.max_long;
+    plan.max_chunks = (int)w.max_chunks;
+  }
+  if (n_rows == 0) return GNNPN_OK;
   const SpmmEpilogue ep{self_scale, mean, bias, scale, shift, act};
-  return spmm_dispatch(rowptr, col, val, x, ldx, y, ldy, n_rows, F, ep, long_row_threshold, &plan, (cudaStream_t)stream);
+  return with_spmm_shape(F / 4, [&](auto s) {
+    using S = decltype(s);
+    return launch_spmm<S::GROUP, S::VPL, S::UNROLL>(rowptr, col, val, x, ldx, y, ldy, n_rows, F / 4, ep, T,
+                                                    T ? &plan : nullptr, (cudaStream_t)stream);
+  });
 }
 
 }  // extern "C"

@@ -10,7 +10,6 @@ struct Options {
   std::atomic<int> scan{-1};         // "scan": -1 auto (by batch size), 0 CTA-pair scan, 1 column-split cluster scan   [GNNPN_COLSPLIT]
   std::atomic<int> scan_groups{0};   // "scan_groups": 0 auto, 1 / 2 / 3 instance groups per column-split encoder cluster  [GNNPN_COLSPLIT_G]
   std::atomic<int> persistent{3};    // "persistent": bit 0 encoder, bit 1 decoder run as ONE persistent launch           [GNNPN_SEQ]
-  std::atomic<int> spmm_chunk{0};    // "spmm_chunk": edges per chunk of a split row, 0 = auto (threshold / 8, at least 32)   (tuning)
   std::atomic<int> bptt{1};          // "bptt": 1 = REINFORCE backward as two persistent cluster scans, 0 = two launches per step   [GNNPN_BPTT]
   std::atomic<int> prof{0};          // "prof": in-kernel wait-cycle counters, printed to stderr (debug, synchronous)     [GNNPN_SEQ_PROF]
 };

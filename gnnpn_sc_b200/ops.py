@@ -539,43 +539,22 @@ def embed_concat(x: torch.Tensor, table: torch.Tensor, pad_to: int = 4) -> torch
     return out
 
 
-SPLIT_MIN_NNZ = 1 << 22          # below this the three extra (tiny) launches of the split path cost more than a hub row
-SPLIT_THRESHOLD = 2048           # rows with more edges are split into chunks of 256 edges (hub rows: at most ~4096 chunks per row);
-                                 # the QWS co-usage graph's largest row has 1,378 edges -> never split, bit-identical to index_add_
-SPLIT_THRESHOLD_NARROW = 256     # F <= 64: 4 / 2 rows share a warp, so a 10^3-edge row idles its warp mates -- split earlier
-                                 # (in-degree-Zipf sweep, F = 32: 0.53 -> 0.59 of the HBM peak, F = 64: 0.68 -> 0.72)
-
-
-def split_threshold(F: int) -> int:
-    return SPLIT_THRESHOLD_NARROW if F <= 64 else SPLIT_THRESHOLD
-
-
 def spmm_csr(rowptr, col, val, x, n_rows: Optional[int] = None, self_scale: float = 0.0, mean: bool = False,
-             bias=None, scale=None, shift=None, act=None, out=None, long_row_threshold: Optional[int] = None,
-             workspace: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """CSR aggregation.  ``long_row_threshold``: rows with more edges are split into chunks (hub destinations of a skewed
-    graph, ``gnnpn_spmm_csr_split_f32``); None = ``split_threshold(F)`` for graphs of at least ``SPLIT_MIN_NNZ`` edges, no
-    splitting below; 0 = never."""
+             bias=None, scale=None, shift=None, act=None, out=None, long_row_threshold: Optional[int] = None) -> torch.Tensor:
+    """CSR aggregation (``gnnpn_spmm_csr_f32``).  ``long_row_threshold``: rows with more edges are split into chunks (hub
+    destinations of a skewed graph); None = the library's choice by edge count and feature width; 0 = never split."""
     x = _f32(x, "x")
     F = x.shape[1]
     assert F % 4 == 0, "feature dim must be padded to a multiple of 4"
     n_rows = rowptr.numel() - 1 if n_rows is None else n_rows
     y = torch.empty(n_rows, F, device=x.device, dtype=torch.float32) if out is None else out
     nnz = int(col.numel())
-    if long_row_threshold is None:
-        long_row_threshold = split_threshold(F) if nnz >= SPLIT_MIN_NNZ else 0
-    if long_row_threshold:
-        need = int(lib().gnnpn_spmm_csr_split_workspace_bytes(nnz, F, int(long_row_threshold)))
-        if workspace is None or workspace.numel() < need:
-            workspace = torch.empty(need, device=x.device, dtype=torch.uint8)
-        check(lib().gnnpn_spmm_csr_split_f32(rowptr.data_ptr(), col.data_ptr(), _ptr(val), x.data_ptr(), x.stride(0),
-                                             y.data_ptr(), y.stride(0), n_rows, nnz, F, float(self_scale), int(mean),
-                                             _ptr(bias), _ptr(scale), _ptr(shift), ACT[act], int(long_row_threshold),
-                                             workspace.data_ptr(), workspace.numel(), _stream()), "spmm_csr_split")
-        return y
-    check(lib().gnnpn_spmm_csr_f32(rowptr.data_ptr(), col.data_ptr(), _ptr(val), x.data_ptr(), x.stride(0),
-                                   y.data_ptr(), y.stride(0), n_rows, F, float(self_scale), int(mean),
-                                   _ptr(bias), _ptr(scale), _ptr(shift), ACT[act], _stream()), "spmm_csr")
+    T = -1 if long_row_threshold is None else int(long_row_threshold)
+    need = int(lib().gnnpn_spmm_csr_workspace_bytes(nnz, F, T))
+    ws = torch.empty(need, device=x.device, dtype=torch.uint8) if need > 0 else None
+    check(lib().gnnpn_spmm_csr_f32(rowptr.data_ptr(), col.data_ptr(), _ptr(val), x.data_ptr(), x.stride(0), y.data_ptr(),
+                                   y.stride(0), n_rows, nnz, F, float(self_scale), int(mean), _ptr(bias), _ptr(scale),
+                                   _ptr(shift), ACT[act], T, _ptr(ws), need, _stream()), "spmm_csr")
     return y
 
 

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define GNNPN_ABI_VERSION 10
+#define GNNPN_ABI_VERSION 11
 
 #if defined(__GNUC__)
 #define GNNPN_API __attribute__((visibility("default")))
@@ -59,7 +59,6 @@ GNNPN_API uint64_t gnnpn_launch_count(void);
  *   "scan_groups"   0 auto | 1 | 2 | 3 instance groups per column-split encoder cluster
  *   "persistent"    bit 0: encoder, bit 1: decoder run as one persistent launch (default 3; 0 = one launch per step)
  *   "bptt"          1: REINFORCE backward as two persistent cluster scans (default) | 0: two launches per step
- *   "spmm_chunk"    edges per chunk of a split aggregation row (default 0 = auto)
  *   "prof"          1: in-kernel wait-cycle counters printed to stderr (debug; makes the call synchronous)
  * Initial values are taken once, at load time, from GNNPN_COLSPLIT / GNNPN_COLSPLIT_G / GNNPN_SEQ / GNNPN_BPTT /
  * GNNPN_SEQ_PROF.
@@ -414,24 +413,25 @@ GNNPN_API int gnnpn_embed_concat_f32(const float* x, int64_t n, int n_cols, cons
  *                 [+ bias] [* scale + shift] )
  * Covers GINConv's sum + (1+eps)*x (self_scale = 1+eps), GCNConv's normalised sum + bias with the
  * following eval-mode BatchNorm + ReLU folded in, and scatter(reduce='mean') (modelML.py:166,172).
- * F must be a multiple of 4; x, y 16-byte aligned with leading dimensions ldx, ldy (floats). */
-GNNPN_API int gnnpn_spmm_csr_f32(const int64_t* rowptr, const int32_t* col, const float* val,
-                       const float* x, int64_t ldx, float* y, int64_t ldy, int64_t n_rows, int F,
-                       float self_scale, int mean, const float* bias, const float* scale,
-                       const float* shift, int act, void* stream);
-
-/* Same aggregation with LONG-ROW SPLITTING for skewed in-degree distributions (hub destinations: the service co-usage
- * graph of src/loadData.py:55-65 gives popular services rows of 10^4..10^5 edges).  Rows with more than
- * `long_row_threshold` (>= 32) edges are cut into chunks of threshold / 8 consecutive edges, each chunk is summed by one
- * lane group like a short row, and the chunk sums are added in chunk order: deterministic, no atomics in the arithmetic.
- * Rows at or below the threshold stay bit-identical to gnnpn_spmm_csr_f32 (index_add_ order); split rows differ from the
- * strictly sequential sum by re-association only.  `nnz` = rowptr[n_rows] (known to the caller, not read from the
- * device); workspace: gnnpn_spmm_csr_split_workspace_bytes(nnz, F, threshold) bytes, 256-byte aligned. */
-GNNPN_API size_t gnnpn_spmm_csr_split_workspace_bytes(int64_t nnz, int F, int64_t long_row_threshold);
-GNNPN_API int gnnpn_spmm_csr_split_f32(const int64_t* rowptr, const int32_t* col, const float* val, const float* x,
-                             int64_t ldx, float* y, int64_t ldy, int64_t n_rows, int64_t nnz, int F, float self_scale,
-                             int mean, const float* bias, const float* scale, const float* shift, int act,
-                             int64_t long_row_threshold, void* workspace, size_t workspace_bytes, void* stream);
+ * F must be a multiple of 4; x, y 16-byte aligned with leading dimensions ldx, ldy (floats).  `nnz` is rowptr[n_rows]
+ * or any upper bound of it (known to the caller, not read from the device).
+ * LONG-ROW SPLITTING for skewed in-degree distributions (hub destinations: the service co-usage graph of
+ * src/loadData.py:55-65 gives popular services rows of 10^4..10^5 edges): rows with more than T edges are cut into
+ * chunks of max(256, T / 8) consecutive edges (longer for a row that would otherwise have more than 4096 chunks), each
+ * chunk is summed by one lane group like a short row, and the chunk sums are added in chunk order: deterministic, no
+ * atomics in the arithmetic.  Rows of at most T edges are bit-identical to the sequential index_add_ order; split rows
+ * differ from the strictly sequential sum by re-association only.
+ *   long_row_threshold < 0 : the library chooses T from nnz and F (no split below 2^22 edges)
+ *                      0   : never split: every row in index_add_ order
+ *                   >= 32  : T = long_row_threshold (1..31: GNNPN_ESHAPE)
+ * workspace: gnnpn_spmm_csr_workspace_bytes(nnz, F, long_row_threshold) bytes, 256-byte aligned.  The query returns 0
+ * when the call does not split; workspace may then be NULL. */
+GNNPN_API size_t gnnpn_spmm_csr_workspace_bytes(int64_t nnz, int F, int64_t long_row_threshold);
+GNNPN_API int gnnpn_spmm_csr_f32(const int64_t* rowptr, const int32_t* col, const float* val, const float* x,
+                                 int64_t ldx, float* y, int64_t ldy, int64_t n_rows, int64_t nnz, int F,
+                                 float self_scale, int mean, const float* bias, const float* scale, const float* shift,
+                                 int act, int64_t long_row_threshold, void* workspace, size_t workspace_bytes,
+                                 void* stream);
 
 /* Train-mode BatchNorm1d (+ optional fused ReLU) for the ML stage's training path (torch.nn.BatchNorm1d in training mode,
  * src/models/modelML.py:75-93,98-104 under TrainML.train, trainML.py:34-47).

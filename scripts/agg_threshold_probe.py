@@ -1,9 +1,8 @@
 """Long-row threshold probe: in-degree-Zipf graph (bench_agg.make_csr_indegree_zipf, E ~ 2^28), whole-call time of
-ops.spmm_csr over split thresholds T (chunks of T / 8 edges) and feature widths, next to the uniform graph of the same size."""
+ops.spmm_csr over split thresholds T (chunks of max(256, T / 8) edges) and feature widths, next to the uniform graph of the same size."""
 import json, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
-from gnnpn_sc_b200 import ops
 from scripts.bench_agg import make_csr, make_csr_indegree_zipf, time_point, peak
 
 dev = torch.device("cuda")
@@ -29,12 +28,10 @@ for F in (32, 64, 128, 256):
     for fam, floor in (("indeg_zipf", 8), ("indeg_zipf_pure", 0)):
         rowptr, col, val, E, dmax = make_csr_indegree_zipf(N, E_t, True, dev, floor=floor)
         alg = E * (8 + 4 * F) + N * 4 * F + (N + 1) * 8
-        for T, C, dyn in ((128, 0, 0), (256, 0, 0), (2048, 0, 0)):
-            ops.set_option("spmm_chunk", C)
+        for T, dyn in ((128, 0), (256, 0), (2048, 0)):
             ms = time_point(rowptr, col, val, x, y, 3, flush, False, long_row_threshold=T)
-            print(json.dumps({"family": fam, "F": F, "E": E, "T": T, "chunk": C, "dyn": dyn, "ms": ms,
+            print(json.dumps({"family": fam, "F": F, "E": E, "T": T, "dyn": dyn, "ms": ms,
                               "frac": alg / ms / 1e6 / pk, "dmax": dmax}), flush=True)
-        ops.set_option("spmm_chunk", 0)
         del rowptr, col, val
     rowptr = col = val = None
     del rowptr, col, val, x, y

@@ -144,7 +144,7 @@ def main():
                             y = torch.empty(N, F, device=dev)
                             ms = time_point(rowptr, col, val, x, y, iters, flush, args.one_launch)
                             ms0 = time_point(rowptr, col, val, x, y, iters, flush, args.one_launch, long_row_threshold=0)
-                            emit(record(family, E, N, F, weighted, ms, max_in_degree=dmax, long_row_threshold=ops.split_threshold(F),
+                            emit(record(family, E, N, F, weighted, ms, max_in_degree=dmax, long_row_threshold="auto",
                                         ms_without_split=ms0))
                         else:
                             rowptr, col, val, E = make_csr(N, d, 1.0 if family == "src_zipf" else 0.0, weighted, dev)
@@ -158,12 +158,12 @@ def main():
                     torch.cuda.empty_cache()
         for B in (8, 256):
             rowptr, col, val, E, dmax, N = make_qws_cousage(B, dev)
-            for F in (256,):
+            for F, T in ((256, 2048),):   # the split path at F = 256's automatic threshold, also for B = 8 (< 2^22 edges)
                 x = torch.empty(N, F, device=dev).uniform_(-1, 1)
                 y = torch.empty(N, F, device=dev)
-                ms = time_point(rowptr, col, val, x, y, 7, flush, args.one_launch, long_row_threshold=ops.split_threshold(F))
+                ms = time_point(rowptr, col, val, x, y, 7, flush, args.one_launch, long_row_threshold=T)
                 ms0 = time_point(rowptr, col, val, x, y, 7, flush, args.one_launch, long_row_threshold=0)
-                emit(record("qws_cousage", E, N, F, True, ms, max_in_degree=dmax, copies=B, long_row_threshold=ops.split_threshold(F),
+                emit(record("qws_cousage", E, N, F, True, ms, max_in_degree=dmax, copies=B, long_row_threshold=T,
                             ms_without_split=ms0))
 
 

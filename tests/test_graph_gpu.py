@@ -339,3 +339,51 @@ def test_long_row_split_hub_destinations():
     assert ((ym.double() - want).abs() / want.abs().clamp(min=1)).max() <= 1e-5
     y0 = ops.spmm_csr(rp, col, val, x.cuda(), long_row_threshold=0).cpu()  # unsplit path: whole matrix bit-identical
     assert torch.equal(y0, ref)
+
+
+def test_automatic_long_row_threshold():
+    """With long_row_threshold=None the library picks the threshold: a graph of exactly 2^22 edges is split at 256 edges
+    for F = 64 (lane groups narrower than a warp) and at 2048 for F = 128, one edge fewer is not split at all.  The graph
+    has rows of 257..2,000 edges and rows above 2,048, so the three explicit choices give three different results."""
+    from gnnpn_sc_b200 import _lib, ops
+    g = torch.Generator().manual_seed(17)
+    n, E = 1 << 16, 1 << 22
+    deg = torch.zeros(n, dtype=torch.int64)
+    mid = torch.randperm(n, generator=g)[:304]
+    deg[mid[:300]] = torch.randint(257, 2001, (300,), generator=g)
+    deg[mid[300:]] = torch.randint(3000, 10001, (4,), generator=g)
+    rest = (deg == 0).nonzero().flatten()
+    deg[rest] = (E - int(deg.sum())) // rest.numel()
+    deg[rest[:E - int(deg.sum())]] += 1
+    assert int(deg.sum()) == E and int(deg[rest].max()) <= 256
+    col = torch.randint(0, n, (E,), generator=g, dtype=torch.int32).cuda()
+    val = (torch.rand(E, generator=g) + 0.05).cuda()
+
+    def csr(d):
+        rp = torch.zeros(n + 1, dtype=torch.int64)
+        rp[1:] = d.cumsum(0)
+        return rp.cuda(), col[:int(d.sum())], val[:int(d.sum())]
+
+    def default_call(rp, c, v, x):                                         # -> (y, kernels launched)
+        before = _lib.launch_count()
+        y = ops.spmm_csr(rp, c, v, x)
+        torch.cuda.synchronize()
+        return y, _lib.launch_count() - before
+
+    rp, c, v = csr(deg)
+    for F, T in ((64, 256), (128, 2048)):
+        x = torch.randn(n, F, generator=g).cuda()
+        y, k = default_call(rp, c, v, x)
+        assert k == 4                                                      # find, short rows, chunks, combine
+        assert torch.equal(y, ops.spmm_csr(rp, c, v, x, long_row_threshold=T))
+        for other in (256, 0):
+            if other != T:
+                assert not torch.equal(y, ops.spmm_csr(rp, c, v, x, long_row_threshold=other))
+    deg1 = deg.clone()
+    deg1[rest[0]] -= 1
+    rp1, c1, v1 = csr(deg1)
+    for F in (64, 128):
+        x = torch.randn(n, F, generator=g).cuda()
+        y, k = default_call(rp1, c1, v1, x)
+        assert k == 1
+        assert torch.equal(y, ops.spmm_csr(rp1, c1, v1, x, long_row_threshold=0))

@@ -143,7 +143,26 @@ def test_anyh_fold_reproduces_the_lstm_preactivations():
     assert ops.anyh_fold(w_ih, w_hh, b_ih, b_hh, w_emb, b_emb)[2] is None          # an encoder has no start token
 
 
-def test_split_threshold_policy():
-    from gnnpn_sc_b200 import ops
-    assert ops.split_threshold(32) == ops.SPLIT_THRESHOLD_NARROW and ops.split_threshold(64) == ops.SPLIT_THRESHOLD_NARROW
-    assert ops.split_threshold(128) == ops.SPLIT_THRESHOLD and ops.SPLIT_THRESHOLD_NARROW < ops.SPLIT_THRESHOLD
+def test_long_row_threshold_policy():
+    """The aggregation's automatic long-row threshold, read through the library's workspace query: no split below 2^22
+    edges, 256 where a lane group is narrower than a warp (F <= 64), 2048 above.  Argument errors are refused before any
+    CUDA call."""
+    from gnnpn_sc_b200 import _lib
+    L = _lib.lib()
+    ws = L.gnnpn_spmm_csr_workspace_bytes
+    for F in (32, 64, 128, 256):
+        assert ws(2**22 - 1, F, -1) == 0
+        assert ws(2**22, F, -1) == ws(2**22, F, 256 if F <= 64 else 2048) > 0
+        assert ws(2**22, F, 0) == ws(100, F, 0) == 0
+    assert ws(2**22, 64, 256) != ws(2**22, 64, 2048)
+    assert ws(2**22, 64, 31) == 0
+    p = 1 << 12                                            # any 256-byte aligned address: nothing is dereferenced
+    need = ws(2**22, 64, 256)
+    call = lambda T, wsb: L.gnnpn_spmm_csr_f32(p, p, p, p, 64, p, 64, 1000, 2**22, 64, 0.0, 0, None, None, None, 0, T, p,
+                                               wsb, None)
+    before = _lib.launch_count()
+    for T in (1, 31):
+        assert call(T, need) == -2                         # GNNPN_ESHAPE
+    assert call(256, need - 1) == -4                       # GNNPN_EWORKSPACE
+    assert call(-1, need - 1) == -4                        # the automatic choice splits here too
+    assert _lib.launch_count() == before
