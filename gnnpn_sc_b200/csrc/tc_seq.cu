@@ -3,15 +3,21 @@
 // (modelPN.py:157-158,191,205) and the decode loop modelPN.py:204-239.
 //
 // A CTA owns 128 composition instances for the whole scan, so the step-to-step dependency is CTA-local:
-//   * A operand  [h | x]  lives in SHARED MEMORY as fp16 hi/lo pairs (error-compensated 3xFP16, fp32 accumulate:
-//     a.w ~= a_lo.w_hi + a_hi.w_hi + a_hi.w_lo) in the 128B-swizzled K-major UMMA layout; the epilogue of step t
-//     writes h'(t) there directly -- h never goes through global memory between steps;
+//   * A operand  [h | x]  as fp16 hi/lo pairs (error-compensated 3xFP16, fp32 accumulate:
+//     a.w ~= a_lo.w_hi + a_hi.w_hi + a_hi.w_lo).  The h part is DOUBLE-BUFFERED: step t reads buffer t&1 and its
+//     epilogue writes h'(t) straight into buffer (t+1)&1 -- h never goes through global memory between steps, and
+//     nothing is staged or copied at the step boundary.  h_hi sits in TENSOR MEMORY (columns [256,384) and
+//     [384,512), lane = instance, two halfs per column; the a_hi MMAs, 8 of every 12, read A from there), h_lo in
+//     shared memory (two 64 KB blocks in the 128B-swizzled K-major UMMA layout).  The x block is single-buffered;
 //   * B operand (the 4H x (H+F) folded weights, fp16 hi/lo, 1.1 MB, L2-resident) is streamed by TMA through a
 //     ring of 8 slots; a slot holds one (N tile, k block, hi|lo) box, each CTA of the pair 8 KB = half its gate columns;
 //   * accumulators: two 128-column TMEM buffers (N tile = 128 gate columns = 32 hidden units), so the
 //     epilogue of tile j overlaps the MMAs of tile j+1;
-//   * h'(t) of tiles 0..6 cannot be written over A while the MMAs of step t still read it: it is staged in the
-//     other 256 TMEM columns (tcgen05.st) and copied to shared memory once the last MMA of the step has retired.
+//   * step t+1 starts one k-block at a time: k-block kb of h'(t) is complete once tiles 2kb and 2kb+1 of both CTAs
+//     have been written, and tile 0 of step t+1 issues each k-block's 12 MMAs behind its own barrier, so k-blocks
+//     0..2 run under the epilogue of tile 7.  Writing buffer (t+1)&1 needs no barrier of its own: the epilogue of
+//     tile j of step t waits for that tile's commit, which retires after every MMA of step t-1, the buffer's last
+//     readers.
 // Warp roles: 0 = TMA producer, 1 = MMA issuer, 2 = TMEM allocator, 3 = x producer (encoder inputs),
 // 4..19 = epilogue (TMEM lane quarter = warp & 3, column group = (warp - 4) / 4).
 //
@@ -57,12 +63,13 @@ constexpr int RING = 8;                    // weight ring slots
 constexpr int SLOT_ROWS = TILE_N / 2;      // each CTA of the pair loads half of a tile's gate columns
 constexpr int SLOT_BYTES = BLK_BYTES / 2;  // [64 gate columns x 64 halfs]
 constexpr int RING_BYTES = RING * SLOT_BYTES;
-constexpr int TMEM_COLS = 512;             // [0,256): 2 accumulator buffers; [256,512): h' staging
-constexpr int STAGE_COL0 = 256;
+constexpr int TMEM_COLS = 512;             // [0,256): 2 accumulator buffers; [256,512): 2 h_hi buffers
+constexpr int AHI_COL0 = 2 * TILE_N;
+constexpr int AHI_COLS = kH / 2;           // 128: two halfs per 32-bit column
 
-constexpr uint32_t OFF_A_HI = 0;
-constexpr uint32_t OFF_A_LO = OFF_A_HI + KB_H * BLK_BYTES;
-constexpr uint32_t OFF_AX_HI = OFF_A_LO + KB_H * BLK_BYTES;
+constexpr uint32_t A_LO_BYTES = KB_H * BLK_BYTES;                // one h_lo buffer, [128 rows x kH halfs]
+constexpr uint32_t OFF_A_LO = 0;                                 // two h_lo buffers
+constexpr uint32_t OFF_AX_HI = OFF_A_LO + 2 * A_LO_BYTES;
 constexpr uint32_t OFF_AX_LO = OFF_AX_HI + BM * XROW_BYTES;
 constexpr uint32_t OFF_RING = OFF_AX_LO + BM * XROW_BYTES;
 constexpr uint32_t OFF_HBUF = OFF_RING + RING_BYTES;      // [128 rows x 32 fp32] h' tile for the TMA store
@@ -214,16 +221,15 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
   auto empty_bar = [&](int s) { return bar0 + 8u * (RING + s); };
   auto tfull_bar = [&](int b) { return bar0 + 8u * (2 * RING + b); };
   auto tempty_bar = [&](int b) { return bar0 + 8u * (2 * RING + 2 + b); };
-  const uint32_t a_ready_bar = bar0 + 8u * (2 * RING + 4);
+  const uint32_t a_ready_bar = bar0 + 8u * (2 * RING + 4);   // x(t+1) is in the x block
   const uint32_t mma_done_bar = bar0 + 8u * (2 * RING + 5);
   const uint32_t hfull_bar = bar0 + 8u * (2 * RING + 6);
   const uint32_t hempty_bar = bar0 + 8u * (2 * RING + 7);
   const uint32_t tmem_slot = bar0 + 8u * (2 * RING + 8);
-  const uint32_t h_ready_bar = bar0 + 8u * (2 * RING + 9);   // decoder: h'(t) is in the A tiles (the pointer phase follows)
+  auto h_ready_bar = [&](int kb) { return bar0 + 8u * (2 * RING + 9 + kb); };   // k-block kb of h'(t) is in A
   const uint32_t rank = cluster_ctarank();
   // barriers the MMA issuer (rank 0) waits on collect arrivals from both CTAs of the pair
   const uint32_t a_ready_remote = mapa_rank(a_ready_bar, 0);
-  const uint32_t h_ready_remote = mapa_rank(h_ready_bar, 0);
   float* sbias = reinterpret_cast<float*>(sgen + OFF_BIAS);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -240,8 +246,8 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < RING; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
     for (int b = 0; b < 2; ++b) { mbar_init(tfull_bar(b), 1); mbar_init(tempty_bar(b), 2 * EPI_WARPS); }
-    mbar_init(a_ready_bar, 2 * (EPI_WARPS + (DEC ? 0 : 1)));
-    mbar_init(h_ready_bar, 2 * EPI_WARPS);
+    mbar_init(a_ready_bar, DEC ? 2 * EPI_WARPS : 2);        // decoder: the epilogue writes x; encoder: warp 3
+    for (int kb = 0; kb < KB_H; ++kb) mbar_init(h_ready_bar(kb), 2 * EPI_WARPS);
     mbar_init(mma_done_bar, 1);
     mbar_init(hfull_bar, EPI_WARPS);
     mbar_init(hempty_bar, 1);
@@ -249,31 +255,11 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
   }
   if (warp == 2) tmem_alloc_cg2(tmem_slot, TMEM_COLS);
 
-  // ---- initial A operand: h(-1) split to fp16 hi/lo (zeros for the encoder), x block of step 0
-  {
-    for (int it = threadIdx.x; it < BM * 32; it += THREADS) {       // (row, 8-unit chunk)
-      const int r = FUSED ? (it & (BM - 1)) : (it >> 5), ch = FUSED ? (it >> 7) : (it & 31);
-      uint32_t hi[4] = {0, 0, 0, 0}, lo[4] = {0, 0, 0, 0};
-      if (FUSED ? cta_ok : (p.h0 && m0 + r < p.n)) {
-        float hv[8];
-        if (FUSED) {
-          // decoder start state = the encoder's last hidden state (modelPN.py:191,205): position L-1 of the block
-          ldg256(p.pa.enc_out + enc_blk_off(blockIdx.x, p.L, p.L - 1, ch >> 2, ch & 3) + r * 8, hv);
-        } else {
-          ldg256(p.h0 + (m0 + r) * p.h0_ld + ch * 8, hv);
-        }
-        split_f16x8(hv, hi, lo);
-      }
-      const uint32_t off = (uint32_t)(ch >> 3) * BLK_BYTES + sw128_off(r, ch & 7);
-      st_shared_v4(sbase + OFF_A_HI + off, hi[0], hi[1], hi[2], hi[3]);
-      st_shared_v4(sbase + OFF_A_LO + off, lo[0], lo[1], lo[2], lo[3]);
-    }
-    // transformed biases: (i,f,o) * -log2e, g * -2log2e
-    for (int i = threadIdx.x; i < 2 * kG; i += THREADS) {
-      const int col = i & (kG - 1);
-      const float b = __ldg((i < kG ? p.bias0 : p.bias) + col);
-      sbias[i] = b * ((col & 3) == 2 ? -2.0f * kLog2e : -kLog2e);
-    }
+  // ---- transformed biases: (i,f,o) * -log2e, g * -2log2e; x block of step 0 (h(-1) is written by the epilogue warps)
+  for (int i = threadIdx.x; i < 2 * kG; i += THREADS) {
+    const int col = i & (kG - 1);
+    const float b = __ldg((i < kG ? p.bias0 : p.bias) + col);
+    sbias[i] = b * ((col & 3) == 2 ? -2.0f * kLog2e : -kLog2e);
   }
 
   // load_x_rows is called through this lambda: calling it directly at the two sites changes the register allocation
@@ -344,16 +330,23 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
       const uint32_t leader = elect_one();
       const uint32_t idesc = idesc_f16(2 * BM, TILE_N);
       auto mma = [&](uint32_t d, uint64_t a, uint64_t b, uint32_t acc) { mma_f16_ss_cg2(d, a, b, idesc, acc); };
+      auto mma_ts = [&](uint32_t d, uint32_t a, uint64_t b) { mma_f16_ts_cg2(d, a, b, idesc, 1u); };
       const uint64_t ax_hi = smem_desc_k_sw32(sbase + OFF_AX_HI), ax_lo = smem_desc_k_sw32(sbase + OFF_AX_LO);
       int s = 0; uint32_t ph = 0;
       uint32_t uses = 0;                                   // per-buffer use count = uses >> 1 (tiles alternate)
       const bool prof = p.prof != nullptr;
       long long w_aready = 0, w_tempty = 0, w_full = 0;
       const long long t_begin = clock64();
-      auto mma_h = [&](uint32_t d) {                     // h part of one tile: 8 ring slots, 48 MMAs
+      // h part of one tile of step t: 8 ring slots, 48 MMAs.  The first tile of a step waits for each k-block of h(t-1).
+      auto mma_h = [&](uint32_t d, int t, bool first) {
+        const uint32_t hb = (uint32_t)t & 1u;
         for (int kb = 0; kb < KB_H; ++kb) {
-          const uint64_t a_hi = smem_desc_k_sw128(sbase + OFF_A_HI + kb * BLK_BYTES);
-          const uint64_t a_lo = smem_desc_k_sw128(sbase + OFF_A_LO + kb * BLK_BYTES);
+          if (first) {
+            mbar_wait_t<true>(h_ready_bar(kb), hb, prof, w_aready);
+            tc_fence_after();
+          }
+          const uint32_t a_hi = tmem_base + (uint32_t)(AHI_COL0 + hb * AHI_COLS + kb * 32);   // 64 halfs = 32 columns
+          const uint64_t a_lo = smem_desc_k_sw128(sbase + OFF_A_LO + hb * A_LO_BYTES + kb * BLK_BYTES);
           mbar_wait_t(full_bar(s), ph, prof, w_full);
           tc_fence_after();
           const uint64_t b_hi = smem_desc_k_sw128(sbase + OFF_RING + s * SLOT_BYTES);
@@ -363,7 +356,7 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
               mma(d, a_lo + (uint64_t)(ks * 2), b_hi + (uint64_t)(ks * 2), (uint32_t)((kb | ks) != 0));
 #pragma unroll
             for (int ks = 0; ks < 4; ++ks)
-              mma(d, a_hi + (uint64_t)(ks * 2), b_hi + (uint64_t)(ks * 2), 1u);
+              mma_ts(d, a_hi + (uint32_t)(ks * 8), b_hi + (uint64_t)(ks * 2));
             mma_commit_cg2(empty_bar(s));
           }
           __syncwarp();
@@ -374,7 +367,7 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
           if (leader) {
 #pragma unroll
             for (int ks = 0; ks < 4; ++ks)
-              mma(d, a_hi + (uint64_t)(ks * 2), b_lo + (uint64_t)(ks * 2), 1u);
+              mma_ts(d, a_hi + (uint32_t)(ks * 8), b_lo + (uint64_t)(ks * 2));
             mma_commit_cg2(empty_bar(s));
           }
           __syncwarp();
@@ -401,16 +394,12 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
         int nt0 = 0;
         if (DEC) {
           // Only the K = 16 x part of a step depends on the pick.  TMEM has two accumulator buffers, so the h parts of
-          // tiles 0 and 1 (96 of the step's 408 MMAs) are issued as soon as h'(t-1) is in the A tiles, i.e. while the
+          // tiles 0 and 1 (96 of the step's 408 MMAs) are issued as soon as h'(t-1) is in A, i.e. while the
           // pointer phase of step t-1 still runs; their x parts follow once the picked rows are in the x block.
-          if (t > 0) {
-            mbar_wait_t<true>(h_ready_bar, (uint32_t)(t - 1) & 1u, prof, w_aready);
-            tc_fence_after();
-          }
           for (int b = 0; b < 2; ++b) {
             mbar_wait_t<true>(tempty_bar(b), (((uses + b) >> 1) & 1u) ^ 1u, prof, w_tempty);
             tc_fence_after();
-            mma_h(tmem_base + (uint32_t)(b * TILE_N));
+            mma_h(tmem_base + (uint32_t)(b * TILE_N), t, b == 0);
           }
           if (t > 0) {
             mbar_wait_t<true>(a_ready_bar, (uint32_t)(t - 1) & 1u, prof, w_aready);   // x(t) is in the x block
@@ -419,16 +408,17 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
           for (int b = 0; b < 2; ++b) mma_x(tmem_base + (uint32_t)(b * TILE_N), b, false);
           uses += 2;
           nt0 = 2;
-        } else if (t > 0) {
-          mbar_wait_t<true>(a_ready_bar, (uint32_t)(t - 1) & 1u, prof, w_aready);  // h'(t-1), x(t) are in smem
-          tc_fence_after();
         }
         for (int nt = nt0; nt < N_TILES; ++nt, ++uses) {
           const int buf = nt & 1;
           mbar_wait_t<true>(tempty_bar(buf), ((uses >> 1) & 1u) ^ 1u, prof, w_tempty);
           tc_fence_after();
           const uint32_t d = tmem_base + (uint32_t)(buf * TILE_N);
-          mma_h(d);
+          mma_h(d, t, nt == 0);
+          if (!DEC && nt == 0 && t > 0) {
+            mbar_wait_t<true>(a_ready_bar, (uint32_t)(t - 1) & 1u, prof, w_aready);  // x(t) is in the x block
+            tc_fence_after();
+          }
           mma_x(d, buf, nt == N_TILES - 1);
         }
       }
@@ -527,6 +517,30 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
       for (int u = 0; u < CHK; ++u)
         if (u < N) ldg256_stream(e_in + ((int64_t)t_ * N + u) * ENC_BLK_ROW + nt_ * ENC_BLK_TILE, ea[u], eb[u], pol_stream);
     };
+    // this thread's 8 units of tile nt -> h buffer nb: hi into TMEM (4 columns), lo into shared memory.  After the odd
+    // tile of k-block kb the warp has written its whole part of the k-block, and says so to the MMA issuer.
+    auto publish_h = [&](uint32_t nb, int nt, const float* hv) {
+      uint32_t hi[4], lo[4];
+      split_f16x8(hv, hi, lo);
+      tmem_st_32x32_x4(t_lane + (uint32_t)(AHI_COL0 + nb * AHI_COLS + nt * 16 + grp * 4), hi);
+      st_shared_v4(sbase + OFF_A_LO + nb * A_LO_BYTES + (uint32_t)(nt >> 1) * BLK_BYTES + sw128_off(r, (nt & 1) * 4 + grp),
+                   lo[0], lo[1], lo[2], lo[3]);
+      if (nt & 1) {
+        tmem_st_wait();
+        fence_proxy_async_smem();
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive_cluster(mapa_rank(h_ready_bar(nt >> 1), 0));
+      }
+    };
+    // h(-1) into buffer 0: zeros for the encoder; the decoder starts from the encoder's last hidden state
+    // (modelPN.py:191,205), with blocked encodings position L-1 of the block
+    for (int nt = 0; nt < N_TILES; ++nt) {
+      float hv[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+      if (FUSED && cta_ok) ldg256(e_in + (int64_t)(p.L - 1) * ENC_BLK_ROW + nt * ENC_BLK_TILE, hv);
+      else if (!FUSED && p.h0 && ok) ldg256(p.h0 + m * p.h0_ld + nt * 32 + grp * 8, hv);
+      publish_h(0u, nt, hv);
+    }
     if (do_dot) request_rows(0, 0);
     uint32_t uses = 0;
     const bool prof = p.prof != nullptr;
@@ -564,6 +578,7 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
         if (lane == 0) mbar_arrive_cluster(mapa_rank(tempty_bar(buf), 0));
         float cn[8], hn[8];
         lstm_cell8(v, bias4 + u0, c_old, cn, hn);
+        if (!last) publish_h((uint32_t)(t + 1) & 1u, nt, hn);
         if (!last && keep_c) {
           stg128_hint(c_t, cn[0], cn[1], cn[2], cn[3], pol_keep);
           stg128_hint(c_t + BM * 4, cn[4], cn[5], cn[6], cn[7], pol_keep);
@@ -589,34 +604,6 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
           fence_proxy_async_smem();
           __syncwarp();
           if (lane == 0) mbar_arrive(hfull_bar);
-        }
-        uint32_t pk[8];                                  // {hi01, hi23, hi45, hi67, lo01, lo23, lo45, lo67}
-        split_f16x8(hn, pk, pk + 4);
-        if (it < N_TILES - 1) {
-          tmem_st_32x32_x8(t_lane + (uint32_t)(STAGE_COL0 + nt * 32 + grp * 8), pk);
-        } else {
-          // tile 7's accumulators were committed after the last MMA of the step: nothing reads A any more.
-          const uint32_t off7 = (uint32_t)(nt >> 1) * BLK_BYTES + sw128_off(r, (nt & 1) * 4 + grp);
-          st_shared_v4(sbase + OFF_A_HI + off7, pk[0], pk[1], pk[2], pk[3]);
-          st_shared_v4(sbase + OFF_A_LO + off7, pk[4], pk[5], pk[6], pk[7]);
-          tmem_st_wait();
-#pragma unroll
-          for (int jj = 1; jj < N_TILES; ++jj) {
-            const int j = (nt + jj) & (N_TILES - 1);        // the seven tiles staged earlier in this step
-            uint32_t sg[8];
-            tmem_ld_32x32_x8(t_lane + (uint32_t)(STAGE_COL0 + j * 32 + grp * 8), sg);
-            tmem_ld_wait8(sg);
-            const uint32_t off = (uint32_t)(j >> 1) * BLK_BYTES + sw128_off(r, (j & 1) * 4 + grp);
-            st_shared_v4(sbase + OFF_A_HI + off, sg[0], sg[1], sg[2], sg[3]);
-            st_shared_v4(sbase + OFF_A_LO + off, sg[4], sg[5], sg[6], sg[7]);
-          }
-          if (DEC) {
-            // h'(t) is in the A tiles: the MMA warp may start the h parts of the next step's first two tiles now
-            fence_proxy_async_smem();
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_cluster(h_ready_remote);
-          }
         }
         if (do_dot) {
           // canonical dot (pointer.cuh): s[nt][g] = fma chain over the 8 units, p[g] sequential over the tiles
@@ -683,10 +670,12 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
         }
         if (prof) w_ptr += clock64() - tp0;
       }
-      fence_proxy_async_smem();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_cluster(a_ready_remote);
+      if (DEC) {                                          // x(t+1) is in the x block
+        fence_proxy_async_smem();
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive_cluster(a_ready_remote);
+      }
     }
     if (prof && warp == 4 && lane == 0) {
       unsigned long long* o = p.prof + (size_t)blockIdx.x * 16;

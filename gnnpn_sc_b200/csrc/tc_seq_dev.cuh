@@ -79,6 +79,17 @@ __device__ __forceinline__ void mma_f16_ss_cg2(uint32_t tmem_d, uint64_t adesc, 
       "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
       "}" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
 }
+// the same with A read from tensor memory: lane = row (each CTA of the pair holds its 128 rows at a_tmem), 32-bit
+// column c = halfs 2c (low 16 bits) and 2c+1 of the K-major row
+__device__ __forceinline__ void mma_f16_ts_cg2(uint32_t tmem_d, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc,
+                                               uint32_t accumulate) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], [%1], %2, %3, p;\n\t"
+      "}" ::"r"(tmem_d), "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
+}
 // arrives (once all previously issued MMAs retire) on the barrier at this CTA-relative offset in BOTH CTAs of the pair
 __device__ __forceinline__ void mma_commit_cg2(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
@@ -105,21 +116,11 @@ __device__ __forceinline__ void fence_proxy_async_smem() {
 __device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
   asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
 }
-__device__ __forceinline__ void tmem_st_32x32_x8(uint32_t taddr, const uint32_t* r) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"r"(taddr), "r"(r[0]),
-               "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]) : "memory");
+__device__ __forceinline__ void tmem_st_32x32_x4(uint32_t taddr, const uint32_t* r) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};" ::"r"(taddr), "r"(r[0]), "r"(r[1]),
+               "r"(r[2]), "r"(r[3]) : "memory");
 }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void tmem_ld_32x32_x8(uint32_t taddr, uint32_t* r) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "r"(taddr) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait8(uint32_t* r) {
-  asm volatile("tcgen05.wait::ld.sync.aligned;"
-               : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7])
-               :: "memory");
-}
 __device__ __forceinline__ void tma_store_3d(const CUtensorMap* map, uint32_t smem_src, int c0, int c1, int c2) {
   asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];" ::"l"(map),
                "r"(smem_src), "r"(c0), "r"(c1), "r"(c2) : "memory");
