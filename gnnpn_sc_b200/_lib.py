@@ -39,6 +39,10 @@ SIGNATURES = {
     "gnnpn_pn_workspace_bytes": (C.c_size_t, [_i64, _i]),
     "gnnpn_pn_decode_greedy_f32": (_i, [_p, _p, _p, _p, _f, _p, _i, _p, _i, _f, _i64, _i, _i, _i, _i, _i,
                                         _p, _p, _p, _p, _p, _p, _p, C.c_size_t, _i, _p]),
+    "gnnpn_pn_rollouts_workspace_bytes": (C.c_size_t, [_i64, _i, _i]),
+    "gnnpn_pn_decode_rollouts_f32": (_i, [_p, _p, _p, _p, _f, _p, _i, _p, _i, _f, _i64, _i, _i, _i, _i, _i,
+                                          _p, _p, _p, _p, _p, _p, C.c_size_t, _i, _i, _p]),
+    "gnnpn_pn_best_rollout_f32": (_i, [_p, _p, _i64, _i, _i, _i, _i, _i, _i, _p, _p, _p, _p, _p]),
     "gnnpn_pn_train_forward_workspace_bytes": (C.c_size_t, [_i64, _i, _i, _i, _i, _i]),
     "gnnpn_pn_train_forward_f32": (_i, [_p, _p, _p, _p, _p, _p, _f, _i, _f, _i64, _i, _i, _i, _i, _i] + [_p] * 10 +
                                    [C.c_size_t, _p]),
@@ -99,7 +103,7 @@ def lib():
                 fn = getattr(h, name)          # AttributeError if the ABI lost a symbol
                 fn.restype = res
                 fn.argtypes = args
-            if h.gnnpn_abi_version() != 11:
+            if h.gnnpn_abi_version() != 12:
                 raise GnnpnError("libgnnpn_b200.so ABI version mismatch")
             _lib = h
     return _lib

@@ -1,5 +1,5 @@
-// Pointer-network entry points: weight packing, encoder scan, fused greedy decode, composition objective / reward
-// (the dense logits are in pn_general.cu).
+// Pointer-network entry points: weight packing, encoder scan, fused greedy decode and its rollouts, composition
+// objective / reward and the best rollout (the dense logits are in pn_general.cu).
 #include <math.h>
 #include <cuda_fp16.h>
 #include "lstm_step.cuh"
@@ -104,11 +104,14 @@ int launch_pointer_steps(const PointerStepArgs& pa, int K, const float* dec_h, c
 // ---------------------------------------------------------------------------
 constexpr int kMaxTasks = 512;
 
-__global__ void reward_kernel(const float* __restrict__ inputs, const int32_t* __restrict__ idx, int64_t n,
-                              int L, int F, int K, int tag, int32_t* __restrict__ viol_out,
-                              float* __restrict__ obj_out, float* __restrict__ rew_out) {
-  const int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (b >= n) return;
+struct Reward {
+  int viol;        // violated global constraints (the "Low" reward)
+  float obj;       // objFunc
+  float high;      // float32(round(viol + obj, 5)) (the "High" reward)
+};
+// the objective of instance b's picks idx[k * n + b]
+__device__ __forceinline__ Reward composition_reward(const float* __restrict__ inputs, const int32_t* __restrict__ idx,
+                                                     int64_t n, int64_t b, int L, int F, int K, int tag) {
   float q0s[kMaxTasks];
   float prod[2] = {1.f, 1.f};
   float min_q1 = INFINITY;
@@ -131,12 +134,40 @@ __global__ void reward_kernel(const float* __restrict__ inputs, const int32_t* _
   obj = __fadd_rn(obj, 1.0f);
   obj = __fsub_rn(obj, min_q1);
   obj = __fdiv_rn(obj, 2.0f);
-  if (viol_out) viol_out[b] = viol;
-  if (obj_out) obj_out[b] = obj;
-  if (rew_out) {
-    const double v = (double)viol + (double)obj;          // python: round(violate + objFunc, 5)
-    rew_out[b] = (float)(rint(v * 1e5) / 1e5);
+  const double v = (double)viol + (double)obj;            // python: round(violate + objFunc, 5)
+  return Reward{viol, obj, (float)(rint(v * 1e5) / 1e5)};
+}
+
+__global__ void reward_kernel(const float* __restrict__ inputs, const int32_t* __restrict__ idx, int64_t n,
+                              int L, int F, int K, int tag, int32_t* __restrict__ viol_out,
+                              float* __restrict__ obj_out, float* __restrict__ rew_out) {
+  const int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (b >= n) return;
+  const Reward r = composition_reward(inputs, idx, n, b, L, F, K, tag);
+  if (viol_out) viol_out[b] = r.viol;
+  if (obj_out) obj_out[b] = r.obj;
+  if (rew_out) rew_out[b] = r.high;
+}
+
+// Best of R rollouts idx [R, K, n] per instance: the lowest reward of `level` (0: Low, 1: High), the lowest rollout on a tie
+__global__ void best_rollout_kernel(const float* __restrict__ inputs, const int32_t* __restrict__ idx, int64_t n, int L,
+                                    int F, int K, int tag, int level, int R, int32_t* __restrict__ best_idx,
+                                    float* __restrict__ best_reward, int32_t* __restrict__ best_rollout,
+                                    float* __restrict__ rollout_rewards) {
+  const int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (b >= n) return;
+  float best = 0.f;
+  int best_r = 0;
+  for (int r = 0; r < R; ++r) {
+    const Reward rw = composition_reward(inputs, idx + (int64_t)r * K * n, n, b, L, F, K, tag);
+    const float s = level ? rw.high : (float)rw.viol;
+    if (rollout_rewards) rollout_rewards[(int64_t)r * n + b] = s;
+    if (r == 0 || s < best) { best = s; best_r = r; }
   }
+  const int32_t* src = idx + (int64_t)best_r * K * n;
+  for (int k = 0; k < K; ++k) best_idx[(int64_t)k * n + b] = src[(int64_t)k * n + b];
+  best_reward[b] = best;
+  best_rollout[b] = best_r;
 }
 
 // raw input range check: *flag |= 1 if any value is NaN / inf or has |x| >= limit
@@ -165,7 +196,7 @@ __global__ void enc_unblock_kernel(const float* __restrict__ blk, int64_t n, int
 // "persistent" option says; it runs when a workspace is given and it takes the batch (the reference trains with 128).
 // Otherwise forced picks are replayed on the strict-fp32 FFMA per-step kernels (kStep); free-running is kUnsupported.
 ScanPlan plan_train_forward(int64_t n, int F, int N, bool has_workspace, bool forced) {
-  ScanPlan p = plan_scans(n, F, N, GNNPN_ENC_ROWMAJOR, has_workspace, 3);
+  ScanPlan p = plan_scans(n, F, N, GNNPN_ENC_ROWMAJOR, has_workspace, 1, 3);
   if (p.enc.kind != ScanKind::kColsplit) p.enc = p.dec = {forced ? ScanKind::kStep : ScanKind::kUnsupported, 0};
   return p;
 }
@@ -292,6 +323,41 @@ int gnnpn_pn_decode_greedy_f32(const float* inputs, const float* enc_out, float*
   return scan.kind == ScanKind::kPair ? tc_seq_decode(sa, scan.variant, st) : GNNPN_EUNSUPPORTED;
 }
 
+size_t gnnpn_pn_rollouts_workspace_bytes(int64_t n, int hidden, int rollouts) {
+  return hidden == kH && n >= 0 && rollouts >= 1 ? tc_seq_rollouts_workspace_bytes(n, rollouts) : 0;
+}
+
+// The decode of gnnpn_pn_decode_greedy_f32 `rollouts` times per instance in one launch of the persistent scan that
+// plan_scans picks for the n * rollouts rows; the encodings, c_state and latent are read by every rollout.
+int gnnpn_pn_decode_rollouts_f32(const float* inputs, const float* enc_out, const float* c_state,
+                                 const float* latent_win, float alpha, const float* packed,
+                                 int attention, const float* att_params, int use_tanh, float C,
+                                 int64_t n, int L, int in_features, int hidden, int K, int N,
+                                 float* dec_h, int32_t* idx_out, float* win_logits, float* win_probs,
+                                 const float* sample_uniform, void* workspace, size_t workspace_bytes,
+                                 int enc_layout, int rollouts, void* stream) {
+  GNNPN_REQUIRE(enc_layout == GNNPN_ENC_ROWMAJOR || enc_layout == GNNPN_ENC_BLOCKED128, GNNPN_ESHAPE);
+  GNNPN_REQUIRE(rollouts >= 1 && hidden == kH && in_features >= 1 && in_features <= 8, GNNPN_ESHAPE);
+  GNNPN_REQUIRE(K >= 1 && N >= 1 && N <= kMaxWindow && (int64_t)K * N == L, GNNPN_ESHAPE);
+  GNNPN_REQUIRE(inputs && enc_out && c_state && packed && idx_out && win_logits && win_probs, GNNPN_ENULL);
+  GNNPN_REQUIRE(dec_h || enc_layout == GNNPN_ENC_BLOCKED128, GNNPN_ENULL);   // optional only in the fused decoder
+  GNNPN_REQUIRE(sample_uniform || rollouts == 1, GNNPN_ENULL);
+  GNNPN_REQUIRE(n >= 0 && n * rollouts < (1ll << 31), GNNPN_ERANGE);
+  GNNPN_REQUIRE(attention == GNNPN_ATT_DOT, GNNPN_EUNSUPPORTED);
+  (void)att_params;
+  GNNPN_REQUIRE(aligned32(enc_out) && aligned32(dec_h) && aligned32(c_state) && aligned16(packed), GNNPN_EALIGN);
+  if (n == 0) return GNNPN_OK;
+  const ScanChoice scan = plan_scans(n, in_features, N, enc_layout, workspace != nullptr, rollouts).dec;
+  GNNPN_REQUIRE(scan.kind == ScanKind::kPair || scan.kind == ScanKind::kColsplit, GNNPN_EUNSUPPORTED);
+  GNNPN_REQUIRE(workspace_bytes >= tc_seq_rollouts_workspace_bytes(n, rollouts), GNNPN_EWORKSPACE);
+  SeqDecodeArgs sa{inputs, enc_out, const_cast<float*>(c_state), latent_win, alpha, packed, use_tanh, C, n, L,
+                   in_features, K, N, dec_h, idx_out, win_logits, win_probs, nullptr, nullptr, align_ws<float>(workspace)};
+  sa.rollouts = rollouts;                    // c_state is read, not written
+  sa.sampled = sample_uniform;
+  cudaStream_t st = (cudaStream_t)stream;
+  return scan.kind == ScanKind::kColsplit ? tc_colsplit_decode(sa, scan.variant, st) : tc_seq_decode(sa, scan.variant, st);
+}
+
 size_t gnnpn_pn_train_forward_workspace_bytes(int64_t n, int L, int in_features, int hidden, int K, int N) {
   (void)L; (void)K;
   if (hidden != kH || n < 0) return 0;
@@ -377,6 +443,19 @@ int gnnpn_pn_reward_f32(const float* inputs, const int32_t* idx, int64_t n, int 
   if (n == 0) return GNNPN_OK;
   reward_kernel<<<(unsigned)ceil_div(n, 128), 128, 0, (cudaStream_t)stream>>>(
       inputs, idx, n, L, in_features, K, tag, viol_out, obj_out, reward_high_out);
+  return after_launch();
+}
+
+int gnnpn_pn_best_rollout_f32(const float* inputs, const int32_t* idx, int64_t n, int L, int in_features, int K, int tag,
+                              int level, int rollouts, int32_t* best_idx, float* best_reward, int32_t* best_rollout,
+                              float* rollout_rewards, void* stream) {
+  GNNPN_REQUIRE(rollouts >= 1 && (level == 0 || level == 1), GNNPN_ESHAPE);
+  GNNPN_REQUIRE(K >= 1 && K <= kMaxTasks && (tag == 0 || tag == 1) && in_features >= tag + 8, GNNPN_ESHAPE);
+  GNNPN_REQUIRE(inputs && idx && best_idx && best_reward && best_rollout, GNNPN_ENULL);
+  GNNPN_REQUIRE(n >= 0, GNNPN_ESHAPE);
+  if (n == 0) return GNNPN_OK;
+  best_rollout_kernel<<<(unsigned)ceil_div(n, 128), 128, 0, (cudaStream_t)stream>>>(
+      inputs, idx, n, L, in_features, K, tag, level, rollouts, best_idx, best_reward, best_rollout, rollout_rewards);
   return after_launch();
 }
 

@@ -33,6 +33,21 @@ struct PointerStepArgs {
 };
 // The decode step k is passed separately so that the argument block itself can stay in constant memory.
 
+// Rollout r of a rollout launch (gnnpn_pn_decode_rollouts_f32): the encodings, latent and input rows are the instance's,
+// the outputs rollout r's slices of idx_out [R, K, n] and win_logits / win_probs [R, n, L].  Rollout 0 decodes with
+// a.uniform (NULL in a rollout launch: greedy), rollout r >= 1 draws with the uniforms [r-1] of `sampled` [R-1, K, n].
+// r = 0 leaves the block as it is, so a launch of one rollout is the plain decode.
+__device__ __forceinline__ PointerStepArgs rollout_args(const PointerStepArgs& a, int r, int K, const float* sampled) {
+  PointerStepArgs o = a;
+  if (r > 0) {
+    o.idx_out += (int64_t)r * K * a.n;
+    o.win_logits += (int64_t)r * a.n * a.L;
+    o.win_probs += (int64_t)r * a.n * a.L;
+    o.uniform = sampled + (int64_t)(r - 1) * K * a.n;
+  }
+  return o;
+}
+
 // argument block of the pointer steps over row-major encodings [n, L, kH]
 inline PointerStepArgs pointer_step_args(const float* enc_out, const float* latent_win, float alpha, int use_tanh, float C,
                                          int64_t n, int L, int N, int32_t* idx_out, float* win_logits, float* win_probs,

@@ -66,7 +66,12 @@ struct Params {
   const float* inputs; int64_t x_inst_ld;
   const float* bias0;      // [kG] gate-interleaved bias of step 0 (decoder: start-token bias)
   const float* bias;       // [kG] bias of steps >= 1
-  float* c;                // [n, kH] cell state: out (encoder), in/out (decoder)
+  const float* c;          // [n, kH] decoder: initial cell state
+  float* c_out;            // [n, kH] final cell state, or nullptr (rollout launches: c is shared by the rollouts)
+  // Rollout launches (decoder, as in tc_seq.cu): cluster -> (instance groups, rollout) with the rollouts of one set of
+  // groups adjacent; rollout r has its own dec_h slice and exchange scratch.  1 for every other launch.
+  int rollouts;
+  const float* sampled;    // [rollouts-1, K, n] uniforms of rollouts 1.. (pointer.cuh::rollout_args)
   const float* h0; int64_t h0_ld;          // decoder: initial hidden rows
   float* h_out; int64_t h_out_inst_ld;     // step t of instance m at h_out + m*ld + t*kH (enc_out / dec_h)
   __half* scratch;         // [groups][parity 2][hi|lo][128][kH] halfs
@@ -117,7 +122,10 @@ lstm_colsplit_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid
   auto ax_lo_off = [&](int g) { return ax_hi_off(g) + BM * XROW_BYTES; };
   const uint32_t rank = cluster_ctarank();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int64_t group0 = (int64_t)(blockIdx.x / CL) * G;                  // first instance group of this cluster
+  const int64_t cluster = blockIdx.x / CL;
+  const int roll = (int)(cluster % p.rollouts);
+  const int64_t group0 = (cluster / p.rollouts) * G;                      // first instance group of this cluster
+  const int64_t sgroup0 = cluster * G;                                    // its first group of the exchange scratch
   float* sbias = reinterpret_cast<float*>(sgen + LY::OFF_BIAS);
   constexpr int PUB0 = DEC ? 1 : 0;                    // publish index of h'(t) = t + PUB0
 
@@ -181,7 +189,7 @@ lstm_colsplit_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid
         const int par = j & 1;
         const uint32_t rph = (uint32_t)(j >> 1) & 1u;
         for (int g = 0; g < G; ++g) {
-          const int row_base = (int)(((group0 + g) * 2 + par) * 2) * BM;       // hi rows; lo rows follow BM later
+          const int row_base = (int)(((sgroup0 + g) * 2 + par) * 2) * BM;      // hi rows; lo rows follow BM later
           for (int kb = 0; kb < KB_H; ++kb) {
             const long long t0 = prof ? clock64() : 0;
             mbar_wait_cluster(a_rdy(g, par, kb), rph);                   // both producers of units [64kb, 64kb+64) have published
@@ -300,11 +308,12 @@ lstm_colsplit_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid
     const float4* const bias4_0 = reinterpret_cast<const float4*>(sbias) + grp * 8;
     const float4* const bias4_1 = reinterpret_cast<const float4*>(sbias + TILE_N) + grp * 8;
     auto row_of = [&](int g) { return (group0 + g) * BM + r; };
+    float* const h_out = p.h_out + roll * p.n * p.h_out_inst_ld;      // this rollout's enc_out / dec_h
     // split 8 fp32 values to fp16 hi/lo and store them to scratch parity (j & 1) of group g
     auto stage = [&](int g, const float* hv, int j) {
       uint32_t pk[8];
       split_f16x8(hv, pk, pk + 4);
-      __half* dst = p.scratch + (size_t)(group0 + g) * (2 * 2 * BM * kH) + (size_t)(j & 1) * (2 * BM * kH) + (size_t)r * kH + u0;
+      __half* dst = p.scratch + (size_t)(sgroup0 + g) * (2 * 2 * BM * kH) + (size_t)(j & 1) * (2 * BM * kH) + (size_t)r * kH + u0;
       stg128_u(dst, pk[0], pk[1], pk[2], pk[3]);                    // hi rows
       stg128_u(dst + BM * kH, pk[4], pk[5], pk[6], pk[7]);          // lo rows
     };
@@ -351,7 +360,7 @@ lstm_colsplit_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid
       for (int g = 0; g < G; ++g) {
         const int64_t m = row_of(g);
         const bool ok = m < p.n;
-        float* const h_dst = p.h_out + (ok ? m : 0) * p.h_out_inst_ld + (int64_t)t * kH + u0;
+        float* const h_dst = h_out + (ok ? m : 0) * p.h_out_inst_ld + (int64_t)t * kH + u0;
         const long long t0 = prof ? clock64() : 0;
         mbar_wait(tfull(g), (uint32_t)t & 1u);
         const long long t1 = prof ? clock64() : 0;
@@ -398,8 +407,8 @@ lstm_colsplit_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid
           int fed = 0;
           if (b < p.n) {                                                        // warp-uniform
             float4 q0, q1;
-            ld_row8(p.h_out + b * p.h_out_inst_ld + (int64_t)t * kH, lane, q0, q1);
-            fed = pointer_step_warp(p.pa, t, b, q0, q1, lane);
+            ld_row8(h_out + b * p.h_out_inst_ld + (int64_t)t * kH, lane, q0, q1);
+            fed = pointer_step_warp(rollout_args(p.pa, roll, p.steps, p.sampled), t, b, q0, q1, lane);
           }
           if (t + 1 < p.steps) {
             if (lane < CL) {
@@ -438,7 +447,7 @@ lstm_colsplit_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid
 #pragma unroll
     for (int g = 0; g < G; ++g) {
       const int64_t m = row_of(g);
-      if (m < p.n) stg256(p.c + m * kH + u0, c[g]);
+      if (m < p.n && p.c_out) stg256(p.c_out + m * kH + u0, c[g]);
     }
     if (prof && warp == 4 && lane == 0) {
       unsigned long long* o = p.prof + (size_t)blockIdx.x * 8;
@@ -478,7 +487,7 @@ namespace cs {
 
 template <bool DEC, int G>
 static int launch(const float* packed, Params p, cudaStream_t st) {
-  const int64_t clusters = ceil_div(ceil_div(p.n, BM), G);
+  const int64_t clusters = ceil_div(ceil_div(p.n, BM), G) * p.rollouts;
   CUtensorMap maps[5];
   int rc = make_weight_maps(maps, packed, TILE_N);
   // exchange scratch as one 2-D fp16 tensor [groups * 2 parities * (hi|lo) * 128 rows, kH]; box = one k-block
@@ -506,7 +515,8 @@ int tc_colsplit_encode(const SeqEncodeArgs& a, int groups, cudaStream_t st) {
   p.n = a.n; p.steps = a.L; p.F = a.F; p.L = a.L;
   p.inputs = a.inputs; p.x_inst_ld = (int64_t)a.L * a.F;
   p.bias0 = p.bias = a.packed + kOffBias;
-  p.c = a.c_state;
+  p.c_out = a.c_state;
+  p.rollouts = 1;
   p.h_out = a.enc_out; p.h_out_inst_ld = (int64_t)a.L * kH;
   p.scratch = reinterpret_cast<__half*>(a.c_scratch);
   p.save_gates = a.save_gates; p.save_c = a.save_c;
@@ -522,7 +532,9 @@ int tc_colsplit_decode(const SeqDecodeArgs& a, int groups, cudaStream_t st) {
   p.n = a.n; p.steps = a.K; p.F = a.F; p.L = a.L;
   p.inputs = a.inputs; p.x_inst_ld = (int64_t)a.L * a.F;
   p.bias0 = a.packed + kOffStart; p.bias = a.packed + kOffBias;
-  p.c = a.c_state;
+  p.c = a.c_state; p.c_out = a.rollouts ? nullptr : a.c_state;
+  p.rollouts = a.rollouts ? a.rollouts : 1;
+  p.sampled = a.sampled;
   p.h0 = a.enc_out + (int64_t)(a.L - 1) * kH; p.h0_ld = (int64_t)a.L * kH;
   p.h_out = a.dec_h; p.h_out_inst_ld = (int64_t)a.K * kH;
   p.scratch = reinterpret_cast<__half*>(a.c_scratch);

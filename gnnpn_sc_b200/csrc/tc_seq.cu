@@ -87,8 +87,14 @@ struct SeqParams {
   const float* inputs; int64_t x_inst_ld;
   const float* bias0;      // [kG] gate-interleaved bias of step 0 (decoder: start-token bias)
   const float* bias;       // [kG] bias of steps >= 1
-  float* c;                // [n, kH]
+  const float* c;          // [n, kH] initial cell state (unless c_zero_init)
+  float* c_out;            // [n, kH] final cell state, or nullptr (rollout launches: c is shared by the rollouts)
   int c_zero_init;
+  // Rollout launches (decoder): clusters are ordered (instance pair block, rollout) with the rollouts of one block adjacent,
+  // so they run in the same wave and their window-row reads meet in L2.  Rollout r writes its own dec_h slice
+  // (h_out + r * n * h_out_inst_ld) and the pointer outputs of pointer.cuh::rollout_args.  1 for every other launch.
+  int rollouts;
+  const float* sampled;    // [rollouts-1, K, n] uniforms of rollouts 1.. (rollout_args)
   const float* h0; int64_t h0_ld;          // initial hidden rows or nullptr (zeros)
   float* h_out; int64_t h_out_inst_ld;     // step t of instance m at h_out + m*ld + t*kH
   PointerStepArgs pa;      // decoder only
@@ -117,14 +123,13 @@ __device__ __forceinline__ void store_ax(uint8_t* sgen, int rr, int f, float xv)
 
 // Pointer phase of decode step t for the 8 instances of one epilogue warp (rows rr0..rr0+7 of the CTA); see
 // pointer_steps_batched in pointer.cuh.
-__device__ __forceinline__ void pointer_phase(const SeqParams& p, int t, int rr0, int64_t m0, int lane, uint8_t* sgen
-                                              ) {
-  const PointerStepArgs& pa = p.pa;                 // stays in constant memory (p is a __grid_constant__ parameter)
+__device__ __forceinline__ void pointer_phase(const SeqParams& p, const PointerStepArgs& pa, const float* h_out, int t,
+                                              int rr0, int64_t m0, int lane, uint8_t* sgen) {
   const int64_t b0 = m0 + rr0;
   const int64_t left = p.n - b0;
   const int count = left <= 0 ? 0 : (left < BM / EPI_WARPS ? (int)left : BM / EPI_WARPS);
   const bool feed_next = t + 1 < p.steps;
-  const float* q_base = p.h_out + (int64_t)t * kH;
+  const float* q_base = h_out + (int64_t)t * kH;
   // the raw rows of the picks (next decoder inputs) of a whole pass are fetched together and written
   // to the x block after the last pass, so their latency is paid once
   float pend_x[kWarpInstances];
@@ -233,7 +238,10 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
   float* sbias = reinterpret_cast<float*>(sgen + OFF_BIAS);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int64_t m0 = (int64_t)blockIdx.x * BM;
+  const int cluster = (int)(blockIdx.x >> 1);
+  const int roll = cluster % p.rollouts;
+  const int blk = cluster / p.rollouts * 2 + (int)(blockIdx.x & 1);   // this CTA's block of 128 instances
+  const int64_t m0 = (int64_t)blk * BM;
   constexpr bool BLK = NR > 0;                         // blocked encodings (see the file header)
   constexpr bool FUSED = DEC && BLK;                   // pointer dots fused into the cell epilogue
   const bool cta_ok = m0 < p.n;                        // a pair's second CTA may be all padding
@@ -452,10 +460,10 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
         // windows keep the prefetched-but-unused footprint (dist x N x 16 KB per CTA) at the same ~24 MB: at N = 10 two tiles
         // ahead made the kernel re-read 35 % of the rows from DRAM (ncu: 13.1 GB for 9.7 GB algorithmic)
         const int dist = p.pa.N > 5 ? 1 : 2;
-        const float* const blk = p.pa.enc_out + enc_blk_off(blockIdx.x, p.L, 0, 0, 0);
+        const float* const rows = p.pa.enc_out + enc_blk_off(blk, p.L, 0, 0, 0);
         const int N = p.pa.N;
         for (int a = 0; a < dist; ++a)
-          for (int j = 0; j < N; ++j) bulk_prefetch_l2(blk + (int64_t)j * ENC_BLK_ROW + a * ENC_BLK_TILE, ENC_BLK_TILE * 4);
+          for (int j = 0; j < N; ++j) bulk_prefetch_l2(rows + (int64_t)j * ENC_BLK_ROW + a * ENC_BLK_TILE, ENC_BLK_TILE * 4);
         uint32_t uses = 0;
         for (int t = 0; t < p.steps; ++t) {
           for (int it = 0; it < N_TILES; ++it, ++uses) {
@@ -464,7 +472,7 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
             const int t2 = t + (it + dist >= N_TILES ? 1 : 0);
             if (t2 < p.steps)
               for (int j = 0; j < N; ++j)
-                bulk_prefetch_l2(blk + ((int64_t)t2 * N + j) * ENC_BLK_ROW + nt2 * ENC_BLK_TILE, ENC_BLK_TILE * 4);
+                bulk_prefetch_l2(rows + ((int64_t)t2 * N + j) * ENC_BLK_ROW + nt2 * ENC_BLK_TILE, ENC_BLK_TILE * 4);
           }
         }
       }
@@ -492,12 +500,13 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
     const int64_t m = m0 + r;
     const bool ok = m < p.n;
     const uint32_t t_lane = tmem_base + ((uint32_t)(q * 32) << 16);
-    float* const c_row = p.c + (ok ? m : 0) * kH;
-    float* const h_row = p.h_out + (ok ? m : 0) * p.h_out_inst_ld;
+    const float* const c_row = p.c + (ok ? m : 0) * kH;
+    float* const h_out = p.h_out ? p.h_out + roll * p.n * p.h_out_inst_ld : nullptr;     // this rollout's dec_h
+    float* const h_row = h_out + (ok ? m : 0) * p.h_out_inst_ld;
     // blocked scratch: float4 index (((cta*8 + nt)*4 + grp)*2 + half)*128 + row  -> a warp touches 512 contiguous bytes
     float* const c_blk = p.c_scr + ((int64_t)blockIdx.x * (BM * kH) + (int64_t)grp * (2 * BM * 4) + r * 4);
     // blocked encodings of this thread (8 consecutive units): + position * ENC_BLK_ROW + nt * ENC_BLK_TILE
-    const int64_t blk_thread = enc_blk_off(blockIdx.x, p.L, 0, 0, grp) + r * 8;
+    const int64_t blk_thread = enc_blk_off(blk, p.L, 0, 0, grp) + r * 8;
     float* const e_out = BLK && !DEC ? p.h_out + blk_thread : nullptr;
     const float* const e_in = FUSED ? p.pa.enc_out + blk_thread : nullptr;
     const int N = DEC ? p.pa.N : 0;
@@ -585,8 +594,8 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
         } else if (!last) {
           stg128(c_t, cn[0], cn[1], cn[2], cn[3]);
           stg128(c_t + BM * 4, cn[4], cn[5], cn[6], cn[7]);
-        } else if (ok) {
-          stg256(c_row + u0, cn);
+        } else if (ok && p.c_out) {
+          stg256(p.c_out + m * kH + u0, cn);
         }
         if (DEC) {
           if (ok && p.h_out) stg256(h_row + (int64_t)t * kH + u0, hn);        // dec_h is optional in the fused decoder
@@ -637,7 +646,8 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
         const long long tp0 = prof ? clock64() : 0;
         __threadfence_block();
         asm volatile("bar.sync 1, %0;" ::"n"(32 * EPI_WARPS) : "memory");
-        pointer_phase(p, t, (warp - 4) * (BM / EPI_WARPS), m0, lane, sgen);
+        pointer_phase(p, rollout_args(p.pa, roll, p.steps, p.sampled), h_out, t, (warp - 4) * (BM / EPI_WARPS), m0, lane,
+                      sgen);
         if (prof) w_ptr += clock64() - tp0;
       }
       if (FUSED) {
@@ -656,7 +666,7 @@ lstm_seq_kernel(const __grid_constant__ CUtensorMap map_wh_hi, const __grid_cons
           for (int j = 0; j < NR; ++j)
             d[j] = j < N ? __fadd_rn(__fadd_rn(acc[j], part[(0 * NR + j) * BM + r]),
                                       __fadd_rn(part[(1 * NR + j) * BM + r], part[(2 * NR + j) * BM + r])) : 0.f;
-          const int fed = pointer_finish_thread<NRA>(p.pa, t, m, ok, d);
+          const int fed = pointer_finish_thread<NRA>(rollout_args(p.pa, roll, p.steps, p.sampled), t, m, ok, d);
           if (t + 1 < p.steps) {                        // the fed row is the x block row of the next step
             float xv[8];
 #pragma unroll
@@ -705,7 +715,7 @@ int launch_seq(const float* packed, SeqParams p, cudaStream_t st) {
                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
       return GNNPN_ESHAPE;
   }
-  const unsigned grid = (unsigned)(ceil_div(p.n, 2 * BM) * 2);
+  const unsigned grid = (unsigned)(ceil_div(p.n, 2 * BM) * 2 * p.rollouts);
   if ((rc = prof_alloc(grid, 16, st, &p.prof))) return rc;
   rc = launch_cluster<lstm_seq_kernel<DEC, NR>>(grid, 2, THREADS, SMEM_BYTES, st, maps[0], maps[1], maps[2], maps[3], map_h,
                                                 p);
@@ -729,7 +739,8 @@ int tc_seq_encode(const SeqEncodeArgs& a, int nr, cudaStream_t st) {
   p.n = a.n; p.steps = a.L; p.L = a.L; p.F = a.F;
   p.inputs = a.inputs; p.x_inst_ld = (int64_t)a.L * a.F;
   p.bias0 = p.bias = a.packed + kOffBias;
-  p.c = a.c_state; p.c_zero_init = 1;
+  p.c = p.c_out = a.c_state; p.c_zero_init = 1;
+  p.rollouts = 1;
   p.h0 = nullptr; p.h0_ld = 0;
   p.h_out = a.enc_out; p.h_out_inst_ld = (int64_t)a.L * kH;
   p.c_scr = a.c_scratch;
@@ -742,6 +753,9 @@ int tc_seq_decode(const SeqDecodeArgs& a, int nr, cudaStream_t st) {
   p.inputs = a.inputs; p.x_inst_ld = (int64_t)a.L * a.F;
   p.bias0 = a.packed + kOffStart; p.bias = a.packed + kOffBias;
   p.c = a.c_state; p.c_zero_init = 0;
+  p.c_out = a.rollouts ? nullptr : a.c_state;
+  p.rollouts = a.rollouts ? a.rollouts : 1;
+  p.sampled = a.sampled;
   p.h_out = a.dec_h; p.h_out_inst_ld = (int64_t)a.K * kH;
   p.pa = pointer_step_args(a.enc_out, a.latent_win, a.alpha, a.use_tanh, a.C, a.n, a.L, a.N, a.idx_out, a.win_logits,
                            a.win_probs, a.forced_idx, a.sample_uniform);
@@ -787,12 +801,14 @@ int colsplit_groups(int64_t n) {
 // A/B reference).  The blocked encodings layout exists for the CTA-pair scan's fused decoder, so it is asked for only
 // when both scans are persistent, the batch is not the column-split scan's, and the window fits the fused decoder's
 // row capacity (N <= 10).  Encodings that are already blocked go to the CTA-pair scan before the column-split test.
-ScanPlan plan_scans(int64_t n, int F, int N, int layout, bool has_workspace, int persistent) {
+// A rollout launch decodes n * rollouts rows from the encodings of n instances: the encoder's choice and the layout come
+// from n, the decoder's from the n * rollouts rows and the layout the encoder wrote.
+ScanPlan plan_scans(int64_t n, int F, int N, int layout, bool has_workspace, int rollouts, int persistent) {
   ScanPlan p{{ScanKind::kStep, 0}, {ScanKind::kStep, 0}, GNNPN_ENC_ROWMAJOR};
   if (!has_workspace || F < 1 || F > 8) return p;
   if (persistent < 0) persistent = options().persistent.load(std::memory_order_relaxed);
   const bool blocked = layout == GNNPN_ENC_BLOCKED128;
-  const int g = colsplit_groups(n);
+  const int g = colsplit_groups(n), g_dec = colsplit_groups(n * rollouts);
   if (persistent == 3 && N >= 1 && N <= 10 && g == 0) p.layout = GNNPN_ENC_BLOCKED128;
   if (persistent & 1) {
     if (blocked) p.enc = {ScanKind::kPair, 1};
@@ -802,7 +818,7 @@ ScanPlan plan_scans(int64_t n, int F, int N, int layout, bool has_workspace, int
   if (persistent & 2) {
     if (blocked && N > 10) p.dec = {ScanKind::kUnsupported, 0};
     else if (blocked) p.dec = {ScanKind::kPair, N == 5 ? 5 : (N <= 8 ? 8 : 10)};
-    else if (g) p.dec = {ScanKind::kColsplit, std::min(g, 2)};
+    else if (g_dec) p.dec = {ScanKind::kColsplit, std::min(g_dec, 2)};
     else p.dec = {ScanKind::kPair, 0};
   }
   return p;

@@ -28,9 +28,10 @@ struct ScanPlan {
   int layout;     // the encodings layout gnnpn_pn_enc_layout reports for the batch
 };
 // Encoder and decoder choice for n instances with F input columns and windows of N candidates, whose encodings are in
-// `layout`, under the current "scan" and "scan_groups" options and the "persistent" bits (-1: the option).  A step
-// choice with blocked encodings is GNNPN_EUNSUPPORTED for the caller.
-ScanPlan plan_scans(int64_t n, int F, int N, int layout, bool has_workspace, int persistent = -1);
+// `layout`, under the current "scan" and "scan_groups" options and the "persistent" bits (-1: the option); the decoder of
+// a rollout launch runs `rollouts` rows per instance.  A step choice with blocked encodings is GNNPN_EUNSUPPORTED for
+// the caller.
+ScanPlan plan_scans(int64_t n, int F, int N, int layout, bool has_workspace, int rollouts = 1, int persistent = -1);
 
 // ---- host launch code shared by the two scans (tc_seq.cu) ---------------------------------------------------------
 // The packed block's fp16 hi/lo weights as TMA maps, boxes of `box_rows` gate columns: {h hi, h lo} (64 halfs,
@@ -92,8 +93,20 @@ struct SeqDecodeArgs {
   float* c_scratch;              // as SeqEncodeArgs::c_scratch
   float* save_gates;             // training (column-split scan only): [K, n, 4H] post-activation gates, or nullptr
   float* save_c;                 // [K, n, H] cell state after every step, or nullptr
+  // rollout launch (gnnpn_pn_decode_rollouts_f32), 0 for a plain decode: `rollouts` decodes of every instance, c_state
+  // read only; dec_h [rollouts, n, K, H], idx_out [rollouts, K, n], win_logits / win_probs [rollouts, n, L]; rollout 0
+  // greedy, rollout r >= 1 drawn with sampled[r-1] (sample_uniform is NULL).  The workspace c_scratch lies in is
+  // tc_seq_rollouts_workspace_bytes(n, rollouts) long.
+  int rollouts;
+  const float* sampled;          // [rollouts-1, K, n]
 };
 // nr: 0 row-major encodings; 5 / 8 / 10 blocked encodings, window row capacity of the fused decoder (N <= nr)
 int tc_seq_decode(const SeqDecodeArgs& a, int nr, cudaStream_t st);
+
+// Workspace of a rollout launch: every rollout has the per-CTA scratch of a decode of n instances (the CTA-pair scan's
+// cell state, the column-split scan's h' exchange), so it is sized from rollouts * n rows padded to whole pair blocks.
+inline size_t tc_seq_rollouts_workspace_bytes(int64_t n, int rollouts) {
+  return tc_lstm_workspace_bytes(rollouts * ((n + 255) / 256) * 256);
+}
 
 }  // namespace gnnpn

@@ -229,6 +229,7 @@ class PointerNet(nn.Module):
                                                   # the caller reads it with ``raise_if_out_of_range`` when convenient
         self.replay_impl = "own"                  # REINFORCE gradient: "own" = library kernels (fast configuration), "torch"
         self._train_saves = None                  # (saves, inputs, latent window) of a training-mode forward, consumed by the replay
+        self.last_rollouts = None                 # (encoded handle, latent window) of the most recent decode_rollouts
 
     # -- the kernels' weights are a cache over the parameters; rebuilt when any of them changes
     def _weights(self):
@@ -381,12 +382,7 @@ class PointerNet(nn.Module):
             if encoded is None:
                 encoded = self.encode(inputs)
         else:
-            cur = torch.cuda.current_stream(inputs.device)
-            if encoded.stream != cur:                      # encoded on a side stream: order after it, keep its buffers alive
-                cur.wait_stream(encoded.stream)
-                for t in (encoded.x, encoded.ws, encoded.enc_out, encoded.c):
-                    if t is not None:
-                        t.record_stream(cur)
+            self._join(encoded)
         path, x, ws, layout, enc_out, c = encoded.path, encoded.x, encoded.ws, encoded.layout, encoded.enc_out, encoded.c
         _, dec_w = self._weights()
         att = self.pointer.name
@@ -462,6 +458,52 @@ class PointerNet(nn.Module):
         prev_logits = WindowLogits(K, win_logits, dense_logits)
         return prev_probs, list(idx64.unbind(0)), prev_logits
 
+
+    @staticmethod
+    def _join(encoded):
+        """Orders the current stream after an ``encode`` enqueued on another stream and keeps its buffers alive."""
+        cur = torch.cuda.current_stream(encoded.x.device)
+        if encoded.stream != cur:
+            cur.wait_stream(encoded.stream)
+            for t in (encoded.x, encoded.ws, encoded.enc_out, encoded.c):
+                if t is not None:
+                    t.record_stream(cur)
+
+    def decode_rollouts(self, inputs, latent, rollouts: int, encoded=None):
+        """``rollouts`` decodes of every instance from ONE encoder pass (``gnnpn_pn_decode_rollouts_f32``): rollout 0 is the
+        greedy decode (``forward(..., sample="greedy")``), rollouts 1.. draw every pick from the window distribution with
+        uniforms from ``self.generator``, as ``sample="sample"`` does.  ``encoded``: optional handle from ``encode``.
+        Returns (idx int32 [R, K, B], win_logits [R, B, L], win_probs [R, B, L]) and leaves the handle in
+        ``self.last_rollouts``.  The fast configuration only (hidden_size 256, Dot attention, no glimpses, no category
+        embedding, at most 32 candidates per window, the tensor-core kernels): anything else raises NotImplementedError."""
+        B, L, F = inputs.shape
+        assert L == self.seq_len
+        if int(rollouts) != rollouts or rollouts < 1:
+            raise ValueError(f"decode_rollouts: rollouts must be an integer >= 1, got {rollouts!r}")
+        if self._path(F) != "fast" or self._impl != "tc":
+            raise NotImplementedError(
+                "best-of-R decoding runs on the fused scan kernels only: hidden_size = 256, Dot attention, n_glimpses = 0, "
+                f"embedding_size = 0, at most 32 candidates per window and 8 input columns, impl 'tc' (this network: "
+                f"hidden_size = {self.hidden_size}, attention = {self.pointer.name}, n_glimpses = {self.n_glimpses}, "
+                f"embedding_size = {self.embedding_size}, {self.serNumber} candidates, {F} columns, impl {self._impl!r})")
+        K, N = self.serCategory, self.serNumber
+        R = int(rollouts)
+        if encoded is None:
+            encoded = self.encode(inputs)
+        else:
+            self._join(encoded)
+        _, dec_w = self._weights()
+        with torch.no_grad():
+            lat = _window_of(latent, K, N) if latent else None
+            uniform = torch.rand(R - 1, K, B, device=inputs.device, generator=self.generator) if R > 1 else None
+            _, idx, win_logits, win_probs = ops.pn_decode_rollouts(
+                encoded.x, encoded.enc_out, encoded.c, dec_w, K, N, R, sample_uniform=uniform, latent_win=lat,
+                alpha=float(self.alpha), use_tanh=bool(self.pointer.use_tanh), C=float(self.pointer.C),
+                enc_layout=encoded.layout, hidden=self.hidden_size)
+        if not self.defer_range_check:
+            self.raise_if_out_of_range(encoded.range_flag)
+        self.last_rollouts = (encoded, lat)
+        return idx, win_logits, win_probs
 
     @staticmethod
     def raise_if_out_of_range(range_flag):
@@ -616,3 +658,39 @@ class CombinatorialRL(nn.Module):
                             embedding_size=self.embedding_size)
             return R, action_probs, actions, action_idxs, latent_p
         return probs, action_probs, actions, action_idxs, latent_p
+
+    @torch.no_grad()
+    def best_of(self, inputs, labs, latent=None, rollouts: int = 16, encoded=None):
+        """Best-of-M sampled decoding (the "Sampling" inference of a REINFORCE-trained pointer network): ``rollouts`` decodes
+        of every instance (``PointerNet.decode_rollouts``: rollout 0 greedy, the others sampled) scored by this module's
+        reward -- "Low": violated constraints, "High": round(viol + objFunc, 5) (``gnnpn_pn_best_rollout_f32``, the
+        arithmetic of ``reward``) -- keeping the lowest, the lowest rollout on a tie, so the result is never worse than
+        the greedy decode and ``rollouts=1`` is the greedy decode.  Returns (R_best [B], actions K x [B, F], action_idxs
+        K x [B], rollout int32 [B]); ``self.actor.last`` then holds the chosen rollout's picks, window logits and
+        probabilities.  ``labs`` is unused, as in ``reward``."""
+        actor = self.actor
+        idx_all, wl_all, wp_all = actor.decode_rollouts(inputs, latent, rollouts, encoded=encoded)
+        encoded, lat = actor.last_rollouts
+        x = encoded.x
+        idx, R_best, rollout, _ = ops.pn_best_rollout(x, idx_all, level="Low" if self.level == "Low" else "High")
+        B, L, _ = inputs.shape
+        rows = torch.arange(B, device=inputs.device)
+        chosen = rollout.long()
+        win_logits, win_probs = wl_all[chosen, rows], wp_all[chosen, rows]
+        K, N = self.serCategory, self.sNumber
+        _, dec_w = actor._weights()
+        kw = dict(latent_win=lat, alpha=float(actor.alpha), attention="Dot", use_tanh=bool(actor.pointer.use_tanh),
+                  C=float(actor.pointer.C), workspace=encoded.ws, enc_layout=encoded.layout, hidden=actor.hidden_size)
+
+        def replay():       # the chosen rollout's decoder states: the decode teacher-forced on its picks
+            return ops.pn_decode_greedy(x, encoded.enc_out, encoded.c.clone(), dec_w, K, N, forced_idx=idx, want_dec_h=True,
+                                        **kw)[0]
+        actor.last = _Last({"idx": idx, "win_logits": win_logits, "win_probs": win_probs, "latent_win": lat,
+                            "enc_buf": encoded.enc_out, "enc_layout": encoded.layout,
+                            "enc_shape": (B, L, actor.hidden_size), "range_flag": encoded.range_flag,
+                            "replay_dec_h": replay})
+        if encoded.layout == ops.ENC_ROWMAJOR:
+            actor.last["enc_out"] = encoded.enc_out
+        idx64 = idx.long()
+        actions = list(inputs[rows.unsqueeze(0), idx64].unbind(0))
+        return (R_best if self.use_cuda else R_best.cpu()), actions, list(idx64.unbind(0)), rollout

@@ -161,6 +161,59 @@ def pn_decode_greedy(inputs, enc_out, c_state, packed_dec, K: int, N: int, laten
     return dec_h, idx, wl, wp
 
 
+def pn_decode_rollouts(inputs, enc_out, c_state, packed_dec, K: int, N: int, rollouts: int, sample_uniform=None,
+                       latent_win=None, alpha: float = 1.0, use_tanh: bool = True, C: float = 10.0,
+                       enc_layout: int = ENC_ROWMAJOR, hidden: int = 256, want_dec_h: bool = False):
+    """``rollouts`` decodes of every instance from one set of encodings (``gnnpn_pn_decode_rollouts_f32``): rollout 0
+    greedy, rollout r >= 1 drawn with ``sample_uniform[r-1]`` (fp32 [rollouts-1, K, n]).  ``c_state`` is read, not
+    updated.  Returns (dec_h [R, n, K, H] | None, idx int32 [R, K, n], win_logits [R, n, L], win_probs [R, n, L]); dec_h
+    is allocated when the decoder needs it (row-major encodings) or ``want_dec_h``."""
+    x = _f32(inputs, "inputs")
+    n, L, F = x.shape
+    R = int(rollouts)
+    if R < 1:
+        raise ValueError(f"pn_decode_rollouts: rollouts must be >= 1, got {R}")
+    dev = x.device
+    dec_h = (torch.empty(R, n, K, hidden, device=dev, dtype=torch.float32)
+             if (want_dec_h or enc_layout == ENC_ROWMAJOR) else None)
+    idx = torch.empty(R, K, n, device=dev, dtype=torch.int32)
+    wl = torch.empty(R, n, L, device=dev, dtype=torch.float32)
+    wp = torch.empty(R, n, L, device=dev, dtype=torch.float32)
+    if latent_win is not None:
+        latent_win = _f32(latent_win, "latent_win")
+        assert latent_win.shape == (n, L)
+    if sample_uniform is not None:
+        sample_uniform = _f32(sample_uniform, "sample_uniform")
+        assert sample_uniform.shape == (R - 1, K, n)
+    ws = torch.empty(int(lib().gnnpn_pn_rollouts_workspace_bytes(n, hidden, R)), device=dev, dtype=torch.uint8)
+    check(lib().gnnpn_pn_decode_rollouts_f32(
+        x.data_ptr(), enc_out.data_ptr(), c_state.data_ptr(), _ptr(latent_win), float(alpha), packed_dec.data_ptr(),
+        ATT["Dot"], None, int(bool(use_tanh)), float(C), n, L, F, hidden, K, N, _ptr(dec_h), idx.data_ptr(),
+        wl.data_ptr(), wp.data_ptr(), _ptr(sample_uniform), *_ws(ws), int(enc_layout), R, _stream()),
+        "pn_decode_rollouts")
+    return dec_h, idx, wl, wp
+
+
+def pn_best_rollout(inputs, idx, level: str = "High", tag: int = 0, want_rollout_rewards: bool = False):
+    """Best rollout of picks ``idx`` int32 [R, K, n] by the reward of ``level`` ("Low": violations, "High":
+    round(viol + obj, 5)), lowest rollout on a tie (``gnnpn_pn_best_rollout_f32``).  Returns (best picks int32 [K, n],
+    best reward fp32 [n], chosen rollout int32 [n], every rollout's reward fp32 [R, n] | None)."""
+    x = _f32(inputs, "inputs")
+    n, L, F = x.shape
+    idx = idx.to(torch.int32).contiguous()
+    R, K, _ = idx.shape
+    if level not in ("Low", "High"):
+        raise ValueError(f"pn_best_rollout: level must be 'Low' or 'High', got {level!r}")
+    best_idx = torch.empty(K, n, device=x.device, dtype=torch.int32)
+    best_rew = torch.empty(n, device=x.device, dtype=torch.float32)
+    best_r = torch.empty(n, device=x.device, dtype=torch.int32)
+    rews = torch.empty(R, n, device=x.device, dtype=torch.float32) if want_rollout_rewards else None
+    check(lib().gnnpn_pn_best_rollout_f32(x.data_ptr(), idx.data_ptr(), n, L, F, K, tag, int(level == "High"), R,
+                                          best_idx.data_ptr(), best_rew.data_ptr(), best_r.data_ptr(), _ptr(rews),
+                                          _stream()), "pn_best_rollout")
+    return best_idx, best_rew, best_r, rews
+
+
 # ------------------------------------------------------------------ any hidden size (strict fp32, per-step launches)
 def anyh_fold(w_ih, w_hh, b_ih, b_hh, w_embed, b_embed, start_input=None):
     """Folded weights of the any-hidden-size kernels: ``w_cat [4H, H+F] = [W_hh | W_ih . W_emb]``, ``bias = b_ih + b_hh +

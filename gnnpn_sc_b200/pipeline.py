@@ -65,8 +65,10 @@ def _one_batch_behind(host_batches, upload, enqueue, device) -> Iterator[Tuple[t
 
 
 class GreedyLowHigh:
-    def __init__(self, low, high, device=None):
+    def __init__(self, low, high, device=None, rollouts: int = 1):
+        """``rollouts``: PNHigh decodes best-of-``rollouts`` (``low_high``); 1 is the greedy decode."""
         self.low, self.high = low.eval(), high.eval()
+        self.rollouts = rollouts
         self.high.actor.check_inputs = False      # PNHigh decodes the rows PNLow has just range-checked
         self.device = torch.device(device if device is not None else "cuda")
         if self.device.type != "cuda":
@@ -93,7 +95,8 @@ class GreedyLowHigh:
     def _enqueue(self, slot: int):
         main = torch.cuda.current_stream(self.device)
         main.wait_event(self._ready[slot])
-        latent, R, idx, flag = low_high(self.low, self.high, self._stage[slot], self._side, check="defer")
+        latent, R, idx, flag = low_high(self.low, self.high, self._stage[slot], self._side, check="defer",
+                                        rollouts=self.rollouts)
         self._consumed[slot] = torch.cuda.Event()
         self._consumed[slot].record(main)                 # after every kernel that reads the staging buffer
         return (torch.stack(idx).to(torch.int32), R), flag
@@ -104,13 +107,15 @@ class GreedyLowHigh:
         return _one_batch_behind(host_batches, self._upload, self._enqueue, self.device)
 
 
-def low_high(low, high, x, side_stream, own_buffers: bool = True, check: str = "now"):
+def low_high(low, high, x, side_stream, own_buffers: bool = True, check: str = "now", rollouts: int = 1):
     """PNLow greedy -> latent -> PNHigh greedy on the rows ``x`` (trainPNHigh.py:131-144).  The two encoders are independent
     (same rows, different weights): PNHigh's is enqueued on ``side_stream`` and runs concurrently with PNLow's whenever the
     batch leaves SMs free (one encoder occupies ceil(n / 128) SMs); the decoders follow on the current stream.
     ``own_buffers``: both actors keep their encodings buffer across calls (``actor.last["enc_out"]`` of a call is then only
     valid until the next call).  The input range flag is read ONCE, after everything is enqueued (no mid-pipeline sync);
     ``check="defer"`` does not read it at all and returns it as a fourth value (device int32 [1] or None) for the caller.
+    ``rollouts`` > 1: PNHigh decodes best-of-``rollouts`` (``CombinatorialRL.best_of``: rollout 0 greedy, the others
+    sampled, the lowest reward kept) from its one encoder pass; PNLow stays greedy, its latent is what PNHigh consumes.
     Returns (latent, reward, K-list of picks)."""
     from . import ops
     main = torch.cuda.current_stream(x.device)
@@ -148,7 +153,10 @@ def low_high(low, high, x, side_stream, own_buffers: bool = True, check: str = "
         _, _, _, _, latent = low(x, None, sample="greedy", training="SL", encoded=enc_lo)
     finally:
         low.actor.defer_range_check = deferred
-    R, _, _, idx, _ = high(x, None, latent, sample="greedy", training="RL", encoded=enc_hi)
+    if rollouts == 1:
+        R, _, _, idx, _ = high(x, None, latent, sample="greedy", training="RL", encoded=enc_hi)
+    else:
+        R, _, idx, _ = high.best_of(x, None, latent, rollouts=rollouts, encoded=enc_hi)
     flag = low.actor.last["range_flag"]
     if check == "defer":
         return latent, R, idx, flag
@@ -231,9 +239,12 @@ class ML2PN:
 
     ``woa``: optional ESWOA fine-tuning stage after the objective (the third stage of ``ML2PNWOATest``,
     gnnpn_sc_b200/WOA.py), a dict with ``popSize``, ``MAX_Iter`` and ``reduct`` (0, or 0.55 in the Normal ini
-    sections).  PNHigh's picks seed it, as ``WOA.start`` seeds it from ``allActions`` files."""
+    sections).  PNHigh's picks seed it, as ``WOA.start`` seeds it from ``allActions`` files.
 
-    def __init__(self, net, low, high, service_sample, serviceFeature, device=None, woa=None):
+    ``rollouts``: PNHigh decodes best-of-``rollouts`` (``low_high``; 1, the default, is the greedy decode); the best
+    rollout's picks are the ones scored and the ones that seed ESWOA."""
+
+    def __init__(self, net, low, high, service_sample, serviceFeature, device=None, woa=None, rollouts: int = 1):
         self.device = torch.device(device if device is not None else "cuda")
         self.net, self.low, self.high = net.eval(), low.eval(), high.eval()
         self.high.actor.check_inputs = False      # same rows as PNLow
@@ -243,6 +254,7 @@ class ML2PN:
         self.max_category_size = int((ptr[1:] - ptr[:-1]).max())         # static: no device read per call
         self.K = len(ptr) - 1
         self.N = low.sNumber
+        self.rollouts = rollouts
         self.service_enc = net.service_encodings(service_sample)          # static: encoded once
         self._side = torch.cuda.Stream(self.device)
         self._copy = torch.cuda.Stream(self.device)                       # host->device uploads of run()
@@ -329,7 +341,7 @@ class ML2PN:
                                              max_category_size=self.max_category_size)          # [B, K*N, 8]
         mark()
         # defer_check: the input range flag is returned (``range_flag``) instead of being read here (one host sync less)
-        latent, R, idx, flag = low_high(self.low, self.high, rows, self._side, check="defer")
+        latent, R, idx, flag = low_high(self.low, self.high, rows, self._side, check="defer", rollouts=self.rollouts)
         if not defer_check:
             self.low.actor.raise_if_out_of_range(flag)
         idx = torch.stack(idx)                                                                # [K, B]

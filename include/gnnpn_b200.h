@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define GNNPN_ABI_VERSION 11
+#define GNNPN_ABI_VERSION 12
 
 #if defined(__GNUC__)
 #define GNNPN_API __attribute__((visibility("default")))
@@ -161,6 +161,43 @@ GNNPN_API int gnnpn_pn_decode_greedy_f32(const float* inputs, const float* enc_o
                                float* dec_h, int32_t* idx_out, float* win_logits, float* win_probs,
                                const int32_t* forced_idx, const float* sample_uniform,
                                void* workspace, size_t workspace_bytes, int enc_layout, void* stream);
+
+/* Best-of-R sampled decoding ("Sampling" inference of a REINFORCE-trained pointer network): R rollouts of every instance
+ * decoded from ONE set of encodings (encoder run once, each extra rollout costs one decoder pass), then the rollout with
+ * the best objective.  Scope: the fused configuration above (H = 256, Dot attention, in_features <= 8, N <= 32).
+ *
+ * gnnpn_pn_decode_rollouts_f32: the arguments of gnnpn_pn_decode_greedy_f32 without forced_idx, plus `rollouts` = R >= 1.
+ * Rollout r of instance b is row r * n + b.  Rollout 0 is the greedy decode (first-max picks); rollout r >= 1 draws with
+ * sample_uniform[r-1] as gnnpn_pn_decode_greedy_f32 draws with its sample_uniform, so every rollout is bit for bit the
+ * single decode with those inputs.  The rollouts of an instance share enc_out, c_state (read only: not updated),
+ * latent_win and the input rows.
+ *   sample_uniform fp32 [R-1, K, n]  (may be NULL when R = 1)
+ *   dec_h          fp32 [R, n, K, H] or NULL with enc_layout = GNNPN_ENC_BLOCKED128
+ *   idx_out        int32 [R, K, n];  win_logits, win_probs  fp32 [R, n, L]
+ *   workspace      gnnpn_pn_rollouts_workspace_bytes(n, H, R) bytes (per-rollout scan scratch); required
+ * The launch is the persistent scan plan for n * R decoder rows (the CTA-pair scan, fused with blocked encodings, or the
+ * column-split scan); without a workspace, or with the "persistent" option's decoder bit off, GNNPN_EUNSUPPORTED.  The
+ * CTAs of an instance block's rollouts are scheduled next to each other, so their encodings reads coincide in L2.
+ * GNNPN_ESHAPE for R < 1 or shapes outside the scope. */
+GNNPN_API size_t gnnpn_pn_rollouts_workspace_bytes(int64_t n, int hidden, int rollouts);
+GNNPN_API int gnnpn_pn_decode_rollouts_f32(const float* inputs, const float* enc_out, const float* c_state,
+                                 const float* latent_win, float alpha, const float* packed_decoder,
+                                 int attention, const float* att_params, int use_tanh, float C,
+                                 int64_t n, int L, int in_features, int hidden, int K, int N,
+                                 float* dec_h, int32_t* idx_out, float* win_logits, float* win_probs,
+                                 const float* sample_uniform, void* workspace, size_t workspace_bytes,
+                                 int enc_layout, int rollouts, void* stream);
+
+/* gnnpn_pn_best_rollout_f32: scores every rollout idx int32 [R, K, n] with gnnpn_pn_reward_f32's arithmetic (one device
+ * function serves both) -- level 0 ("Low"): the violations as fp32, level 1 ("High"): float32(round(viol + obj, 5)) --
+ * and keeps the lowest score; ties go to the lowest rollout, so the greedy rollout 0 wins them and the result is never
+ * worse than greedy.
+ *   best_idx int32 [K, n] (the chosen rollout's picks), best_reward fp32 [n], best_rollout int32 [n],
+ *   rollout_rewards fp32 [R, n] or NULL (every rollout's score)
+ * GNNPN_ESHAPE for R < 1, a level other than 0 / 1, or gnnpn_pn_reward_f32's shape errors. */
+GNNPN_API int gnnpn_pn_best_rollout_f32(const float* inputs, const int32_t* idx, int64_t n, int L, int in_features, int K,
+                              int tag, int level, int rollouts, int32_t* best_idx, float* best_reward,
+                              int32_t* best_rollout, float* rollout_rewards, void* stream);
 
 /* ---- REINFORCE training: differentiable replay of a sampled decode (src/models/trainPNLow.py:77-106,
  * trainPNHigh.py:77-112 back-propagate sum_k log p_k(a_k) with torch autograd through the K-step python graph).
